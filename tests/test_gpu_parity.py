@@ -508,16 +508,3 @@ def test_enqueue_only_step_equals_the_synchronous_step(pkg):
         for i in range(3):
             assert gd[i, :gc[i]].tobytes() == wd[i, :wc[i]].tobytes()
     gm.close()
-
-
-def test_opt_in_pipeline_variants_stay_bit_exact():
-    """MARS_TC_HALO2 (one pipeline step per tile on stride-2 layers) and MARS_TC_TPS (several taps per step) are read once per process:
-    the conv micro shapes and the yolov5-shaped batch run again in a child process with both switched on"""
-    import subprocess
-    import sys
-    env = dict(os.environ, MARS_TC_HALO2="1", MARS_TC_TPS="3")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-x", "-m", "gpu", "-p", "no:cacheprovider",
-                        "-k", "(test_micro_models and conv) or (test_generated_yolov5_batch and 320)"], env=env, capture_output=True, text=True,
-                       cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert " passed" in r.stdout

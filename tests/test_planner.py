@@ -46,7 +46,7 @@ def test_level2_fuses_but_never_drops_or_moves_a_store(headline):
     assert sum(o["impl"] == 1 for o in convs) == len(convs) - 1  # all but the in-place 1x1 layer run on the tensor pipe
     assert sum(o["fused"] == 2 for o in convs) == 54             # every conv + sigmoid + mul chain but three (below), the in-place conv included
     assert not any(re.search(r" -[YSZ]\b|\+fwd|forwarded", o["note"]) for o in ops)  # whole-arena parity holds at levels 0-2
-    assert sum(o["kind"] == "sigmoid_i8" for o in ops) == sum(o["kind"] == "mul_i8" for o in ops) == 3  # two-N-tile layers whose outputs overwrite their input: fusing needs a private input copy (opt-in, no gain)
+    assert sum(o["kind"] == "sigmoid_i8" for o in ops) == sum(o["kind"] == "mul_i8" for o in ops) == 3  # two-N-tile layers whose outputs overwrite their input are not fused
 
 
 def test_level3_elides_forwards_and_trims(headline):

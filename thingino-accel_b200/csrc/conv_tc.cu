@@ -68,13 +68,9 @@ struct TcParams {
     int q_m, q_s;            /* RQ 3 (integer requantisation): multiplier m = cs * 2^(32 + q_s), shift */
     long long q_c;           /* RQ 3: rounding addend c; the kernel forms c64[ch] = bias[ch] * m + c */
     uint32_t cm_off;         /* RQ 3: offset of the int64 per-channel addends in dynamic shared memory */
-    /* TST (plane stores through shared memory + TMA): staging area [team][2][NST][16 channels][128 pixels] in dynamic shared
-     * memory; st_wp = row pitch of the tile's pixel index in the store tensor's (x, y) space (the padded width of kxk layers;
-     * "one long row" for flat 1x1 tiles), st_magic = floor(2^32 / st_wp) + 1 */
+    /* TST (plane stores through shared memory): staging area [team][2][NST][16 channels][128 pixels] in dynamic shared memory,
+     * copied out by the team's threads, 16 pixels of one channel each */
     uint32_t stg_off;
-    int st_manual;           /* TST: the staged block is written by the team's threads, 16 pixels of one channel each (padded tiles: TMA stores cannot clip on the left) */
-    int st_wp;
-    unsigned st_magic;
     const uint32_t *lutw;    /* 256-entry word table: index = r + 128, byte k = value of output stream k, byte 3 = side-output stream */
     uint32_t tab_off, tab_rep; /* offset of the replicated table ([256][tab_rep] words) in dynamic shared memory; copies (8, 16 or 32) */
     uint8_t *out_base;       /* slot 0 of the launch */
@@ -88,12 +84,7 @@ struct TcParams {
     unsigned wp_magic;       /* floor(2^32 / Wp) + 1 */
     int a_row_bytes;         /* bytes of one A row in a halo stage: bk, or 16 in s2d mode */
     int toep;                /* s2d mode: A rows are 16-byte pixels read as overlapping 32-byte K rows (no swizzle) */
-    int halo, halo_min, halo_rb, halo_nb; /* kxk stride 1: one A load per (tile, k block) covers all taps: rows q0+halo_min .., halo_nb boxes of halo_rb rows */
-    /* halo regions: region r = halo_reg_nb[r] boxes of halo_rb rows starting at flat row q0 + halo_reg_row[r], stored back to back in
-     * the stage.  Stride 1 / s2d: one region.  halo == 2 (stride 2 over the phase-split copy): one region per 2x2 phase that has
-     * taps, and a_shift[tap] already is the tap's offset inside the stage in 16-byte units */
-    int halo_nreg, halo_reg_row[4], halo_reg_nb[4];
-    int tps;                 /* taps per pipeline step (copy-based kxk layers with one k block per tap, no halo): a stage holds the A tiles -- and, when the weights are not resident, the B tiles -- of tps consecutive taps */
+    int halo, halo_min, halo_rb, halo_nb; /* kxk stride 1 / s2d: one A load per (tile, k block) covers all taps: rows q0+halo_min .., halo_nb boxes of halo_rb rows */
     int halo_wide;           /* s2d: the halo region travels as 256-byte rows (16 pixels): halo_rb counts those rows, halo_min is a multiple of 16 */
     int acc_bufs;            /* TMEM accumulator ring depth */
     int grp, m_groups;       /* M tiles (128 rows each) per pipeline step and accumulator hand-over; groups per image */
@@ -128,17 +119,6 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-#ifdef MARS_SPIN_WAIT
-    uint32_t done;
-    do {
-        asm volatile(
-            "{\n\t"
-            ".reg .pred p;\n\t"
-            "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t"
-            "}\n" : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    } while (!done);
-#else
     asm volatile(
         "{\n\t"
         ".reg .pred p;\n\t"
@@ -148,7 +128,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
         "bra WAIT_LOOP;\n\t"                                              /* issue slots the epilogue warps need     */
         "WAIT_DONE:\n\t"
         "}\n" ::"r"(bar), "r"(parity), "r"(0x989680u) : "memory");
-#endif
 }
 __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0, int c1, int c2) {
     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
@@ -157,11 +136,6 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *map
 __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0, int c1, int c2, int c3) {
     asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
                  ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-/* shared -> global tile store (bulk async group of the issuing thread); coordinates beyond the tensor are clipped */
-__device__ __forceinline__ void tma_store_4d(const CUtensorMap *map, uint32_t src, int c0, int c1, int c2, int c3) {
-    asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-                 ::"l"(map), "r"(src), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
 }
 __device__ __forceinline__ void sts_u8(uint32_t addr, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(addr), "r"(v) : "memory"); }
 /* D[tmem] (+)= A[smem] * B[smem]; the two 64-bit shared-memory matrix descriptors are given as 32-bit halves (the high
@@ -204,17 +178,11 @@ __device__ __forceinline__ void mbar_wait_relaxed(uint32_t bar, uint32_t parity)
         asm volatile(
             "{\n\t"
             ".reg .pred p;\n\t"
-#ifdef MARS_SPIN_WAIT
-            "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-#else
             "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-#endif
             "selp.u32 %0, 1, 0, p;\n\t"
             "}\n" : "=r"(done) : "r"(bar), "r"(parity) : "memory");
         if (done) break;
-#ifndef MARS_SPIN_WAIT
         __nanosleep(64);
-#endif
     }
 }
 
@@ -428,7 +396,7 @@ __device__ __forceinline__ void epilogue_unit(const uint32_t (&v)[16], uint32_t 
 }
 
 /* TST: the NCHW streams of the unit go into the team's staging block [stream][16 channels][128 pixels] (this thread's pixel =
- * byte r of every row; immediate offsets, no pointer arithmetic); a TMA store writes the block afterwards.  The side output
+ * byte r of every row; immediate offsets, no pointer arithmetic); the team's threads copy the block out afterwards.  The side output
  * (NHWC) is stored directly as before. */
 template <int RQ, bool TAB, int NST, bool NHWC>
 __device__ __forceinline__ void epilogue_unit_staged(const uint32_t (&v)[16], uint32_t cm, uint32_t tab_lane, uint32_t tab_stride, float cs, int qs,
@@ -493,8 +461,7 @@ __device__ __forceinline__ void epilogue_unit_nhwc(const uint32_t (&v)[16], uint
  * 128-byte K rows of the A operand from it, in the 128B-swizzled K-major layout TMA would have produced. */
 template <int RQ, bool GATHER, bool TAB, int NST, int OUT, int EPI, bool TST = false>
 __global__ void __launch_bounds__((EPI + (GATHER ? 5 : 2)) * 32, EPI == 8 ? 2 : 1)
-k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const __grid_constant__ CUtensorMap mapO0,
-          const __grid_constant__ CUtensorMap mapO1, const __grid_constant__ CUtensorMap mapO2, const TcParams p) {
+k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const TcParams p) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bar_full[8], bar_empty[8], bar_tmem_full[8], bar_tmem_empty[8], bar_b;
     __shared__ uint32_t tmem_base_slot;
@@ -502,7 +469,6 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
     __shared__ __align__(16) int s_koff[GATHER ? 128 : 4]; /* gather: patch-relative byte offset of tap k */
     __shared__ int s_shift[TC_MAX_TAPS];
 
-    pdl_release_dependents(); /* the next kernel of the step may be scheduled as CTAs of this one retire (mars_internal.h) */
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     uint8_t *smem_al = smem_raw + (smem_base - smem_u32(smem_raw));
@@ -540,7 +506,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
         for (int i = threadIdx.x; i < (256 << sh); i += blockDim.x) tab[i] = __ldg(p.lutw + (i >> sh));
     }
     /* per tap: flat pixel shift (TMA coordinate); halo mode: start of the tap's rows inside the stage, in 16-byte units */
-    if (threadIdx.x < TC_MAX_TAPS) s_shift[threadIdx.x] = p.halo == 1 ? ((p.a_shift[threadIdx.x] - p.halo_min) * p.a_row_bytes) >> 4 : p.a_shift[threadIdx.x];
+    if (threadIdx.x < TC_MAX_TAPS) s_shift[threadIdx.x] = p.halo ? ((p.a_shift[threadIdx.x] - p.halo_min) * p.a_row_bytes) >> 4 : p.a_shift[threadIdx.x];
     if (GATHER) {
         const int PP = p.gPWW * 4;
         for (int k = threadIdx.x; k < 128; k += blockDim.x) {
@@ -559,9 +525,6 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_d = tmem_base_slot;
-    /* everything above read only weights, biases and tables (written at load time); the activations this kernel reads, and the
-     * buffers it overwrites, belong to the previous kernel of the step until it has completed */
-    pdl_wait_prior_grid();
     if (TC_DBG(p) == 6) goto teardown; /* tuning aid: prologue + teardown only */
 
     if (warp < EPI) {
@@ -603,11 +566,10 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
             const int g_last = (i_hi - 1) / n_units, u_last_end = i_hi - g_last * n_units; /* units [0, u_last_end) of the last M tile */
             int ab = 0, aph = 0;
             uint32_t va[16], vb[16];
-            /* TST: the four warps of a part (one per TMEM lane quadrant) form a team that fills one staging block per unit;
-             * the team's leader thread issues the block's TMA stores and, before the next barrier, waits until the previous
-             * block has been read (its buffer is the one the unit after this one fills) */
+            /* TST: the four warps of a part (one per TMEM lane quadrant) form a team that fills one staging block per unit and,
+             * behind a barrier, copies it out; consecutive units alternate between two blocks, so the writes of the next unit
+             * cannot meet the copy-out of this one */
             const uint32_t stg_team = smem_base + p.stg_off + (uint32_t)part * (2u * NST * 2048u) + (uint32_t)r;
-            const bool leader = quad == 0 && lane == 0;
             uint32_t cnt = 0;
             for (TileIter ti(blockIdx.x, gridDim.x, tiles_per_img); ti.img < p.n_img; ti.next()) {
                 mbar_wait_relaxed(sa_full + 8u * ab, aph);
@@ -660,39 +622,23 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
                     const long long plane16 = OUT == 2 ? 16 : plane * 16;
                     const uint32_t acc_g = acc_grp + (uint32_t)(g * p.n_tile);
                     const bool last_g = g == g_last;
-                    /* TST: where the tile's pixel 0 sits in the store tensor: (x0, y0) = (q0 % st_wp, q0 / st_wp); flat tiles: one long row */
-                    const int q0 = mt * TC_BM, ty0 = (int)__umulhi((unsigned)q0, p.st_magic), tx0 = q0 - ty0 * p.st_wp;
-                    const int nseg = (int)__umulhi((unsigned)(tx0 + TC_BM - 1), p.st_magic) + 1; /* rows the 128 pixels touch */
-                    /* manual copy-out: thread r of the team owns the 16-pixel chunk (r & 7) of channel (r >> 3) of every unit */
-                    const int cq = q0 + (r & 7) * 16, cy = (int)__umulhi((unsigned)cq, p.st_magic), cx = cq - cy * p.st_wp;
-                    const bool c_ok = p.st_magic ? (cx < p.Wo && cy < p.Ho) : (cq < p.plane);
+                    /* TST copy-out: thread r of the team owns the 16-pixel chunk (r & 7) of channel (r >> 3) of every unit (the
+                     * chunk starts on a 16-pixel boundary of its row: Wo and Wp are multiples of 16) */
+                    const int cq = mt * TC_BM + (r & 7) * 16, cy = (int)__umulhi((unsigned)cq, p.wp_magic), cx = cq - cy * p.Wp;
+                    const bool c_ok = cx < p.Wo && cy < p.Ho;
                     const long long c_off = (long long)(unsigned long long)ti.img * (long long)p.slot_stride + (long long)cy * p.Wo + cx;
                     auto staged = [&](const uint32_t (&v)[16], int uu) {
                         const uint32_t sb = stg_team + (cnt & 1u) * (NST * 2048u);
                         epilogue_unit_staged<RQ, TAB, NST, OUT == 1>(v, cm0 + 16u * CMB * (uint32_t)uu, tab_lane, tab_stride, cs, qs, sb, valid, nh + uu * 16);
-                        asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); /* generic-proxy writes -> visible to the TMA store */
-                        if (leader && !p.st_manual) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); /* the previous block has left shared memory */
                         asm volatile("bar.sync %0, 128;" ::"r"(1 + part) : "memory");
-                        if (p.st_manual) {
-                            const int c = n0 + uu * 16 + (r >> 3);
-                            const uint32_t src = sb - (uint32_t)r + (uint32_t)(r >> 3) * 128u + (uint32_t)(r & 7) * 16u;
-                            if (c_ok && c < p.Co) {
-                                uint8_t *dst = p.out_base + (c_off + (long long)c * plane);
-                                const int4 d0 = lds_v4(src);
-                                *reinterpret_cast<int4 *>(dst + p.out_off[0]) = d0;
-                                if (NST > 1) { const int4 d1 = lds_v4(src + 2048u); *reinterpret_cast<int4 *>(dst + p.out_off[1]) = d1; }
-                                if (NST > 2) { const int4 d2 = lds_v4(src + 4096u); *reinterpret_cast<int4 *>(dst + p.out_off[2]) = d2; }
-                            }
-                        } else if (leader) {
-                            const uint32_t src = sb - (uint32_t)r;
-                            const int c = n0 + uu * 16, zi = p.img0 + ti.img;
-                            for (int sg = 0; sg < nseg; sg++) { /* one store per image row the tile touches; pad columns and rows beyond the image are clipped */
-                                const int xs = tx0 - sg * p.st_wp;
-                                tma_store_4d(&mapO0, src, xs, ty0 + sg, c, zi);
-                                if (NST > 1) tma_store_4d(&mapO1, src + 2048u, xs, ty0 + sg, c, zi);
-                                if (NST > 2) tma_store_4d(&mapO2, src + 4096u, xs, ty0 + sg, c, zi);
-                            }
-                            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                        const int c = n0 + uu * 16 + (r >> 3);
+                        const uint32_t src = sb - (uint32_t)r + (uint32_t)(r >> 3) * 128u + (uint32_t)(r & 7) * 16u;
+                        if (c_ok && c < p.Co) {
+                            uint8_t *dst = p.out_base + (c_off + (long long)c * plane);
+                            const int4 d0 = lds_v4(src);
+                            *reinterpret_cast<int4 *>(dst + p.out_off[0]) = d0;
+                            if (NST > 1) { const int4 d1 = lds_v4(src + 2048u); *reinterpret_cast<int4 *>(dst + p.out_off[1]) = d1; }
+                            if (NST > 2) { const int4 d2 = lds_v4(src + 4096u); *reinterpret_cast<int4 *>(dst + p.out_off[2]) = d2; }
                         }
                         cnt++;
                     };
@@ -735,7 +681,6 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
                 }
                 if (++ab == p.acc_bufs) { ab = 0; aph ^= 1; }
             }
-            if (TST && leader) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); /* every store of this team has completed */
         }
     } else if (warp == WARP_MMA) {
         if (lane < p.grp) { /* ===== MMA issuers: lane g issues the MMAs of M tile g of every group =====
@@ -790,15 +735,13 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
                         if (++s == stages) { s = 0; ph ^= 1; }
                     }
                 } else {
-                    const int T = p.tps; /* taps per step (1 unless the plan merged taps: then one k block per tap) */
-                    for (int i = 0; i < nsteps; i += T) {
+                    for (int i = 0; i < nsteps; i++) {
                         mbar_wait(sa_full + 8u * s, ph);
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        uint32_t a_st = a_lo0 + s * a_st16 + lane * a_tile16, b_lo = b_lo0 + (b_res ? i : s * T) * b_st16;
+                        const uint32_t a_st = a_lo0 + s * a_st16 + lane * a_tile16, b_lo = b_lo0 + (b_res ? i : s) * b_st16;
                         if (TC_DBG(p) != 4 && TC_DBG(p) != 9)
-                            for (int t = 0; t < T; t++, a_st += G * a_tile16, b_lo += b_st16)
-                                for (int j = 0; j < nj; j++)
-                                    umma_i8_parts(acc + (uint32_t)(lane * n_tile), a_st + a_j16 * j, hi_a, b_lo + 2u * j, hi_k, idesc, (uint32_t)((i | t | j) != 0));
+                            for (int j = 0; j < nj; j++)
+                                umma_i8_parts(acc + (uint32_t)(lane * n_tile), a_st + a_j16 * j, hi_a, b_lo + 2u * j, hi_k, idesc, (uint32_t)((i | j) != 0));
                         umma_commit(sa_empty + 8u * s); /* frees the stage when these MMAs retire */
                         if (++s == stages) { s = 0; ph ^= 1; }
                     }
@@ -822,46 +765,28 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
             }
             int s = 0, ph = 1; /* waits on the empty barriers start with the opposite parity */
             if (p.halo) {
-                const int nb = p.halo_nb, rb = p.halo_rb, nreg = p.halo_nreg;
+                const int nb = p.halo_nb, rb = p.halo_rb;
                 /* wide mode: the same bytes as 256-byte rows of 16 pixels (TMA's cost is per row: measured ~2 cycles per 16-byte row) */
                 const int wide = p.halo_wide ? 16 : 1;
                 const uint32_t tx = (uint32_t)(nb * rb * p.a_row_bytes * wide), box_b = (uint32_t)(rb * p.a_row_bytes * wide);
                 for (TileIter ti(blockIdx.x, gridDim.x, tiles_per_img); ti.img < n_img; ti.next()) {
-                    const int q0 = ti.rem * G * TC_BM, zc = p.img0 + ti.img; /* n_tiles == 1 with resident weights; q0 and the region rows are multiples of 16 in wide mode */
+                    const int q0 = ti.rem * G * TC_BM, zc = p.img0 + ti.img; /* n_tiles == 1 with resident weights; q0 and halo_min are multiples of 16 in wide mode */
+                    const int qr = (q0 + p.halo_min) / wide;
                     for (int kb = 0; kb < ksteps; kb++) {
                         mbar_wait(sa_empty + 8u * s, ph);
                         const uint32_t full = sa_full + 8u * s, dst = a_base + s * a_stb;
                         if (TC_DBG(p) == 3 || TC_DBG(p) == 9) { mbar_arrive(full); if (++s == stages) { s = 0; ph ^= 1; } continue; }
                         mbar_expect_tx(full, tx);
-                        for (int r = 0, bi = 0; r < nreg; r++) {
-                            const int qr = (q0 + p.halo_reg_row[r]) / wide, nbr = p.halo_reg_nb[r];
-                            for (int b = 0; b < nbr; b++, bi++) tma_load_3d(dst + bi * box_b, &mapA, full, kb * bk, qr + b * rb, zc);
-                        }
+                        for (int b = 0; b < nb; b++) tma_load_3d(dst + b * box_b, &mapA, full, kb * bk, qr + b * rb, zc);
                         if (++s == stages) { s = 0; ph ^= 1; }
                     }
                 }
             } else {
-                const int T = p.tps;
-                const uint32_t tx = p.a_tx_bytes + (b_res ? 0u : (uint32_t)(T * p.n_tile * bk));
+                const uint32_t tx = p.a_tx_bytes + (b_res ? 0u : (uint32_t)(p.n_tile * bk));
                 const bool rect = p.rect != 0;
                 for (TileIter ti(blockIdx.x, gridDim.x, tiles_per_img); ti.img < n_img; ti.next()) {
                     const int mg = n_tiles == 1 ? ti.rem : ti.rem / n_tiles, n0 = (ti.rem - mg * n_tiles) * p.n_tile;
                     const int q0 = mg * G * TC_BM, zc = p.img0 + ti.img;
-                    if (T > 1) { /* several taps per step (K-major copy, one k block per tap): the step's loads share one barrier */
-                        for (int tap = 0; tap < ntaps; tap += T) {
-                            mbar_wait(sa_empty + 8u * s, ph);
-                            const uint32_t full = sa_full + 8u * s;
-                            if (TC_DBG(p) == 3 || TC_DBG(p) == 9) { mbar_arrive(full); if (++s == stages) { s = 0; ph ^= 1; } continue; }
-                            mbar_expect_tx(full, tx);
-                            for (int t = 0; t < T; t++) {
-                                const int qa = q0 + s_shift[tap + t];
-                                for (int g = 0; g < G; g++) tma_load_3d(a_base + s * a_stb + (t * G + g) * a_tb, &mapA, full, 0, qa + g * TC_BM, zc);
-                                if (!b_res) tma_load_3d(b_base + (s * T + t) * b_stb, &mapB, full, 0, n0, tap + t);
-                            }
-                            if (++s == stages) { s = 0; ph ^= 1; }
-                        }
-                        continue;
-                    }
                     for (int tap = 0; tap < ntaps; tap++) {
                         const int sh = s_shift[tap], qa = q0 + sh; /* rect mode: sh = kh << 16 | kw */
                         for (int kb = 0; kb < ksteps; kb++) {
@@ -986,7 +911,6 @@ teardown:
 __global__ void __launch_bounds__(256) k_to_nhwc(const uint8_t *src_base, unsigned long long src_stride, uint8_t *dst_base,
                                                  unsigned long long dst_stride, int C, int Cp, int H, int W, int Wp, int plane, int npix,
                                                  int stride2, int pt, int pl) { /* Cp >= C: bytes per pixel of the copy */
-    pdl_begin();
     __shared__ uint8_t tile[32][33];
     const uint8_t *src = src_base + (unsigned long long)blockIdx.z * src_stride;
     uint8_t *dst = dst_base + (unsigned long long)blockIdx.z * dst_stride;
@@ -1022,7 +946,6 @@ __global__ void __launch_bounds__(256) k_to_nhwc(const uint8_t *src_base, unsign
  * zero border and zero beyond 4*C bytes.  One thread per P pixel. */
 __global__ void __launch_bounds__(256) k_s2d16(const uint8_t *__restrict__ src_base, unsigned long long src_stride, uint8_t *__restrict__ dst_base,
                                                unsigned long long dst_stride, int C, int H, int W, int Wp, int npix, int src_nhwc) {
-    pdl_begin();
     const uint8_t *src = src_base + (unsigned long long)blockIdx.y * src_stride;
     uint4 *dst = reinterpret_cast<uint4 *>(dst_base + (unsigned long long)blockIdx.y * dst_stride);
     /* four pixels per thread, 256 apart: all their loads are issued before the first store (the kernel is pure latency) */
@@ -1090,16 +1013,15 @@ __global__ void k_repack_weights(const int8_t *w, int8_t *dst, int Co, int Co_pa
 }
 
 /* ---- host side ------------------------------------------------------------------ */
-typedef void (*TcKernel)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const TcParams);
+typedef void (*TcKernel)(const CUtensorMap, const CUtensorMap, const TcParams);
 struct TcPlanImpl {
     CUtensorMap mapA, mapB, mapA_linked;
-    CUtensorMap mapO[3];   /* TST: store tensors of the NCHW output streams (x, y, channel, image) */
-    bool tst = false;      /* plane stores through shared memory + TMA */
+    bool tst = false;      /* plane stores through shared memory (the space-to-depth stem) */
     bool has_linked = false;
     TcParams p;
     int prepass = 0;
     int rq = 0;     /* requantisation variant of the epilogue (requant_pair) */
-    bool fast = false, tab = false; /* tab: the epilogue looks its byte up in the per-lane word table */
+    bool tab = false; /* the epilogue looks its byte up in the per-lane word table */
     int C = 0, Cp = 0, H = 0, W = 0, pt = 0, pl = 0, plane = 0, npix = 0; /* Cp: bytes per pixel of the channel-innermost copy */
     const uint8_t *src_slot0 = nullptr; /* input tensor in slot 0 */
     uint8_t *scratch = nullptr;
@@ -1116,7 +1038,6 @@ struct TcPlanImpl {
     int sms = 0; /* multiprocessors of the device the plan was built on */
     int nhwc_in = 0;  /* channel-innermost activations / OHWI weights (OP_CONV_I8_NHWC) */
     bool gather_direct = false; /* gather mode reads the input tensor in the arena itself (no private copy needed) */
-    bool private_in = false;    /* 1x1 from NCHW planes: the planes are copied to the scratch area before every launch */
 };
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
@@ -1175,39 +1096,16 @@ static bool make_map4(CUtensorMap *m, void *base, uint64_t C, uint64_t W, uint64
     return true;
 }
 
-/* store tensor of one NCHW output stream: dims (X, Y, C, images) = (row, rows, channels, slots), box {128 pixels, 1 row, 16 channels,
- * 1 image}, no swizzle: the shared-memory source is a dense [16][128] byte block */
-static bool make_map_store(CUtensorMap *m, void *base, uint64_t X, uint64_t Y, uint64_t C, uint64_t N, uint64_t plane, uint64_t img_stride) {
-    EncodeTiledFn enc = encode_tiled();
-    if (!enc) return false;
-    cuuint64_t dims[4] = {X, Y, C, N};
-    cuuint64_t strides[3] = {X, plane, img_stride};
-    cuuint32_t box[4] = {128, 1, 16, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { cudaGetLastError(); return false; }
-    return true;
-}
-
 static int round_up(int x, int a) { return (x + a - 1) / a * a; }
 
-/* MARS_TC_TST: which layers send their NCHW streams through the shared-memory staging block -- bit 0: tiles without pad columns,
- * TMA stores; bit 1: padded tiles (kxk layers), written out by the team's threads in 16-byte pieces; bit 2: tiles without pad
- * columns, written out by the threads; bit 3: only the space-to-depth stem, by the threads (the default: the stem writes the largest
- * planes next to a side output and is the one layer class where staging pays, -7 %; profiles/r02l_staged_stores.txt) */
-static int tst_modes() {
-    static const int m = getenv("MARS_TC_TST") ? atoi(getenv("MARS_TC_TST")) : 8; /* default: only the space-to-depth stem (bit 3), the one layer class where it pays (-7 %) */
-    return m;
-}
-
-/* Row pitch of the padded / phase-split pixel index.  TMA stores need a 16-byte aligned innermost coordinate (byte elements:
- * anything else faults, measured), so when the output rows are a multiple of 16 pixels the pitch is rounded up to one as well:
- * every 128-pixel tile then starts on a 16-pixel boundary of its row.  The extra pad columns are computed and discarded; the
- * rounding is skipped when they would add more than MARS_TC_WPWASTE percent (default 20) to the layer. */
-static int store_pitch(int wp_min, int ow, bool stem = false) {
-    static const int max_waste = getenv("MARS_TC_WPWASTE") ? atoi(getenv("MARS_TC_WPWASTE")) : 20;
-    if (!(tst_modes() & (stem ? 10 : 2)) || ow % 16 || wp_min % 16 == 0) return wp_min;
+/* Row pitch of the space-to-depth stem's bordered pixel index.  The stem's NCHW streams leave through a shared-memory staging
+ * block (TST: the stem writes the largest planes next to a side output and is the one layer class where staging pays, -7 %;
+ * profiles/r02l_staged_stores.txt), copied out in 16-pixel pieces of one row.  So when the output rows are a multiple of 16
+ * pixels the pitch is rounded up to one as well: every 128-pixel tile then starts on a 16-pixel boundary of its row.  The extra
+ * pad columns are computed and discarded; the rounding is skipped when they would add more than 20 % to the layer. */
+static int store_pitch(int wp_min, int ow) {
+    constexpr int max_waste = 20; /* percent */
+    if (ow % 16 || wp_min % 16 == 0) return wp_min;
     const int wp = (wp_min + 15) / 16 * 16;
     return (wp - wp_min) * 100 <= max_waste * wp_min ? wp : wp_min;
 }
@@ -1233,11 +1131,10 @@ static TcGeom tc_geometry(const Op &o) {
         if (o.pt < 0 || o.pl < 0 || o.pt >= o.kh || o.pl >= o.kw) return g;
         g.ntaps = o.kh * o.kw;
         if (g.ntaps > TC_MAX_TAPS) return g;
-        static const bool s2d_enabled = !(getenv("MARS_TC_S2D") && atoi(getenv("MARS_TC_S2D")) == 0);
-        if (s2d_enabled && o.sh == 2 && o.kh == 6 && (o.pt == 0 || o.pt == 2) && (o.pl == 0 || o.pl == 2) && o.ic <= 4 && o.ih % 2 == 0 &&
+        if (o.sh == 2 && o.kh == 6 && (o.pt == 0 || o.pt == 2) && (o.pl == 0 || o.pl == 2) && o.ic <= 4 && o.ih % 2 == 0 &&
             o.iw % 2 == 0 && o.oh <= o.ih / 2 && o.ow <= o.iw / 2 && round_up(o.oc, 16) <= 128 && (long long)o.oh * o.ow >= 4096) {
             /* the stem: the same space-to-depth copy as the NCHW stem, gathered from interleaved pixels */
-            g.prepass = 4; g.Wp = store_pitch(o.iw / 2 + 2, o.ow, true); g.plane = (o.ih / 2 + 2) * g.Wp; g.npix = g.plane; g.ntaps = 6; g.Kp = 32;
+            g.prepass = 4; g.Wp = store_pitch(o.iw / 2 + 2, o.ow); g.plane = (o.ih / 2 + 2) * g.Wp; g.npix = g.plane; g.ntaps = 6; g.Kp = 32;
             g.scratch_bytes = (size_t)g.npix * 16;
             g.ok = true;
             return g;
@@ -1271,7 +1168,7 @@ static TcGeom tc_geometry(const Op &o) {
     if (o.ic >= 16 && o.ic % 32 && o.kh == 1 && o.kw == 1 && o.sh == 1 && o.pt == 0 && o.pl == 0 && o.oh <= o.ih && o.ow == o.iw) {
         g.ntaps = 1; g.Wp = o.iw;
         g.kpad = o.ic > 64 ? round_up(o.ic, 128) : round_up(o.ic, 32);
-        if (((long long)o.ih * o.iw) % 16 == 0) { g.prepass = 0; g.scratch_bytes = o.private_in ? (size_t)o.ic * o.ih * o.iw : 0; }
+        if (((long long)o.ih * o.iw) % 16 == 0) g.prepass = 0;
         else { /* planes that TMA cannot address (stride not a multiple of 16 bytes, e.g. 10 x 10): channel-innermost copy, kpad bytes per pixel */
             g.prepass = 1; g.plane = o.ih * g.Wp; g.npix = g.plane;
             g.scratch_bytes = (size_t)g.npix * g.kpad;
@@ -1282,11 +1179,10 @@ static TcGeom tc_geometry(const Op &o) {
     if (o.ic < 32 || o.ic % 32 || o.kh != o.kw) {
         auto small_k = [&]() -> bool {
         /* the YOLOv5 stem shape: 6x6 stride 2 pad 2 over <= 4 channels == 3x3 stride 1 pad 1 over the 2x2 space-to-depth image */
-        static const bool s2d_enabled = !(getenv("MARS_TC_S2D") && atoi(getenv("MARS_TC_S2D")) == 0);
-        if (s2d_enabled && o.sh == 2 && o.sw == 2 && o.kh == 6 && o.kw == 6 && (o.pt == 0 || o.pt == 2) && (o.pl == 0 || o.pl == 2) &&
+        if (o.sh == 2 && o.sw == 2 && o.kh == 6 && o.kw == 6 && (o.pt == 0 || o.pt == 2) && (o.pl == 0 || o.pl == 2) &&
             o.ic <= 4 && o.ih % 2 == 0 && o.iw % 2 == 0 && o.oh <= o.ih / 2 && o.ow <= o.iw / 2 && round_up(o.oc, 16) <= 128 &&
             (long long)o.oh * o.ow >= 4096) {
-            g.prepass = 4; g.Wp = store_pitch(o.iw / 2 + 2, o.ow, true); g.plane = (o.ih / 2 + 2) * g.Wp; g.npix = g.plane; g.ntaps = 6; g.Kp = 32;
+            g.prepass = 4; g.Wp = store_pitch(o.iw / 2 + 2, o.ow); g.plane = (o.ih / 2 + 2) * g.Wp; g.npix = g.plane; g.ntaps = 6; g.Kp = 32;
             g.scratch_bytes = (size_t)g.npix * 16;
             g.ok = true;
             return true;
@@ -1325,17 +1221,17 @@ static TcGeom tc_geometry(const Op &o) {
         g.prepass = 0; g.Wp = o.iw;
     } else if (o.sh == 1) {
         if (o.pl >= o.kw || o.pt >= o.kh) return g;
-        g.prepass = 1; g.Wp = store_pitch(o.iw + o.kw - 1, o.ow); g.plane = o.ih * g.Wp; g.npix = g.plane;
+        g.prepass = 1; g.Wp = o.iw + o.kw - 1; g.plane = o.ih * g.Wp; g.npix = g.plane;
     } else if (o.sh == 2) {
         if (o.pl >= o.kw || o.pt >= o.kh) return g;
         /* phase plane: rows a = 0 .. , pitch Wp >= ow + (k-1)/2; enough zero rows below that the
          * deepest tap of the last output row stays inside its own plane */
-        g.prepass = 2; g.Wp = store_pitch(o.ow + (o.kw - 1) / 2, o.ow);
+        g.prepass = 2; g.Wp = o.ow + (o.kw - 1) / 2;
         const int rows = std::max((o.ih - 1 + o.pt) / 2 + 1, o.oh + (o.kh - 1) / 2);
         g.plane = rows * g.Wp; g.npix = 4 * g.plane;
     } else return g;
     if (o.ow > g.Wp) return g;
-    g.scratch_bytes = g.prepass ? (size_t)g.npix * (g.kpad ? g.kpad : o.ic) : (o.private_in ? (size_t)o.ic * o.ih * o.iw : 0);
+    g.scratch_bytes = g.prepass ? (size_t)g.npix * (g.kpad ? g.kpad : o.ic) : 0;
     g.ok = true;
     return g;
 }
@@ -1354,7 +1250,6 @@ int tc_n_tiles(int oc) {
     const int nt = co_pad <= 256 ? co_pad : (co_pad % 256 == 0 ? 256 : 128);
     return (co_pad + nt - 1) / nt;
 }
-bool tc_private_input_ok(const Op &o) { const TcGeom g = tc_geometry(o); return g.ok && g.prepass == 0; }
 bool tc_uses_copy(const Op &o) { return tc_geometry(o).prepass != 0; } /* (NHWC layers: a private copy on demand, see tc_plan) */
 bool tc_linkable(const Op &o) { const TcGeom g = tc_geometry(o); return g.ok && (g.prepass == 1 || g.prepass == 2) && !g.kpad; }
 
@@ -1511,7 +1406,8 @@ static bool int_requant_fit(float cs, long long tmax, int *m_out, int *s_out, lo
 }
 
 /* kernel variants: requantisation x GATHER producer x word table x number of stored streams x output mode (0 NCHW planes,
- * 1 + side copy, 2 channel-innermost tensors).  Without a table (plain conv, no byte-ReLU) there is one stream at most. */
+ * 1 + side copy, 2 channel-innermost tensors) x TST (staged plane stores: only the space-to-depth stem, i.e. EPI 8, no
+ * gather, output mode 0 / 1, at least one stream).  Without a table (plain conv, no byte-ReLU) there is one stream at most. */
 template <int RQ, bool GATHER, int EPI, bool TST>
 static TcKernel pick_kernel2(bool tab, int nst, int out) {
     if (out == 2) {
@@ -1548,8 +1444,9 @@ static TcKernel pick_kernel2(bool tab, int nst, int out) {
 template <int RQ>
 static TcKernel pick_kernel1(bool gather, bool tab, int nst, int out, int epi, bool tst) {
     if (gather) return pick_kernel2<RQ, true, 8, false>(tab, nst, out);
-    if (epi == 16) return tst ? pick_kernel2<RQ, false, 16, true>(tab, nst, out) : pick_kernel2<RQ, false, 16, false>(tab, nst, out);
-    return tst ? pick_kernel2<RQ, false, 8, true>(tab, nst, out) : pick_kernel2<RQ, false, 8, false>(tab, nst, out);
+    if (tst) return epi == 8 ? pick_kernel2<RQ, false, 8, true>(tab, nst, out) : nullptr;
+    if (epi == 16) return pick_kernel2<RQ, false, 16, false>(tab, nst, out);
+    return pick_kernel2<RQ, false, 8, false>(tab, nst, out);
 }
 static TcKernel pick_kernel(int rq, bool gather, bool tab, int nst, int out, int epi, bool tst) {
     if (rq == 3) return pick_kernel1<3>(gather, tab, nst, out, epi, tst);
@@ -1590,8 +1487,7 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     p.tmem_cols = t->ctas_per_sm == 1 ? 512 : 256;
     p.grp = 1;
     if (p.n_tiles == 1 && t->ctas_per_sm == 2) {
-        static const int gmax = getenv("MARS_TC_GROUP") ? std::max(1, atoi(getenv("MARS_TC_GROUP"))) : 4;
-        while (p.grp * 2 <= gmax && 2 * (p.grp * 2) * p.n_tile <= p.tmem_cols) p.grp *= 2;
+        while (p.grp < 4 && 2 * (p.grp * 2) * p.n_tile <= p.tmem_cols) p.grp *= 2; /* up to four M tiles per group */
     }
     p.acc_bufs = std::max(2, std::min(4, p.tmem_cols / (p.grp * p.n_tile)));
     p.a_stage_bytes = p.grp * p.a_tile_bytes;
@@ -1616,27 +1512,17 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
             t->stream_byte[k] = t->nst; p.out_off[t->nst++] = stream_off[k] - (int64_t)ag.W;
         }
     if (t->nst > 1) t->tab = true; /* a plain conv with a forwarded second copy: the bytes of the streams come from the (identity) table */
-    /* TST: the NCHW streams leave through a shared-memory staging block and TMA stores (full 128-byte rows) instead of one byte per
-     * lane and channel.  Needs the tile's pixel index to be row-major over (oh, ow) with pitch Wp (every copy-based and plane-based
-     * mode; not the gather / rect tiles), 16-byte aligned stream bases, and a store tensor TMA can address: the planes as one long
-     * row when the tile has no pad columns, else rows of Wo bytes (Wo a multiple of 16). */
-
-    const bool st_flat = g.Wp == o.ow && ((long long)o.oh * o.ow) % 16 == 0;
-    /* TMA stores fault on negative coordinates (measured), which clipping the left end of a row segment would need: padded tiles
-     * are copied out by the threads instead */
-    const bool st_padded = !st_flat && g.Wp != o.ow && o.ow % 16 == 0 && g.Wp % 16 == 0;
-    t->tst = !gather && !rect && !nhwc_in && t->nst >= 1 && ((st_flat && (tst_modes() & 5)) || (st_padded && (tst_modes() & (s2d ? 10 : 2))));
-    p.st_manual = (t->tst && (st_padded || (tst_modes() & 4))) ? 1 : 0;
+    /* TST (the NCHW space-to-depth stem, see store_pitch): the NCHW streams leave through a shared-memory staging block, copied out
+     * by the threads in 16-byte pieces of one row, instead of one byte per lane and channel.  Needs rows and pitch in whole 16-pixel
+     * pieces and 16-byte aligned stream bases */
+    t->tst = s2d && !nhwc_in && t->nst >= 1 && o.ow % 16 == 0 && g.Wp % 16 == 0;
     for (int k = 0; k < t->nst; k++) if (p.out_off[k] % 16) t->tst = false;
     const int epi_warps = (!gather && t->ctas_per_sm == 1) ? 16 : 8;
     const int stg_bytes = t->tst ? (epi_warps / 4) * 2 * t->nst * 2048 : 0;
     { /* requantisation variant of the epilogue (requant_pair / requant_int) */
-        static const int rq_max = getenv("MARS_TC_RQ") ? atoi(getenv("MARS_TC_RQ")) : 3; /* tuning / test aid: cap the variant */
         const long long bound = fast_requant_bound(o, ag);
-        t->fast = bound >= 0;
-        t->rq = !t->fast ? 0 : ((rq_max >= 2 && halfup_requant_ok(o.f0, bound)) ? 2 : 1);
-        if (rq_max == 0) { t->rq = 0; t->fast = false; }
-        if (rq_max >= 3 && int_requant_fit(o.f0, std::max(1ll, acc_bound(o, ag)), &p.q_m, &p.q_s, &p.q_c)) t->rq = 3;
+        t->rq = bound < 0 ? 0 : (halfup_requant_ok(o.f0, bound) ? 2 : 1);
+        if (int_requant_fit(o.f0, std::max(1ll, acc_bound(o, ag)), &p.q_m, &p.q_s, &p.q_c)) t->rq = 3;
     }
     const int cm64_bytes = t->rq == 3 ? 8 * p.n_tiles * p.n_tile : 0; /* RQ 3: per-channel int64 addends behind the table */
     const int nsteps = g.ntaps * p.ksteps_per_tap;
@@ -1646,7 +1532,7 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     /* dynamic shared memory of a CTA: stages + weights + table (+ 1 KiB alignment slack); 227 KiB per SM, ~7 KiB static */
     auto plan_smem = [&](int tab_bytes) {
         const int budget = (t->ctas_per_sm == 1 ? 200 * 1024 : 104 * 1024) - tab_bytes;
-        p.grp = grp0; p.acc_bufs = acc0; p.a_stage_bytes = a_stage0; p.halo = 0; p.halo_wide = 0; p.halo_nreg = 0; p.b_resident = 0; p.tps = 1; plan_ok = true;
+        p.grp = grp0; p.acc_bufs = acc0; p.a_stage_bytes = a_stage0; p.halo = 0; p.halo_wide = 0; p.b_resident = 0; plan_ok = true;
         if (gather) { /* + 3 x 4 KiB patch ring + 8 KiB patch-word tables */
             if (p.grp > 2) { p.grp = 2; p.a_stage_bytes = p.grp * p.a_tile_bytes; p.acc_bufs = std::max(2, std::min(4, p.tmem_cols / (p.grp * p.n_tile))); }
             p.stages = std::max(2, std::min(8, (budget - (int)p.b_stage_bytes - 20480 - 1024) / (int)p.a_stage_bytes));
@@ -1657,16 +1543,14 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
             p.b_resident = (p.n_tiles == 1 && b_all <= (size_t)budget / 2) ? 1 : 0;
             /* kxk stride 1 over the padded channel-innermost copy: every tap is a row shift of the same pixel rows, so one
              * load of the tile's rows plus its halo (128 + (kh-1)*Wp + kw-1 rows) serves all taps of a k block */
-            static const bool halo_enabled = !(getenv("MARS_TC_HALO") && atoi(getenv("MARS_TC_HALO")) == 0);
             if (s2d && !p.b_resident) { plan_ok = false; return; }
-            if ((halo_enabled && g.prepass == 1 && p.b_resident && g.ntaps > 1) || s2d) {
+            if ((g.prepass == 1 && p.b_resident && g.ntaps > 1) || s2d) {
                 /* s2d: the copy has a one-pixel zero border, so tap (ky2, pair) of output pixel q = oh*Wp + ow starts at row
                  * q + (ky2 + 1 - pt/2)*Wp + (2*pair + 1 - pl/2) and reads two pixels; taps that leave the image hit the border, the
                  * next row's border column, or rows beyond the copy (zero-filled by TMA) */
                 const int s2d_min = (1 - o.pt / 2) * g.Wp + (1 - o.pl / 2);
                 const int smin = s2d ? s2d_min : -o.pt * g.Wp, smax = s2d ? s2d_min + 2 * g.Wp + 3 : (o.kh - 1 - o.pt) * g.Wp + o.kw - 1;
-                static const bool wide_enabled = !(getenv("MARS_TC_WIDE") && atoi(getenv("MARS_TC_WIDE")) == 0);
-                if (s2d && wide_enabled && g.npix % 16 == 0 && (p.grp * TC_BM) % 16 == 0) {
+                if (s2d && g.npix % 16 == 0 && (p.grp * TC_BM) % 16 == 0) {
                     /* the region starts on a 16-pixel boundary and travels as 256-byte rows: same shared-memory image, 1/16 of the rows */
                     const int smin_al = (smin >= 0 ? smin / 16 : -((-smin + 15) / 16)) * 16;
                     const int R16 = (p.grp * TC_BM + smax - smin_al + 15) / 16;
@@ -1674,7 +1558,6 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
                     const uint32_t bytes = (uint32_t)round_up(nb * rb * 256, 1024);
                     if ((size_t)2 * bytes + b_all <= (size_t)budget) {
                         p.halo = 1; p.halo_min = smin_al; p.halo_rb = rb; p.halo_nb = nb; p.halo_wide = 1;
-                        p.halo_nreg = 1; p.halo_reg_row[0] = smin_al; p.halo_reg_nb[0] = nb;
                         p.a_stage_bytes = bytes;
                     }
                 }
@@ -1683,63 +1566,15 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
                 const uint32_t bytes = (uint32_t)round_up(nb * rb * p.a_row_bytes, 1024);
                 if (!p.halo && rb <= 256 && (size_t)2 * bytes + b_all <= (size_t)budget) {
                     p.halo = 1; p.halo_min = smin; p.halo_rb = rb; p.halo_nb = nb;
-                    p.halo_nreg = 1; p.halo_reg_row[0] = smin; p.halo_reg_nb[0] = nb;
                     p.a_stage_bytes = bytes;
                 }
-            }
-            /* kxk stride 2 over the 2x2 phase-split copy: the taps of one phase are row shifts of the same rows (0, 1, Wp, Wp + 1 for a
-             * 3x3 kernel), so one region per phase -- tile rows plus that phase's halo -- serves all taps in ONE pipeline step instead of
-             * one step per tap.  Fewer M tiles per step are accepted to make the regions fit */
-            static const bool halo2_enabled = getenv("MARS_TC_HALO2") && atoi(getenv("MARS_TC_HALO2")) != 0; /* opt-in: measured slower (32->64 s2 at 160^2: 2.65 ms against 2.15 ms with one step per tap -- the halo of a flat 128-pixel tile is a whole image row per phase, and only two such stages fit) */
-            if (halo_enabled && halo2_enabled && g.prepass == 2 && p.b_resident && g.ntaps > 1 && p.ksteps_per_tap >= 1) {
-                int rmin[4], rmax[4], used = 0;
-                for (int ph = 0; ph < 4; ph++) { rmin[ph] = 1 << 30; rmax[ph] = -(1 << 30); }
-                for (int kh = 0; kh < o.kh; kh++)
-                    for (int kw = 0; kw < o.kw; kw++) {
-                        const int ph = (kh & 1) * 2 + (kw & 1), loc = (kh / 2) * g.Wp + kw / 2;
-                        rmin[ph] = std::min(rmin[ph], loc); rmax[ph] = std::max(rmax[ph], loc);
-                    }
-                for (int ph = 0; ph < 4; ph++) used += rmax[ph] >= rmin[ph];
-                for (int gtry = p.grp; gtry >= 1 && !p.halo; gtry /= 2) {
-                    int best_rb = 0, best_boxes = 0; long long best_rows = -1;
-                    for (int rb = 8; rb <= 256; rb += 8) {
-                        int boxes = 0;
-                        for (int ph = 0; ph < 4; ph++) if (rmax[ph] >= rmin[ph]) boxes += (gtry * TC_BM + rmax[ph] - rmin[ph] + rb - 1) / rb;
-                        if (boxes > 12) continue;
-                        if (best_rows < 0 || (long long)boxes * rb < best_rows) { best_rows = (long long)boxes * rb; best_rb = rb; best_boxes = boxes; }
-                    }
-                    if (best_rows < 0) continue;
-                    const uint32_t bytes = (uint32_t)round_up((int)best_rows * p.a_row_bytes, 1024);
-                    if ((size_t)2 * bytes + b_all > (size_t)budget) continue;
-                    p.halo = 2; p.halo_min = 0; p.halo_rb = best_rb; p.halo_nb = best_boxes; p.halo_nreg = 0;
-                    for (int ph = 0; ph < 4; ph++)
-                        if (rmax[ph] >= rmin[ph]) {
-                            p.halo_reg_row[p.halo_nreg] = ph * g.plane + rmin[ph];
-                            p.halo_reg_nb[p.halo_nreg++] = (gtry * TC_BM + rmax[ph] - rmin[ph] + best_rb - 1) / best_rb;
-                        }
-                    p.grp = gtry; p.acc_bufs = std::max(2, std::min(4, p.tmem_cols / (p.grp * p.n_tile)));
-                    p.a_stage_bytes = bytes;
-                }
-                (void)used;
             }
             if (s2d && !p.halo) { plan_ok = false; return; }
-            /* several taps per pipeline step: a step costs the single MMA / producer lanes 0.2-0.5 us of barrier hand-overs whatever it
-             * holds (profiles/r03a), and a tap of a Ci = 32 / 64 layer is only 4-16 KiB */
-            static const int tps_max = getenv("MARS_TC_TPS") ? atoi(getenv("MARS_TC_TPS")) : 1; /* opt-in: measured no gain (32->64 3x3 s2 with three taps per step: 2.26 ms against 2.18 ms) -- under load the SM's issue slots, not the hand-overs, are what the layer waits for */
-            static const int tps_minst = getenv("MARS_TC_TPS_MINST") ? atoi(getenv("MARS_TC_TPS_MINST")) : 2;
-            if (!p.halo && !rect && (g.prepass == 1 || g.prepass == 2) && g.ntaps > 1 && p.ksteps_per_tap == 1) {
-                for (int T = std::min(tps_max, g.ntaps); T > 1; T--) {
-                    if (g.ntaps % T) continue;
-                    const long long stage = (long long)T * (p.a_stage_bytes + (p.b_resident ? 0 : p.b_stage_bytes));
-                    const long long room = (long long)budget - (p.b_resident ? (long long)b_all : 0);
-                    if (stage * tps_minst <= room) { p.tps = T; p.a_stage_bytes *= T; break; }
-                }
-            }
             if (p.b_resident) {
                 p.stages = std::max(2, std::min(8, (budget - (int)b_all) / (int)p.a_stage_bytes));
                 t->smem = 1024 + (size_t)p.stages * p.a_stage_bytes + b_all;
             } else {
-                const int stage_bytes = (int)(p.a_stage_bytes + p.tps * p.b_stage_bytes);
+                const int stage_bytes = (int)(p.a_stage_bytes + p.b_stage_bytes);
                 p.stages = std::max(2, std::min(8, budget / stage_bytes));
                 t->smem = 1024 + (size_t)p.stages * stage_bytes;
             }
@@ -1754,13 +1589,10 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     }
     if (!plan_ok) { delete t; return false; }
     if (t->tab) { /* widen the replication while the pipeline keeps its shape (resident weights, halo loads, >= 3 stages) */
-        const int res8 = p.b_resident, halo8 = p.halo, st8 = p.stages, grp8 = p.grp, tps8 = p.tps;
-        static const int rep_max = getenv("MARS_TC_TABREP") ? atoi(getenv("MARS_TC_TABREP")) : 32;
+        const int res8 = p.b_resident, halo8 = p.halo, st8 = p.stages, grp8 = p.grp;
         for (int r2 = 32; r2 > 8; r2 >>= 1) {
-            if (r2 > rep_max) continue;
             plan_smem(r2 * 1024 + cm64_bytes + stg_bytes);
-            static const int min_st = getenv("MARS_TC_MINST") ? atoi(getenv("MARS_TC_MINST")) : 3;
-            if (plan_ok && !over && p.b_resident == res8 && p.halo == halo8 && p.grp == grp8 && p.tps == tps8 && p.stages >= std::min(st8, min_st)) { rep = r2; break; }
+            if (plan_ok && !over && p.b_resident == res8 && p.halo == halo8 && p.grp == grp8 && p.stages >= std::min(st8, 3)) { rep = r2; break; }
         }
         if (rep == 8) plan_smem(8 * 1024 + cm64_bytes + stg_bytes);
         p.tab_rep = (uint32_t)rep;
@@ -1774,8 +1606,6 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     if (stg_bytes) {
         p.stg_off = (uint32_t)round_up((int)(t->smem - 1024), 128);
         t->smem = 1024 + (size_t)p.stg_off + (size_t)stg_bytes;
-        p.st_wp = st_flat ? (1 << 30) : g.Wp;
-        p.st_magic = st_flat ? 0u : (unsigned)((1ull << 32) / (unsigned)g.Wp) + 1u;
     }
     /* keep residency at ctas_per_sm: a further CTA would fit the registers but stall in tcgen05.alloc */
     t->smem = std::max<size_t>(t->smem, t->ctas_per_sm == 1 ? 120 * 1024 : 80 * 1024);
@@ -1793,16 +1623,6 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
             else if (g.prepass == 1) p.a_shift[tap] = (kh - o.pt) * g.Wp + kw;
             else p.a_shift[tap] = ((kh & 1) * 2 + (kw & 1)) * g.plane + (kh / 2) * g.Wp + kw / 2;
         }
-    if (p.halo == 2) { /* the tap's offset inside the stage, in 16-byte units: its phase's region + its shift inside the region */
-        for (int kh = 0; kh < o.kh; kh++)
-            for (int kw = 0; kw < o.kw; kw++) {
-                const int ph = (kh & 1) * 2 + (kw & 1), loc = (kh / 2) * g.Wp + kw / 2;
-                int boxes = 0, r = 0;
-                for (; r < p.halo_nreg; r++) { if (p.halo_reg_row[r] / g.plane == ph && p.halo_reg_row[r] - ph * g.plane <= loc) break; boxes += p.halo_reg_nb[r]; }
-                if (r == p.halo_nreg) { delete t; return false; }
-                p.a_shift[kh * o.kw + kw] = ((boxes * p.halo_rb + loc - (p.halo_reg_row[r] - ph * g.plane)) * p.a_row_bytes) >> 4;
-            }
-    }
     p.bias = o.bias >= 0 ? reinterpret_cast<const int32_t *>(ag.d_weights + o.bias) : nullptr;
     if (o.bias >= 0 && (o.bias % 4 || o.bias + 4 * (int64_t)o.oc > (int64_t)ag.W)) { delete t; return false; }
     p.cs = o.f0;
@@ -1894,10 +1714,9 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     bool ok = cudaDeviceSynchronize() == cudaSuccess;
 
     const CUtensorMapSwizzle ksw = p.bk == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (p.bk == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-    t->private_in = g.prepass == 0 && o.private_in;
-    if (ok && g.prepass == 0) /* the NCHW planes in the arena, or their private copy (Op::private_in) */
-        ok = make_map3(&t->mapA, t->private_in ? (void *)scratch : (void *)t->src_slot0, (uint64_t)o.ih * o.iw, (uint64_t)o.ic, (uint64_t)ag.capacity,
-                       (uint64_t)o.ih * o.iw, t->private_in ? scratch_stride : ag.slot_stride, TC_BM, (uint32_t)p.bk, CU_TENSOR_MAP_SWIZZLE_128B);
+    if (ok && g.prepass == 0) /* the NCHW planes in the arena */
+        ok = make_map3(&t->mapA, (void *)t->src_slot0, (uint64_t)o.ih * o.iw, (uint64_t)o.ic, (uint64_t)ag.capacity,
+                       (uint64_t)o.ih * o.iw, ag.slot_stride, TC_BM, (uint32_t)p.bk, CU_TENSOR_MAP_SWIZZLE_128B);
     else if (ok && s2d) /* 16-byte pixels, linear rows (no swizzle): the MMA reads them as overlapping 32-byte K rows */
         ok = p.halo_wide ? make_map3(&t->mapA, scratch, 256, (uint64_t)g.npix / 16, (uint64_t)ag.capacity, 256, scratch_stride, 256, (uint32_t)p.halo_rb,
                                      CU_TENSOR_MAP_SWIZZLE_NONE)
@@ -1923,14 +1742,6 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
                          (uint64_t)co_pad * ci_eff, (uint32_t)p.bk, (uint32_t)p.n_tile, ksw);
     { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&t->sms, cudaDevAttrMultiProcessorCount, dev); }
     t->epi = epi_warps;
-    for (int k = 0; ok && t->tst && k < t->nst; k++) {
-        uint8_t *base = ag.d_slots + p.out_off[k];
-        const uint64_t plane_b = (uint64_t)o.oh * o.ow;
-        if (!(st_flat ? make_map_store(&t->mapO[k], base, plane_b, 1, (uint64_t)o.oc, (uint64_t)ag.capacity, plane_b, ag.slot_stride)
-                      : make_map_store(&t->mapO[k], base, (uint64_t)o.ow, (uint64_t)o.oh, (uint64_t)o.oc, (uint64_t)ag.capacity, plane_b, ag.slot_stride)))
-            ok = false;
-    }
-    for (int k = t->tst ? t->nst : 0; k < 3; k++) t->mapO[k] = t->mapB; /* unused slots: any valid map */
     t->kernel = pick_kernel(t->rq, gather, t->tab, t->nst, nhwc_in ? 2 : (p.nhwc_sel >= 0 ? 1 : 0), t->epi, t->tst);
     ok = ok && t->kernel != nullptr;
     ok = ok && cudaFuncSetAttribute((const void *)t->kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 210 * 1024) == cudaSuccess;
@@ -1953,19 +1764,16 @@ bool tc_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, bool u
         /* private copy of the input tensor: the fused outputs may overwrite the input's work buffer (SURVEY C.2) */
         if (cudaMemcpy2DAsync(scr, t->scratch_stride, src, t->slot_stride, (size_t)t->C * t->H * t->W, (size_t)n,
                               cudaMemcpyDeviceToDevice, s) != cudaSuccess) return false;
-    } else if (t->prepass == 0 && t->private_in) {
-        if (cudaMemcpy2DAsync(scr, t->scratch_stride, src, t->slot_stride, (size_t)t->C * t->H * t->W, (size_t)n, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return false;
-        (*launches)++;
     } else if (t->prepass == 4) {
-        launch_pdl(k_s2d16, dim3((t->npix + 1023) / 1024, n), dim3(256), 0, s, src, (unsigned long long)t->slot_stride, scr, (unsigned long long)t->scratch_stride, t->C, t->H, t->W, t->p.Wp, t->npix, t->nhwc_in);
+        k_s2d16<<<dim3((t->npix + 1023) / 1024, n), 256, 0, s>>>(src, (unsigned long long)t->slot_stride, scr, (unsigned long long)t->scratch_stride, t->C, t->H, t->W, t->p.Wp, t->npix, t->nhwc_in);
         (*launches)++;
     } else if (t->prepass == 6 || t->prepass == 5) {
         if (!t->gather_direct && cudaMemcpy2DAsync(scr, t->scratch_stride, src, t->slot_stride, (size_t)t->C * t->H * t->W, (size_t)n,
                                                   cudaMemcpyDeviceToDevice, s) != cudaSuccess) return false;
     } else if (t->prepass && t->prepass != 3 && !(use_linked && t->has_linked)) {
         dim3 g((t->npix + 31) / 32, (t->Cp + 31) / 32, n);
-        launch_pdl(k_to_nhwc, g, dim3(256), 0, s, src, (unsigned long long)t->slot_stride, scr, (unsigned long long)t->scratch_stride, t->C, t->Cp, t->H, t->W,
-                   t->p.Wp, t->plane, t->npix, (int)(t->prepass == 2), t->pt, t->pl);
+        k_to_nhwc<<<g, 256, 0, s>>>(src, (unsigned long long)t->slot_stride, scr, (unsigned long long)t->scratch_stride, t->C, t->Cp, t->H, t->W,
+                                    t->p.Wp, t->plane, t->npix, (int)(t->prepass == 2), t->pt, t->pl);
         (*launches)++;
     }
     TcParams p = t->p;
@@ -1981,7 +1789,7 @@ bool tc_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, bool u
     int sms = t->sms;
     if (sms <= 0) sms = 148;
     const unsigned grid = (unsigned)std::min<long long>(total_tiles, (long long)sms * t->ctas_per_sm);
-    launch_pdl(t->kernel, dim3(grid), dim3((t->epi + (t->prepass == 3 ? 5 : 2)) * 32), t->smem, s, (use_linked && t->has_linked) ? t->mapA_linked : t->mapA, t->mapB, t->mapO[0], t->mapO[1], t->mapO[2], p);
+    t->kernel<<<grid, (t->epi + (t->prepass == 3 ? 5 : 2)) * 32, t->smem, s>>>((use_linked && t->has_linked) ? t->mapA_linked : t->mapA, t->mapB, p);
     (*launches)++;
     return cudaGetLastError() == cudaSuccess;
 }

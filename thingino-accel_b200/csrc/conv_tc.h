@@ -33,8 +33,6 @@ struct TcPlan {
 bool tc_supported(const Op &o);
 /* how many N tiles the kernel would use for `oc` output channels */
 int tc_n_tiles(int oc);
-/* can the kernel read a private copy of its input instead of the arena planes (1x1 layers read straight from the arena otherwise)? */
-bool tc_private_input_ok(const Op &o);
 /* does the kernel read its activations from a private copy (pre-pass) rather than the arena? */
 bool tc_uses_copy(const Op &o);
 /* is that copy the padded / phase-split channel-innermost layout a producing conv's epilogue can write directly? */

@@ -19,7 +19,6 @@ __device__ __forceinline__ uint32_t lut4(const uint8_t *lut, uint32_t w) {
 
 /* out[i] = table[in[i]] (sigmoid / relu / fused unary chains), table index = value + 128 */
 __global__ void __launch_bounds__(256) k_lut16(ArenaView v, KOp o) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     __shared__ uint8_t lut[256];
     lut[threadIdx.x] = v.cpool[o.lut + threadIdx.x];
     __syncthreads();
@@ -75,7 +74,6 @@ __device__ __forceinline__ uint32_t bin4(uint32_t a, uint32_t b, int is_mul, flo
 
 /* int8 mul / add (reference src/mars/mars_runtime.c:818-835, :885-902) */
 __global__ void __launch_bounds__(256) k_bin16(ArenaView v, KOp o) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     const Img im = make_img(v, blockIdx.y);
     const uint8_t *a = im.s_minus_W + o.in0, *b = im.s_minus_W + o.in1;
     uint8_t *out = im.s_minus_W + o.out;
@@ -105,7 +103,6 @@ __global__ void __launch_bounds__(256) k_bin16(ArenaView v, KOp o) {
  * a kernel row is shared by the four (L1), every tap weight is loaded once for all of them, one 4-byte store.  Same arithmetic as dw_i8_point (int32 wrap-around accumulation in tap order, requant_conv);
  * selected for hazard-free layers with ow % 4 == 0 and kernels up to 7 wide. */
 __global__ void __launch_bounds__(256) k_dw_nchw4(ArenaView v, KOp o) {
-    pdl_begin();
     const Img im = make_img(v, blockIdx.y);
     const int ow4 = o.ow >> 2;
     const int64_t total = (int64_t)o.oc * o.oh * ow4;
@@ -149,7 +146,6 @@ static inline bool dw_nchw4_ok(const ArenaView &v, const KOp &o) {
  * SURVEY C.4): out[t + coff] = in[t], a shifted flat copy.  VEC = bytes per access. */
 template <int VEC>
 __global__ void __launch_bounds__(256) k_shift_copy(ArenaView v, KOp o, int periodic) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     const Img im = make_img(v, blockIdx.y);
     uint8_t *out = im.s_minus_W + o.out + o.coff;
     const uint8_t *in = periodic ? (const uint8_t *)(im.s_minus_W + o.out) : (const uint8_t *)(im.s_minus_W + o.in0);
@@ -176,7 +172,6 @@ __global__ void __launch_bounds__(256) k_shift_copy(ArenaView v, KOp o, int peri
  * smem = (Co * CI4 + Co) * 4 bytes. */
 template <int CI4>
 __global__ void __launch_bounds__(128) k_conv1x1_inplace_reg(ArenaView v, KOp o) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     extern __shared__ uint32_t smem_w[];
     const Img im = make_img(v, blockIdx.y);
     uint32_t *ws = smem_w;                                        /* [oc][CI4] */
@@ -256,9 +251,9 @@ static inline void launch_inplace_reg(const ArenaView &v, const KOp &o, int n_im
         cudaFuncSetAttribute(k_conv1x1_inplace_reg<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
         cudaFuncSetAttribute(k_conv1x1_inplace_reg<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
     }
-    if (o.ic == 32) launch_pdl(k_conv1x1_inplace_reg<8>, dim3(g), dim3(128), (size_t)(smem), s, v, o);
-    else if (o.ic == 64) launch_pdl(k_conv1x1_inplace_reg<16>, dim3(g), dim3(128), (size_t)(smem), s, v, o);
-    else launch_pdl(k_conv1x1_inplace_reg<32>, dim3(g), dim3(128), (size_t)(smem), s, v, o);
+    if (o.ic == 32) k_conv1x1_inplace_reg<8><<<g, 128, smem, s>>>(v, o);
+    else if (o.ic == 64) k_conv1x1_inplace_reg<16><<<g, 128, smem, s>>>(v, o);
+    else k_conv1x1_inplace_reg<32><<<g, 128, smem, s>>>(v, o);
 }
 
 static inline unsigned fast_grid(uint64_t items, unsigned per_block = 256) {
@@ -270,7 +265,6 @@ static inline unsigned fast_grid(uint64_t items, unsigned per_block = 256) {
 /* shifted flat copy whose source and destination are only 4-byte aligned relative to each other: 16-byte stores on the
  * destination's alignment, four 4-byte loads each; head and tail words one by one.  n4 = words to copy. */
 __global__ void __launch_bounds__(256) k_shift_copy_d16(ArenaView v, KOp o) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     const Img im = make_img(v, blockIdx.y);
     uint32_t *out = reinterpret_cast<uint32_t *>(im.s_minus_W + o.out + o.coff);
     const uint32_t *in = reinterpret_cast<const uint32_t *>(im.s_minus_W + o.in0);
@@ -295,7 +289,6 @@ __global__ void __launch_bounds__(256) k_shift_copy_d16(ArenaView v, KOp o) {
  * L = lcm(s, 16) bytes, so every 16-byte aligned destination vector is one aligned 16-byte read of it; write-only traffic.
  * grid = (chunks, images), smem = L bytes. */
 __global__ void __launch_bounds__(256) k_fill_periodic(ArenaView v, KOp o, int L) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     extern __shared__ __align__(16) uint8_t fp_pat[];
     const Img im = make_img(v, blockIdx.y);
     uint8_t *base = im.s_minus_W + o.out; /* pattern at [0, s), destination [s, s + n) */
@@ -343,15 +336,14 @@ static inline bool fast_flat_ok(const ArenaView &v, const KOp &o) {
 }
 static inline void launch_fast_flat(const ArenaView &v, const KOp &o, int n_img, cudaStream_t s) {
     dim3 g(fast_grid(o.n >> 4), n_img);
-    if (o.kind == OP_MUL_I8 || o.kind == OP_ADD_I8) launch_pdl(k_bin16, dim3(g), dim3(256), (size_t)(0), s, v, o);
-    else launch_pdl(k_lut16, dim3(g), dim3(256), (size_t)(0), s, v, o);
+    if (o.kind == OP_MUL_I8 || o.kind == OP_ADD_I8) k_bin16<<<g, 256, 0, s>>>(v, o);
+    else k_lut16<<<g, 256, 0, s>>>(v, o);
 }
 
 /* maxpool / upsample over 4 channels per thread (reference src/mars/mars_runtime.c:934-956, :1027-1040; NHWC indexing of
  * shape[1..3] whatever the tag, SURVEY C.4): signed per-byte max with __vmaxs4, window clipped at the bottom/right edge,
  * pads ignored, exactly like the point functions. */
 __global__ void __launch_bounds__(256) k_spatial_vec4(ArenaView v, KOp o) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     const Img im = make_img(v, blockIdx.y);
     const uint32_t *in = reinterpret_cast<const uint32_t *>(im.s_minus_W + o.in0);
     uint32_t *out = reinterpret_cast<uint32_t *>(im.s_minus_W + o.out);
@@ -384,7 +376,6 @@ __global__ void __launch_bounds__(256) k_spatial_vec4(ArenaView v, KOp o) {
  * clipped at the right / bottom edge and pads are ignored, exactly like maxpool_point.  grid = (strips, images),
  * smem = 2 * (TH + kh - 1) * RW words. */
 __global__ void __launch_bounds__(256) k_maxpool_sep(ArenaView v, KOp o, int TH) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     extern __shared__ uint32_t mp_smem[];
     const Img im = make_img(v, blockIdx.y);
     const uint32_t *in = reinterpret_cast<const uint32_t *>(im.s_minus_W + o.in0);
@@ -423,7 +414,6 @@ __device__ __forceinline__ S16x4 s16x4_from_s8x4(uint32_t w) { return {__byte_pe
 __device__ __forceinline__ S16x4 s16x4_max3(S16x4 a, S16x4 b, S16x4 c) { return {__vimax3_s16x2(a.lo, b.lo, c.lo), __vimax3_s16x2(a.hi, b.hi, c.hi)}; }
 __device__ __forceinline__ uint32_t s8x4_from_s16x4(S16x4 a) { return __byte_perm(a.lo, a.hi, 0x6420u); }
 __global__ void __launch_bounds__(128) k_maxpool5_col(ArenaView v, KOp o, int rows_per_block) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     const Img im = make_img(v, blockIdx.z);
     const int c4 = o.ic >> 2, RW = o.iw * c4, OW = o.ow * c4;
     const int xw = blockIdx.x * 128 + threadIdx.x;
@@ -465,7 +455,6 @@ __global__ void __launch_bounds__(128) k_maxpool5_col(ArenaView v, KOp o, int ro
  * through L1.  Divisions by multiplication. */
 #define UPS_ROWS 8
 __global__ void __launch_bounds__(256) k_upsample_rep(ArenaView v, KOp o) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     const Img im = make_img(v, blockIdx.y);
     const int c4 = o.ic >> 2, orw = o.ow * c4;
     const unsigned m_c4 = 0xFFFFFFFFu / (unsigned)c4 + 1u, m_sw = 0xFFFFFFFFu / (unsigned)o.sw + 1u; /* floor(a / d) = umulhi(a, m) */
@@ -485,7 +474,6 @@ __global__ void __launch_bounds__(256) k_upsample_rep(ArenaView v, KOp o) {
  * src/mars/mars_runtime.c:963-1000): pixel p copies its ic bytes to out[p * oc + coff]; 16 bytes per thread, consecutive
  * threads walk the channel chunks of a pixel and then the next pixel (coalesced on both sides) */
 __global__ void __launch_bounds__(256) k_concat_strided16(ArenaView v, KOp o) {
-    pdl_begin(); /* dependents may be scheduled; wait for the previous kernel of the step before touching the arena */
     const Img im = make_img(v, blockIdx.y);
     const uint4 *in = reinterpret_cast<const uint4 *>(im.s_minus_W + o.in0);
     uint8_t *out = im.s_minus_W + o.out + o.coff;
@@ -521,7 +509,6 @@ static inline bool upsample_ranges_overlap(const KOp &o) {
  * index split per input word instead of two divisions per output word (ncu on k_upsample_rep: alu 64 %, xu 28 %, 47
  * instructions per output warp-word).  Only the input rows / columns the output reads are visited. */
 __global__ void __launch_bounds__(256) k_upsample_exact(ArenaView v, KOp o) {
-    pdl_begin();
     const Img im = make_img(v, blockIdx.z);
     const int c4 = o.ic >> 2, irw = o.iw * c4, orw = o.ow * c4;
     const int w = blockIdx.x * 256 + threadIdx.x, yi = blockIdx.y;
@@ -537,7 +524,7 @@ __global__ void __launch_bounds__(256) k_upsample_exact(ArenaView v, KOp o) {
 static inline void launch_fast_spatial(const ArenaView &v, const KOp &o, int n_img, cudaStream_t s) {
     if (o.kind == OP_MAXPOOL && o.sh == 1 && o.sw == 1 && o.kh == 5 && o.kw == 5 && o.oh <= o.ih && o.ow <= o.iw && n_img <= 65535) {
         const int OW = o.ow * (o.ic >> 2), rows = 64;
-        launch_pdl(k_maxpool5_col, dim3(dim3((OW + 127) / 128, (o.oh + rows - 1) / rows, n_img)), dim3(128), (size_t)(0), s, v, o, rows);
+        k_maxpool5_col<<<dim3((OW + 127) / 128, (o.oh + rows - 1) / rows, n_img), 128, 0, s>>>(v, o, rows);
         return;
     }
     if (o.kind == OP_MAXPOOL && o.sh == 1 && o.sw == 1 && o.kh >= 1 && o.kw >= 1 && o.oh <= o.ih && o.ow <= o.iw) {
@@ -548,28 +535,28 @@ static inline void launch_fast_spatial(const ArenaView &v, const KOp &o, int n_i
             static unsigned long long attr = 0;
             if (first_time_on_device(&attr)) cudaFuncSetAttribute(k_maxpool_sep, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
             dim3 g((o.oh + TH - 1) / TH, n_img);
-            launch_pdl(k_maxpool_sep, dim3(g), dim3(256), (size_t)((size_t)2 * (TH + o.kh - 1) * RW * 4), s, v, o, TH);
+            k_maxpool_sep<<<g, 256, (size_t)2 * (TH + o.kh - 1) * RW * 4, s>>>(v, o, TH);
             return;
         }
     }
     if (o.kind == OP_UPSAMPLE && o.sh >= 1 && o.sw >= 1 && o.sw <= 4 && o.sh <= 4 && o.oh <= o.ih * o.sh && o.ow <= o.iw * o.sw && o.oh <= 65535 * o.sh &&
         n_img <= 65535 && !upsample_ranges_overlap(o)) {
         const int rows_in = (o.oh + o.sh - 1) / o.sh, cols_in = (o.ow + o.sw - 1) / o.sw; /* the input rows / pixels the output reads */
-        launch_pdl(k_upsample_exact, dim3(dim3((cols_in * (o.ic >> 2) + 255) / 256, rows_in, n_img)), dim3(256), (size_t)(0), s, v, o);
+        k_upsample_exact<<<dim3((cols_in * (o.ic >> 2) + 255) / 256, rows_in, n_img), 256, 0, s>>>(v, o);
         return;
     }
     if (o.kind == OP_UPSAMPLE && o.oh <= 65535 && (long long)o.ow * (o.ic >> 2) < 65536) {
-        launch_pdl(k_upsample_rep, dim3(dim3((o.oh + UPS_ROWS - 1) / UPS_ROWS, n_img)), dim3(256), (size_t)(0), s, v, o);
+        k_upsample_rep<<<dim3((o.oh + UPS_ROWS - 1) / UPS_ROWS, n_img), 256, 0, s>>>(v, o);
         return;
     }
     if (o.kind == OP_MAXPOOL || o.kind == OP_UPSAMPLE) {
         /* one output word per thread: the loads of a thread are dependent, so parallelism comes from the number of warps */
         dim3 g((unsigned)(((uint64_t)o.oh * o.ow * (o.ic >> 2) + 255) / 256), n_img);
-        launch_pdl(k_spatial_vec4, dim3(g), dim3(256), (size_t)(0), s, v, o);
+        k_spatial_vec4<<<g, 256, 0, s>>>(v, o);
         return;
     }
     if (o.kind == OP_CONCAT && o.ic != o.oc) {
-        launch_pdl(k_concat_strided16, dim3(dim3(fast_grid(o.n >> 4), n_img)), dim3(256), (size_t)(0), s, v, o);
+        k_concat_strided16<<<dim3(fast_grid(o.n >> 4), n_img), 256, 0, s>>>(v, o);
         return;
     }
     const int periodic = o.kind == OP_CONCAT_PERIODIC;
@@ -578,7 +565,7 @@ static inline void launch_fast_spatial(const ArenaView &v, const KOp &o, int n_i
         while (b) { int t = g % b; g = b; b = t; } /* gcd(coff, 16) */
         const long long L = (long long)o.coff / g * 16;
         if (L <= 16384) {
-            launch_pdl(k_fill_periodic, dim3(dim3(fast_grid(o.n >> 4), n_img)), dim3(256), (size_t)((size_t)L), s, v, o, (int)L);
+            k_fill_periodic<<<dim3(fast_grid(o.n >> 4), n_img), 256, L, s>>>(v, o, (int)L);
             return;
         }
     }
@@ -590,10 +577,10 @@ static inline void launch_fast_spatial(const ArenaView &v, const KOp &o, int n_i
     if (((rel_d | rel_s) & 15) == 0 && (!periodic || (o.coff & 15) == 0)) vec = 16;
     else if (((rel_d | rel_s) & 3) == 0 && (!periodic || (o.coff & 3) == 0)) vec = 4;
     dim3 g(fast_grid(o.n / vec), n_img);
-    if (vec == 16) launch_pdl(k_shift_copy<16>, dim3(g), dim3(256), (size_t)(0), s, v, o, periodic);
-    else if (vec == 4 && !periodic && o.n >= 1024) launch_pdl(k_shift_copy_d16, dim3(dim3(fast_grid(o.n / 16), n_img)), dim3(256), (size_t)(0), s, v, o);
-    else if (vec == 4) launch_pdl(k_shift_copy<4>, dim3(g), dim3(256), (size_t)(0), s, v, o, periodic);
-    else launch_pdl(k_shift_copy<1>, dim3(g), dim3(256), (size_t)(0), s, v, o, periodic);
+    if (vec == 16) k_shift_copy<16><<<g, 256, 0, s>>>(v, o, periodic);
+    else if (vec == 4 && !periodic && o.n >= 1024) k_shift_copy_d16<<<dim3(fast_grid(o.n / 16), n_img), 256, 0, s>>>(v, o);
+    else if (vec == 4) k_shift_copy<4><<<g, 256, 0, s>>>(v, o, periodic);
+    else k_shift_copy<1><<<g, 256, 0, s>>>(v, o, periodic);
 }
 
 static inline bool fast_conv_nchw_ok(const KOp &) { return false; }

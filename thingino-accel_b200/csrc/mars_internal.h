@@ -94,9 +94,6 @@ struct Op {
      * own layout pre-pass (copy_from = producer op, copy_off = byte offset of its region in the per-image link area) */
     int copy_from = -1, nhwc_consumer = -1, nhwc_stream = -1;
     int64_t copy_off = 0;
-    /* 1x1 tensor-core conv whose fused outputs overwrite its own input buffer while other CTAs (a second N tile) still read it:
-     * the kernel reads a private device copy of the input made just before the launch (round-robin work buffers, SURVEY C.2) */
-    bool private_in = false;
     /* concat forwarding (opt level 3): the op's stream fwd_stream (0 = Z, 1 = S, 2 = Y) is ALSO written at arena offset fwd_out --
      * its place in the output of the concat that would copy it there later (program.cpp forward_concat_inputs) */
     int64_t fwd_out = -1;
@@ -126,32 +123,6 @@ struct ArenaView {
 };
 
 struct Model; /* defined in runtime.cu */
-
-#ifdef __CUDACC__
-/* ---- programmatic dependent launch (PDL) -----------------------------------------------------------------------------
- * The ~110 kernels of a step run back to back on one stream; each is launched with
- * cudaLaunchAttributeProgrammaticStreamSerialization, so the next kernel's CTAs may be scheduled (and run their prologue:
- * barrier init, TMEM allocation, table fill) while the tail of the current one drains, instead of after it.  Every such kernel
- * releases its dependents at its very start and executes griddepcontrol.wait before its first access to memory another
- * kernel of the step writes or reads -- the wait returns once the preceding grid has completed and its writes are visible.
- * Opt-in (MARS_PDL=1): measured slower than plain stream order on this workload, see pdl_enabled() in runtime.cu; without the
- * attribute the wait is a no-op. */
-__device__ __forceinline__ void pdl_release_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait_prior_grid() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_begin() { pdl_release_dependents(); pdl_wait_prior_grid(); }
-bool pdl_enabled();
-template <typename... KArgs, typename... Args>
-static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-#endif
 
 /* ---- host-side helpers shared between translation units ---- */
 size_t tensor_byte_size(const mars_tensor_t *t);

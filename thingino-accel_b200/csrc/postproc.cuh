@@ -63,7 +63,6 @@ __device__ __forceinline__ int block_excl_scan(int v, int *total, int *warp_sums
 __global__ void __launch_bounds__(256) k_parse_output(const int8_t *data, size_t img_stride, int npred, float scale,
                                                       const DecodeTables *tab, mars_det_t *dets, int32_t *counts,
                                                       int maxd, int det_stride) {
-    pdl_begin();
     __shared__ int warp_sums[32];
     const int8_t *rows = data + (size_t)blockIdx.x * img_stride;
     mars_det_t *out = dets + (size_t)blockIdx.x * det_stride;
@@ -123,105 +122,16 @@ __device__ __forceinline__ float iou_corner(const mars_box_t &a, const mars_box_
 }
 
 /*
- * Exchange-sort emulation, one PASS at a time, the whole block working on each pass.
- * Pass i of `for i: for j>i: if d[j].conf > d[i].conf swap` (reference
- * src/mars/mars_yolo_test.c:108-110) walks the strict prefix-maximum records
- * r0 = i < r1 < ... < rk of key[i..n): afterwards position r0 holds the element of rk and every
- * other record position holds the previous record's element (SURVEY A.4; NOT a stable sort).
- * Thread j owns position j and keeps its element in registers.  Per pass: a warp-level prefix
- * max + one barrier gives every thread the maximum of all earlier positions, hence the records;
- * the last record of every warp + a second barrier gives every record its predecessor, whose
- * element it then reads from the shared copy of the array as it stood before the pass.  The shared
- * copy is double buffered (written after the reads of a pass, read again only behind the next
- * pass's barriers), so a pass costs two barriers whatever the data looks like.  NaN keys never
- * compare greater, exactly as in the C loop.  blockDim.x = NMS_THREADS >= n.
- */
-#define NMS_THREADS 1024
-
-struct NmsSortShared {
-    float key[2][MARS_MAX_DETS];
-    uint16_t idx[2][MARS_MAX_DETS];
-    float wmax[32];
-    int wlast[32];
-    int skip[2];
-};
-
-/* on return thread j < n holds the index (into the unsorted input) of sorted element j */
-__device__ __forceinline__ int exchange_sort_block(NmsSortShared &sh, float myk, int n) {
-    const int j = threadIdx.x, lane = j & 31, wid = j >> 5;
-    const float NEG_INF = -__int_as_float(0x7f800000);
-    int myi = j, cur = 0;
-    sh.key[0][j] = myk;
-    sh.idx[0][j] = (uint16_t)j;
-    __syncthreads();
-    bool parked = false;
-    for (int i = 0; i + 1 < n; i++) {
-        /* a warp whose positions are all final (below i) or beyond n only keeps the barrier count: it publishes
-         * neutral values once and then skips the arithmetic of every further pass */
-        if ((wid + 1) * 32 <= i || wid * 32 >= n) {
-            if (!parked) {
-                if (lane == 0) { sh.wmax[wid] = NEG_INF; sh.wlast[wid] = -1; }
-                parked = true;
-            }
-            __syncthreads();
-            if (!sh.skip[i & 1]) __syncthreads();
-            continue;
-        }
-        const bool act = j >= i && j < n;
-        const float v = (act && myk == myk) ? myk : NEG_INF;
-        float inc = v; /* inclusive prefix max inside the warp */
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const float y = __shfl_up_sync(0xffffffffu, inc, d);
-            if (lane >= d) inc = fmaxf(inc, y);
-        }
-        if (lane == 31) sh.wmax[wid] = inc;
-        if (j == i) sh.skip[i & 1] = (myk != myk); /* NaN in hand: no comparison succeeds, the pass moves nothing */
-        __syncthreads();
-        if (sh.skip[i & 1]) continue; /* uniform; slot i & 1 is rewritten two passes later, behind the next pass's barrier */
-        float before = (lane < wid) ? sh.wmax[lane] : NEG_INF; /* max over all earlier warps */
-#pragma unroll
-        for (int d = 16; d; d >>= 1) before = fmaxf(before, __shfl_xor_sync(0xffffffffu, before, d));
-        float excl = __shfl_up_sync(0xffffffffu, inc, 1);
-        excl = lane ? fmaxf(excl, before) : before;
-        const bool rec = act && (j == i || myk > excl);
-        const unsigned m = __ballot_sync(0xffffffffu, rec);
-        if (lane == 0) sh.wlast[wid] = m ? (wid * 32 + 31 - __clz(m)) : -1;
-        __syncthreads();
-        /* predecessor record of each record; the first record (position i) takes the LAST record's element */
-        const int wl = sh.wlast[lane];
-        const unsigned has = __ballot_sync(0xffffffffu, wl >= 0);
-        float nk = myk;
-        int ni = myi;
-        /* every lane computes the warp-level predecessor (convergent shuffle), record lanes then select */
-        {
-            const unsigned prevw = has & ((1u << wid) - 1u);
-            const int w = prevw ? 31 - __clz(prevw) : 31 - __clz(has | 1u);
-            const int from_prev = __shfl_sync(0xffffffffu, wl, w);
-            if (rec) {
-                const unsigned lower = m & ((1u << lane) - 1u);
-                const int src = lower ? wid * 32 + 31 - __clz(lower) : from_prev;
-                if (src != j) { nk = sh.key[cur][src]; ni = sh.idx[cur][src]; }
-            }
-        }
-        myk = nk; myi = ni;
-        cur ^= 1;
-        sh.key[cur][j] = myk;
-        sh.idx[cur][j] = (uint16_t)myi;
-    }
-    return myi;
-}
-
-
-/*
- * The same exchange-sort permutation, one WARP per image and no barriers (the default path; the block-wide version
- * above is kept as a cross-check, MARS_NMS_BLOCKSORT=1).
+ * Exchange-sort emulation, one WARP per image and no barriers.  Pass i of `for i: for j>i: if d[j].conf > d[i].conf swap`
+ * (reference src/mars/mars_yolo_test.c:108-110) walks the strict prefix-maximum records r0 = i < r1 < ... < rk of key[i..n):
+ * afterwards position r0 holds the element of rk and every other record position holds the previous record's element
+ * (SURVEY A.4; NOT a stable sort).
  *
  * Lane L holds positions [32L, 32L+32) in registers (key k[], input index x[]); the 32 positions of the lane that
  * contains the current pass index i are spread one per lane (Bk, Bx: "the block"), so that the hand d[i] is a shuffle
- * from lane i % 32 and nothing is indexed dynamically.  Pass i, as in exchange_sort_block, rotates the chain of strict
- * prefix-maximum records of d[i..n): every record takes its predecessor's element, the first record takes the hand and
- * position i takes the last record's element.  The chain is found in two levels:
+ * from lane i % 32 and nothing is indexed dynamically.  Pass i rotates the chain of strict prefix-maximum records of d[i..n):
+ * every record takes its predecessor's element, the first record takes the hand and position i takes the last record's
+ * element.  The chain is found in two levels:
  *   block    : prefix max over the 32 lanes (retired positions hold -inf and are inert);
  *   registers: each lane keeps the first-occurrence maximum (lm, lmx) of its 32 positions; a prefix max over the lanes
  *              (seeded with the block's outgoing maximum) tells which lanes contain records and what enters them, and those
@@ -368,7 +278,6 @@ __device__ __forceinline__ void nms_sort_image(const mars_det_t *in, int n, uint
 
 __global__ void __launch_bounds__(32) k_nms_sort_warp(const mars_det_t *dets_in, const int32_t *counts_in, int det_stride,
                                                       unsigned *scratch, size_t scratch_stride_words) {
-    pdl_begin();
     const int img = blockIdx.x, lane = threadIdx.x;
     const mars_det_t *in = dets_in + (size_t)img * det_stride;
     uint16_t *order = reinterpret_cast<uint16_t *>(scratch + (size_t)img * scratch_stride_words + (size_t)MARS_MAX_DETS * 32);
@@ -386,9 +295,10 @@ __global__ void __launch_bounds__(32) k_nms_sort_warp(const mars_det_t *dets_in,
 #define NMS_CLASS_ROWS 128 /* class ids -1..126 get a member bitset; anything else takes the dense pair loop */
 #define NMS_SCRATCH_WORDS ((size_t)MARS_MAX_DETS * 32 + MARS_MAX_DETS / 2 + NMS_CLASS_ROWS * 32)
 
+#define NMS_THREADS 1024 /* threads of k_nms_center: one per sorted position */
+
 /* dynamic shared memory of k_nms_center */
 struct NmsShared {
-    NmsSortShared sort;
     float x0[MARS_MAX_DETS], y0[MARS_MAX_DETS], x1[MARS_MAX_DETS], y1[MARS_MAX_DETS], area[MARS_MAX_DETS];
     int cls[MARS_MAX_DETS];
     unsigned members[NMS_CLASS_ROWS][32]; /* bit j of row c: sorted element j has class c - 1 */
@@ -416,8 +326,7 @@ __device__ __forceinline__ float iou_pre(float ax0, float ay0, float ax1, float 
  * the same result as the sequential double loop. */
 __global__ void __launch_bounds__(NMS_THREADS, 2) k_nms_center(const mars_det_t *dets_in, const int32_t *counts_in,
                                                                mars_det_t *dets_out, int32_t *counts_out, int det_stride,
-                                                               float thresh, unsigned *mask_scratch, int presorted) {
-    pdl_begin();
+                                                               float thresh, unsigned *mask_scratch) {
     extern __shared__ __align__(16) uint8_t nms_smem[];
     NmsShared &sh = *reinterpret_cast<NmsShared *>(nms_smem);
     const mars_det_t *in = dets_in + (size_t)blockIdx.x * det_stride;
@@ -427,9 +336,8 @@ __global__ void __launch_bounds__(NMS_THREADS, 2) k_nms_center(const mars_det_t 
     int n = counts_in[blockIdx.x];
     if (n > MARS_MAX_DETS) n = MARS_MAX_DETS;
     const int j = threadIdx.x, lane = j & 31, wid = j >> 5;
-    const float NEG_INF = -__int_as_float(0x7f800000);
-    /* sorted position j holds input element src: from k_nms_sort_warp, or (cross-check path) sorted here by the block */
-    const int src = presorted ? (j < n ? order[j] : j) : exchange_sort_block(sh.sort, j < n ? in[j].conf : NEG_INF, n);
+    /* sorted position j holds input element src (k_nms_sort_warp) */
+    const int src = j < n ? order[j] : j;
     for (int q = j; q < NMS_CLASS_ROWS * 32; q += NMS_THREADS) (&sh.members[0][0])[q] = 0u;
     if (j == 0) sh.dense = 0;
     mars_det_t me;
@@ -534,7 +442,6 @@ struct NmsSupShared {
 __global__ void __launch_bounds__(NMS_SUP_THREADS, 8) k_nms_suppress(const mars_det_t *dets_in, const int32_t *counts_in,
                                                                      mars_det_t *dets_out, int32_t *counts_out, int det_stride,
                                                                      float thresh, unsigned *scratch) {
-    pdl_begin();
     __shared__ NmsSupShared sh;
     const mars_det_t *in = dets_in + (size_t)blockIdx.x * det_stride;
     mars_det_t *out = dets_out + (size_t)blockIdx.x * det_stride;
@@ -653,22 +560,17 @@ __global__ void __launch_bounds__(NMS_SUP_THREADS, 8) k_nms_suppress(const mars_
 
 static inline cudaError_t launch_nms_center(const mars_det_t *dets_in, const int32_t *counts_in, mars_det_t *dets_out,
                                             int32_t *counts_out, int det_stride, float thresh, int n_img, unsigned *scratch /* NMS_SCRATCH_WORDS per image */,
-                                            cudaStream_t s, int *launches = nullptr) {
+                                            cudaStream_t s) {
     static unsigned long long attr = 0; /* function attributes are per device */
-    static const bool block_sort = getenv("MARS_NMS_BLOCKSORT") && atoi(getenv("MARS_NMS_BLOCKSORT")) != 0;
     if (first_time_on_device(&attr)) {
         cudaError_t e = cudaFuncSetAttribute(k_nms_center, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(NmsShared));
         if (e != cudaSuccess) return e;
     }
-    if (!block_sort) {
-        launch_pdl(k_nms_sort_warp, dim3(n_img), dim3(32), 0, s, dets_in, counts_in, det_stride, scratch, NMS_SCRATCH_WORDS);
-        /* many images: eight 256-thread blocks per SM keep the whole batch resident (throughput); few images: 1024 threads
-         * per image finish each one sooner (latency) */
-        static const int force = getenv("MARS_NMS_SUPPRESS") ? atoi(getenv("MARS_NMS_SUPPRESS")) : -1; /* 1 / 0: always / never (tests) */
-        if (force == 1 || (force != 0 && n_img > 2 * 296)) launch_pdl(k_nms_suppress, dim3(n_img), dim3(NMS_SUP_THREADS), 0, s, dets_in, counts_in, dets_out, counts_out, det_stride, thresh, scratch);
-        else launch_pdl(k_nms_center, dim3(n_img), dim3(NMS_THREADS), sizeof(NmsShared), s, dets_in, counts_in, dets_out, counts_out, det_stride, thresh, scratch, 1);
-    } else launch_pdl(k_nms_center, dim3(n_img), dim3(NMS_THREADS), sizeof(NmsShared), s, dets_in, counts_in, dets_out, counts_out, det_stride, thresh, scratch, 0);
-    if (launches) *launches = block_sort ? 1 : 2;
+    k_nms_sort_warp<<<n_img, 32, 0, s>>>(dets_in, counts_in, det_stride, scratch, NMS_SCRATCH_WORDS);
+    /* many images: eight 256-thread blocks per SM keep the whole batch resident (throughput); few images: 1024 threads
+     * per image finish each one sooner (latency) */
+    if (n_img > 2 * 296) k_nms_suppress<<<n_img, NMS_SUP_THREADS, 0, s>>>(dets_in, counts_in, dets_out, counts_out, det_stride, thresh, scratch);
+    else k_nms_center<<<n_img, NMS_THREADS, sizeof(NmsShared), s>>>(dets_in, counts_in, dets_out, counts_out, det_stride, thresh, scratch);
     return cudaGetLastError();
 }
 

@@ -586,16 +586,8 @@ static void fuse_silu(Program *p, int64_t W) {
             const bool same_tile = c.kh == 1 && c.kw == 1 && tc_n_tiles(c.oc) == 1 && c.oh == c.ih && c.ow == c.iw &&
                                    (s.out == c.in0 || !overlap(s.out, s.out + numel, x0, x1)) &&
                                    (m.out == c.in0 || !overlap(m.out, m.out + numel, x0, x1));
-            if (!tc_uses_copy(c) && !same_tile) {
-                /* several N tiles (Co > 256): a CTA's outputs would overwrite input pixels the other N tile's CTAs still read.
-                 * A private copy of the input (one device-to-device copy per launch, a fraction of the two element-wise passes
-                 * it saves) makes the fusion legal */
-                /* opt-in (MARS_FUSE_PRIVATE=1): measured a wash on the 20 x 20 layers it applies to in the headline model -- the copy
-                 * and the slower table epilogue cost what the two element-wise passes did (profiles/r02r) */
-                static const bool fuse_private = getenv("MARS_FUSE_PRIVATE") && atoi(getenv("MARS_FUSE_PRIVATE")) != 0;
-                if (fuse_private && c.kind == OP_CONV_I8_NCHW && c.kh == 1 && c.kw == 1 && !c.xlat && tc_private_input_ok(c)) c.private_in = true;
-                else continue;
-            }
+            /* several N tiles (Co > 256): a CTA's outputs would overwrite input pixels the other N tile's CTAs still read */
+            if (!tc_uses_copy(c) && !same_tile) continue;
         }
         /* neither follower may clobber the weights or the bias the kernel is still reading: both live below W */
         int8_t lut[256];
@@ -611,7 +603,7 @@ static void fuse_silu(Program *p, int64_t W) {
         c.store_y = c.out != m.out;
         c.fused_layers = 2;
         c.whi = std::max(c.whi, std::max(s.whi, m.whi));
-        c.note = c.private_in ? "conv+sigmoid+mul fused (reads a private copy of its input)" : "conv+sigmoid+mul fused";
+        c.note = "conv+sigmoid+mul fused";
         s.kind = OP_NOP; s.note = "folded into the conv epilogue";
         m.kind = OP_NOP; m.note = "folded into the conv epilogue";
     }
@@ -890,12 +882,9 @@ mars_error_t compile_program(const mars_header_t &h, const mars_runtime_tensor_t
             int64_t es = (d.dtype == MARS_DTYPE_FLOAT32 || d.dtype == MARS_DTYPE_INT32) ? 4 : (d.dtype == MARS_DTYPE_INT16 ? 2 : 1);
             host_written.add((int64_t)toff[ti], (int64_t)toff[ti] + (int64_t)numel_of(d) * es);
         }
-        static const bool fwd_enabled = !(getenv("MARS_CONCAT_FWD") && atoi(getenv("MARS_CONCAT_FWD")) == 0);
         elide_dead_stores(out, observed, host_written); /* first: which streams of a conv are stored at all */
-        if (fwd_enabled) {
-            forward_concat_inputs(out);
-            elide_dead_stores(out, observed, host_written); /* again: the original of a forwarded stream is usually dead now */
-        }
+        forward_concat_inputs(out);
+        elide_dead_stores(out, observed, host_written); /* again: the original of a forwarded stream is usually dead now */
     }
     /* tables are addressed in 256-byte units; keep the pool non-empty so the upload is uniform */
     if (out->const_pool.empty()) out->const_pool.resize(256, 0);

@@ -61,14 +61,6 @@ void set_last_error(const char *fmt, ...) {
         }                                                                                      \
     } while (0)
 
-bool pdl_enabled() {
-    /* measured on B200 (one_step.py, yolov5s-shaped graph, CUDA-graph replay): 5.93 ms with PDL against 5.58 ms without at 128
-     * images, 39.0 against 37.6 ms at 1024 -- the early CTAs of the next kernel take shared memory and TMEM from the persistent
-     * CTAs still running.  Off unless MARS_PDL=1. */
-    static const bool on = getenv("MARS_PDL") && atoi(getenv("MARS_PDL")) != 0;
-    return on;
-}
-
 bool first_time_on_device(unsigned long long *mask) {
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev > 63) return true;
@@ -457,7 +449,7 @@ static mars_error_t launch_op(Model *m, size_t op_index, int first, int n, bool 
             if (o.kind == OP_CONV_I8_NCHW && !xl && fast_conv_nchw_ok(k)) {
                 launch_fast_conv_nchw(v, k, n, s);
             } else if (o.kind == OP_DW_I8 && !xl && m->opt_level >= 1 && dw_nchw4_ok(v, k)) {
-                launch_pdl(k_dw_nchw4, dim3(blocks_for((uint64_t)o.oc * o.oh * (o.ow >> 2), 256), n), dim3(256), (size_t)0, s, v, k);
+                k_dw_nchw4<<<dim3(blocks_for((uint64_t)o.oc * o.oh * (o.ow >> 2), 256), n), 256, 0, s>>>(v, k);
             } else {
                 dim3 g(blocks_for(P * o.oc, 256), n);
                 if (xl) k_conv_point<true><<<g, 256, 0, s>>>(v, k); else k_conv_point<false><<<g, 256, 0, s>>>(v, k);
@@ -524,18 +516,11 @@ static mars_error_t launch_op(Model *m, size_t op_index, int first, int n, bool 
     return MARS_OK;
 }
 
-/* all ops (or the ops of one layer, or the ops [op_lo, op_hi)) over slots [first, first+n) on m->stream */
-static mars_error_t enqueue_ops(Model *m, int first, int n, int only_layer, size_t op_lo = 0, size_t op_hi = (size_t)-1) {
+/* all ops (or the ops of one layer) over slots [first, first+n) on m->stream */
+static mars_error_t enqueue_ops(Model *m, int first, int n, int only_layer) {
     mars_error_t e = compile_model(m);
     if (e != MARS_OK) return e;
     const size_t nops = m->prog.ops.size();
-    if (op_lo != 0 || op_hi < nops) { /* a slice of the op list (micro-batched head / full-batch tail): no per-op events */
-        for (size_t i = op_lo; i < std::min(op_hi, nops); i++) {
-            e = launch_op(m, i, first, n, true);
-            if (e != MARS_OK) return e;
-        }
-        return MARS_OK;
-    }
     if (m->profile && m->prof_ev.size() < nops + 1) {
         while (m->prof_ev.size() < nops + 1) {
             cudaEvent_t ev;
@@ -622,14 +607,12 @@ static mars_error_t enqueue_detect(Model *m, int first, int n, float thresh) {
     mars_error_t e = ensure_tables(m, d.scale);
     if (e != MARS_OK) return e;
     const int8_t *data = reinterpret_cast<const int8_t *>(dev_addr(m, m->toff[oi], first));
-    int nms_launches = 1;
-    launch_pdl(k_parse_output, dim3(n), dim3(256), 0, m->stream, data, m->slot_stride, d.shape[1], d.scale, m->d_tab,
-                                            m->d_raw + (size_t)first * MARS_MAX_DETS, m->d_raw_cnt + first, 1000,
-                                            MARS_MAX_DETS);
+    k_parse_output<<<n, 256, 0, m->stream>>>(data, m->slot_stride, d.shape[1], d.scale, m->d_tab, m->d_raw + (size_t)first * MARS_MAX_DETS,
+                                             m->d_raw_cnt + first, 1000, MARS_MAX_DETS);
     CU_OK(launch_nms_center(m->d_raw + (size_t)first * MARS_MAX_DETS, m->d_raw_cnt + first, m->d_det + (size_t)first * MARS_MAX_DETS,
-                            m->d_det_cnt + first, MARS_MAX_DETS, thresh, n, m->d_nms_mask + (size_t)first * NMS_SCRATCH_WORDS, m->stream, &nms_launches),
+                            m->d_det_cnt + first, MARS_MAX_DETS, thresh, n, m->d_nms_mask + (size_t)first * NMS_SCRATCH_WORDS, m->stream),
           MARS_ERR_LAYER_FAILED);
-    m->launches += 1 + nms_launches;
+    m->launches += 3; /* parse, NMS sort, NMS suppression */
     CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
 }
@@ -1178,53 +1161,13 @@ mars_error_t mars_b200_preprocess_batch(mars_model_t *model, int first, int n, c
     return MARS_OK;
 }
 
-/* Layer-group micro-batching (replaces the reference's one-image-at-a-time schedule, src/mars/mars_runtime.c:439-459): the
- * head of the op list -- the layers at the large resolutions, whose activations dominate the traffic -- runs over
- * MARS_MICRO_BATCH images at a time, all its layers back to back, so that a layer finds its producer's output in L2 instead
- * of HBM; the tail (small planes, where a micro-batch would not fill the 296 persistent CTAs) runs over the whole batch.
- * MARS_MICRO_OPS = number of head ops (default: everything in front of the first conv whose output plane is <= 80 x 80;
- * 0 = the whole list per micro-batch).  Images are independent, so any order across images is the same computation.
- * Off by default (MARS_MICRO_BATCH unset): profiles/r02h_micro_batch_sweep.txt has the measurement. */
-static int micro_batch() {
-    static int mb = -1;
-    if (mb < 0) {
-        const char *e = getenv("MARS_MICRO_BATCH");
-        mb = (e && *e) ? atoi(e) : 0;
-    }
-    return mb;
-}
-static size_t micro_split(Model *m) {
-    const char *e = getenv("MARS_MICRO_OPS");
-    if (e && *e) return (size_t)std::max(0, atoi(e));
-    for (size_t i = 0; i < m->prog.ops.size(); i++) {
-        const Op &o = m->prog.ops[i];
-        if ((o.kind == OP_CONV_I8_NCHW || o.kind == OP_CONV_I8_NHWC) && (long long)o.oh * o.ow <= 6400) return i;
-    }
-    return 0;
-}
-
-static mars_error_t enqueue_run(Model *m, int first, int n) {
-    const int mb = micro_batch();
-    if (mb <= 0 || mb >= n || m->profile) return enqueue_ops(m, first, n, -1);
-    mars_error_t e = compile_model(m);
-    if (e != MARS_OK) return e;
-    const size_t nops = m->prog.ops.size(), split = micro_split(m);
-    const size_t head = (split == 0 || split > nops) ? nops : split;
-    for (int i = 0; i < n; i += mb) {
-        e = enqueue_ops(m, first + i, std::min(mb, n - i), -1, 0, head);
-        if (e != MARS_OK) return e;
-    }
-    if (head < nops) e = enqueue_ops(m, first, n, -1, head, nops);
-    return e;
-}
-
 mars_error_t mars_b200_run_resident(mars_model_t *model, int first, int n) {
     Model *m = as_model(model);
     if (!m) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
     cudaEventRecord(m->ev0, m->stream);
-    mars_error_t e = enqueue_run(m, first, n);
+    mars_error_t e = enqueue_ops(m, first, n, -1);
     cudaEventRecord(m->ev1, m->stream);
     cudaError_t ce = cudaStreamSynchronize(m->stream);
     if (e == MARS_OK && ce != cudaSuccess) {
@@ -1262,7 +1205,7 @@ static bool graphs_enabled() {
 }
 
 static mars_error_t enqueue_step(Model *m, int first, int n, float nms_thresh, int with_detect) {
-    mars_error_t e = enqueue_run(m, first, n);
+    mars_error_t e = enqueue_ops(m, first, n, -1);
     if (e == MARS_OK && with_detect) e = enqueue_detect(m, first, n, nms_thresh);
     return e;
 }
@@ -1386,7 +1329,7 @@ static mars_error_t batch_pipeline(Model *m, int n, const void *inputs, size_t i
         if (e != MARS_OK) break;
         cudaEventRecord(m->ev_in[h], m->h2d_stream);
         cudaStreamWaitEvent(m->stream, m->ev_in[h], 0);
-        e = enqueue_run(m, first, cnt);
+        e = enqueue_ops(m, first, cnt, -1);
         if (e == MARS_OK && dets) e = enqueue_detect(m, first, cnt, thresh);
         if (e != MARS_OK) break;
         cudaEventRecord(m->ev_done[h], m->stream);

@@ -1,4 +1,4 @@
-"""tools/tst_probe.py -- one single-layer conv model through the CUDA path against the restatement (debug aid for the TMA-store epilogue).
+"""tools/tst_probe.py -- one single-layer conv model through the CUDA path against the restatement (debug aid for the conv epilogue).
 usage: python tools/tst_probe.py "dict(k=1, s=1, c=32, co=64, h=20, w=20)" """
 import sys
 
