@@ -36,6 +36,7 @@
 
 #include "conv_tc.h"
 #include "conv_tf32.h"
+#include "tc_common.cuh"
 
 namespace marsb200 {
 
@@ -47,11 +48,8 @@ namespace marsb200 {
 #else
 #define TC_DBG(p) 0
 #endif
-#define TC_MAX_TAPS 36
-#define TC_BM 128
 /* warp roles: warps 0..EPI-1 epilogue (EPI = 8, or 16 when one CTA owns the SM; quadrant = warp & 3), warp EPI = TMEM
  * allocator + MMA issuer (one elected lane), warp EPI+1 = TMA producer (lane 0) -- gather mode: warps EPI+1..EPI+4 */
-#define TC_MAX_CO 1024
 
 struct TcParams {
     int Co, Ho, Wo, Wp;      /* Wp = row pitch of the flat pixel index */
@@ -107,113 +105,6 @@ struct TcParams {
     int onhwc_vec;           /* OUT 2: 16-byte stores are legal (Co % 16 == 0, 16-byte aligned tensors) */
 };
 
-/* ---- PTX wrappers ------------------------------------------------------------- */
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t" /* suspend-time hint: the warp sleeps in the */
-        "@p bra WAIT_DONE;\n\t"                                          /* barrier unit instead of spinning through */
-        "bra WAIT_LOOP;\n\t"                                              /* issue slots the epilogue warps need     */
-        "WAIT_DONE:\n\t"
-        "}\n" ::"r"(bar), "r"(parity), "r"(0x989680u) : "memory");
-}
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0, int c1, int c2) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-                 ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0, int c1, int c2, int c3) {
-    asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-                 ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void sts_u8(uint32_t addr, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(addr), "r"(v) : "memory"); }
-/* D[tmem] (+)= A[smem] * B[smem]; the two 64-bit shared-memory matrix descriptors are given as 32-bit halves (the high
- * halves are loop invariants of the issuing thread) */
-__device__ __forceinline__ void umma_i8_parts(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc,
-                                              uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        ".reg .b64 da, db;\n\t"
-        "setp.ne.b32 p, %6, 0;\n\t"
-        "mov.b64 da, {%1, %2};\n\t"
-        "mov.b64 db, {%3, %4};\n\t"
-        "tcgen05.mma.cta_group::1.kind::i8 [%0], da, db, %5, {%7, %7, %7, %7}, p;\n\t"
-        "}\n" ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate), "r"(0u) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-/* split form: issue the load, and later wait for it; the wait takes the destination registers as in/out operands so
- * that no use of them can be scheduled before it */
-__device__ __forceinline__ void tmem_ld16_issue(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-          "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait(uint32_t (&v)[16]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]), "+r"(v[8]),
-                   "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15])
-                 :: "memory");
-}
-/* wait used by warps that are not on the critical path (epilogue, gather producers): back off between polls so the
- * spin does not take issue slots from the warps doing the work */
-__device__ __forceinline__ void mbar_wait_relaxed(uint32_t bar, uint32_t parity) {
-    for (;;) {
-        uint32_t done;
-        asm volatile(
-            "{\n\t"
-            ".reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t"
-            "}\n" : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (done) break;
-        __nanosleep(64);
-    }
-}
-
-/* one non-blocking probe */
-__device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity) {
-    uint32_t done;
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t"
-        "}\n" : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    return done != 0;
-}
-
-/* shared-memory loads through a 32-bit shared address kept in a register (the generic->shared conversion of a
- * __shared__ object is otherwise re-materialised at every use in the epilogue's hot loop) */
-__device__ __forceinline__ uint32_t lds_u32(uint32_t addr) {
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ int4 lds_v4(uint32_t addr) {
-    int4 v;
-    asm volatile("ld.shared.v4.s32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
-    return v;
-}
-
-/* UMMA shared-memory matrix descriptor (cute/arch/mma_sm100_desc.hpp layout), assembled in the MMA issuer from halves:
- * [0,14) start>>4, [16,30) LBO>>4, [32,46) SBO>>4, [46,48) version=1, [61,64) layout type (2 = SW128, 4 = SW64, 6 = SW32) */
-
 /* ---- requantisation ------------------------------------------------------------
  * reference src/mars/mxu_conv.c:663-666: r = (int32)(sc + (sc >= 0 ? 0.5f : -0.5f)), sc = (float)acc * cs, clamped to
  * int8, with the x86 cvttss2si rule (NaN and |v| >= 2^31 become INT_MIN, hence -128).  Both variants return the clamped
@@ -264,19 +155,6 @@ __device__ __forceinline__ void requant_pair(int32_t t0, int32_t t1, float cs, i
         if (!(h1 < 2147483648.0f)) r1 = -128;
     }
 }
-
-/* walks the tiles b, b + G, b + 2G, ... of a launch as (image, tile inside the image) without divisions in the loop */
-struct TileIter {
-    int img, rem, tpi, step_img, step_rem;
-    __device__ __forceinline__ TileIter(int first, int G, int tiles_per_img) : tpi(tiles_per_img) {
-        img = first / tpi; rem = first - img * tpi;
-        step_img = G / tpi; step_rem = G - step_img * tpi;
-    }
-    __device__ __forceinline__ void next() {
-        img += step_img; rem += step_rem;
-        if (rem >= tpi) { rem -= tpi; img++; }
-    }
-};
 
 /* ---- requantisation, integer form (RQ 3) ----------------------------------------
  * The reference's r(t) = clamp((int32)(fl(t * cs) + copysign(0.5f, .))) (src/mars/mxu_conv.c:663-666) is a monotone step function
@@ -485,12 +363,11 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
         for (int s = 0; s < p.stages; s++) { mbar_init(smem_u32(&bar_full[s]), GATHER ? 4 : 1); mbar_init(smem_u32(&bar_empty[s]), p.grp); }
         for (int b = 0; b < p.acc_bufs; b++) { mbar_init(smem_u32(&bar_tmem_full[b]), p.grp); mbar_init(smem_u32(&bar_tmem_empty[b]), EPI); }
         mbar_init(smem_u32(&bar_b), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_fence_init();
     }
     constexpr int WARP_MMA = EPI, WARP_PROD = EPI + 1; /* then: TMA producer (lane 0) or four gather producer warps */
     if (warp == WARP_MMA) { /* TMEM allocation is a warp-wide operation; this warp also frees it */
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"((uint32_t)p.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc(smem_u32(&tmem_base_slot), (uint32_t)p.tmem_cols);
     }
     if (RQ == 3) { /* int64 addends c64[ch] = bias[ch] * m + c in dynamic shared memory (p.cm_off), all N tiles */
         long long *cm64 = reinterpret_cast<long long *>(smem_al + p.cm_off);
@@ -521,9 +398,9 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
             g_pyx[i] = (py << 16) | (4 * wi);
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem_d = tmem_base_slot;
     if (TC_DBG(p) == 6) goto teardown; /* tuning aid: prologue + teardown only */
 
@@ -573,7 +450,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
             uint32_t cnt = 0;
             for (TileIter ti(blockIdx.x, gridDim.x, tiles_per_img); ti.img < p.n_img; ti.next()) {
                 mbar_wait_relaxed(sa_full + 8u * ab, aph);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tcgen05_fence_after();
                 const int mg = p.n_tiles == 1 ? ti.rem : ti.rem / p.n_tiles;
                 const int n0 = (ti.rem - mg * p.n_tiles) * p.n_tile;
                 const uint32_t acc_grp = acc_lane + (uint32_t)(ab * gcols);
@@ -650,7 +527,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
                         tmem_ld_wait(va);
                         if (u + 1 < u_hi) tmem_ld16_issue(acc_g + (uint32_t)((u + 1) * 16), vb);
                         else if (last_g) { /* last read of this accumulator group by this warp: hand it back */
-                            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                            tcgen05_fence_before();
                             __syncwarp();
                             if (lane == 0) mbar_arrive(sa_empty + 8u * ab);
                         }
@@ -665,7 +542,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
                         tmem_ld_wait(vb);
                         if (u + 1 < u_hi) tmem_ld16_issue(acc_g + (uint32_t)((u + 1) * 16), va);
                         else if (last_g) {
-                            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                            tcgen05_fence_before();
                             __syncwarp();
                             if (lane == 0) mbar_arrive(sa_empty + 8u * ab);
                         }
@@ -712,7 +589,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
             int s = 0, ph = 0, buf = 0, aph = 1; /* waits on the accumulator-empty barriers start with the opposite parity */
             for (TileIter ti(blockIdx.x, gridDim.x, tiles_per_img); ti.img < n_img; ti.next()) {
                 mbar_wait(sa_tempty + 8u * buf, aph); /* epilogue drained this accumulator */
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tcgen05_fence_after();
                 const uint32_t acc = tmem_d + (uint32_t)(buf * G * n_tile);
                 if (halo) {
                     /* a tap = the same rows shifted: the operand simply starts (shift) rows further down.  The swizzle is a
@@ -720,7 +597,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
                      * the 8-row atom needs NO descriptor base offset), so TMA's layout is read back as is */
                     for (int kb = 0; kb < ksteps; kb++) {
                         mbar_wait(sa_full + 8u * s, ph);
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                        tcgen05_fence_after();
                         const uint32_t a_st = a_lo0 + s * a_st16;
                         { /* M tile g of the group starts 128 rows further down the same stage */
                             const int g = lane;
@@ -728,7 +605,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
                             for (int tap = 0; tap < ntaps; tap++, b_lo += ksteps * b_st16) {
                                 const uint32_t a_lo = a_st + g * g_rows16 + (uint32_t)s_shift[tap]; /* halo mode: row shift in 16-byte units */
                                 for (int j = 0; j < nj; j++)
-                                    umma_i8_parts(acc + (uint32_t)(g * n_tile), a_lo + 2u * j, hi_a, b_lo + 2u * j, hi_k, idesc, (uint32_t)((kb | tap | j) != 0));
+                                    umma_i8(acc + (uint32_t)(g * n_tile), a_lo + 2u * j, hi_a, b_lo + 2u * j, hi_k, idesc, (uint32_t)((kb | tap | j) != 0));
                             }
                         }
                         umma_commit(sa_empty + 8u * s);
@@ -737,11 +614,11 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
                 } else {
                     for (int i = 0; i < nsteps; i++) {
                         mbar_wait(sa_full + 8u * s, ph);
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                        tcgen05_fence_after();
                         const uint32_t a_st = a_lo0 + s * a_st16 + lane * a_tile16, b_lo = b_lo0 + (b_res ? i : s) * b_st16;
                         if (TC_DBG(p) != 4 && TC_DBG(p) != 9)
                             for (int j = 0; j < nj; j++)
-                                umma_i8_parts(acc + (uint32_t)(lane * n_tile), a_st + a_j16 * j, hi_a, b_lo + 2u * j, hi_k, idesc, (uint32_t)((i | j) != 0));
+                                umma_i8(acc + (uint32_t)(lane * n_tile), a_st + a_j16 * j, hi_a, b_lo + 2u * j, hi_k, idesc, (uint32_t)((i | j) != 0));
                         umma_commit(sa_empty + 8u * s); /* frees the stage when these MMAs retire */
                         if (++s == stages) { s = 0; ph ^= 1; }
                     }
@@ -894,18 +771,16 @@ k_conv_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUte
         }
     }
 teardown:
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
     if (warp == WARP_MMA) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "r"((uint32_t)p.tmem_cols) : "memory");
+        tcgen05_fence_after();
+        tmem_dealloc(tmem_d, (uint32_t)p.tmem_cols);
     }
 }
 
 /* ---- pre-pass: arena NCHW -> channel-innermost copy with zero padding --------------- */
-/* dst[pix][c] for pix < npix; source pixel of `pix`:
- *   stride 1: ih = pix / Wp, iw = pix % Wp - pl                          (rows padded to Wp)
- *   stride 2: ph = pix / plane, a = (pix % plane) / Wp, b = .. % Wp, ih = 2a + ph/2 - pt, iw = 2b + ph%2 - pl
+/* dst[pix][c] for pix < npix (source pixel: copy_src_pixel).
  * 32 pixels x 32 channels per block through shared memory: coalesced reads along pixels,
  * coalesced writes along channels. */
 __global__ void __launch_bounds__(256) k_to_nhwc(const uint8_t *src_base, unsigned long long src_stride, uint8_t *dst_base,
@@ -919,14 +794,7 @@ __global__ void __launch_bounds__(256) k_to_nhwc(const uint8_t *src_base, unsign
     {
         const int pix = p0 + tx;
         int ih = -1, iw = -1;
-        if (pix < npix) {
-            if (stride2) {
-                int ph = pix / plane, r = pix - ph * plane, a = r / Wp, b = r - a * Wp;
-                ih = 2 * a + (ph >> 1) - pt; iw = 2 * b + (ph & 1) - pl;
-            } else {
-                ih = pix / Wp; iw = pix - ih * Wp - pl;
-            }
-        }
+        if (pix < npix) copy_src_pixel(pix, stride2, Wp, plane, pt, pl, ih, iw);
         const bool inb = ih >= 0 && ih < H && iw >= 0 && iw < W;
 #pragma unroll
         for (int k = 0; k < 4; k++) {
@@ -1022,7 +890,8 @@ struct TcPlanImpl {
     int prepass = 0;
     int rq = 0;     /* requantisation variant of the epilogue (requant_pair) */
     bool tab = false; /* the epilogue looks its byte up in the per-lane word table */
-    int C = 0, Cp = 0, H = 0, W = 0, pt = 0, pl = 0, plane = 0, npix = 0; /* Cp: bytes per pixel of the channel-innermost copy */
+    int C = 0, Cp = 0, H = 0, W = 0, npix = 0; /* Cp: bytes per pixel of the channel-innermost copy */
+    PixelCopy copy; /* prepass 1 / 2 */
     const uint8_t *src_slot0 = nullptr; /* input tensor in slot 0 */
     uint8_t *scratch = nullptr;
     size_t scratch_stride = 0, slot_stride = 0;
@@ -1040,10 +909,7 @@ struct TcPlanImpl {
     bool gather_direct = false; /* gather mode reads the input tensor in the arena itself (no private copy needed) */
 };
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_tiled() {
+EncodeTiledFn encode_tiled() {
     static EncodeTiledFn fn = nullptr;
     static bool tried = false;
     if (!tried) {
@@ -1057,8 +923,8 @@ static EncodeTiledFn encode_tiled() {
     return fn;
 }
 
-static bool make_map3(CUtensorMap *m, void *base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t s1, uint64_t s2, uint32_t b0,
-                      uint32_t b1, CUtensorMapSwizzle sw) {
+bool make_map3(CUtensorMap *m, void *base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t s1, uint64_t s2, uint32_t b0, uint32_t b1,
+               CUtensorMapSwizzle sw) {
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return false;
     cuuint64_t dims[3] = {d0, d1, d2};
@@ -1076,10 +942,8 @@ static bool make_map3(CUtensorMap *m, void *base, uint64_t d0, uint64_t d1, uint
     return true;
 }
 
-/* 4-d map over channel-innermost activations: dims (C, W, H, images), box {bc channels, bw, bh, 1} traversed with stride es in W
- * and H (the box covers bw / es x bh / es pixels); coordinates outside the tensor read as zeros */
-static bool make_map4(CUtensorMap *m, void *base, uint64_t C, uint64_t W, uint64_t H, uint64_t N, uint64_t img_stride, uint32_t bc,
-                      uint32_t bw, uint32_t bh, uint32_t es, CUtensorMapSwizzle sw) {
+bool make_map4(CUtensorMap *m, void *base, uint64_t C, uint64_t W, uint64_t H, uint64_t N, uint64_t img_stride, uint32_t bc, uint32_t bw,
+               uint32_t bh, uint32_t es, CUtensorMapSwizzle sw) {
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return false;
     cuuint64_t dims[4] = {C, W, H, N};
@@ -1096,7 +960,38 @@ static bool make_map4(CUtensorMap *m, void *base, uint64_t C, uint64_t W, uint64
     return true;
 }
 
-static int round_up(int x, int a) { return (x + a - 1) / a * a; }
+int tc_n_tile(int oc) {
+    const int co_pad = round_up(oc, 16);
+    return co_pad <= 256 ? co_pad : (co_pad % 256 == 0 ? 256 : 128);
+}
+int tc_n_tiles(int oc) { return (round_up(oc, 16) + tc_n_tile(oc) - 1) / tc_n_tile(oc); }
+int tc_bk(int kbytes) { return kbytes % 128 == 0 ? 128 : (kbytes % 64 == 0 ? 64 : 32); }
+uint32_t tc_umma_layout(int bk) { return bk == 128 ? 2u : (bk == 64 ? 4u : 6u); }
+CUtensorMapSwizzle tc_swizzle(int bk) { return bk == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (bk == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B); }
+int tc_sm_count() {
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return sms > 0 ? sms : 148;
+}
+
+PixelCopy pixel_copy(const Op &o) {
+    PixelCopy c;
+    if (o.sh < 1 || o.sh > 2 || o.pl >= o.kw || o.pt >= o.kh) return c;
+    c.pt = o.pt; c.pl = o.pl;
+    if (o.sh == 1) {
+        c.Wp = o.iw + o.kw - 1; c.plane = o.ih * c.Wp; c.npix = c.plane;
+    } else {
+        /* phase plane: rows a = 0 .. , pitch Wp >= ow + (k-1)/2; enough zero rows below that the
+         * deepest tap of the last output row stays inside its own plane */
+        c.Wp = o.ow + (o.kw - 1) / 2;
+        const int rows = std::max((o.ih - 1 + o.pt) / 2 + 1, o.oh + (o.kh - 1) / 2);
+        c.plane = rows * c.Wp; c.npix = 4 * c.plane;
+    }
+    if (o.ow > c.Wp) return PixelCopy();
+    c.mode = o.sh;
+    return c;
+}
 
 /* Row pitch of the space-to-depth stem's bordered pixel index.  The stem's NCHW streams leave through a shared-memory staging
  * block (TST: the stem writes the largest planes next to a side output and is the one layer class where staging pays, -7 %;
@@ -1116,12 +1011,24 @@ struct TcGeom {
     int prepass = 0; /* 4: space-to-depth copy with 16-byte pixels (stem); 0: A from the arena (1x1); 1: NHWC copy, rows padded (stride 1); 2: NHWC 2x2 phase split (stride 2);
                         3: gather -- A rows built in shared memory from a private NCHW copy of the input (small Ci);
                         5: NHWC 1x1 -- flat tiles, A rows = the arena tensor's pixels; 6: NHWC kxk -- rect tiles, one 4-d TMA box per tap */
-    int Wp = 0, plane = 0, npix = 0, ntaps = 0, Kp = 0;
+    int Wp = 0, npix = 0, ntaps = 0, Kp = 0;
+    PixelCopy copy; /* prepass 1 / 2 */
     int kpad = 0; /* prepass 0 with Ci not a multiple of 32: K extent padded with zeros (TMA fills the missing channel rows, the repacked weights hold zeros) */
     int tw_shift = 0, PH = 0, PWW = 0, dx = 0; /* gather: M tile shape and input patch geometry */
     int rtw = 0, rth = 0; /* rect mode (prepass 6): output pixels per tile row / tile rows, rtw * rth <= 128 */
     size_t scratch_bytes = 0;
 };
+/* the YOLOv5 stem shape: 6x6 stride 2 pad 0 / 2 over <= 4 channels == 3x3 stride 1 over the 2x2 space-to-depth image (prepass 4,
+ * the same copy for NCHW and channel-innermost inputs); fills *g when the op has that shape */
+static bool stem_geometry(const Op &o, TcGeom *g) {
+    if (!(o.sh == 2 && o.sw == 2 && o.kh == 6 && o.kw == 6 && (o.pt == 0 || o.pt == 2) && (o.pl == 0 || o.pl == 2) && o.ic <= 4 &&
+          o.ih % 2 == 0 && o.iw % 2 == 0 && o.oh <= o.ih / 2 && o.ow <= o.iw / 2 && round_up(o.oc, 16) <= 128 && (long long)o.oh * o.ow >= 4096))
+        return false;
+    g->prepass = 4; g->Wp = store_pitch(o.iw / 2 + 2, o.ow); g->npix = (o.ih / 2 + 2) * g->Wp; g->ntaps = 6; g->Kp = 32;
+    g->scratch_bytes = (size_t)g->npix * 16;
+    g->ok = true;
+    return true;
+}
 static TcGeom tc_geometry(const Op &o) {
     TcGeom g;
     if (o.kind == OP_CONV_I8_NHWC) { /* channel-innermost activations and OHWI weights (reference src/mars/mxu_conv.c:713-757) */
@@ -1131,14 +1038,7 @@ static TcGeom tc_geometry(const Op &o) {
         if (o.pt < 0 || o.pl < 0 || o.pt >= o.kh || o.pl >= o.kw) return g;
         g.ntaps = o.kh * o.kw;
         if (g.ntaps > TC_MAX_TAPS) return g;
-        if (o.sh == 2 && o.kh == 6 && (o.pt == 0 || o.pt == 2) && (o.pl == 0 || o.pl == 2) && o.ic <= 4 && o.ih % 2 == 0 &&
-            o.iw % 2 == 0 && o.oh <= o.ih / 2 && o.ow <= o.iw / 2 && round_up(o.oc, 16) <= 128 && (long long)o.oh * o.ow >= 4096) {
-            /* the stem: the same space-to-depth copy as the NCHW stem, gathered from interleaved pixels */
-            g.prepass = 4; g.Wp = store_pitch(o.iw / 2 + 2, o.ow); g.plane = (o.ih / 2 + 2) * g.Wp; g.npix = g.plane; g.ntaps = 6; g.Kp = 32;
-            g.scratch_bytes = (size_t)g.npix * 16;
-            g.ok = true;
-            return g;
-        }
+        if (stem_geometry(o, &g)) return g;
         if (o.ic < 32 || o.ic % 32) return g; /* K rows are the pixels' channel vectors: whole 32-byte k-steps only */
         if (o.kh == 1 && o.sh == 1 && o.pt == 0 && o.pl == 0 && o.oh <= o.ih && o.ow == o.iw) {
             g.prepass = 5; g.Wp = o.iw; /* 1x1: flat 128-pixel tiles, A rows straight from the arena tensor (or a private copy) */
@@ -1170,7 +1070,8 @@ static TcGeom tc_geometry(const Op &o) {
         g.kpad = o.ic > 64 ? round_up(o.ic, 128) : round_up(o.ic, 32);
         if (((long long)o.ih * o.iw) % 16 == 0) g.prepass = 0;
         else { /* planes that TMA cannot address (stride not a multiple of 16 bytes, e.g. 10 x 10): channel-innermost copy, kpad bytes per pixel */
-            g.prepass = 1; g.plane = o.ih * g.Wp; g.npix = g.plane;
+            g.copy = pixel_copy(o);
+            g.prepass = 1; g.npix = g.copy.npix;
             g.scratch_bytes = (size_t)g.npix * g.kpad;
         }
         g.ok = true;
@@ -1178,15 +1079,7 @@ static TcGeom tc_geometry(const Op &o) {
     }
     if (o.ic < 32 || o.ic % 32 || o.kh != o.kw) {
         auto small_k = [&]() -> bool {
-        /* the YOLOv5 stem shape: 6x6 stride 2 pad 2 over <= 4 channels == 3x3 stride 1 pad 1 over the 2x2 space-to-depth image */
-        if (o.sh == 2 && o.sw == 2 && o.kh == 6 && o.kw == 6 && (o.pt == 0 || o.pt == 2) && (o.pl == 0 || o.pl == 2) &&
-            o.ic <= 4 && o.ih % 2 == 0 && o.iw % 2 == 0 && o.oh <= o.ih / 2 && o.ow <= o.iw / 2 && round_up(o.oc, 16) <= 128 &&
-            (long long)o.oh * o.ow >= 4096) {
-            g.prepass = 4; g.Wp = store_pitch(o.iw / 2 + 2, o.ow); g.plane = (o.ih / 2 + 2) * g.Wp; g.npix = g.plane; g.ntaps = 6; g.Kp = 32;
-            g.scratch_bytes = (size_t)g.npix * 16;
-            g.ok = true;
-            return true;
-        }
+        if (stem_geometry(o, &g)) return true;
         /* small / odd channel counts: one 128-byte K row per pixel, built in shared memory from a staged input patch */
         const int Kt = o.ic * o.kh * o.kw;
         if (Kt > 128 || o.kh > 255 || o.kw > 255 || (long long)o.oh * o.ow < 4096 || round_up(o.oc, 16) > 256) return false;
@@ -1219,18 +1112,11 @@ static TcGeom tc_geometry(const Op &o) {
     if (g.ntaps > TC_MAX_TAPS) return g;
     if (!g.kpad && o.kh == 1 && o.sh == 1 && o.pt == 0 && o.pl == 0 && o.oh <= o.ih && o.ow == o.iw && ((long long)o.ih * o.iw) % 16 == 0) {
         g.prepass = 0; g.Wp = o.iw;
-    } else if (o.sh == 1) {
-        if (o.pl >= o.kw || o.pt >= o.kh) return g;
-        g.prepass = 1; g.Wp = o.iw + o.kw - 1; g.plane = o.ih * g.Wp; g.npix = g.plane;
-    } else if (o.sh == 2) {
-        if (o.pl >= o.kw || o.pt >= o.kh) return g;
-        /* phase plane: rows a = 0 .. , pitch Wp >= ow + (k-1)/2; enough zero rows below that the
-         * deepest tap of the last output row stays inside its own plane */
-        g.prepass = 2; g.Wp = o.ow + (o.kw - 1) / 2;
-        const int rows = std::max((o.ih - 1 + o.pt) / 2 + 1, o.oh + (o.kh - 1) / 2);
-        g.plane = rows * g.Wp; g.npix = 4 * g.plane;
-    } else return g;
-    if (o.ow > g.Wp) return g;
+    } else {
+        g.copy = pixel_copy(o);
+        if (!g.copy.mode) return g;
+        g.prepass = g.copy.mode; g.Wp = g.copy.Wp; g.npix = g.copy.npix;
+    }
     g.scratch_bytes = g.prepass ? (size_t)g.npix * (g.kpad ? g.kpad : o.ic) : 0;
     g.ok = true;
     return g;
@@ -1244,11 +1130,6 @@ bool tc_supported(const Op &o) {
     if (!tc_geometry(o).ok) return false;
     return true; /* any Co up to TC_MAX_CO: above 256 the N tiles are 256 or 128 wide and the last one may be ragged (weight rows
                   * beyond Co_pad do not exist in the tensor map and arrive as zeros; the epilogue skips their columns) */
-}
-int tc_n_tiles(int oc) {
-    const int co_pad = round_up(oc, 16);
-    const int nt = co_pad <= 256 ? co_pad : (co_pad % 256 == 0 ? 256 : 128);
-    return (co_pad + nt - 1) / nt;
 }
 bool tc_uses_copy(const Op &o) { return tc_geometry(o).prepass != 0; } /* (NHWC layers: a private copy on demand, see tc_plan) */
 bool tc_linkable(const Op &o) { const TcGeom g = tc_geometry(o); return g.ok && (g.prepass == 1 || g.prepass == 2) && !g.kpad; }
@@ -1470,9 +1351,9 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     const int ci_eff = (gather || s2d) ? g.Kp : (g.kpad ? g.kpad : o.ic); /* K extent of one tap */
     p.Co = o.oc; p.Ho = o.oh; p.Wo = o.ow; p.Wp = g.Wp; p.mflat = o.oh * g.Wp; p.plane = o.oh * o.ow;
     const int co_pad = round_up(o.oc, 16);
-    p.n_tile = co_pad <= 256 ? co_pad : (co_pad % 256 == 0 ? 256 : 128);
-    p.n_tiles = (co_pad + p.n_tile - 1) / p.n_tile;
-    p.bk = ci_eff % 128 == 0 ? 128 : (ci_eff % 64 == 0 ? 64 : 32);
+    p.n_tile = tc_n_tile(o.oc);
+    p.n_tiles = tc_n_tiles(o.oc);
+    p.bk = tc_bk(ci_eff);
     p.ksteps_per_tap = ci_eff / p.bk;
     p.ntaps = g.ntaps;
     p.a_tile_bytes = (uint32_t)(TC_BM * p.bk);
@@ -1611,7 +1492,7 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     t->smem = std::max<size_t>(t->smem, t->ctas_per_sm == 1 ? 120 * 1024 : 80 * 1024);
     /* cute/arch/mma_sm100_desc.hpp InstrDescriptor: c=S32, a=b=signed 8 bit, A MN-major, B K-major, N>>3, M>>4 */
     p.idesc = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.n_tile >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
-    p.b_layout = p.bk == 128 ? 2u : (p.bk == 64 ? 4u : 6u);
+    p.b_layout = tc_umma_layout(p.bk);
     p.a_kmajor = g.prepass != 0;
     if (!p.a_kmajor) p.idesc |= 1u << 15; /* A MN-major */
     if (s2d) for (int t6 = 0; t6 < 6; t6++) p.a_shift[t6] = ((t6 >> 1) + 1 - o.pt / 2) * g.Wp + 2 * (t6 & 1) + 1 - o.pl / 2;
@@ -1620,8 +1501,7 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
             const int tap = kh * o.kw + kw;
             if (g.prepass == 0 || g.prepass == 5 || gather) p.a_shift[tap] = 0;
             else if (rect) p.a_shift[tap] = (kh << 16) | kw;
-            else if (g.prepass == 1) p.a_shift[tap] = (kh - o.pt) * g.Wp + kw;
-            else p.a_shift[tap] = ((kh & 1) * 2 + (kw & 1)) * g.plane + (kh / 2) * g.Wp + kw / 2;
+            else p.a_shift[tap] = g.copy.tap_shift(kh, kw);
         }
     p.bias = o.bias >= 0 ? reinterpret_cast<const int32_t *>(ag.d_weights + o.bias) : nullptr;
     if (o.bias >= 0 && (o.bias % 4 || o.bias + 4 * (int64_t)o.oc > (int64_t)ag.W)) { delete t; return false; }
@@ -1656,18 +1536,17 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     if (consumer && linked) { /* this op's epilogue also writes the consumer's channel-innermost input copy */
         const TcGeom cg = tc_geometry(*consumer);
         const int sidx = o.fused_layers > 0 ? o.nhwc_stream : 0; /* stream index in {Z,S,Y} order; a plain conv only has Y = 0 */
-        if (!cg.ok || (cg.prepass != 1 && cg.prepass != 2) || sidx < 0 || sidx > 2 || consumer->ic != o.oc) { delete t; return false; }
+        if (!cg.ok || !cg.copy.mode || sidx < 0 || sidx > 2 || consumer->ic != o.oc) { delete t; return false; }
         t->nhwc_stream = sidx; /* its value goes into the top byte of every table word */
         p.nhwc_sel = 3;
-        p.nhwc_mode = cg.prepass; p.nhwc_Wp = cg.Wp; p.nhwc_plane = cg.plane; p.nhwc_pt = consumer->pt; p.nhwc_pl = consumer->pl;
+        p.nhwc_mode = cg.copy.mode; p.nhwc_Wp = cg.copy.Wp; p.nhwc_plane = cg.copy.plane; p.nhwc_pt = cg.copy.pt; p.nhwc_pl = cg.copy.pl;
         p.nhwc_C = consumer->ic;
         p.nhwc_base = linked + consumer->copy_off;
         p.nhwc_stride = linked_stride;
         /* the side output leaves in 32-byte pieces (two 16-channel units of a pixel per store) */
         if (consumer->ic % 32 || p.n_tile % 32 || consumer->copy_off % 32 || linked_stride % 32 || ((uintptr_t)linked % 32)) { delete t; return false; }
     }
-    t->prepass = g.prepass; t->C = o.ic; t->Cp = ci_eff; t->H = o.ih; t->W = o.iw; t->pt = o.pt; t->pl = o.pl;
-    t->plane = g.plane; t->npix = g.npix;
+    t->prepass = g.prepass; t->C = o.ic; t->Cp = ci_eff; t->H = o.ih; t->W = o.iw; t->npix = g.npix; t->copy = g.copy;
     t->src_slot0 = ag.d_slots + (o.in0 - (int64_t)ag.W);
     t->scratch = scratch; t->scratch_stride = scratch_stride; t->slot_stride = ag.slot_stride;
     if (gather) {
@@ -1713,7 +1592,7 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
         k_repack_weights<<<256, 256>>>(reinterpret_cast<const int8_t *>(ag.d_weights + o.w), t->d_wr, o.oc, co_pad, o.ic, ci_eff, g.ntaps, nhwc_in);
     bool ok = cudaDeviceSynchronize() == cudaSuccess;
 
-    const CUtensorMapSwizzle ksw = p.bk == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (p.bk == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+    const CUtensorMapSwizzle ksw = tc_swizzle(p.bk);
     if (ok && g.prepass == 0) /* the NCHW planes in the arena */
         ok = make_map3(&t->mapA, (void *)t->src_slot0, (uint64_t)o.ih * o.iw, (uint64_t)o.ic, (uint64_t)ag.capacity,
                        (uint64_t)o.ih * o.iw, ag.slot_stride, TC_BM, (uint32_t)p.bk, CU_TENSOR_MAP_SWIZZLE_128B);
@@ -1740,7 +1619,7 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     }
     ok = ok && make_map3(&t->mapB, t->d_wr, (uint64_t)ci_eff, (uint64_t)co_pad, (uint64_t)g.ntaps, (uint64_t)ci_eff,
                          (uint64_t)co_pad * ci_eff, (uint32_t)p.bk, (uint32_t)p.n_tile, ksw);
-    { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&t->sms, cudaDevAttrMultiProcessorCount, dev); }
+    t->sms = tc_sm_count();
     t->epi = epi_warps;
     t->kernel = pick_kernel(t->rq, gather, t->tab, t->nst, nhwc_in ? 2 : (p.nhwc_sel >= 0 ? 1 : 0), t->epi, t->tst);
     ok = ok && t->kernel != nullptr;
@@ -1750,13 +1629,12 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
         fprintf(stderr, "tc_plan layer %d: %dx%d k%d s%d ci %d co %d | n_tile %d grp %d acc %d stages %d bk %d halo %d b_res %d ctas %d epi %d | rq %d tab %d rep %u nst %d side %d tst %d smem %zu\n",
                 o.layer, o.oh, o.ow, o.kh, o.sh, o.ic, o.oc, p.n_tile, p.grp, p.acc_bufs, p.stages, p.bk, p.halo, p.b_resident, t->ctas_per_sm, t->epi,
                 t->rq, (int)t->tab, p.tab_rep, t->nst, p.nhwc_sel >= 0, (int)t->tst, t->smem);
-    plan->impl = t;
-    plan->valid = true;
+    plan->i8 = t;
     return true;
 }
 
 bool tc_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, bool use_linked, cudaStream_t s, uint64_t *launches) {
-    TcPlanImpl *t = static_cast<TcPlanImpl *>(plan.impl);
+    TcPlanImpl *t = plan.i8;
     if (!t) return false;
     const uint8_t *src = t->src_slot0 + (size_t)first * t->slot_stride;
     uint8_t *scr = t->scratch + (size_t)first * t->scratch_stride;
@@ -1773,7 +1651,7 @@ bool tc_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, bool u
     } else if (t->prepass && t->prepass != 3 && !(use_linked && t->has_linked)) {
         dim3 g((t->npix + 31) / 32, (t->Cp + 31) / 32, n);
         k_to_nhwc<<<g, 256, 0, s>>>(src, (unsigned long long)t->slot_stride, scr, (unsigned long long)t->scratch_stride, t->C, t->Cp, t->H, t->W,
-                                    t->p.Wp, t->plane, t->npix, (int)(t->prepass == 2), t->pt, t->pl);
+                                    t->copy.Wp, t->copy.plane, t->npix, (int)(t->copy.mode == 2), t->copy.pt, t->copy.pl);
         (*launches)++;
     }
     TcParams p = t->p;
@@ -1786,9 +1664,7 @@ bool tc_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, bool u
     }
     if (p.nhwc_sel >= 0) p.nhwc_base += (size_t)first * p.nhwc_stride;
     const long long total_tiles = (long long)p.m_groups * p.n_tiles * n;
-    int sms = t->sms;
-    if (sms <= 0) sms = 148;
-    const unsigned grid = (unsigned)std::min<long long>(total_tiles, (long long)sms * t->ctas_per_sm);
+    const unsigned grid = (unsigned)std::min<long long>(total_tiles, (long long)t->sms * t->ctas_per_sm);
     t->kernel<<<grid, (t->epi + (t->prepass == 3 ? 5 : 2)) * 32, t->smem, s>>>((use_linked && t->has_linked) ? t->mapA_linked : t->mapA, t->mapB, p);
     (*launches)++;
     return cudaGetLastError() == cudaSuccess;
@@ -1796,11 +1672,8 @@ bool tc_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, bool u
 
 void tc_release(std::vector<TcPlan> &plans) {
     for (auto &pl : plans) {
-        if (pl.f32) { tf32_release_one(pl); continue; }
-        TcPlanImpl *t = static_cast<TcPlanImpl *>(pl.impl);
-        if (t) { cudaFree(t->d_wr); cudaFree(t->d_lutw); delete t; }
-        pl.impl = nullptr;
-        pl.valid = false;
+        if (TcPlanImpl *t = pl.i8) { cudaFree(t->d_wr); cudaFree(t->d_lutw); delete t; }
+        tf32_release(pl.f32);
     }
     plans.clear();
 }

@@ -30,19 +30,20 @@
 #include <algorithm>
 
 #include "conv_tf32.h"
+#include "tc_common.cuh"
 
 namespace marsb200 {
 
 namespace {
 
-constexpr int F_BM = 128, F_MAX_TAPS = 36, F_EPI = 8, F_MAX_CO = 1024;
+constexpr int F_EPI = 8;
 
 struct F32Params {
     int Co, Ho, Wo, Wp, mflat, plane;
     int n_tile, n_tiles, m_tiles, ntaps, ksteps, stages, acc_bufs, tmem_cols, x3;
     uint32_t idesc, layout, bk; /* bk: bytes of K per pipeline step (128 / 64 / 32) */
     uint32_t a_tile_bytes, b_tile_bytes, stage_bytes;
-    int a_shift[F_MAX_TAPS];
+    int a_shift[TC_MAX_TAPS];
     int lo_rows;             /* row offset of the `lo` copy inside the A tensor map (tf32x3) */
     const float *bias;
     uint8_t *out_base;       /* slot 0 of the launch */
@@ -52,61 +53,13 @@ struct F32Params {
     int img0, n_img;
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count)); }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) { asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory"); }
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); }
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tWAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t@p bra WAIT_DONE;\n\tbra WAIT_LOOP;\n\tWAIT_DONE:\n\t}\n" ::"r"(bar), "r"(parity), "r"(0x989680u) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_relaxed(uint32_t bar, uint32_t parity) {
-    for (;;) {
-        uint32_t done;
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n" : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (done) break;
-        __nanosleep(64);
-    }
-}
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0, int c1, int c2) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-                 ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\tsetp.ne.b32 p, %6, 0;\n\tmov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], da, db, %5, {%7, %7, %7, %7}, p;\n\t}\n" ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate), "r"(0u) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) { asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory"); }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-        "tcgen05.wait::ld.sync.aligned;\n"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-          "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr) : "memory");
-}
-
-struct TileIter {
-    int img, rem, tpi, step_img, step_rem;
-    __device__ __forceinline__ TileIter(int first, int G, int tiles_per_img) : tpi(tiles_per_img) {
-        img = first / tpi; rem = first - img * tpi;
-        step_img = G / tpi; step_rem = G - step_img * tpi;
-    }
-    __device__ __forceinline__ void next() {
-        img += step_img; rem += step_rem;
-        if (rem >= tpi) { rem -= tpi; img++; }
-    }
-};
-
 __global__ void __launch_bounds__((F_EPI + 2) * 32, 1)
 k_conv_tf32(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const F32Params p) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bar_full[8], bar_empty[8], bar_tfull[4], bar_tempty[4];
     __shared__ uint32_t tmem_base_slot;
-    __shared__ float s_bias[F_MAX_CO];
-    __shared__ int s_shift[F_MAX_TAPS];
+    __shared__ float s_bias[TC_MAX_CO];
+    __shared__ int s_shift[TC_MAX_TAPS];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const int tiles_per_img = p.m_tiles * p.n_tiles;
@@ -114,17 +67,14 @@ k_conv_tf32(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
     if (threadIdx.x == 0) {
         for (int s = 0; s < p.stages; s++) { mbar_init(smem_u32(&bar_full[s]), 1); mbar_init(smem_u32(&bar_empty[s]), 1); }
         for (int b = 0; b < p.acc_bufs; b++) { mbar_init(smem_u32(&bar_tfull[b]), 1); mbar_init(smem_u32(&bar_tempty[b]), F_EPI); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_fence_init();
     }
-    if (warp == F_EPI) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"((uint32_t)p.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    for (int i = threadIdx.x; i < F_MAX_CO; i += blockDim.x) s_bias[i] = (p.bias && i < p.Co) ? p.bias[i] : 0.0f;
-    if (threadIdx.x < F_MAX_TAPS) s_shift[threadIdx.x] = p.a_shift[threadIdx.x];
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    if (warp == F_EPI) tmem_alloc(smem_u32(&tmem_base_slot), (uint32_t)p.tmem_cols);
+    for (int i = threadIdx.x; i < TC_MAX_CO; i += blockDim.x) s_bias[i] = (p.bias && i < p.Co) ? p.bias[i] : 0.0f;
+    if (threadIdx.x < TC_MAX_TAPS) s_shift[threadIdx.x] = p.a_shift[threadIdx.x];
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem_d = tmem_base_slot;
 
     if (warp < F_EPI) {
@@ -137,17 +87,18 @@ k_conv_tf32(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
         int ab = 0, aph = 0;
         for (TileIter ti(blockIdx.x, gridDim.x, tiles_per_img); ti.img < p.n_img; ti.next()) {
             mbar_wait_relaxed(smem_u32(&bar_tfull[ab]), aph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tcgen05_fence_after();
             const int mt = p.n_tiles == 1 ? ti.rem : ti.rem / p.n_tiles, n0 = (ti.rem - mt * p.n_tiles) * p.n_tile;
-            const int q = mt * F_BM + r;
+            const int q = mt * TC_BM + r;
             const int oh = (int)__umulhi((unsigned)q, p.wp_magic), ow = q - oh * p.Wp;
             const bool valid = q < p.mflat && ow < p.Wo;
             float *o = reinterpret_cast<float *>(p.out_base + (unsigned long long)ti.img * p.slot_stride + p.out_off) + ((long long)n0 * plane + (long long)oh * p.Wo + ow);
             for (int u = part; u < n_units; u += parts) {
                 uint32_t v[16];
-                tmem_ld16(acc_lane + (uint32_t)(ab * p.n_tile + u * 16), v);
+                tmem_ld16_issue(acc_lane + (uint32_t)(ab * p.n_tile + u * 16), v);
+                tmem_ld_wait(v);
                 if (u + parts >= n_units) { /* last read of this accumulator by this warp */
-                    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                    tcgen05_fence_before();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(smem_u32(&bar_tempty[ab]));
                 }
@@ -173,11 +124,11 @@ k_conv_tf32(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
             int s = 0, ph = 0, buf = 0, aph = 1;
             for (TileIter ti(blockIdx.x, gridDim.x, tiles_per_img); ti.img < p.n_img; ti.next()) {
                 mbar_wait(smem_u32(&bar_tempty[buf]), aph);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tcgen05_fence_after();
                 const uint32_t acc = tmem_d + (uint32_t)(buf * p.n_tile);
                 for (int i = 0; i < nsteps; i++) {
                     mbar_wait(smem_u32(&bar_full[s]), ph);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    tcgen05_fence_after();
                     /* stage: [A hi | A lo | B hi | B lo] (x3) or [A | B] */
                     const uint32_t a_hi_d = a_lo0 + s * st16, a_lo_d = a_hi_d + at16;
                     const uint32_t b_hi_d = a_hi_d + (p.x3 ? 2u : 1u) * at16, b_lo_d = b_hi_d + bt16;
@@ -200,7 +151,7 @@ k_conv_tf32(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
         int s = 0, ph = 1;
         for (TileIter ti(blockIdx.x, gridDim.x, tiles_per_img); ti.img < p.n_img; ti.next()) {
             const int mt = p.n_tiles == 1 ? ti.rem : ti.rem / p.n_tiles, n0 = (ti.rem - mt * p.n_tiles) * p.n_tile;
-            const int q0 = mt * F_BM, zc = p.img0 + ti.img;
+            const int q0 = mt * TC_BM, zc = p.img0 + ti.img;
             for (int tap = 0; tap < p.ntaps; tap++) {
                 const int qa = q0 + s_shift[tap];
                 for (int kb = 0; kb < p.ksteps; kb++) {
@@ -218,11 +169,11 @@ k_conv_tf32(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
     if (warp == F_EPI) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "r"((uint32_t)p.tmem_cols) : "memory");
+        tcgen05_fence_after();
+        tmem_dealloc(tmem_d, (uint32_t)p.tmem_cols);
     }
 }
 
@@ -232,7 +183,7 @@ __device__ __forceinline__ float tf32_round(float x) { /* round to nearest, ties
     return __uint_as_float(r);
 }
 
-/* pre-pass: arena NCHW fp32 -> channel-innermost fp32 copy (pixel indexing as k_to_nhwc in conv_tc.cu): dst[pix][c] for
+/* pre-pass: arena NCHW fp32 -> channel-innermost fp32 copy (source pixel: copy_src_pixel): dst[pix][c] for
  * pix < npix, c < Cp (channels >= C are zero); split != 0: a second copy behind the first (and `guard` zero rows) holds lo = x - hi;
  * split == 0: the values are rounded to tf32.  32 pixels x 32 channels per block through shared memory. */
 __global__ void __launch_bounds__(256) k_f32_to_kmajor(const uint8_t *src_base, unsigned long long src_stride, uint8_t *dst_base, unsigned long long dst_stride,
@@ -245,14 +196,7 @@ __global__ void __launch_bounds__(256) k_f32_to_kmajor(const uint8_t *src_base, 
     {
         const int pix = p0 + tx;
         int ih = -1, iw = -1;
-        if (pix < npix) {
-            if (stride2) {
-                int ph = pix / plane, r = pix - ph * plane, a = r / Wp, b = r - a * Wp;
-                ih = 2 * a + (ph >> 1) - pt; iw = 2 * b + (ph & 1) - pl;
-            } else {
-                ih = pix / Wp; iw = pix - ih * Wp - pl;
-            }
-        }
+        if (pix < npix) copy_src_pixel(pix, stride2, Wp, plane, pt, pl, ih, iw);
         const bool inb = ih >= 0 && ih < H && iw >= 0 && iw < W;
 #pragma unroll
         for (int k = 0; k < 4; k++) {
@@ -292,92 +236,52 @@ __global__ void k_repack_f32(const float *w, float *dst, int Co, int Co_pad, int
     }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_tiled_f() {
-    static EncodeTiledFn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void *sym = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)sym;
-    }
-    return fn;
-}
-/* byte-typed 3-d map: dims (row bytes, rows, images / taps) */
-bool make_map3b(CUtensorMap *m, void *base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t s1, uint64_t s2, uint32_t b0, uint32_t b1, CUtensorMapSwizzle sw) {
-    EncodeTiledFn enc = encode_tiled_f();
-    if (!enc) return false;
-    cuuint64_t dims[3] = {d0, d1, d2};
-    cuuint64_t strides[2] = {s1, s2};
-    cuuint32_t box[3] = {b0, b1, 1};
-    cuuint32_t es[3] = {1, 1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_last_error("cuTensorMapEncodeTiled (tf32) failed: %d (dims %llu %llu %llu strides %llu %llu box %u %u)", (int)r, (unsigned long long)d0,
-                       (unsigned long long)d1, (unsigned long long)d2, (unsigned long long)s1, (unsigned long long)s2, b0, b1);
-        return false;
-    }
-    return true;
-}
-int round_up_i(int x, int a) { return (x + a - 1) / a * a; }
-
 struct F32Geom {
     bool ok = false;
-    int prepass = 0; /* 1: rows padded with k-1 zero columns (stride 1); 2: 2x2 phase split (stride 2) */
-    int Wp = 0, plane = 0, npix = 0, ntaps = 0, Cp = 0, guard = 0;
+    PixelCopy copy;
+    int ntaps = 0, Cp = 0, guard = 0;
     size_t scratch_bytes = 0;
 };
 F32Geom f32_geometry(const Op &o, int mode) {
     F32Geom g;
     if (mode <= 0 || o.kind != OP_CONV_F32_NCHW || o.mode != EXEC_PARALLEL || o.xlat) return g;
     if (o.oc < 1 || o.sh != o.sw || o.sh < 1 || o.sh > 2 || o.kh < 1 || o.kh != o.kw) return g;
-    if (o.oh <= 0 || o.ow <= 0 || o.ih <= 0 || o.iw <= 0 || o.ic <= 0 || round_up_i(o.oc, 16) > F_MAX_CO) return g;
+    if (o.oh <= 0 || o.ow <= 0 || o.ih <= 0 || o.iw <= 0 || o.ic <= 0 || round_up(o.oc, 16) > TC_MAX_CO) return g;
     if (o.pt < 0 || o.pl < 0 || o.pl >= o.kw || o.pt >= o.kh) return g;
     if ((long long)o.oh * o.ow * o.oc * o.ic * o.kh * o.kw < (1ll << 22)) return g; /* tiny layers stay on the exact kernel */
     g.ntaps = o.kh * o.kw;
-    if (g.ntaps > F_MAX_TAPS) return g;
-    g.Cp = round_up_i(o.ic, 8);
-    if (o.sh == 1) {
-        g.prepass = 1; g.Wp = o.iw + o.kw - 1; g.plane = o.ih * g.Wp; g.npix = g.plane;
-    } else {
-        g.prepass = 2; g.Wp = o.ow + (o.kw - 1) / 2;
-        const int rows = std::max((o.ih - 1 + o.pt) / 2 + 1, o.oh + (o.kh - 1) / 2);
-        g.plane = rows * g.Wp; g.npix = 4 * g.plane;
-    }
-    if (o.ow > g.Wp) return g;
-    if ((unsigned long long)(o.oh * (long long)g.Wp + 2 * g.Wp) * (unsigned)g.Wp >= (1ull << 32)) return g;
+    if (g.ntaps > TC_MAX_TAPS) return g;
+    g.Cp = round_up(o.ic, 8);
+    g.copy = pixel_copy(o);
+    const PixelCopy &c = g.copy;
+    if (!c.mode) return g;
+    if ((unsigned long long)(o.oh * (long long)c.Wp + 2 * c.Wp) * (unsigned)c.Wp >= (1ull << 32)) return g;
     /* zero rows between the hi and the lo copy: the deepest tap of the last M tile */
-    const int max_shift = g.prepass == 1 ? (o.kh - 1) * g.Wp + o.kw - 1 : 3 * g.plane + ((o.kh - 1) / 2) * g.Wp + (o.kw - 1) / 2;
-    g.guard = mode >= 2 ? F_BM + (g.prepass == 1 ? max_shift : ((o.kh - 1) / 2) * g.Wp + (o.kw - 1) / 2) + 8 : 0;
-    (void)max_shift;
-    g.scratch_bytes = (size_t)(mode >= 2 ? 2 * g.npix + g.guard : g.npix) * g.Cp * 4;
+    g.guard = mode >= 2 ? TC_BM + (c.mode == 1 ? (o.kh - 1) * c.Wp + o.kw - 1 : ((o.kh - 1) / 2) * c.Wp + (o.kw - 1) / 2) + 8 : 0;
+    g.scratch_bytes = (size_t)(mode >= 2 ? 2 * c.npix + g.guard : c.npix) * g.Cp * 4;
     g.ok = true;
     return g;
 }
 
+} // namespace
+
 struct F32PlanImpl {
     CUtensorMap mapA, mapB;
     F32Params p;
-    int prepass = 0, C = 0, Cp = 0, H = 0, W = 0, pt = 0, pl = 0, plane = 0, npix = 0, split = 0, guard = 0, sms = 148;
+    PixelCopy copy;
+    int C = 0, Cp = 0, H = 0, W = 0, split = 0, guard = 0, sms = 148;
     const uint8_t *src_slot0 = nullptr;
     uint8_t *scratch = nullptr;
     size_t scratch_stride = 0, slot_stride = 0, smem = 0;
     float *d_wr = nullptr;
 };
 
-} // namespace
-
 bool tf32_supported(const Op &o, int mode) { return f32_geometry(o, mode).ok; }
 size_t tf32_scratch_need(const Op &o, int mode) { const F32Geom g = f32_geometry(o, mode); return g.ok ? g.scratch_bytes : 0; }
 
 bool tf32_plan(const Op &o, const ArenaGeom &ag, int mode, uint8_t *scratch, size_t scratch_stride, TcPlan *plan) {
     const F32Geom g = f32_geometry(o, mode);
-    if (!g.ok || !encode_tiled_f()) return false;
+    if (!g.ok || !encode_tiled()) return false;
     if (o.in0 < (int64_t)ag.W || o.out < (int64_t)ag.W || o.w >= (int64_t)ag.W || o.w % 4 || g.scratch_bytes > scratch_stride) return false;
     if (o.bias >= 0 && (o.bias % 4 || o.bias + 4 * (int64_t)o.oc > (int64_t)ag.W)) return false;
     F32PlanImpl *t = new F32PlanImpl();
@@ -385,17 +289,18 @@ bool tf32_plan(const Op &o, const ArenaGeom &ag, int mode, uint8_t *scratch, siz
     memset(&p, 0, sizeof p);
     const int x3 = mode >= 2 ? 1 : 0;
     p.x3 = x3;
-    p.Co = o.oc; p.Ho = o.oh; p.Wo = o.ow; p.Wp = g.Wp; p.mflat = o.oh * g.Wp; p.plane = o.oh * o.ow;
-    const int co_pad = round_up_i(o.oc, 16);
-    p.n_tile = co_pad <= 256 ? co_pad : (co_pad % 256 == 0 ? 256 : 128);
-    p.n_tiles = (co_pad + p.n_tile - 1) / p.n_tile;
+    const PixelCopy &c = g.copy;
+    p.Co = o.oc; p.Ho = o.oh; p.Wo = o.ow; p.Wp = c.Wp; p.mflat = o.oh * c.Wp; p.plane = o.oh * o.ow;
+    const int co_pad = round_up(o.oc, 16);
+    p.n_tile = tc_n_tile(o.oc);
+    p.n_tiles = tc_n_tiles(o.oc);
     const int kbytes = g.Cp * 4; /* K extent of one tap in bytes */
-    p.bk = kbytes % 128 == 0 ? 128 : (kbytes % 64 == 0 ? 64 : 32);
+    p.bk = tc_bk(kbytes);
     p.ksteps = kbytes / (int)p.bk;
     p.ntaps = g.ntaps;
-    p.layout = p.bk == 128 ? 2u : (p.bk == 64 ? 4u : 6u);
-    p.a_tile_bytes = (uint32_t)(F_BM * p.bk);
-    p.b_tile_bytes = (uint32_t)round_up_i(p.n_tile * (int)p.bk, 1024);
+    p.layout = tc_umma_layout(p.bk);
+    p.a_tile_bytes = (uint32_t)(TC_BM * p.bk);
+    p.b_tile_bytes = (uint32_t)round_up(p.n_tile * (int)p.bk, 1024);
     p.stage_bytes = (x3 ? 2u : 1u) * (p.a_tile_bytes + p.b_tile_bytes);
     p.stages = std::max(2, std::min(8, (200 * 1024) / (int)p.stage_bytes));
     t->smem = 1024 + (size_t)p.stages * p.stage_bytes;
@@ -403,52 +308,46 @@ bool tf32_plan(const Op &o, const ArenaGeom &ag, int mode, uint8_t *scratch, siz
     if (p.acc_bufs < 2) p.acc_bufs = 2; /* n_tile <= 256: two buffers always fit the 512 columns */
     p.tmem_cols = 512;
     /* cute/arch/mma_sm100_desc.hpp InstrDescriptor: c = F32 (1), a = b = TF32 (2), both K-major, N >> 3, M >> 4 */
-    p.idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(p.n_tile >> 3) << 17) | ((uint32_t)(F_BM >> 4) << 24);
+    p.idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(p.n_tile >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
     for (int kh = 0; kh < o.kh; kh++)
-        for (int kw = 0; kw < o.kw; kw++) {
-            const int tap = kh * o.kw + kw;
-            p.a_shift[tap] = g.prepass == 1 ? (kh - o.pt) * g.Wp + kw : ((kh & 1) * 2 + (kw & 1)) * g.plane + (kh / 2) * g.Wp + kw / 2;
-        }
-    p.lo_rows = g.npix + g.guard;
+        for (int kw = 0; kw < o.kw; kw++) p.a_shift[kh * o.kw + kw] = c.tap_shift(kh, kw);
+    p.lo_rows = c.npix + g.guard;
     p.bias = o.bias >= 0 ? reinterpret_cast<const float *>(ag.d_weights + o.bias) : nullptr;
     p.slot_stride = ag.slot_stride;
     p.out_off = o.out - (int64_t)ag.W;
-    p.m_tiles = (p.mflat + F_BM - 1) / F_BM;
-    p.wp_magic = (unsigned)((1ull << 32) / (unsigned)g.Wp) + 1u;
+    p.m_tiles = (p.mflat + TC_BM - 1) / TC_BM;
+    p.wp_magic = (unsigned)((1ull << 32) / (unsigned)c.Wp) + 1u;
     if ((long long)p.m_tiles * p.n_tiles * ag.capacity >= (1ll << 31)) { delete t; return false; }
-    t->prepass = g.prepass; t->C = o.ic; t->Cp = g.Cp; t->H = o.ih; t->W = o.iw; t->pt = o.pt; t->pl = o.pl; t->plane = g.plane; t->npix = g.npix;
-    t->split = x3; t->guard = g.guard;
+    t->copy = c; t->C = o.ic; t->Cp = g.Cp; t->H = o.ih; t->W = o.iw; t->split = x3; t->guard = g.guard;
     t->src_slot0 = ag.d_slots + (o.in0 - (int64_t)ag.W);
     t->scratch = scratch; t->scratch_stride = scratch_stride; t->slot_stride = ag.slot_stride;
     const size_t wr_floats = (size_t)g.ntaps * (x3 ? 2 : 1) * co_pad * g.Cp;
     if (cudaMalloc(&t->d_wr, wr_floats * 4) != cudaSuccess) { delete t; return false; }
     k_repack_f32<<<256, 256>>>(reinterpret_cast<const float *>(ag.d_weights + o.w), t->d_wr, o.oc, co_pad, o.ic, g.Cp, g.ntaps, x3);
     bool ok = cudaDeviceSynchronize() == cudaSuccess;
-    const CUtensorMapSwizzle ksw = p.bk == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (p.bk == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-    ok = ok && make_map3b(&t->mapA, scratch, (uint64_t)kbytes, (uint64_t)(x3 ? 2 * g.npix + g.guard : g.npix), (uint64_t)ag.capacity, (uint64_t)kbytes, scratch_stride,
-                          p.bk, F_BM, ksw);
-    ok = ok && make_map3b(&t->mapB, t->d_wr, (uint64_t)kbytes, (uint64_t)co_pad, (uint64_t)g.ntaps * (x3 ? 2 : 1), (uint64_t)kbytes,
-                          (uint64_t)co_pad * kbytes, p.bk, (uint32_t)p.n_tile, ksw);
-    { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&t->sms, cudaDevAttrMultiProcessorCount, dev); if (t->sms <= 0) t->sms = 148; }
+    const CUtensorMapSwizzle ksw = tc_swizzle(p.bk);
+    ok = ok && make_map3(&t->mapA, scratch, (uint64_t)kbytes, (uint64_t)(x3 ? 2 * c.npix + g.guard : c.npix), (uint64_t)ag.capacity, (uint64_t)kbytes, scratch_stride,
+                         p.bk, TC_BM, ksw);
+    ok = ok && make_map3(&t->mapB, t->d_wr, (uint64_t)kbytes, (uint64_t)co_pad, (uint64_t)g.ntaps * (x3 ? 2 : 1), (uint64_t)kbytes,
+                         (uint64_t)co_pad * kbytes, p.bk, (uint32_t)p.n_tile, ksw);
+    t->sms = tc_sm_count();
     ok = ok && cudaFuncSetAttribute((const void *)k_conv_tf32, cudaFuncAttributeMaxDynamicSharedMemorySize, 210 * 1024) == cudaSuccess;
     if (!ok) { cudaFree(t->d_wr); delete t; return false; }
     if (getenv("MARS_TC_VERBOSE"))
         fprintf(stderr, "tf32_plan layer %d: %dx%d k%d s%d ci %d co %d | n_tile %d stages %d bk %u x3 %d smem %zu\n", o.layer, o.oh, o.ow, o.kh, o.sh, o.ic,
                 o.oc, p.n_tile, p.stages, p.bk, x3, t->smem);
-    plan->impl = t;
-    plan->valid = true;
-    plan->f32 = true;
+    plan->f32 = t;
     return true;
 }
 
 bool tf32_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, cudaStream_t s, uint64_t *launches) {
-    F32PlanImpl *t = static_cast<F32PlanImpl *>(plan.impl);
+    F32PlanImpl *t = plan.f32;
     if (!t) return false;
     const uint8_t *src = t->src_slot0 + (size_t)first * t->slot_stride;
     uint8_t *scr = t->scratch + (size_t)first * t->scratch_stride;
-    dim3 g((t->npix + t->guard + 31) / 32, (t->Cp + 31) / 32, n);
-    k_f32_to_kmajor<<<g, 256, 0, s>>>(src, t->slot_stride, scr, t->scratch_stride, t->C, t->Cp, t->H, t->W, t->p.Wp, t->plane, t->npix, t->prepass == 2,
-                                      t->pt, t->pl, t->split, t->guard);
+    dim3 g((t->copy.npix + t->guard + 31) / 32, (t->Cp + 31) / 32, n);
+    k_f32_to_kmajor<<<g, 256, 0, s>>>(src, t->slot_stride, scr, t->scratch_stride, t->C, t->Cp, t->H, t->W, t->copy.Wp, t->copy.plane, t->copy.npix,
+                                      t->copy.mode == 2, t->copy.pt, t->copy.pl, t->split, t->guard);
     (*launches)++;
     F32Params p = t->p;
     p.out_base = slots_base + (size_t)first * t->slot_stride;
@@ -461,12 +360,8 @@ bool tf32_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, cuda
     return cudaGetLastError() == cudaSuccess;
 }
 
-void tf32_release_one(TcPlan &pl) {
-    F32PlanImpl *t = static_cast<F32PlanImpl *>(pl.impl);
+void tf32_release(F32PlanImpl *t) {
     if (t) { cudaFree(t->d_wr); delete t; }
-    pl.impl = nullptr;
-    pl.valid = false;
-    pl.f32 = false;
 }
 
 } // namespace marsb200

@@ -12,6 +12,7 @@ bool tf32_supported(const Op &o, int mode);
 size_t tf32_scratch_need(const Op &o, int mode);
 bool tf32_plan(const Op &o, const ArenaGeom &g, int mode, uint8_t *scratch, size_t scratch_stride, TcPlan *plan);
 bool tf32_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, cudaStream_t s, uint64_t *launches);
-void tf32_release_one(TcPlan &plan);
+/* frees a plan tf32_plan built (null: nothing) */
+void tf32_release(F32PlanImpl *t);
 
 } // namespace marsb200

@@ -441,9 +441,9 @@ static mars_error_t launch_op(Model *m, size_t op_index, int first, int n, bool 
     } else if (is_conv) {
         const uint64_t P = (uint64_t)o.oh * o.ow;
         const int es = o.kind == OP_CONV_F32_NCHW ? 4 : 1;
-        if (o.impl == CONV_TC_F32 && m->tc[op_index].valid) {
+        if (o.impl == CONV_TC_F32 && m->tc[op_index].f32) {
             if (!tf32_launch(m->tc[op_index], m->d_slots, first, n, s, &m->launches)) return MARS_ERR_LAYER_FAILED;
-        } else if (o.impl == CONV_TC_NCHW && m->tc[op_index].valid) {
+        } else if (o.impl == CONV_TC_NCHW && m->tc[op_index].i8) {
             if (!tc_launch(m->tc[op_index], m->d_slots, first, n, full_pass, s, &m->launches)) return MARS_ERR_LAYER_FAILED;
         } else if (o.mode == EXEC_PARALLEL) {
             if (o.kind == OP_CONV_I8_NCHW && !xl && fast_conv_nchw_ok(k)) {

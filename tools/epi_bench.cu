@@ -18,9 +18,11 @@
 #include <stdio.h>
 #include <stdlib.h>
 
-#define CK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { printf("CUDA error %s at %s:%d\n", cudaGetErrorString(e_), __FILE__, __LINE__); exit(1); } } while (0)
+#include "../thingino-accel_b200/csrc/tc_common.cuh"
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+using namespace marsb200;
+
+#define CK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { printf("CUDA error %s at %s:%d\n", cudaGetErrorString(e_), __FILE__, __LINE__); exit(1); } } while (0)
 
 __device__ __forceinline__ uint32_t old_index(int32_t t, float cs) {
     const float f = __fsub_rn(__int_as_float(t), 12582912.0f);

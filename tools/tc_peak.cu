@@ -12,21 +12,11 @@
 #include <stdio.h>
 #include <stdlib.h>
 
-#define CK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { printf("CUDA error %s at %s:%d\n", cudaGetErrorString(e_), __FILE__, __LINE__); exit(1); } } while (0)
+#include "../thingino-accel_b200/csrc/tc_common.cuh"
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count)); }
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tWAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t@p bra WAIT_DONE;\n\tbra WAIT_LOOP;\n\tWAIT_DONE:\n\t}\n" ::"r"(bar), "r"(parity), "r"(0x989680u) : "memory");
-}
-__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t acc) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\tsetp.ne.b32 p, %6, 0;\n\tmov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\t"
-        "tcgen05.mma.cta_group::1.kind::i8 [%0], da, db, %5, {%7, %7, %7, %7}, p;\n\t}\n" ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(acc), "r"(0u) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) { asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory"); }
+using namespace marsb200;
+
+#define CK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { printf("CUDA error %s at %s:%d\n", cudaGetErrorString(e_), __FILE__, __LINE__); exit(1); } } while (0)
 
 /* smem: A = 128 rows x 128 B (4 K=32 slices), B = N rows x 128 B, both in the canonical SW128 K-major layout (content is random:
  * the layout does not matter for timing, the power draw of random operands does) */
@@ -37,15 +27,12 @@ __global__ void __launch_bounds__(128) k_peak(int N, int lanes, int chain, int r
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     uint8_t *al = smem_raw + (base - smem_u32(smem_raw));
     for (int i = threadIdx.x; i < (128 + 256) * 128 / 16; i += blockDim.x) reinterpret_cast<uint4 *>(al)[i] = reinterpret_cast<const uint4 *>(rnd)[i];
-    if (threadIdx.x == 0) { for (int i = 0; i < 16; i++) mbar_init(smem_u32(&bar[i]), 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-    if (threadIdx.x < 32) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"((uint32_t)tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (threadIdx.x == 0) { for (int i = 0; i < 16; i++) mbar_init(smem_u32(&bar[i]), 1); mbar_fence_init(); }
+    if (threadIdx.x < 32) tmem_alloc(smem_u32(&tmem_slot), (uint32_t)tmem_cols);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem_d = tmem_slot;
     unsigned long long t0 = 0, t1 = 0;
     if (threadIdx.x < 32) {
@@ -69,11 +56,11 @@ __global__ void __launch_bounds__(128) k_peak(int N, int lanes, int chain, int r
         __syncwarp();
     }
     if (threadIdx.x == 0) cycles[blockIdx.x] = t1 - t0;
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
     if (threadIdx.x < 32) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "r"((uint32_t)tmem_cols) : "memory");
+        tcgen05_fence_after();
+        tmem_dealloc(tmem_d, (uint32_t)tmem_cols);
     }
 }
 
