@@ -111,6 +111,34 @@ mars_error_t mars_b200_enqueue_step_resident(mars_model_t *m, int first, int n, 
  * dets = mars_det_t[capacity][*stride_dets], counts = int32[capacity] */
 void mars_b200_detections_device(mars_model_t *m, void **dets, void **counts, int *stride_dets);
 
+/* ---- YOLOv5 Detect heads on the batched path ------------------------------------------------------------------------------ */
+/* A compiler-emitted YOLOv5 .mars file keeps only the three raw head convolutions of its Detect block; output0 then holds stale
+ * bytes (the Split / Pow / Constant nodes are dropped).  These calls decode the heads inside the program instead: right after each
+ * head conv the anchor grid of examples/yolo_detect.cpp:176-181 (mgk-decompiler/test_yolo_inference.py:136-202) turns it into
+ * corner-box candidates (at most 1000 per image over the three levels), then the corner NMS of examples/yolo_detect.cpp:152-173
+ * and, for slots with a frame size, the letterbox inverse of :208-227 give mars_box_t records. */
+/* host only: tensor ids (mars_tensor_t.id) of the outputs of the three CONV2D layers of a YOLOv5 Detect block, stride 8 / 16 / 32
+ * (int8, 3 (5 + nc) channels, NCHW [1,C,gh,gw] or NHWC [1,gh,gw,C], input size / grid in {8, 16, 32}).  Returns 3, or 0 without heads */
+int mars_b200_find_yolo_heads(const void *data, size_t size, uint32_t *tensor_ids, int cap);
+/* decode these heads (level 0, 1, 2 = stride 8, 16, 32) inside every run; tensor_ids = NULL: mars_b200_find_yolo_heads, n = 0: off
+ * (the default; the program is then the one without heads).  MARS_ERR_INVALID_TENSOR (mars_b200_last_error) when a tensor is not a
+ * conv output, has the wrong channel count or grid, a scale <= 0, or the heads are not produced in level order.  Recompiles and
+ * drops captured graphs like mars_b200_set_opt_level. */
+mars_error_t mars_b200_set_yolo_heads(mars_model_t *m, const uint32_t *tensor_ids, int n, float conf_thresh);
+/* original frame size of slots [first, first+n) for the letterbox inverse (0 x 0: keep network coordinates, the default).
+ * mars_b200_preprocess_batch records it as well. */
+mars_error_t mars_b200_set_frame_size(mars_model_t *m, int first, int n, int w, int h);
+/* corner NMS + letterbox inverse on the candidates of the last pass of slots [first, first+n); results stay resident */
+mars_error_t mars_b200_detect_heads_resident(mars_model_t *m, int first, int n, float nms_thresh);
+/* all layers (with the head decodes), NMS and the letterbox inverse as one device-timed region; a CUDA graph from the second call on */
+mars_error_t mars_b200_step_heads_resident(mars_model_t *m, int first, int n, float nms_thresh);
+mars_error_t mars_b200_enqueue_step_heads_resident(mars_model_t *m, int first, int n, float nms_thresh);
+/* mars_b200_submit_batch with the heads decode: boxes[n][maxd], counts[n]; waited for with mars_b200_wait_batch */
+mars_error_t mars_b200_submit_heads_batch(mars_model_t *m, int pool, int n, const void *inputs, size_t in_stride, mars_box_t *boxes,
+                                          int32_t *counts, int maxd, float nms_thresh);
+/* kept boxes of slots [first, first+n): boxes[n][maxd] (maxd <= 1000), counts[n] */
+mars_error_t mars_b200_download_boxes(mars_model_t *m, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd);
+
 /* ---- several GPUs of one box behind one call (batch sharded over the devices, no inter-GPU traffic on the path) ---------- */
 typedef struct mars_b200_group mars_b200_group_t;
 /* one replica of the model per device (devices = NULL: ordinals 0 .. n_devices-1), `per_gpu_batch` image slots each */

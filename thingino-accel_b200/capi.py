@@ -194,6 +194,14 @@ SIGNATURES = {
     "mars_yolo_nms_boxes": (C.c_int, [C.c_void_p, C.c_int, C.c_float]),
     "mars_yolo_scale_detections": (None, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "mars_yolo_decode_anchor_grid": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_int, C.c_float, C.c_void_p, C.c_int, C.c_int]),
+    "mars_b200_find_yolo_heads": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int]),
+    "mars_b200_set_yolo_heads": (C.c_int, [PM, C.c_void_p, C.c_int, C.c_float]),
+    "mars_b200_set_frame_size": (C.c_int, [PM, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "mars_b200_detect_heads_resident": (C.c_int, [PM, C.c_int, C.c_int, C.c_float]),
+    "mars_b200_step_heads_resident": (C.c_int, [PM, C.c_int, C.c_int, C.c_float]),
+    "mars_b200_enqueue_step_heads_resident": (C.c_int, [PM, C.c_int, C.c_int, C.c_float]),
+    "mars_b200_submit_heads_batch": (C.c_int, [PM, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_float]),
+    "mars_b200_download_boxes": (C.c_int, [PM, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
 }
 
 _lib = None
@@ -400,6 +408,44 @@ class MarsModel:
         """queue a batch without the YOLO post-process (raw output tensors read back); wait with wait_batch(pool)"""
         self._check(lib().mars_b200_submit_run_batch(self.m, pool, n, _addr(inputs), in_stride, _addr(outputs), out_stride), "submit_run_batch")
 
+    # ---- YOLOv5 Detect heads (include/mars_b200.h) ------------------------------------
+    def set_yolo_heads(self, tensor_ids=None, conf_thresh=0.25, enable=True):
+        """decode the three head convs inside every run (tensor_ids None: find them); enable=False switches it off"""
+        if not enable:
+            ids, n = None, 0
+        elif tensor_ids is None:
+            ids, n = None, 3
+        else:
+            ids = np.ascontiguousarray(tensor_ids, dtype=np.uint32)
+            n = ids.size
+        self._check(lib().mars_b200_set_yolo_heads(self.m, None if ids is None else ids.ctypes.data, n, conf_thresh), "set_yolo_heads")
+
+    def set_frame_size(self, first, n, w, h):
+        """original frame size of slots [first, first+n) for the letterbox inverse (0, 0: network coordinates)"""
+        self._check(lib().mars_b200_set_frame_size(self.m, first, n, w, h), "set_frame_size")
+
+    def detect_heads_resident(self, first, n, thresh=0.45):
+        self._check(lib().mars_b200_detect_heads_resident(self.m, first, n, thresh), "detect_heads_resident")
+        return float(lib().mars_b200_last_gpu_ms(self.m))
+
+    def step_heads_resident(self, first, n, thresh=0.45):
+        self._check(lib().mars_b200_step_heads_resident(self.m, first, n, thresh), "step_heads_resident")
+        return float(lib().mars_b200_last_gpu_ms(self.m))
+
+    def enqueue_step_heads_resident(self, first, n, thresh=0.45):
+        self._check(lib().mars_b200_enqueue_step_heads_resident(self.m, first, n, thresh), "enqueue_step_heads_resident")
+
+    def submit_heads_batch(self, pool, n, inputs, in_stride, boxes, counts, maxd=1000, thresh=0.45):
+        """submit_batch with the heads decode: boxes [n, maxd] BOX_DTYPE; buffers must stay alive until wait_batch(pool)"""
+        self._check(lib().mars_b200_submit_heads_batch(self.m, pool, n, _addr(inputs), in_stride, _addr(boxes), _addr(counts), maxd, thresh),
+                    "submit_heads_batch")
+
+    def download_boxes(self, first, n, maxd=1000):
+        boxes = np.zeros((n, maxd), dtype=BOX_DTYPE)
+        counts = np.zeros(n, dtype=np.int32)
+        self._check(lib().mars_b200_download_boxes(self.m, first, n, boxes.ctypes.data, counts.ctypes.data, maxd), "download_boxes")
+        return boxes, counts
+
     def wait_batch(self, pool):
         self._check(lib().mars_b200_wait_batch(self.m, pool), "wait_batch")
 
@@ -480,6 +526,14 @@ def resize_taps(in_size, out_size):
         if n <= cap:
             return start, src[:n].copy(), w[:n].copy()
         cap = n
+
+
+def find_yolo_heads(blob):
+    """tensor ids of the three YOLOv5 Detect head convs of a .mars blob in stride order 8 / 16 / 32, or [] (host only, no GPU)"""
+    b = bytes(blob)
+    ids = (C.c_uint32 * 3)()
+    n = lib().mars_b200_find_yolo_heads(b, len(b), ids, 3)
+    return [int(v) for v in ids[:n]]
 
 
 # ---- post-process on host arrays (runs on the device) ---------------------------------

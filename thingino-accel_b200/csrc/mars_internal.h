@@ -41,6 +41,7 @@ enum OpKind : int {
     OP_CONCAT_PERIODIC,/* in-place concat input with constant shift (SURVEY C.4b) */
     OP_UPSAMPLE,       /* :1003-1044 */
     OP_LUT_I8,         /* fused chain of int8 unary layers as one table */
+    OP_YOLO_HEAD,      /* anchor-grid decode of one YOLO head conv output (mars_b200_set_yolo_heads), right after the conv */
     OP_KIND_COUNT
 };
 
@@ -100,7 +101,21 @@ struct Op {
     int fwd_stream = -1;
     /* write/read extents for hazard analysis and bounds checks */
     int64_t wlo = 0, whi = 0;
+    /* OP_YOLO_HEAD: the head tensor is [in0, in0 + n) with grid oh x ow, `lut` = const-pool offset of its 256-float sigmoid table,
+     * f0 = confidence threshold, sh = stride (8 << head_level) */
+    int head_level = -1, head_nc = 0;
+    bool head_nhwc = false;
     std::string note;
+};
+
+/* one YOLOv5 Detect head as the layer table describes it */
+struct YoloHead {
+    uint32_t id = 0;   /* tensor id (mars_tensor_t.id) of the head conv's output */
+    int tensor = -1;   /* its tensor table index */
+    int layer = -1;    /* the CONV2D layer that writes it */
+    int nc = 0, gh = 0, gw = 0, stride = 0;
+    bool nhwc = false;
+    float scale = 0.0f;
 };
 
 struct Program {
@@ -136,8 +151,13 @@ bool first_time_on_device(unsigned long long *mask);
 mars_error_t compile_program(const mars_header_t &h, const mars_runtime_tensor_t *tensors,
                              const mars_runtime_layer_t *layers, const std::vector<size_t> &toff,
                              size_t weights_size, size_t arena_size, int opt_level, int depthwise_mode,
-                             Program *out, int f32_mode = 0);
+                             Program *out, int f32_mode = 0, const std::vector<YoloHead> *heads = nullptr, float head_conf = 0.25f);
 std::string describe_program(const Program &p);
+/* the outputs of the three CONV2D layers of a YOLOv5 Detect block in stride order 8 / 16 / 32 (host only); 0 when there are none */
+int find_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers, uint32_t *ids, int cap);
+/* checks n head tensor ids for mars_b200_set_yolo_heads: MARS_ERR_INVALID_TENSOR (with mars_b200_last_error) or MARS_OK + *out */
+mars_error_t resolve_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers,
+                                const std::vector<size_t> &toff, size_t weights_size, const uint32_t *ids, int n, std::vector<YoloHead> *out);
 
 } // namespace marsb200
 

@@ -12,13 +12,17 @@
  *                   threads per image for large batches, 1024 for small ones; k_nms_center
  *                   also holds the block-wide sort kept as a cross-check);
  *  k_nms_corner   : nms() of reference examples/yolo_detect.cpp:152-173 (corner boxes);
- *  k_anchor_decode: anchor-grid decode (mgk-decompiler/test_yolo_inference.py:136-202).
+ *  k_anchor_decode: anchor-grid decode (mgk-decompiler/test_yolo_inference.py:136-202);
+ *  k_head_decode, k_nms_corner_batch : the same decode and corner NMS (+ letterbox inverse) over a batch of image slots, reading
+ *                   the raw head convolutions where the program leaves them (OP_YOLO_HEAD, mars_b200_set_yolo_heads).
  * One thread block per image; blocks are independent (images shard with no exchange).
  */
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdlib.h>
+
+#include <cub/block/block_radix_sort.cuh>
 
 #include "kernels_exact.cuh"
 
@@ -666,6 +670,193 @@ __global__ void __launch_bounds__(256) k_anchor_decode(const int8_t *head, int g
         cnt += total;
     }
     if (threadIdx.x == 0) *count_out = cnt < maxd ? cnt : maxd;
+}
+
+/* ---- YOLOv5 Detect heads on the batched path ----------------------------------------------------------------------------- */
+#define HEAD_MAX_CAND 1000 /* candidates per image over the three levels (yolo_detect.cpp keeps an uncapped vector) */
+
+/* anchors of reference examples/yolo_detect.cpp:176-181, (w, h) per anchor, one row per level */
+struct HeadAnchors { float wh[6]; };
+
+/* Anchor-grid decode of one level for every image of the launch: the head of image b is at head + b * img_stride, element
+ * (anchor a, channel c, cell p = y * gw + x) at a * astride + c * cstride + p * pstride (NCHW: cstride = gh * gw, pstride = 1, so a
+ * warp reads one byte plane across adjacent x; NHWC: cstride = 1, pstride = 3 (5 + nc)).  Arithmetic of k_anchor_decode with nc
+ * classes.  Candidates go to boxes[b][...] in (anchor, y, x) order after the image's running count (level 0 starts at 0), capped. */
+__global__ void __launch_bounds__(256) k_head_decode(const int8_t *head, size_t img_stride, int gh, int gw, int nc, int astride, int cstride,
+                                                     int pstride, const float *sig, float stride, HeadAnchors anc, float conf_thresh,
+                                                     int level, mars_box_t *boxes, int32_t *counts, int box_stride, int maxd) {
+    __shared__ int warp_sums[32];
+    const int8_t *hb = head + (size_t)blockIdx.x * img_stride;
+    mars_box_t *out = boxes + (size_t)blockIdx.x * box_stride;
+    const int P = gh * gw, ncell = 3 * P;
+    int cnt = level == 0 ? 0 : min(counts[blockIdx.x], maxd);
+    __syncthreads(); /* every thread has read the count before thread 0 rewrites it */
+    for (int base = 0; base < ncell && cnt < maxd; base += blockDim.x) {
+        const int i = base + threadIdx.x;
+        int pass = 0, best = 0, a = 0, cell = 0;
+        float conf = 0.0f;
+        const int8_t *p = hb;
+        if (i < ncell) {
+            a = i / P; cell = i - a * P;
+            p = hb + (size_t)a * astride + (size_t)cell * pstride;
+            const float obj = sig[(int)p[4 * cstride] + 128];
+            if (!(obj < conf_thresh)) {
+                int bv = p[5 * cstride];
+                for (int c = 1; c < nc; c++) {
+                    const int v = p[(size_t)(5 + c) * cstride];
+                    if (v > bv) { bv = v; best = c; }
+                }
+                conf = __fmul_rn(obj, sig[bv + 128]);
+                pass = !(conf < conf_thresh);
+            }
+        }
+        int total;
+        const int rank = cnt + block_excl_scan(pass, &total, warp_sums);
+        if (pass && rank < maxd) {
+            const int y = cell / gw, x = cell - y * gw;
+            const float aw = anc.wh[2 * a], ah = anc.wh[2 * a + 1];
+            const float cx = __fmul_rn(__fadd_rn(__fsub_rn(__fmul_rn(sig[(int)p[0] + 128], 2.0f), 0.5f), (float)x), stride);
+            const float cy = __fmul_rn(__fadd_rn(__fsub_rn(__fmul_rn(sig[(int)p[cstride] + 128], 2.0f), 0.5f), (float)y), stride);
+            const float tw = __fmul_rn(sig[(int)p[2 * cstride] + 128], 2.0f), th = __fmul_rn(sig[(int)p[3 * cstride] + 128], 2.0f);
+            const float w = __fmul_rn(__fmul_rn(tw, tw), aw), h = __fmul_rn(__fmul_rn(th, th), ah);
+            const float hw = __fdiv_rn(w, 2.0f), hh = __fdiv_rn(h, 2.0f);
+            mars_box_t d;
+            d.x0 = __fsub_rn(cx, hw); d.y0 = __fsub_rn(cy, hh); d.x1 = __fadd_rn(cx, hw); d.y1 = __fadd_rn(cy, hh);
+            d.confidence = conf; d.class_id = best;
+            out[rank] = d;
+        }
+        cnt += total;
+    }
+    if (threadIdx.x == 0) counts[blockIdx.x] = min(cnt, maxd);
+}
+
+/* Corner-box NMS of reference examples/yolo_detect.cpp:152-173 for every image of the launch, one CTA per image.
+ *   order : descending confidence, equal confidences in input order, NaN after every number (as k_nms_corner): a block radix
+ *           sort of (confidence key << 10 | input index), unique keys, so no stability question arises;
+ *   test  : same class and IoU (iou_corner) > thresh, one row of a suppression bit matrix per sorted element (warp per row,
+ *           lane per bit) in the image's global scratch, then the greedy walk of k_nms_suppress;
+ *   output: kept boxes in sorted order; for an image with a frame size (frames[b].x > 0) the letterbox inverse of
+ *           k_scale_detections (reference examples/yolo_detect.cpp:208-227) is applied on the way out. */
+#define NMSB_THREADS 256
+#define NMSB_ITEMS (MARS_MAX_DETS / NMSB_THREADS)
+struct NmsBatchShared {
+    union {
+        typename cub::BlockRadixSort<unsigned long long, NMSB_THREADS, NMSB_ITEMS>::TempStorage sort;
+        struct { float x0[MARS_MAX_DETS], y0[MARS_MAX_DETS], x1[MARS_MAX_DETS], y1[MARS_MAX_DETS]; } box;
+    };
+    uint16_t order[MARS_MAX_DETS];
+    int cls[MARS_MAX_DETS];
+    unsigned removed[32];
+    int removed_before[32];
+};
+
+__global__ void __launch_bounds__(NMSB_THREADS) k_nms_corner_batch(const mars_box_t *in_all, const int32_t *counts_in, mars_box_t *out_all,
+                                                                  int32_t *counts_out, int box_stride, float thresh, unsigned *scratch,
+                                                                  const int2 *frames, int net_w, int net_h) {
+    __shared__ NmsBatchShared sh;
+    const mars_box_t *in = in_all + (size_t)blockIdx.x * box_stride;
+    mars_box_t *out = out_all + (size_t)blockIdx.x * box_stride;
+    unsigned *const mask = scratch + (size_t)blockIdx.x * NMS_SCRATCH_WORDS;
+    const int n = min(counts_in[blockIdx.x], MARS_MAX_DETS);
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    unsigned long long key[NMSB_ITEMS];
+#pragma unroll
+    for (int k = 0; k < NMSB_ITEMS; k++) {
+        const int j = tid * NMSB_ITEMS + k;
+        unsigned u = 0xFFFFFFFFu; /* NaN and padding sort last */
+        if (j < n) {
+            const float c = in[j].confidence;
+            if (c == c) {
+                const unsigned b = __float_as_uint(__fadd_rn(c, 0.0f)); /* -0 == +0: a tie, as the comparison sort sees it */
+                const unsigned asc = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+                u = ~asc;
+            }
+        }
+        key[k] = ((unsigned long long)u << 10) | (unsigned)j;
+    }
+    cub::BlockRadixSort<unsigned long long, NMSB_THREADS, NMSB_ITEMS>(sh.sort).Sort(key, 0, 42);
+#pragma unroll
+    for (int k = 0; k < NMSB_ITEMS; k++) sh.order[tid * NMSB_ITEMS + k] = (uint16_t)(key[k] & 1023u);
+    __syncthreads(); /* the sort's storage is reused for the sorted boxes */
+    for (int j = tid; j < n; j += NMSB_THREADS) {
+        const mars_box_t b = in[sh.order[j]];
+        sh.box.x0[j] = b.x0; sh.box.y0[j] = b.y0; sh.box.x1[j] = b.x1; sh.box.y1[j] = b.y1;
+        sh.cls[j] = b.class_id;
+    }
+    __syncthreads();
+    const int nwords = (n + 31) >> 5;
+    for (int i = wid; i < n; i += NMSB_THREADS / 32) {
+        mars_box_t a;
+        a.x0 = sh.box.x0[i]; a.y0 = sh.box.y0[i]; a.x1 = sh.box.x1[i]; a.y1 = sh.box.y1[i];
+        const int acls = sh.cls[i];
+        for (int w = i >> 5; w < nwords; w++) {
+            const int j = w * 32 + lane;
+            bool sup = false;
+            if (j > i && j < n && sh.cls[j] == acls) {
+                mars_box_t b;
+                b.x0 = sh.box.x0[j]; b.y0 = sh.box.y0[j]; b.x1 = sh.box.x1[j]; b.y1 = sh.box.y1[j];
+                sup = iou_corner(a, b) > thresh;
+            }
+            const unsigned bits = __ballot_sync(0xffffffffu, sup);
+            if (lane == 0) mask[i * 32 + w] = bits;
+        }
+    }
+    __syncthreads();
+    if (wid == 0) {
+        unsigned removed = 0u; /* lane w: bits of sorted elements [32w, 32w+32) */
+        constexpr int CH = 8;  /* rows fetched ahead: the walk is serial in i, the row loads are not */
+        unsigned cur_rows[CH], nxt_rows[CH];
+        auto fetch = [&](unsigned (&rows)[CH], int base) {
+#pragma unroll
+            for (int q = 0; q < CH; q++) {
+                const int i = base + q;
+                rows[q] = (i < n && lane >= (i >> 5) && lane < nwords) ? mask[i * 32 + lane] : 0u;
+            }
+        };
+        fetch(cur_rows, 0);
+        for (int base = 0; base < n; base += CH) {
+            fetch(nxt_rows, base + CH);
+#pragma unroll
+            for (int q = 0; q < CH; q++) {
+                const int i = base + q; /* rows beyond n are zero */
+                const unsigned word = __shfl_sync(0xffffffffu, removed, (i >> 5) & 31);
+                if (!((word >> (i & 31)) & 1u)) removed |= cur_rows[q];
+            }
+#pragma unroll
+            for (int q = 0; q < CH; q++) cur_rows[q] = nxt_rows[q];
+        }
+        const int cnt = __popc(removed);
+        int incl = cnt;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int y = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= d) incl += y;
+        }
+        sh.removed[lane] = removed;
+        sh.removed_before[lane] = incl - cnt;
+        if (lane == 31) counts_out[blockIdx.x] = n - incl;
+    }
+    __syncthreads();
+    const int2 fr = frames[blockIdx.x];
+    float sc = 1.0f, px = 0.0f, py = 0.0f, wmax = 0.0f, hmax = 0.0f;
+    if (fr.x > 0 && fr.y > 0) { /* mo_scale_detections / mars_yolo_scale_detections, one rounding per operation */
+        sc = fminf(__fdiv_rn((float)net_w, (float)fr.x), __fdiv_rn((float)net_h, (float)fr.y));
+        px = __fdiv_rn(__fsub_rn((float)net_w, __fmul_rn((float)fr.x, sc)), 2.0f);
+        py = __fdiv_rn(__fsub_rn((float)net_h, __fmul_rn((float)fr.y, sc)), 2.0f);
+        wmax = __fsub_rn((float)fr.x, 1.0f); hmax = __fsub_rn((float)fr.y, 1.0f);
+    }
+    for (int j = tid; j < n; j += NMSB_THREADS) {
+        const unsigned word = sh.removed[j >> 5];
+        if ((word >> (j & 31)) & 1u) continue;
+        mars_box_t b = in[sh.order[j]];
+        if (fr.x > 0 && fr.y > 0) {
+            b.x0 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.x0, px), sc), wmax));
+            b.y0 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.y0, py), sc), hmax));
+            b.x1 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.x1, px), sc), wmax));
+            b.y1 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.y1, py), sc), hmax));
+        }
+        out[j - sh.removed_before[j >> 5] - __popc(word & ((1u << (j & 31)) - 1u))] = b;
+    }
 }
 
 } // namespace marsb200

@@ -18,6 +18,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 
 #include "conv_tc.h"
 #include "conv_tf32.h"
@@ -512,6 +513,172 @@ static mars_error_t compile_concat(Ctx &c, int li, const mars_layer_t &L) {
 }
 
 
+/* ---- YOLOv5 Detect heads (mars_b200_set_yolo_heads) ------------------------------------------------------------------
+ * The compiler drops the Split / Pow / Constant nodes of the Detect block, so everything after the three head convolutions runs
+ * over zero elements and output0 holds stale bytes (SURVEY Appendix B.2).  The detections are in the raw head convolutions
+ * [1, 3 (5 + nc), gh, gw] (or [1, gh, gw, 3 (5 + nc)] with --nhwc).  The planner's round-robin buffers let later layers overwrite a
+ * head, so each head is decoded by an op placed right after the op that completes it. */
+static const int HEAD_STRIDES[3] = {8, 16, 32};
+
+/* geometry of a head candidate: int8 [1,C,gh,gw] / [1,gh,gw,C] whose grid divides the network input by 8, 16 or 32.  Returns false
+ * when the tensor does not have that shape; *why (optional) says what is wrong */
+static bool head_geometry(const mars_header_t &h, const mars_runtime_tensor_t *tensors, int ti, YoloHead *hd, const char **why) {
+    static const char *dummy;
+    const char *&w = why ? *why : dummy;
+    const mars_tensor_t &d = tensors[ti].desc;
+    if (d.dtype != MARS_DTYPE_INT8 || d.ndims != 4 || d.shape[0] != 1) { w = "is not an int8 [1,C,gh,gw] / [1,gh,gw,C] tensor"; return false; }
+    hd->nhwc = d.format == MARS_FORMAT_NHWC;
+    const int C = hd->nhwc ? d.shape[3] : d.shape[1];
+    hd->gh = hd->nhwc ? d.shape[1] : d.shape[2];
+    hd->gw = hd->nhwc ? d.shape[2] : d.shape[3];
+    if (C < 18 || C % 3) { w = "does not have 3 * (5 + nc) channels (nc >= 1)"; return false; }
+    hd->nc = C / 3 - 5;
+    hd->scale = d.scale;
+    const uint32_t ii = h.num_inputs ? h.input_tensor_ids[0] : 0xFFFFFFFFu;
+    if (ii >= h.num_tensors) { w = "belongs to a model without an input tensor"; return false; }
+    const mars_tensor_t &in = tensors[ii].desc;
+    const bool in_nhwc = in.format == MARS_FORMAT_NHWC;
+    const int H = in_nhwc ? in.shape[1] : in.shape[2], W = in_nhwc ? in.shape[2] : in.shape[3];
+    hd->stride = 0;
+    if (hd->gh > 0 && hd->gw > 0 && H % hd->gh == 0 && W % hd->gw == 0 && H / hd->gh == W / hd->gw)
+        for (int s : HEAD_STRIDES) if (H / hd->gh == s) hd->stride = s;
+    if (!hd->stride) { w = "has a grid that is not the input size divided by 8, 16 or 32"; return false; }
+    return true;
+}
+
+/* the last CONV2D layer that writes tensor `id`, or -1 */
+static int producing_conv(const mars_header_t &h, const mars_runtime_layer_t *layers, uint32_t id) {
+    for (uint32_t i = h.num_layers; i-- > 0;)
+        if ((int)layers[i].desc.type == MARS_LAYER_CONV2D && layers[i].desc.num_outputs >= 1 && layers[i].desc.output_tensor_ids[0] == id) return (int)i;
+    return -1;
+}
+
+/* true when a layer that computes something (not one of the reference's no-op layer types) reads tensor `id` */
+static bool read_by_compute(const mars_header_t &h, const mars_runtime_layer_t *layers, uint32_t id) {
+    for (uint32_t i = 0; i < h.num_layers; i++) {
+        const mars_layer_t &L = layers[i].desc;
+        const int t = (int)L.type;
+        if (t == MARS_LAYER_RESHAPE || t == MARS_LAYER_TRANSPOSE || t == MARS_LAYER_SOFTMAX || t == MARS_LAYER_SILU || t == MARS_LAYER_AVGPOOL) continue;
+        for (uint32_t k = 0; k < L.num_inputs && k < 4; k++)
+            if (L.input_tensor_ids[k] == id) return true;
+    }
+    return false;
+}
+
+int find_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers, uint32_t *ids, int cap) {
+    /* A Detect head is a 1x1 conv without activation whose output only the dropped decode layers read.  The last such conv fixes
+     * nc; each stride then takes its last conv of that channel count. */
+    int nc = -1, found[3] = {-1, -1, -1};
+    for (uint32_t i = h.num_layers; i-- > 0;) {
+        const mars_layer_t &L = layers[i].desc;
+        if ((int)L.type != MARS_LAYER_CONV2D || L.num_outputs < 1) continue;
+        const mars_conv_params_t &p = L.params.conv;
+        if (p.kernel_h != 1 || p.kernel_w != 1 || p.activation != MARS_ACT_NONE || read_by_compute(h, layers, L.output_tensor_ids[0])) continue;
+        const int ti = find_tensor(h, tensors, L.output_tensor_ids[0]);
+        YoloHead hd;
+        if (ti < 0 || !head_geometry(h, tensors, ti, &hd, nullptr)) continue;
+        if (nc < 0) nc = hd.nc;
+        if (hd.nc != nc) continue;
+        for (int k = 0; k < 3; k++)
+            if (hd.stride == HEAD_STRIDES[k] && found[k] < 0) found[k] = (int)i;
+    }
+    if (found[0] < 0 || found[1] < 0 || found[2] < 0) return 0;
+    for (int k = 0; k < 3 && k < cap; k++) if (ids) ids[k] = layers[found[k]].desc.output_tensor_ids[0];
+    return 3;
+}
+
+mars_error_t resolve_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers,
+                                const std::vector<size_t> &toff, size_t weights_size, const uint32_t *ids, int n, std::vector<YoloHead> *out) {
+    out->clear();
+    if (n != 3) {
+        set_last_error("set_yolo_heads: %d heads given; a YOLOv5 Detect block has 3 (n = 0 switches the decode off)", n);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    for (int k = 0; k < n; k++) {
+        YoloHead hd;
+        hd.id = ids[k];
+        hd.tensor = find_tensor(h, tensors, ids[k]);
+        hd.layer = hd.tensor < 0 ? -1 : producing_conv(h, layers, ids[k]);
+        const char *why = "";
+        if (hd.layer < 0) {
+            set_last_error("set_yolo_heads: head %d (tensor id %u) is not the output of a CONV2D layer", k, ids[k]);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (!head_geometry(h, tensors, hd.tensor, &hd, &why)) {
+            set_last_error("set_yolo_heads: head %d (tensor id %u) %s", k, ids[k], why);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (k > 0 && hd.nc != (*out)[0].nc) {
+            set_last_error("set_yolo_heads: head %d (tensor id %u) has %d channels, head 0 has %d: the channel count must be the same 3 * (5 + nc)",
+                           k, ids[k], 3 * (5 + hd.nc), 3 * (5 + (*out)[0].nc));
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (!(hd.scale > 0.0f) || !std::isfinite(hd.scale)) { /* the class argmax runs on raw bytes: it needs a monotone dequantisation */
+            set_last_error("set_yolo_heads: head %d (tensor id %u) has scale %g; the decode needs a finite scale > 0", k, ids[k], (double)hd.scale);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (toff[hd.tensor] < weights_size) {
+            set_last_error("set_yolo_heads: head %d (tensor id %u) lives in the weight blob", k, ids[k]);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        out->push_back(hd);
+    }
+    const std::vector<YoloHead> &v = *out;
+    for (int k = 1; k < n; k++)
+        if (v[k].layer <= v[k - 1].layer) {
+            set_last_error("set_yolo_heads: head %d (layer %d) is not produced after head %d (layer %d): heads are decoded in level order",
+                           k, v[k].layer, k - 1, v[k - 1].layer);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+    for (int k = 0; k < n; k++)
+        if (v[k].stride != HEAD_STRIDES[k]) {
+            set_last_error("set_yolo_heads: head %d (tensor id %u) has stride %d; level %d needs stride %d", k, ids[k], v[k].stride, k, HEAD_STRIDES[k]);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+    return MARS_OK;
+}
+
+/* one OP_YOLO_HEAD behind the last op of each head's layer (its conv, or the byte-ReLU that follows it); the sigmoid table is the
+ * host libm's, built like k_anchor_decode's (seam.inc) */
+static mars_error_t insert_yolo_heads(Ctx &c, const std::vector<YoloHead> &heads, float conf) {
+    std::vector<Op> &ops = c.prog->ops;
+    for (size_t k = heads.size(); k-- > 0;) {
+        const YoloHead &hd = heads[k];
+        size_t at = 0;
+        for (size_t i = ops.size(); i-- > 0;)
+            if (ops[i].layer == hd.layer) { at = i + 1; break; }
+        if (!at) { set_last_error("YOLO head %zu: layer %d compiled to no device op", k, hd.layer); return MARS_ERR_INVALID_TENSOR; }
+        Op o;
+        o.kind = OP_YOLO_HEAD;
+        o.layer = hd.layer;
+        o.in0 = c.off(hd.tensor);
+        o.oc = 3 * (5 + hd.nc); o.oh = hd.gh; o.ow = hd.gw;
+        o.sh = o.sw = hd.stride;
+        o.n = (uint64_t)o.oc * hd.gh * hd.gw;
+        o.f0 = conf; o.f1 = hd.scale;
+        o.head_level = (int)k; o.head_nc = hd.nc; o.head_nhwc = hd.nhwc;
+        mars_error_t e;
+        if ((e = check_read(c, hd.layer, o.in0, o.in0 + (int64_t)o.n))) return e;
+        float sig[256];
+        for (int v = -128; v < 128; v++) {
+            volatile float x = (float)v * hd.scale;
+            volatile float ex = expf(-x);
+            volatile float den = 1.0f + ex;
+            volatile float r = 1.0f / den;
+            sig[v + 128] = r;
+        }
+        o.lut = (int)c.prog->const_pool.size(); /* four 256-byte units, float-aligned */
+        c.prog->const_pool.resize(c.prog->const_pool.size() + sizeof sig);
+        memcpy(&c.prog->const_pool[o.lut], sig, sizeof sig);
+        char note[160];
+        snprintf(note, sizeof note, "level %zu stride %d nc %d %s conf %g: decodes [in, in+n), the head store is kept", k, hd.stride, hd.nc,
+                 hd.nhwc ? "nhwc" : "nchw", (double)conf);
+        o.note = note;
+        ops.insert(ops.begin() + (ptrdiff_t)at, o);
+    }
+    return MARS_OK;
+}
+
 /* ---- opt_level >= 1: route hazard-free GEMM-shaped convs to the tcgen05 kernel ---------- */
 static void select_tensor_core_convs(Program *p, int f32_mode) {
     for (auto &o : p->ops)
@@ -740,6 +907,7 @@ static void op_access(const Op &o, Access *a) {
             if (o.ic == o.oc) K(o.out + o.coff, (int64_t)o.n); /* strided writes kill nothing (conservative) */
             break;
         case OP_CONCAT_PERIODIC: R(o.out, o.coff); K(o.out + o.coff, (int64_t)o.n); break;
+        case OP_YOLO_HEAD: R(o.in0, (int64_t)o.n); break; /* keeps the head conv's store alive through dead-store elision */
         default: break;
     }
 }
@@ -836,7 +1004,7 @@ static void elide_dead_stores(Program *p, const IvSet &observed, const IvSet &ho
 mars_error_t compile_program(const mars_header_t &h, const mars_runtime_tensor_t *tensors,
                              const mars_runtime_layer_t *layers, const std::vector<size_t> &toff,
                              size_t weights_size, size_t arena_size, int opt_level, int depthwise_mode,
-                             Program *out, int f32_mode) {
+                             Program *out, int f32_mode, const std::vector<YoloHead> *heads, float head_conf) {
     out->ops.clear();
     out->const_pool.clear();
     out->scratch_bytes = 0;
@@ -864,6 +1032,10 @@ mars_error_t compile_program(const mars_header_t &h, const mars_runtime_tensor_t
                 out->ops.push_back(fail_op((int)i, MARS_ERR_INVALID_LAYER, "unknown layer type"));
                 break;
         }
+        if (e != MARS_OK) return e;
+    }
+    if (heads && !heads->empty()) {
+        mars_error_t e = insert_yolo_heads(c, *heads, head_conf);
         if (e != MARS_OK) return e;
     }
     if (opt_level >= 1) select_tensor_core_convs(out, f32_mode);
@@ -894,7 +1066,8 @@ mars_error_t compile_program(const mars_header_t &h, const mars_runtime_tensor_t
 static const char *kind_name(int k) {
     static const char *n[] = {"nop", "conv_i8_nchw", "conv_i8_nhwc", "conv_f32_nchw", "dw_i8", "byte_relu",
                               "sigmoid_i8", "sigmoid_f32", "mul_i8", "add_i8", "mul_f32", "add_f32", "relu_i8",
-                              "relu_f32", "bn_i8", "bn_f32", "maxpool", "concat", "concat_periodic", "upsample", "lut_i8"};
+                              "relu_f32", "bn_i8", "bn_f32", "maxpool", "concat", "concat_periodic", "upsample", "lut_i8",
+                              "yolo_head"};
     return (k >= 0 && k < OP_KIND_COUNT) ? n[k] : "?";
 }
 static const char *mode_name(int m) {

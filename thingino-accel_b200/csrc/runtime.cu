@@ -191,6 +191,12 @@ struct Model {
     mars_det_t *d_raw = nullptr, *d_det = nullptr;
     int32_t *d_raw_cnt = nullptr, *d_det_cnt = nullptr;
     unsigned *d_nms_mask = nullptr; /* capacity x 1024 x 32 words: suppression bit matrices */
+    /* YOLO heads (mars_b200_set_yolo_heads): decoded candidates, kept boxes, and the original frame size per slot (0 = none) */
+    std::vector<YoloHead> heads;
+    float head_conf = 0.25f;
+    mars_box_t *d_box_raw = nullptr, *d_box = nullptr;
+    int32_t *d_box_raw_cnt = nullptr, *d_box_cnt = nullptr;
+    int2 *d_frame = nullptr;
     DecodeTables *d_tab = nullptr;
     float tab_scale = 0.0f;
     bool tab_valid = false;
@@ -237,6 +243,7 @@ static void model_release(Model *m) {
     for (auto e : m->prof_ev) cudaEventDestroy(e);
     cudaFree(m->d_weights); cudaFree(m->d_slots); cudaFree(m->d_scratch); cudaFree(m->d_cpool); cudaFree(m->d_tc_scratch); cudaFree(m->d_linked);
     cudaFree(m->d_raw); cudaFree(m->d_det); cudaFree(m->d_raw_cnt); cudaFree(m->d_det_cnt); cudaFree(m->d_tab); cudaFree(m->d_nms_mask);
+    cudaFree(m->d_box_raw); cudaFree(m->d_box); cudaFree(m->d_box_raw_cnt); cudaFree(m->d_box_cnt); cudaFree(m->d_frame);
     if (m->h_arena) cudaFreeHost(m->h_arena);
     if (m->ev0) cudaEventDestroy(m->ev0);
     if (m->ev1) cudaEventDestroy(m->ev1);
@@ -284,7 +291,23 @@ static mars_error_t set_capacity(Model *m, int capacity) {
     CU_OK(cudaMalloc(&ndc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaMemsetAsync(nrc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaMemsetAsync(ndc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
+    mars_box_t *nbraw = nullptr, *nbox = nullptr;
+    int32_t *nbrc = nullptr, *nbc = nullptr;
+    int2 *nfr = nullptr;
+    CU_OK(cudaMalloc(&nbraw, (size_t)capacity * MARS_MAX_DETS * sizeof(mars_box_t)), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMalloc(&nbox, (size_t)capacity * MARS_MAX_DETS * sizeof(mars_box_t)), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMalloc(&nbrc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMalloc(&nbc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMalloc(&nfr, (size_t)capacity * sizeof(int2)), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMemsetAsync(nbrc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMemsetAsync(nbc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMemsetAsync(nfr, 0, (size_t)capacity * sizeof(int2), m->stream), MARS_ERR_ALLOC_FAILED);
+    if (m->d_frame)
+        CU_OK(cudaMemcpyAsync(nfr, m->d_frame, (size_t)std::min(capacity, m->capacity) * sizeof(int2), cudaMemcpyDeviceToDevice, m->stream),
+              MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
+    cudaFree(m->d_box_raw); cudaFree(m->d_box); cudaFree(m->d_box_raw_cnt); cudaFree(m->d_box_cnt); cudaFree(m->d_frame);
+    m->d_box_raw = nbraw; m->d_box = nbox; m->d_box_raw_cnt = nbrc; m->d_box_cnt = nbc; m->d_frame = nfr;
     cudaFree(m->d_slots); cudaFree(m->d_scratch); cudaFree(m->d_raw); cudaFree(m->d_det);
     cudaFree(m->d_raw_cnt); cudaFree(m->d_det_cnt); cudaFree(m->d_nms_mask);
     m->d_nms_mask = nmask;
@@ -309,7 +332,7 @@ static mars_error_t compile_model(Model *m) {
     release_graphs(m); /* kernel parameters (slot addresses, tensor maps, tables) are about to change */
     Program p;
     mars_error_t e = compile_program(m->pub.header, m->pub.tensors, m->pub.layers, m->toff, m->weights_size,
-                                     m->arena_size, m->opt_level, m->depthwise_mode, &p, m->f32_mode);
+                                     m->arena_size, m->opt_level, m->depthwise_mode, &p, m->f32_mode, &m->heads, m->head_conf);
     if (e != MARS_OK) return e;
     m->prog = std::move(p);
     cudaFree(m->d_cpool);
@@ -423,6 +446,18 @@ static mars_error_t launch_op(Model *m, size_t op_index, int first, int n, bool 
         return (mars_error_t)(-(o.mode - 1000));
     }
     if (o.kind == OP_NOP || n <= 0) return MARS_OK;
+    if (o.kind == OP_YOLO_HEAD) {
+        static const HeadAnchors ANC[3] = {{{10, 13, 16, 30, 33, 23}}, {{30, 61, 62, 45, 59, 119}}, {{116, 90, 156, 198, 373, 326}}};
+        const int C = o.oc, P = o.oh * o.ow;
+        k_head_decode<<<n, 256, 0, m->stream>>>(reinterpret_cast<const int8_t *>(dev_addr(m, (size_t)o.in0, first)), m->slot_stride, o.oh, o.ow,
+                                                o.head_nc, o.head_nhwc ? 5 + o.head_nc : (5 + o.head_nc) * P, o.head_nhwc ? 1 : P,
+                                                o.head_nhwc ? C : 1, reinterpret_cast<const float *>(m->d_cpool + o.lut), (float)o.sh,
+                                                ANC[o.head_level], o.f0, o.head_level, m->d_box_raw + (size_t)first * MARS_MAX_DETS,
+                                                m->d_box_raw_cnt + first, MARS_MAX_DETS, HEAD_MAX_CAND);
+        m->launches++;
+        CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
+        return MARS_OK;
+    }
     ArenaView v;
     v.wbase = m->d_weights;
     v.sbase = m->d_slots + (size_t)first * m->slot_stride;
@@ -617,6 +652,23 @@ static mars_error_t enqueue_detect(Model *m, int first, int n, float thresh) {
     return MARS_OK;
 }
 
+/* corner NMS + letterbox inverse over the candidates the program's OP_YOLO_HEAD ops left for slots [first, first+n) */
+static mars_error_t enqueue_heads_nms(Model *m, int first, int n, float thresh) {
+    if (m->heads.empty()) {
+        set_last_error("no YOLO heads configured (mars_b200_set_yolo_heads)");
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    const mars_tensor_t &in = m->pub.tensors[m->pub.header.input_tensor_ids[0]].desc; /* checked by set_yolo_heads */
+    const bool nhwc = in.format == MARS_FORMAT_NHWC;
+    const int net_h = nhwc ? in.shape[1] : in.shape[2], net_w = nhwc ? in.shape[2] : in.shape[3];
+    k_nms_corner_batch<<<n, NMSB_THREADS, 0, m->stream>>>(m->d_box_raw + (size_t)first * MARS_MAX_DETS, m->d_box_raw_cnt + first,
+                                                         m->d_box + (size_t)first * MARS_MAX_DETS, m->d_box_cnt + first, MARS_MAX_DETS, thresh,
+                                                         m->d_nms_mask + (size_t)first * NMS_SCRATCH_WORDS, m->d_frame + first, net_w, net_h);
+    m->launches++;
+    CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
+    return MARS_OK;
+}
+
 static inline double now_us() {
     struct timespec ts;
     clock_gettime(CLOCK_MONOTONIC, &ts);
@@ -683,6 +735,24 @@ size_t mars_b200_plan_describe(const void *data, size_t size, size_t arena_bytes
         dst[n] = 0;
     }
     return s.size();
+}
+
+/* The outputs of the three CONV2D layers of a YOLOv5 Detect block, stride 8 / 16 / 32, without touching a device */
+int mars_b200_find_yolo_heads(const void *data, size_t size, uint32_t *tensor_ids, int cap) {
+    if (!data || size < sizeof(mars_header_t)) return 0;
+    mars_header_t h;
+    memcpy(&h, data, sizeof h);
+    if (h.magic != MARS_MAGIC || h.version_major != MARS_VERSION_MAJOR) return 0;
+    const size_t tables = sizeof h + (size_t)h.num_tensors * sizeof(mars_tensor_t) + (size_t)h.num_layers * sizeof(mars_layer_t);
+    if (size < tables) return 0;
+    std::vector<mars_runtime_tensor_t> tensors(h.num_tensors ? h.num_tensors : 1);
+    std::vector<mars_runtime_layer_t> layers(h.num_layers ? h.num_layers : 1);
+    memset(tensors.data(), 0, tensors.size() * sizeof(mars_runtime_tensor_t));
+    memset(layers.data(), 0, layers.size() * sizeof(mars_runtime_layer_t));
+    const uint8_t *p = (const uint8_t *)data + sizeof h;
+    for (uint32_t i = 0; i < h.num_tensors; i++, p += sizeof(mars_tensor_t)) memcpy(&tensors[i].desc, p, sizeof(mars_tensor_t));
+    for (uint32_t i = 0; i < h.num_layers; i++, p += sizeof(mars_layer_t)) memcpy(&layers[i].desc, p, sizeof(mars_layer_t));
+    return find_yolo_heads(h, tensors.data(), layers.data(), tensor_ids, cap);
 }
 
 mars_error_t mars_load_memory(const void *data, size_t size, mars_model_t **out_model) {
@@ -1026,6 +1096,46 @@ void mars_b200_set_opt_level(mars_model_t *model, int level) {
     m->compiled = false;
 }
 void mars_b200_set_strict(int on) { g_strict = on ? 1 : 0; }
+
+mars_error_t mars_b200_set_yolo_heads(mars_model_t *model, const uint32_t *tensor_ids, int n, float conf_thresh) {
+    Model *m = as_model(model);
+    if (!m) return MARS_ERR_INVALID_FILE;
+    std::vector<YoloHead> heads;
+    if (n != 0) {
+        uint32_t found[3];
+        if (!tensor_ids) {
+            n = find_yolo_heads(m->pub.header, m->pub.tensors, m->pub.layers, found, 3);
+            if (n == 0) { set_last_error("set_yolo_heads: the model has no YOLOv5 Detect head convolutions"); return MARS_ERR_INVALID_TENSOR; }
+            tensor_ids = found;
+        }
+        mars_error_t e = resolve_yolo_heads(m->pub.header, m->pub.tensors, m->pub.layers, m->toff, m->weights_size, tensor_ids, n, &heads);
+        if (e != MARS_OK) return e;
+    }
+    bool same = heads.size() == m->heads.size() && (heads.empty() || memcmp(&conf_thresh, &m->head_conf, 4) == 0);
+    for (size_t k = 0; same && k < heads.size(); k++) same = heads[k].id == m->heads[k].id;
+    if (same) return MARS_OK;
+    cudaSetDevice(m->device);
+    cudaStreamSynchronize(m->stream);
+    m->heads = std::move(heads);
+    m->head_conf = conf_thresh;
+    m->compiled = false; /* the next call recompiles and drops the captured graphs */
+    return MARS_OK;
+}
+
+mars_error_t mars_b200_set_frame_size(mars_model_t *model, int first, int n, int w, int h) {
+    Model *m = as_model(model);
+    if (!m) return MARS_ERR_INVALID_FILE;
+    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
+    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
+    if (w < 0 || h < 0 || (w == 0) != (h == 0)) {
+        set_last_error("set_frame_size: %d x %d is not a frame size (0 x 0 clears it)", w, h);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    std::vector<int2> fr((size_t)n, make_int2(w, h));
+    if (n > 0) CU_OK(cudaMemcpyAsync(m->d_frame + first, fr.data(), (size_t)n * sizeof(int2), cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
+    CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
+    return MARS_OK;
+}
 void mars_b200_set_f32_mode(mars_model_t *model, int mode) {
     Model *m = as_model(model);
     if (!m || m->f32_mode == mode) return;
@@ -1156,6 +1266,9 @@ mars_error_t mars_b200_preprocess_batch(mars_model_t *model, int first, int n, c
         m->launches += 2;
     }
     cudaEventRecord(m->ev1, m->stream);
+    /* the frame size of every slot, for the letterbox inverse of the heads decode (mars_b200_set_frame_size) */
+    std::vector<int2> fr((size_t)n, make_int2(w, h));
+    if (n > 0) CU_OK(cudaMemcpyAsync(m->d_frame + first, fr.data(), (size_t)n * sizeof(int2), cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1);
     return MARS_OK;
@@ -1204,9 +1317,13 @@ static bool graphs_enabled() {
     return on;
 }
 
+/* what follows the layers of a step; also the graph cache key */
+enum StepFlavour : int { STEP_LAYERS = 0, STEP_DETECT = 1 /* parse_output of output0 + centre NMS */, STEP_HEADS = 2 /* corner NMS of the heads */ };
+
 static mars_error_t enqueue_step(Model *m, int first, int n, float nms_thresh, int with_detect) {
     mars_error_t e = enqueue_ops(m, first, n, -1);
-    if (e == MARS_OK && with_detect) e = enqueue_detect(m, first, n, nms_thresh);
+    if (e == MARS_OK && with_detect == STEP_DETECT) e = enqueue_detect(m, first, n, nms_thresh);
+    if (e == MARS_OK && with_detect == STEP_HEADS) e = enqueue_heads_nms(m, first, n, nms_thresh);
     return e;
 }
 
@@ -1251,16 +1368,14 @@ static mars_error_t enqueue_step_graphed(Model *m, int first, int n, float nms_t
     return MARS_OK;
 }
 
-/* run + detect as one timed region (the bench's resident step) */
-mars_error_t mars_b200_step_resident(mars_model_t *model, int first, int n, float nms_thresh, int with_detect) {
-    Model *m = as_model(model);
+static mars_error_t step_resident(Model *m, int first, int n, float nms_thresh, int flavour) {
     if (!m) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
     mars_error_t e = compile_model(m);
     if (e != MARS_OK) return e;
     cudaEventRecord(m->ev0, m->stream);
-    e = enqueue_step_graphed(m, first, n, nms_thresh, with_detect);
+    e = enqueue_step_graphed(m, first, n, nms_thresh, flavour);
     cudaEventRecord(m->ev1, m->stream);
     cudaError_t ce = cudaStreamSynchronize(m->stream);
     if (e == MARS_OK && ce != cudaSuccess) {
@@ -1271,39 +1386,88 @@ mars_error_t mars_b200_step_resident(mars_model_t *model, int first, int n, floa
     return e;
 }
 
+static mars_error_t enqueue_step_resident(Model *m, int first, int n, float nms_thresh, int flavour) {
+    if (!m) return MARS_ERR_INVALID_FILE;
+    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
+    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
+    mars_error_t e = compile_model(m);
+    if (e != MARS_OK) return e;
+    return enqueue_step_graphed(m, first, n, nms_thresh, flavour);
+}
+
+/* run + detect as one timed region (the bench's resident step) */
+mars_error_t mars_b200_step_resident(mars_model_t *model, int first, int n, float nms_thresh, int with_detect) {
+    return step_resident(as_model(model), first, n, nms_thresh, with_detect ? STEP_DETECT : STEP_LAYERS);
+}
+
 /* the same step, enqueued only: the call returns as soon as the launches (one CUDA-graph replay from the second time on) are on the
  * model's compute stream; the caller orders its own work behind them there (mars_b200_compute_stream) and synchronises itself */
 mars_error_t mars_b200_enqueue_step_resident(mars_model_t *model, int first, int n, float nms_thresh, int with_detect) {
+    return enqueue_step_resident(as_model(model), first, n, nms_thresh, with_detect ? STEP_DETECT : STEP_LAYERS);
+}
+
+/* all layers (with the head decodes the program holds), corner NMS and the letterbox inverse as one timed region */
+mars_error_t mars_b200_step_heads_resident(mars_model_t *model, int first, int n, float nms_thresh) {
+    Model *m = as_model(model);
+    if (m && m->heads.empty()) { set_last_error("step_heads_resident: no YOLO heads configured (mars_b200_set_yolo_heads)"); return MARS_ERR_INVALID_TENSOR; }
+    return step_resident(m, first, n, nms_thresh, STEP_HEADS);
+}
+mars_error_t mars_b200_enqueue_step_heads_resident(mars_model_t *model, int first, int n, float nms_thresh) {
+    Model *m = as_model(model);
+    if (m && m->heads.empty()) { set_last_error("enqueue_step_heads_resident: no YOLO heads configured (mars_b200_set_yolo_heads)"); return MARS_ERR_INVALID_TENSOR; }
+    return enqueue_step_resident(m, first, n, nms_thresh, STEP_HEADS);
+}
+
+mars_error_t mars_b200_detect_heads_resident(mars_model_t *model, int first, int n, float nms_thresh) {
     Model *m = as_model(model);
     if (!m) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
     mars_error_t e = compile_model(m);
     if (e != MARS_OK) return e;
-    return enqueue_step_graphed(m, first, n, nms_thresh, with_detect);
+    cudaEventRecord(m->ev0, m->stream);
+    e = enqueue_heads_nms(m, first, n, nms_thresh);
+    cudaEventRecord(m->ev1, m->stream);
+    cudaError_t ce = cudaStreamSynchronize(m->stream);
+    if (e == MARS_OK && ce != cudaSuccess) {
+        set_last_error("detect_heads_resident: %s", cudaGetErrorString(ce));
+        e = MARS_ERR_LAYER_FAILED;
+    }
+    if (e == MARS_OK) cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1);
+    return e;
 }
 
-static mars_error_t copy_dets(Model *m, int first, int n, mars_det_t *dets, int32_t *counts, int maxd, cudaStream_t s) {
+/* kept records of slots [first, first+n): mars_det_t of the output0 path, or (boxes) mars_box_t of the heads path (both 24 bytes) */
+static mars_error_t copy_dets(Model *m, int first, int n, void *dets, int32_t *counts, int maxd, cudaStream_t s, bool boxes = false) {
+    static_assert(sizeof(mars_det_t) == sizeof(mars_box_t), "one record size");
     if (maxd > 1000) maxd = 1000;
     if (maxd < 0) maxd = 0;
-    CU_OK(cudaMemcpyAsync(counts, m->d_det_cnt + first, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
+    const int32_t *dcnt = boxes ? m->d_box_cnt : m->d_det_cnt;
+    const void *drec = boxes ? (const void *)(m->d_box + (size_t)first * MARS_MAX_DETS) : (const void *)(m->d_det + (size_t)first * MARS_MAX_DETS);
+    CU_OK(cudaMemcpyAsync(counts, dcnt + first, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
     if (maxd > 0)
-        CU_OK(cudaMemcpy2DAsync(dets, (size_t)maxd * sizeof(mars_det_t), m->d_det + (size_t)first * MARS_MAX_DETS,
+        CU_OK(cudaMemcpy2DAsync(dets, (size_t)maxd * sizeof(mars_det_t), drec,
                                 (size_t)MARS_MAX_DETS * sizeof(mars_det_t), (size_t)maxd * sizeof(mars_det_t), (size_t)n,
                                 cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
 }
 
-mars_error_t mars_b200_download_detections(mars_model_t *model, int first, int n, mars_det_t *dets, int32_t *counts, int maxd) {
+static mars_error_t download_records(mars_model_t *model, int first, int n, void *dets, int32_t *counts, int maxd, bool boxes) {
     Model *m = as_model(model);
     if (!m || !dets || !counts) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    mars_error_t e = copy_dets(m, first, n, dets, counts, maxd, m->stream);
+    mars_error_t e = copy_dets(m, first, n, dets, counts, maxd, m->stream, boxes);
     if (e != MARS_OK) return e;
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     for (int i = 0; i < n; i++) if (counts[i] > maxd) counts[i] = maxd;
     return MARS_OK;
+}
+mars_error_t mars_b200_download_detections(mars_model_t *model, int first, int n, mars_det_t *dets, int32_t *counts, int maxd) {
+    return download_records(model, first, n, dets, counts, maxd, false);
+}
+mars_error_t mars_b200_download_boxes(mars_model_t *model, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd) {
+    return download_records(model, first, n, boxes, counts, maxd, true);
 }
 
 /* end to end from host buffers, double-buffered over the two halves of the slot pool:
@@ -1371,9 +1535,8 @@ mars_error_t mars_b200_run_batch(mars_model_t *model, int n, const void *inputs,
  * detection records on the read-back stream -- and the call returns.  While it runs the caller submits the next batch to the
  * other half, so the host->device copy of batch k+1 and the read-back of batch k-1 overlap the kernels of batch k.
  * inputs / dets / counts must stay valid (and should be pinned, e.g. nna_malloc) until mars_b200_wait_batch(pool) returns. */
-mars_error_t mars_b200_submit_batch(mars_model_t *model, int pool, int n, const void *inputs, size_t in_stride, mars_det_t *dets,
-                                    int32_t *counts, int maxd, float nms_thresh) {
-    Model *m = as_model(model);
+static mars_error_t submit_batch(Model *m, int pool, int n, const void *inputs, size_t in_stride, void *dets, int32_t *counts, int maxd,
+                                 float nms_thresh, int flavour) {
     if (!m || !inputs || !dets || !counts || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     const int half = m->capacity / 2;
@@ -1398,17 +1561,29 @@ mars_error_t mars_b200_submit_batch(mars_model_t *model, int pool, int n, const 
         if (e != MARS_OK) return e;
         cudaEventRecord(m->ev_in[pool], m->h2d_stream);
         cudaStreamWaitEvent(m->stream, m->ev_in[pool], 0);
-        e = enqueue_step_graphed(m, first, n, nms_thresh, 1);
+        e = enqueue_step_graphed(m, first, n, nms_thresh, flavour);
         if (e != MARS_OK) { cudaStreamSynchronize(m->stream); return e; }
         cudaEventRecord(m->ev_done[pool], m->stream);
         cudaStreamWaitEvent(m->d2h_stream, m->ev_done[pool], 0);
-        e = copy_dets(m, first, n, dets, counts, maxd, m->d2h_stream);
+        e = copy_dets(m, first, n, dets, counts, maxd, m->d2h_stream, flavour == STEP_HEADS);
         if (e != MARS_OK) return e;
     }
     cudaEventRecord(m->ev_out[pool], m->d2h_stream);
     m->pending[pool].active = true;
     m->pending[pool].n = n; m->pending[pool].maxd = maxd; m->pending[pool].counts = counts;
     return MARS_OK;
+}
+mars_error_t mars_b200_submit_batch(mars_model_t *model, int pool, int n, const void *inputs, size_t in_stride, mars_det_t *dets,
+                                    int32_t *counts, int maxd, float nms_thresh) {
+    return submit_batch(as_model(model), pool, n, inputs, in_stride, dets, counts, maxd, nms_thresh, STEP_DETECT);
+}
+/* mars_b200_submit_batch with the YOLO heads decode (mars_b200_set_yolo_heads): boxes[n][maxd] corner boxes, frame coordinates for
+ * slots with a frame size */
+mars_error_t mars_b200_submit_heads_batch(mars_model_t *model, int pool, int n, const void *inputs, size_t in_stride, mars_box_t *boxes,
+                                          int32_t *counts, int maxd, float nms_thresh) {
+    Model *m = as_model(model);
+    if (m && m->heads.empty()) { set_last_error("submit_heads_batch: no YOLO heads configured (mars_b200_set_yolo_heads)"); return MARS_ERR_INVALID_TENSOR; }
+    return submit_batch(m, pool, n, inputs, in_stride, boxes, counts, maxd, nms_thresh, STEP_HEADS);
 }
 
 /* mars_b200_submit_batch without the YOLO post-process: the raw output tensor 0 of every image is read back instead
