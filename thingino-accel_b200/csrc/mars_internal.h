@@ -118,6 +118,15 @@ struct YoloHead {
     float scale = 0.0f;
 };
 
+/* the three YOLOv5 Detect levels of reference examples/yolo_detect.cpp:176-181: stride and (w, h) of each of the level's anchors */
+struct HeadAnchors { float wh[6]; };
+struct YoloLevel {
+    int stride;
+    HeadAnchors anchors;
+};
+static const YoloLevel YOLO_LEVELS[3] = {
+    {8, {{10, 13, 16, 30, 33, 23}}}, {16, {{30, 61, 62, 45, 59, 119}}}, {32, {{116, 90, 156, 198, 373, 326}}}};
+
 struct Program {
     std::vector<Op> ops;
     std::vector<uint8_t> const_pool; /* 256-byte tables, uploaded once */
@@ -146,6 +155,8 @@ void set_last_error(const char *fmt, ...);
 /* once per CUDA device: true the first time it is called with this mask on the current device (function attributes and
  * SM counts are per device; the API supports several devices in one process) */
 bool first_time_on_device(unsigned long long *mask);
+/* sig[v + 128] = 1 / (1 + expf(-(v * scale))) for v = -128..127: the host libm's expf, one rounding per operation */
+void build_sigmoid_table(float scale, float sig[256]);
 
 /* compile the layer table into ops (program.cpp) */
 mars_error_t compile_program(const mars_header_t &h, const mars_runtime_tensor_t *tensors,

@@ -9,12 +9,12 @@
  *                   sort is emulated pass by pass (its permutation under ties is NOT a
  *                   stable sort, SURVEY A.4) by one warp per image, then greedy same-class
  *                   suppression through per-class member bitsets and a bit matrix (256
- *                   threads per image for large batches, 1024 for small ones; k_nms_center
- *                   also holds the block-wide sort kept as a cross-check);
- *  k_nms_corner   : nms() of reference examples/yolo_detect.cpp:152-173 (corner boxes);
- *  k_anchor_decode: anchor-grid decode (mgk-decompiler/test_yolo_inference.py:136-202);
- *  k_head_decode, k_nms_corner_batch : the same decode and corner NMS (+ letterbox inverse) over a batch of image slots, reading
- *                   the raw head convolutions where the program leaves them (OP_YOLO_HEAD, mars_b200_set_yolo_heads).
+ *                   threads per image for large batches, 1024 for small ones);
+ *  k_head_decode  : anchor-grid decode (mgk-decompiler/test_yolo_inference.py:136-202) of one head level, reading the raw
+ *                   head convolution where the program leaves it (OP_YOLO_HEAD, mars_b200_set_yolo_heads);
+ *  k_nms_corner_batch : nms() of reference examples/yolo_detect.cpp:152-173 (corner boxes), with the letterbox inverse;
+ *  k_scale_detections : the letterbox inverse alone (reference examples/yolo_detect.cpp:208-227).
+ * The host-pointer entry points (seam.inc) run these kernels on a batch of one image.
  * One thread block per image; blocks are independent (images shard with no exchange).
  */
 #pragma once
@@ -301,10 +301,15 @@ __global__ void __launch_bounds__(32) k_nms_sort_warp(const mars_det_t *dets_in,
 
 #define NMS_THREADS 1024 /* threads of k_nms_center: one per sorted position */
 
-/* dynamic shared memory of k_nms_center */
-struct NmsShared {
+/* the sorted elements of one image as the centre-box suppression reads them: corners, area and class id */
+struct NmsBoxes {
     float x0[MARS_MAX_DETS], y0[MARS_MAX_DETS], x1[MARS_MAX_DETS], y1[MARS_MAX_DETS], area[MARS_MAX_DETS];
     int cls[MARS_MAX_DETS];
+};
+
+/* dynamic shared memory of k_nms_center */
+struct NmsShared {
+    NmsBoxes b;
     unsigned members[NMS_CLASS_ROWS][32]; /* bit j of row c: sorted element j has class c - 1 */
     unsigned removed[32];
     int warp_sums[32];
@@ -320,14 +325,113 @@ __device__ __forceinline__ float iou_pre(float ax0, float ay0, float ax1, float 
     return __fdiv_rn(inter, __fadd_rn(__fsub_rn(__fadd_rn(aarea, barea), inter), 1e-6f));
 }
 
+/* sorted element j is d: the corner and area terms of iou_pre (d by value: the caller's loads all issue before these stores) */
+__device__ __forceinline__ void nms_set_box(NmsBoxes &b, int j, const mars_det_t d) {
+    const float hw = __fdiv_rn(d.w, 2.0f), hh = __fdiv_rn(d.h, 2.0f);
+    b.x0[j] = __fsub_rn(d.x, hw); b.x1[j] = __fadd_rn(d.x, hw);
+    b.y0[j] = __fsub_rn(d.y, hh); b.y1[j] = __fadd_rn(d.y, hh);
+    b.area[j] = __fmul_rn(d.w, d.h);
+    b.cls[j] = d.cls;
+}
+
+/* sorted element j has class cls: bit j of the class's member row members[(cls + 1) * 32 + word] (rows zeroed beforehand), or
+ * *dense = 1 when the class has no row */
+__device__ __forceinline__ void nms_add_member(unsigned *members, int cls, int j, int *dense) {
+    const unsigned c = (unsigned)(cls + 1);
+    if (c < NMS_CLASS_ROWS) atomicOr(&members[c * 32 + (j >> 5)], 1u << (j & 31));
+    else *dense = 1;
+}
+
+/* rows i = row0, row0 + rstep, ... of the suppression bit matrix, one warp per row: bit j of row i is set when sorted element
+ * j > i has i's class and IoU(i, j) > thresh.  Only same-class pairs can suppress: the member row of i's class turns row i
+ * into "members of i's class behind i" -- one word per lane -- and each lane evaluates the IoU of the few bits set in its
+ * word.  With dense set (class ids without a member row) every pair behind i is tested, lane = bit. */
+__device__ __forceinline__ void nms_build_rows(const NmsBoxes &b, const unsigned *members, bool dense, int n, float thresh,
+                                               unsigned *mask, int row0, int rstep, int lane) {
+    const int nwords = (n + 31) >> 5;
+    if (!dense) {
+        for (int i = row0; i < n; i += rstep) {
+            const int w0 = i >> 5;
+            unsigned cand = (lane >= w0 && lane < nwords) ? members[(b.cls[i] + 1) * 32 + lane] : 0u;
+            if (lane == w0) cand &= ~((2u << (i & 31)) - 1u); /* only elements behind i */
+            unsigned bits = 0u;
+            if (__any_sync(0xffffffffu, cand != 0u)) {
+                const float ax0 = b.x0[i], ay0 = b.y0[i], ax1 = b.x1[i], ay1 = b.y1[i], aarea = b.area[i];
+                while (cand) {
+                    const int q = __ffs(cand) - 1;
+                    cand &= cand - 1u;
+                    const int jj = lane * 32 + q;
+                    if (iou_pre(ax0, ay0, ax1, ay1, aarea, b.x0[jj], b.y0[jj], b.x1[jj], b.y1[jj], b.area[jj]) > thresh) bits |= 1u << q;
+                }
+            }
+            if (lane >= w0 && lane < nwords) mask[i * 32 + lane] = bits;
+        }
+    } else {
+        for (int i = row0; i < n; i += rstep) {
+            const float ax0 = b.x0[i], ay0 = b.y0[i], ax1 = b.x1[i], ay1 = b.y1[i], aarea = b.area[i];
+            const int acls = b.cls[i];
+            for (int w = i >> 5; w < nwords; w++) {
+                const int jj = w * 32 + lane;
+                bool sup = false;
+                if (jj > i && jj < n && b.cls[jj] == acls)
+                    sup = iou_pre(ax0, ay0, ax1, ay1, aarea, b.x0[jj], b.y0[jj], b.x1[jj], b.y1[jj], b.area[jj]) > thresh;
+                const unsigned bits = __ballot_sync(0xffffffffu, sup);
+                if (lane == 0) mask[i * 32 + w] = bits;
+            }
+        }
+    }
+}
+
+/* The greedy walk of one warp over the bit matrix: i ascending, row i is ORed into the removed set iff i is still alive -- the
+ * same result as the sequential double loop.  Returns lane w's removed bits (sorted elements [32w, 32w+32)).  The walk is
+ * serial in i but the rows do not depend on it: they are fetched CH at a time (independent L2 loads in flight together), the
+ * next CH while these are used. */
+template <int CH>
+__device__ __forceinline__ unsigned nms_walk(const unsigned *mask, int n, int lane) {
+    const int nwords = (n + 31) >> 5;
+    unsigned removed = 0u;
+    unsigned cur_rows[CH], nxt_rows[CH];
+    auto fetch = [&](unsigned (&rows)[CH], int base) {
+#pragma unroll
+        for (int q = 0; q < CH; q++) {
+            const int i = base + q;
+            rows[q] = (i < n && lane >= (i >> 5) && lane < nwords) ? mask[i * 32 + lane] : 0u;
+        }
+    };
+    fetch(cur_rows, 0);
+    for (int base = 0; base < n; base += CH) {
+        fetch(nxt_rows, base + CH);
+#pragma unroll
+        for (int q = 0; q < CH; q++) {
+            const int i = base + q; /* rows beyond n are zero */
+            const unsigned word = __shfl_sync(0xffffffffu, removed, (i >> 5) & 31);
+            if (!((word >> (i & 31)) & 1u)) removed |= cur_rows[q];
+        }
+#pragma unroll
+        for (int q = 0; q < CH; q++) cur_rows[q] = nxt_rows[q];
+    }
+    return removed;
+}
+
+/* lane w publishes its removed bits (removed[w]) and the exclusive prefix of the per-word removed counts (before[w]: removed
+ * elements in words 0..w-1); lane 31 writes the kept count of the n elements to *kept */
+__device__ __forceinline__ void nms_publish_removed(unsigned removed, int n, int lane, unsigned *removed_out, int *before, int32_t *kept) {
+    const int cnt = __popc(removed);
+    int incl = cnt;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int y = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += y;
+    }
+    removed_out[lane] = removed;
+    before[lane] = incl - cnt;
+    if (lane == 31) *kept = n - incl;
+}
+
 /* dets_in/dets_out: [det_stride] per image; counts in/out per image.  blockDim.x = NMS_THREADS, dynamic smem = sizeof(NmsShared);
- * mask_scratch: NMS_SCRATCH_WORDS per image: MARS_MAX_DETS x 32 words (row i, bit j: sorted element j > i has i's class and
- * IoU(i, j) > thresh; kept in global memory, L2-resident, written and read once, so that two blocks fit one SM), then the
- * sorted order written by k_nms_sort_warp.
- * Greedy suppression (mars_yolo_test.c:113-123) as a bit matrix.  Only same-class pairs can suppress: a member bitset per
- * class turns row i into "members of i's class behind i" -- one word per lane -- and each lane evaluates the IoU of the
- * few bits set in its word.  Then one warp walks i ascending and ORs row i into the removed set iff i is still alive --
- * the same result as the sequential double loop. */
+ * mask_scratch: NMS_SCRATCH_WORDS per image: the MARS_MAX_DETS x 32 words of the bit matrix (kept in global memory,
+ * L2-resident, written and read once, so that two blocks fit one SM), then the sorted order written by k_nms_sort_warp.
+ * Greedy suppression (mars_yolo_test.c:113-123) as a bit matrix (nms_build_rows) and its walk (nms_walk). */
 __global__ void __launch_bounds__(NMS_THREADS, 2) k_nms_center(const mars_det_t *dets_in, const int32_t *counts_in,
                                                                mars_det_t *dets_out, int32_t *counts_out, int det_stride,
                                                                float thresh, unsigned *mask_scratch) {
@@ -347,79 +451,14 @@ __global__ void __launch_bounds__(NMS_THREADS, 2) k_nms_center(const mars_det_t 
     mars_det_t me;
     if (j < n) {
         me = in[src];
-        const float hw = __fdiv_rn(me.w, 2.0f), hh = __fdiv_rn(me.h, 2.0f);
-        sh.x0[j] = __fsub_rn(me.x, hw); sh.x1[j] = __fadd_rn(me.x, hw);
-        sh.y0[j] = __fsub_rn(me.y, hh); sh.y1[j] = __fadd_rn(me.y, hh);
-        sh.area[j] = __fmul_rn(me.w, me.h);
-        sh.cls[j] = me.cls;
+        nms_set_box(sh.b, j, me);
     }
     __syncthreads();
-    if (j < n) {
-        const unsigned c = (unsigned)(me.cls + 1);
-        if (c < NMS_CLASS_ROWS) atomicOr(&sh.members[c][wid], 1u << lane);
-        else sh.dense = 1;
-    }
+    if (j < n) nms_add_member(&sh.members[0][0], me.cls, j, &sh.dense);
     __syncthreads();
-    const int nwords = (n + 31) >> 5;
-    if (!sh.dense) {
-        for (int i = wid; i < n; i += NMS_THREADS / 32) { /* one warp per row, lane = word of the row */
-            const int w0 = i >> 5;
-            unsigned cand = (lane >= w0 && lane < nwords) ? sh.members[sh.cls[i] + 1][lane] : 0u;
-            if (lane == w0) cand &= ~((2u << (i & 31)) - 1u); /* only elements behind i */
-            unsigned bits = 0u;
-            if (__any_sync(0xffffffffu, cand != 0u)) {
-                const float ax0 = sh.x0[i], ay0 = sh.y0[i], ax1 = sh.x1[i], ay1 = sh.y1[i], aarea = sh.area[i];
-                while (cand) {
-                    const int b = __ffs(cand) - 1;
-                    cand &= cand - 1u;
-                    const int jj = lane * 32 + b;
-                    if (iou_pre(ax0, ay0, ax1, ay1, aarea, sh.x0[jj], sh.y0[jj], sh.x1[jj], sh.y1[jj], sh.area[jj]) > thresh) bits |= 1u << b;
-                }
-            }
-            if (lane >= w0 && lane < nwords) mask[i * 32 + lane] = bits;
-        }
-    } else {
-        for (int i = wid; i < n; i += NMS_THREADS / 32) { /* arbitrary class ids: one warp per row, lane = bit, all pairs */
-            const float ax0 = sh.x0[i], ay0 = sh.y0[i], ax1 = sh.x1[i], ay1 = sh.y1[i], aarea = sh.area[i];
-            const int acls = sh.cls[i];
-            for (int w = i >> 5; w < nwords; w++) {
-                const int jj = w * 32 + lane;
-                bool sup = false;
-                if (jj > i && jj < n && sh.cls[jj] == acls)
-                    sup = iou_pre(ax0, ay0, ax1, ay1, aarea, sh.x0[jj], sh.y0[jj], sh.x1[jj], sh.y1[jj], sh.area[jj]) > thresh;
-                const unsigned bits = __ballot_sync(0xffffffffu, sup);
-                if (lane == 0) mask[i * 32 + w] = bits;
-            }
-        }
-    }
+    nms_build_rows(sh.b, &sh.members[0][0], sh.dense, n, thresh, mask, wid, NMS_THREADS / 32, lane);
     __syncthreads();
-    if (wid == 0) {
-        /* lane w: bits of elements [32w, 32w+32).  The walk is serial in i but the rows do not depend on it: they are
-         * fetched sixteen at a time (independent L2 loads in flight together), the next sixteen while these are used. */
-        unsigned removed = 0u;
-        constexpr int CH = 16;
-        unsigned cur_rows[CH], nxt_rows[CH];
-        auto fetch = [&](unsigned (&rows)[CH], int base) {
-#pragma unroll
-            for (int q = 0; q < CH; q++) {
-                const int i = base + q;
-                rows[q] = (i < n && lane >= (i >> 5) && lane < nwords) ? mask[i * 32 + lane] : 0u;
-            }
-        };
-        fetch(cur_rows, 0);
-        for (int base = 0; base < n; base += CH) {
-            fetch(nxt_rows, base + CH);
-#pragma unroll
-            for (int q = 0; q < CH; q++) {
-                const int i = base + q; /* rows beyond n are zero */
-                const unsigned word = __shfl_sync(0xffffffffu, removed, (i >> 5) & 31);
-                if (!((word >> (i & 31)) & 1u)) removed |= cur_rows[q];
-            }
-#pragma unroll
-            for (int q = 0; q < CH; q++) cur_rows[q] = nxt_rows[q];
-        }
-        sh.removed[lane] = removed;
-    }
+    if (wid == 0) sh.removed[lane] = nms_walk<16>(mask, n, lane);
     __syncthreads();
     /* ordered compaction */
     const int keep = j < n && !((sh.removed[wid] >> lane) & 1u);
@@ -430,14 +469,12 @@ __global__ void __launch_bounds__(NMS_THREADS, 2) k_nms_center(const mars_det_t 
 }
 
 /* ---- suppression for presorted images: 256 threads per image, ~24 KiB of shared memory ----------------------------------
- * Same algorithm as the second half of k_nms_center (member bitsets -> bit matrix -> ordered walk -> ordered compaction),
- * sized so that eight images share an SM and a whole 1024-image batch is resident at once: the per-class member bitsets live
- * in the image's global scratch (L2), each thread owns four sorted positions, and the compaction rank comes from population
- * counts over the removed set instead of a block scan. */
+ * The algorithm of k_nms_center sized so that eight images share an SM and a whole 1024-image batch is resident at once: the
+ * per-class member bitsets live in the image's global scratch (L2), each thread owns four sorted positions, and the compaction
+ * rank comes from population counts over the removed set instead of a block scan. */
 #define NMS_SUP_THREADS 256
 struct NmsSupShared {
-    float x0[MARS_MAX_DETS], y0[MARS_MAX_DETS], x1[MARS_MAX_DETS], y1[MARS_MAX_DETS], area[MARS_MAX_DETS];
-    int cls[MARS_MAX_DETS];
+    NmsBoxes b;
     unsigned removed[32];
     int removed_before[32]; /* removed elements in words 0..w-1 */
     int dense;
@@ -462,94 +499,18 @@ __global__ void __launch_bounds__(NMS_SUP_THREADS, 8) k_nms_suppress(const mars_
 #pragma unroll
     for (int k = 0; k < PER; k++) {
         const int j = tid + k * NMS_SUP_THREADS;
-        if (j < n) {
-            const mars_det_t me = in[order[j]];
-            const float hw = __fdiv_rn(me.w, 2.0f), hh = __fdiv_rn(me.h, 2.0f);
-            sh.x0[j] = __fsub_rn(me.x, hw); sh.x1[j] = __fadd_rn(me.x, hw);
-            sh.y0[j] = __fsub_rn(me.y, hh); sh.y1[j] = __fadd_rn(me.y, hh);
-            sh.area[j] = __fmul_rn(me.w, me.h);
-            sh.cls[j] = me.cls;
-        }
+        if (j < n) nms_set_box(sh.b, j, in[order[j]]);
     }
     __syncthreads(); /* members zeroed (global writes of this block are visible to it after the barrier), dense flag reset */
 #pragma unroll
     for (int k = 0; k < PER; k++) {
         const int j = tid + k * NMS_SUP_THREADS;
-        if (j < n) {
-            const unsigned c = (unsigned)(sh.cls[j] + 1);
-            if (c < NMS_CLASS_ROWS) atomicOr(&members[c * 32 + (j >> 5)], 1u << (j & 31));
-            else sh.dense = 1;
-        }
+        if (j < n) nms_add_member(members, sh.b.cls[j], j, &sh.dense);
     }
     __syncthreads();
-    const int nwords = (n + 31) >> 5;
-    if (!sh.dense) {
-        for (int i = wid; i < n; i += NW) { /* one warp per row, lane = word of the row */
-            const int w0 = i >> 5;
-            unsigned cand = (lane >= w0 && lane < nwords) ? members[(sh.cls[i] + 1) * 32 + lane] : 0u;
-            if (lane == w0) cand &= ~((2u << (i & 31)) - 1u); /* only elements behind i */
-            unsigned bits = 0u;
-            if (__any_sync(0xffffffffu, cand != 0u)) {
-                const float ax0 = sh.x0[i], ay0 = sh.y0[i], ax1 = sh.x1[i], ay1 = sh.y1[i], aarea = sh.area[i];
-                while (cand) {
-                    const int b = __ffs(cand) - 1;
-                    cand &= cand - 1u;
-                    const int jj = lane * 32 + b;
-                    if (iou_pre(ax0, ay0, ax1, ay1, aarea, sh.x0[jj], sh.y0[jj], sh.x1[jj], sh.y1[jj], sh.area[jj]) > thresh) bits |= 1u << b;
-                }
-            }
-            if (lane >= w0 && lane < nwords) mask[i * 32 + lane] = bits;
-        }
-    } else {
-        for (int i = wid; i < n; i += NW) { /* arbitrary class ids: lane = bit, all pairs */
-            const float ax0 = sh.x0[i], ay0 = sh.y0[i], ax1 = sh.x1[i], ay1 = sh.y1[i], aarea = sh.area[i];
-            const int acls = sh.cls[i];
-            for (int w = i >> 5; w < nwords; w++) {
-                const int jj = w * 32 + lane;
-                bool sup = false;
-                if (jj > i && jj < n && sh.cls[jj] == acls)
-                    sup = iou_pre(ax0, ay0, ax1, ay1, aarea, sh.x0[jj], sh.y0[jj], sh.x1[jj], sh.y1[jj], sh.area[jj]) > thresh;
-                const unsigned bits = __ballot_sync(0xffffffffu, sup);
-                if (lane == 0) mask[i * 32 + w] = bits;
-            }
-        }
-    }
+    nms_build_rows(sh.b, members, sh.dense, n, thresh, mask, wid, NW, lane);
     __syncthreads();
-    if (wid == 0) {
-        unsigned removed = 0u; /* lane w: bits of elements [32w, 32w+32) */
-        constexpr int CH = 8;
-        unsigned cur_rows[CH], nxt_rows[CH];
-        auto fetch = [&](unsigned (&rows)[CH], int base) {
-#pragma unroll
-            for (int q = 0; q < CH; q++) {
-                const int i = base + q;
-                rows[q] = (i < n && lane >= (i >> 5) && lane < nwords) ? mask[i * 32 + lane] : 0u;
-            }
-        };
-        fetch(cur_rows, 0);
-        for (int base = 0; base < n; base += CH) {
-            fetch(nxt_rows, base + CH);
-#pragma unroll
-            for (int q = 0; q < CH; q++) {
-                const int i = base + q; /* rows beyond n are zero */
-                const unsigned word = __shfl_sync(0xffffffffu, removed, (i >> 5) & 31);
-                if (!((word >> (i & 31)) & 1u)) removed |= cur_rows[q];
-            }
-#pragma unroll
-            for (int q = 0; q < CH; q++) cur_rows[q] = nxt_rows[q];
-        }
-        /* exclusive prefix of the per-word removed counts */
-        const int cnt = __popc(removed);
-        int incl = cnt;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const int y = __shfl_up_sync(0xffffffffu, incl, d);
-            if (lane >= d) incl += y;
-        }
-        sh.removed[lane] = removed;
-        sh.removed_before[lane] = incl - cnt;
-        if (lane == 31) counts_out[blockIdx.x] = n - incl;
-    }
+    if (wid == 0) nms_publish_removed(nms_walk<8>(mask, n, lane), n, lane, sh.removed, sh.removed_before, &counts_out[blockIdx.x]);
     __syncthreads();
     /* ordered compaction: a kept element moves up by the number of removed elements in front of it */
 #pragma unroll
@@ -578,118 +539,49 @@ static inline cudaError_t launch_nms_center(const mars_det_t *dets_in, const int
     return cudaGetLastError();
 }
 
-/* corner-box variant: descending by confidence, equal confidences keep input order */
-__global__ void __launch_bounds__(128) k_nms_corner(const mars_box_t *in, int n, mars_box_t *out, int32_t *count_out,
-                                                    float thresh) {
-    __shared__ uint16_t idx[MARS_MAX_DETS];
-    __shared__ unsigned char sup[MARS_MAX_DETS];
-    __shared__ int warp_sums[32];
-    for (int j = threadIdx.x; j < n; j += blockDim.x) {
-        float c = in[j].confidence;
-        int r = 0;
-        for (int k = 0; k < n; k++) {
-            float ck = in[k].confidence;
-            r += (ck > c) || (ck == c && k < j) || (c != c && ck == ck) || (c != c && ck != ck && k < j);
-        }
-        idx[r] = (uint16_t)j;
-        sup[j] = 0;
-    }
-    __syncthreads();
-    for (int i = 0; i < n; i++) {
-        if (sup[i]) continue;
-        mars_box_t a = in[idx[i]];
-        for (int j = i + 1 + threadIdx.x; j < n; j += blockDim.x) {
-            if (sup[j]) continue;
-            mars_box_t b = in[idx[j]];
-            if (a.class_id == b.class_id && iou_corner(a, b) > thresh) sup[j] = 1;
-        }
-        __syncthreads();
-    }
-    int cnt = 0;
-    for (int base = 0; base < n; base += blockDim.x) {
-        int j = base + threadIdx.x;
-        int keep = j < n && !sup[j];
-        int total;
-        int r = cnt + block_excl_scan(keep, &total, warp_sums);
-        if (keep) out[r] = in[idx[j]];
-        cnt += total;
-    }
-    if (threadIdx.x == 0) *count_out = cnt;
+/* ---- letterbox inverse of reference examples/yolo_detect.cpp:208-227 (mo_scale_detections), one rounding per operation ---- */
+struct Letterbox { float sc, px, py, wmax, hmax; };
+
+/* the scale and padding that letterboxed an orig_w x orig_h frame into the net_w x net_h input, and the frame's last pixel */
+__device__ __forceinline__ Letterbox letterbox_params(int orig_w, int orig_h, int net_w, int net_h) {
+    Letterbox l;
+    l.sc = fminf(__fdiv_rn((float)net_w, (float)orig_w), __fdiv_rn((float)net_h, (float)orig_h));
+    l.px = __fdiv_rn(__fsub_rn((float)net_w, __fmul_rn((float)orig_w, l.sc)), 2.0f);
+    l.py = __fdiv_rn(__fsub_rn((float)net_h, __fmul_rn((float)orig_h, l.sc)), 2.0f);
+    l.wmax = __fsub_rn((float)orig_w, 1.0f); l.hmax = __fsub_rn((float)orig_h, 1.0f);
+    return l;
 }
 
-/* reference examples/yolo_detect.cpp:208-227; sc/px/py computed on the host */
-__global__ void k_scale_detections(mars_box_t *d, int n, float sc, float px, float py, float wmax, float hmax) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    mars_box_t b = d[i];
-    b.x0 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.x0, px), sc), wmax));
-    b.y0 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.y0, py), sc), hmax));
-    b.x1 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.x1, px), sc), wmax));
-    b.y1 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.y1, py), sc), hmax));
-    d[i] = b;
+/* a box in input pixels -> frame pixels, clamped to the frame */
+__device__ __forceinline__ mars_box_t letterbox_inverse(mars_box_t b, const Letterbox &l) {
+    b.x0 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.x0, l.px), l.sc), l.wmax));
+    b.y0 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.y0, l.py), l.sc), l.hmax));
+    b.x1 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.x1, l.px), l.sc), l.wmax));
+    b.y1 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.y1, l.py), l.sc), l.hmax));
+    return b;
 }
 
-/* anchor-grid decode of one head [3,gh,gw,85]; sig[v+128] = 1/(1+expf(-(v*scale))) from the host.
- * Ordered compaction in (anchor, y, x) order appended after cnt0, capped at maxd. */
-__global__ void __launch_bounds__(256) k_anchor_decode(const int8_t *head, int gh, int gw, const float *sig,
-                                                       float stride, float aw0, float ah0, float aw1, float ah1,
-                                                       float aw2, float ah2, float conf_thresh, mars_box_t *dets,
-                                                       int cnt0, int maxd, int32_t *count_out) {
-    __shared__ int warp_sums[32];
-    const int ncell = 3 * gh * gw;
-    int cnt = cnt0;
-    for (int base = 0; base < ncell && cnt < maxd; base += blockDim.x) {
-        int i = base + threadIdx.x;
-        int pass = 0, best = 0;
-        float conf = 0.0f;
-        const int8_t *p = head + (size_t)i * 85;
-        if (i < ncell) {
-            float obj = sig[(int)p[4] + 128];
-            if (!(obj < conf_thresh)) {
-                int bv = p[5];
-                for (int c = 1; c < 80; c++) if (p[5 + c] > bv) { bv = p[5 + c]; best = c; }
-                conf = __fmul_rn(obj, sig[bv + 128]);
-                pass = !(conf < conf_thresh);
-            }
-        }
-        int total;
-        int rank = cnt + block_excl_scan(pass, &total, warp_sums);
-        if (pass && rank < maxd) {
-            int a = i / (gh * gw), rem = i % (gh * gw), y = rem / gw, x = rem % gw;
-            float aw = a == 0 ? aw0 : (a == 1 ? aw1 : aw2), ah = a == 0 ? ah0 : (a == 1 ? ah1 : ah2);
-            float cx = __fmul_rn(__fadd_rn(__fsub_rn(__fmul_rn(sig[(int)p[0] + 128], 2.0f), 0.5f), (float)x), stride);
-            float cy = __fmul_rn(__fadd_rn(__fsub_rn(__fmul_rn(sig[(int)p[1] + 128], 2.0f), 0.5f), (float)y), stride);
-            float tw = __fmul_rn(sig[(int)p[2] + 128], 2.0f), th = __fmul_rn(sig[(int)p[3] + 128], 2.0f);
-            float w = __fmul_rn(__fmul_rn(tw, tw), aw), h = __fmul_rn(__fmul_rn(th, th), ah);
-            float hw = __fdiv_rn(w, 2.0f), hh = __fdiv_rn(h, 2.0f);
-            mars_box_t d;
-            d.x0 = __fsub_rn(cx, hw); d.y0 = __fsub_rn(cy, hh); d.x1 = __fadd_rn(cx, hw); d.y1 = __fadd_rn(cy, hh);
-            d.confidence = conf; d.class_id = best;
-            dets[rank] = d;
-        }
-        cnt += total;
-    }
-    if (threadIdx.x == 0) *count_out = cnt < maxd ? cnt : maxd;
+__global__ void k_scale_detections(mars_box_t *d, int n, int orig_w, int orig_h, int net_w, int net_h) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) d[i] = letterbox_inverse(d[i], letterbox_params(orig_w, orig_h, net_w, net_h));
 }
 
-/* ---- YOLOv5 Detect heads on the batched path ----------------------------------------------------------------------------- */
+/* ---- YOLOv5 Detect heads ------------------------------------------------------------------------------------------------ */
 #define HEAD_MAX_CAND 1000 /* candidates per image over the three levels (yolo_detect.cpp keeps an uncapped vector) */
-
-/* anchors of reference examples/yolo_detect.cpp:176-181, (w, h) per anchor, one row per level */
-struct HeadAnchors { float wh[6]; };
 
 /* Anchor-grid decode of one level for every image of the launch: the head of image b is at head + b * img_stride, element
  * (anchor a, channel c, cell p = y * gw + x) at a * astride + c * cstride + p * pstride (NCHW: cstride = gh * gw, pstride = 1, so a
- * warp reads one byte plane across adjacent x; NHWC: cstride = 1, pstride = 3 (5 + nc)).  Arithmetic of k_anchor_decode with nc
- * classes.  Candidates go to boxes[b][...] in (anchor, y, x) order after the image's running count (level 0 starts at 0), capped. */
+ * warp reads one byte plane across adjacent x; NHWC: cstride = 1, pstride = 3 (5 + nc)); sig[v+128] =
+ * 1/(1+expf(-(v*scale))) from the host.  Candidates go to boxes[b][...] in (anchor, y, x) order, ordered compaction after the
+ * image's running count when `append` is set (else from 0), capped at maxd. */
 __global__ void __launch_bounds__(256) k_head_decode(const int8_t *head, size_t img_stride, int gh, int gw, int nc, int astride, int cstride,
                                                      int pstride, const float *sig, float stride, HeadAnchors anc, float conf_thresh,
-                                                     int level, mars_box_t *boxes, int32_t *counts, int box_stride, int maxd) {
+                                                     int append, mars_box_t *boxes, int32_t *counts, int box_stride, int maxd) {
     __shared__ int warp_sums[32];
     const int8_t *hb = head + (size_t)blockIdx.x * img_stride;
     mars_box_t *out = boxes + (size_t)blockIdx.x * box_stride;
     const int P = gh * gw, ncell = 3 * P;
-    int cnt = level == 0 ? 0 : min(counts[blockIdx.x], maxd);
+    int cnt = append ? min(counts[blockIdx.x], maxd) : 0;
     __syncthreads(); /* every thread has read the count before thread 0 rewrites it */
     for (int base = 0; base < ncell && cnt < maxd; base += blockDim.x) {
         const int i = base + threadIdx.x;
@@ -731,12 +623,12 @@ __global__ void __launch_bounds__(256) k_head_decode(const int8_t *head, size_t 
 }
 
 /* Corner-box NMS of reference examples/yolo_detect.cpp:152-173 for every image of the launch, one CTA per image.
- *   order : descending confidence, equal confidences in input order, NaN after every number (as k_nms_corner): a block radix
- *           sort of (confidence key << 10 | input index), unique keys, so no stability question arises;
+ *   order : descending confidence, equal confidences in input order, -0 == +0, NaN after every number: a block radix sort of
+ *           (confidence key << 10 | input index), unique keys, so no stability question arises;
  *   test  : same class and IoU (iou_corner) > thresh, one row of a suppression bit matrix per sorted element (warp per row,
- *           lane per bit) in the image's global scratch, then the greedy walk of k_nms_suppress;
- *   output: kept boxes in sorted order; for an image with a frame size (frames[b].x > 0) the letterbox inverse of
- *           k_scale_detections (reference examples/yolo_detect.cpp:208-227) is applied on the way out. */
+ *           lane per bit) in the image's global scratch, then the greedy walk (nms_walk);
+ *   output: kept boxes in sorted order; for an image with a frame size (frames[b].x > 0 and frames[b].y > 0) the letterbox
+ *           inverse is applied on the way out. */
 #define NMSB_THREADS 256
 #define NMSB_ITEMS (MARS_MAX_DETS / NMSB_THREADS)
 struct NmsBatchShared {
@@ -802,59 +694,16 @@ __global__ void __launch_bounds__(NMSB_THREADS) k_nms_corner_batch(const mars_bo
         }
     }
     __syncthreads();
-    if (wid == 0) {
-        unsigned removed = 0u; /* lane w: bits of sorted elements [32w, 32w+32) */
-        constexpr int CH = 8;  /* rows fetched ahead: the walk is serial in i, the row loads are not */
-        unsigned cur_rows[CH], nxt_rows[CH];
-        auto fetch = [&](unsigned (&rows)[CH], int base) {
-#pragma unroll
-            for (int q = 0; q < CH; q++) {
-                const int i = base + q;
-                rows[q] = (i < n && lane >= (i >> 5) && lane < nwords) ? mask[i * 32 + lane] : 0u;
-            }
-        };
-        fetch(cur_rows, 0);
-        for (int base = 0; base < n; base += CH) {
-            fetch(nxt_rows, base + CH);
-#pragma unroll
-            for (int q = 0; q < CH; q++) {
-                const int i = base + q; /* rows beyond n are zero */
-                const unsigned word = __shfl_sync(0xffffffffu, removed, (i >> 5) & 31);
-                if (!((word >> (i & 31)) & 1u)) removed |= cur_rows[q];
-            }
-#pragma unroll
-            for (int q = 0; q < CH; q++) cur_rows[q] = nxt_rows[q];
-        }
-        const int cnt = __popc(removed);
-        int incl = cnt;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const int y = __shfl_up_sync(0xffffffffu, incl, d);
-            if (lane >= d) incl += y;
-        }
-        sh.removed[lane] = removed;
-        sh.removed_before[lane] = incl - cnt;
-        if (lane == 31) counts_out[blockIdx.x] = n - incl;
-    }
+    if (wid == 0) nms_publish_removed(nms_walk<8>(mask, n, lane), n, lane, sh.removed, sh.removed_before, &counts_out[blockIdx.x]);
     __syncthreads();
     const int2 fr = frames[blockIdx.x];
-    float sc = 1.0f, px = 0.0f, py = 0.0f, wmax = 0.0f, hmax = 0.0f;
-    if (fr.x > 0 && fr.y > 0) { /* mo_scale_detections / mars_yolo_scale_detections, one rounding per operation */
-        sc = fminf(__fdiv_rn((float)net_w, (float)fr.x), __fdiv_rn((float)net_h, (float)fr.y));
-        px = __fdiv_rn(__fsub_rn((float)net_w, __fmul_rn((float)fr.x, sc)), 2.0f);
-        py = __fdiv_rn(__fsub_rn((float)net_h, __fmul_rn((float)fr.y, sc)), 2.0f);
-        wmax = __fsub_rn((float)fr.x, 1.0f); hmax = __fsub_rn((float)fr.y, 1.0f);
-    }
+    const bool inv = fr.x > 0 && fr.y > 0;
+    const Letterbox lb = inv ? letterbox_params(fr.x, fr.y, net_w, net_h) : Letterbox{1.0f, 0.0f, 0.0f, 0.0f, 0.0f};
     for (int j = tid; j < n; j += NMSB_THREADS) {
         const unsigned word = sh.removed[j >> 5];
         if ((word >> (j & 31)) & 1u) continue;
         mars_box_t b = in[sh.order[j]];
-        if (fr.x > 0 && fr.y > 0) {
-            b.x0 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.x0, px), sc), wmax));
-            b.y0 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.y0, py), sc), hmax));
-            b.x1 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.x1, px), sc), wmax));
-            b.y1 = fmaxf(0.0f, fminf(__fdiv_rn(__fsub_rn(b.y1, py), sc), hmax));
-        }
+        if (inv) b = letterbox_inverse(b, lb);
         out[j - sh.removed_before[j >> 5] - __popc(word & ((1u << (j & 31)) - 1u))] = b;
     }
 }

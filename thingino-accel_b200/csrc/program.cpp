@@ -44,16 +44,24 @@ static int pool_add(Program *p, const int8_t lut[256]) {
     return (int)o;
 }
 
-/* reference src/mars/mars_runtime.c:752-768 tabulated over the 256 possible inputs;
- * expf is the host libm's, the same one the reference would call */
-static void build_sigmoid_lut(float in_scale, float out_scale_raw, int8_t lut[256]) {
-    float os = out_scale_raw > 0 ? out_scale_raw : 1.0f;
+/* expf is the host libm's, the same one the reference would call (this file is compiled without FP contraction) */
+void build_sigmoid_table(float scale, float sig[256]) {
     for (int v = -128; v < 128; v++) {
-        volatile float x = (float)v * in_scale;
+        volatile float x = (float)v * scale;
         volatile float e = expf(-x);
         volatile float den = 1.0f + e;
-        volatile float y = 1.0f / den;
-        volatile float t = y / os;
+        volatile float r = 1.0f / den;
+        sig[v + 128] = r;
+    }
+}
+
+/* reference src/mars/mars_runtime.c:752-768 tabulated over the 256 possible inputs */
+static void build_sigmoid_lut(float in_scale, float out_scale_raw, int8_t lut[256]) {
+    float os = out_scale_raw > 0 ? out_scale_raw : 1.0f;
+    float sig[256];
+    build_sigmoid_table(in_scale, sig);
+    for (int v = -128; v < 128; v++) {
+        volatile float t = sig[v + 128] / os;
         volatile float u = t + 0.5f;
         lut[v + 128] = clamp_i8(f2i_x86(u));
     }
@@ -518,7 +526,6 @@ static mars_error_t compile_concat(Ctx &c, int li, const mars_layer_t &L) {
  * over zero elements and output0 holds stale bytes (SURVEY Appendix B.2).  The detections are in the raw head convolutions
  * [1, 3 (5 + nc), gh, gw] (or [1, gh, gw, 3 (5 + nc)] with --nhwc).  The planner's round-robin buffers let later layers overwrite a
  * head, so each head is decoded by an op placed right after the op that completes it. */
-static const int HEAD_STRIDES[3] = {8, 16, 32};
 
 /* geometry of a head candidate: int8 [1,C,gh,gw] / [1,gh,gw,C] whose grid divides the network input by 8, 16 or 32.  Returns false
  * when the tensor does not have that shape; *why (optional) says what is wrong */
@@ -541,7 +548,7 @@ static bool head_geometry(const mars_header_t &h, const mars_runtime_tensor_t *t
     const int H = in_nhwc ? in.shape[1] : in.shape[2], W = in_nhwc ? in.shape[2] : in.shape[3];
     hd->stride = 0;
     if (hd->gh > 0 && hd->gw > 0 && H % hd->gh == 0 && W % hd->gw == 0 && H / hd->gh == W / hd->gw)
-        for (int s : HEAD_STRIDES) if (H / hd->gh == s) hd->stride = s;
+        for (const YoloLevel &l : YOLO_LEVELS) if (H / hd->gh == l.stride) hd->stride = l.stride;
     if (!hd->stride) { w = "has a grid that is not the input size divided by 8, 16 or 32"; return false; }
     return true;
 }
@@ -580,7 +587,7 @@ int find_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors
         if (nc < 0) nc = hd.nc;
         if (hd.nc != nc) continue;
         for (int k = 0; k < 3; k++)
-            if (hd.stride == HEAD_STRIDES[k] && found[k] < 0) found[k] = (int)i;
+            if (hd.stride == YOLO_LEVELS[k].stride && found[k] < 0) found[k] = (int)i;
     }
     if (found[0] < 0 || found[1] < 0 || found[2] < 0) return 0;
     for (int k = 0; k < 3 && k < cap; k++) if (ids) ids[k] = layers[found[k]].desc.output_tensor_ids[0];
@@ -631,15 +638,15 @@ mars_error_t resolve_yolo_heads(const mars_header_t &h, const mars_runtime_tenso
             return MARS_ERR_INVALID_TENSOR;
         }
     for (int k = 0; k < n; k++)
-        if (v[k].stride != HEAD_STRIDES[k]) {
-            set_last_error("set_yolo_heads: head %d (tensor id %u) has stride %d; level %d needs stride %d", k, ids[k], v[k].stride, k, HEAD_STRIDES[k]);
+        if (v[k].stride != YOLO_LEVELS[k].stride) {
+            set_last_error("set_yolo_heads: head %d (tensor id %u) has stride %d; level %d needs stride %d", k, ids[k], v[k].stride, k, YOLO_LEVELS[k].stride);
             return MARS_ERR_INVALID_TENSOR;
         }
     return MARS_OK;
 }
 
-/* one OP_YOLO_HEAD behind the last op of each head's layer (its conv, or the byte-ReLU that follows it); the sigmoid table is the
- * host libm's, built like k_anchor_decode's (seam.inc) */
+/* one OP_YOLO_HEAD behind the last op of each head's layer (its conv, or the byte-ReLU that follows it), with the head's sigmoid
+ * table */
 static mars_error_t insert_yolo_heads(Ctx &c, const std::vector<YoloHead> &heads, float conf) {
     std::vector<Op> &ops = c.prog->ops;
     for (size_t k = heads.size(); k-- > 0;) {
@@ -660,13 +667,7 @@ static mars_error_t insert_yolo_heads(Ctx &c, const std::vector<YoloHead> &heads
         mars_error_t e;
         if ((e = check_read(c, hd.layer, o.in0, o.in0 + (int64_t)o.n))) return e;
         float sig[256];
-        for (int v = -128; v < 128; v++) {
-            volatile float x = (float)v * hd.scale;
-            volatile float ex = expf(-x);
-            volatile float den = 1.0f + ex;
-            volatile float r = 1.0f / den;
-            sig[v + 128] = r;
-        }
+        build_sigmoid_table(hd.scale, sig);
         o.lut = (int)c.prog->const_pool.size(); /* four 256-byte units, float-aligned */
         c.prog->const_pool.resize(c.prog->const_pool.size() + sizeof sig);
         memcpy(&c.prog->const_pool[o.lut], sig, sizeof sig);

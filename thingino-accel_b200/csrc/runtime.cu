@@ -447,12 +447,11 @@ static mars_error_t launch_op(Model *m, size_t op_index, int first, int n, bool 
     }
     if (o.kind == OP_NOP || n <= 0) return MARS_OK;
     if (o.kind == OP_YOLO_HEAD) {
-        static const HeadAnchors ANC[3] = {{{10, 13, 16, 30, 33, 23}}, {{30, 61, 62, 45, 59, 119}}, {{116, 90, 156, 198, 373, 326}}};
         const int C = o.oc, P = o.oh * o.ow;
         k_head_decode<<<n, 256, 0, m->stream>>>(reinterpret_cast<const int8_t *>(dev_addr(m, (size_t)o.in0, first)), m->slot_stride, o.oh, o.ow,
                                                 o.head_nc, o.head_nhwc ? 5 + o.head_nc : (5 + o.head_nc) * P, o.head_nhwc ? 1 : P,
                                                 o.head_nhwc ? C : 1, reinterpret_cast<const float *>(m->d_cpool + o.lut), (float)o.sh,
-                                                ANC[o.head_level], o.f0, o.head_level, m->d_box_raw + (size_t)first * MARS_MAX_DETS,
+                                                YOLO_LEVELS[o.head_level].anchors, o.f0, o.head_level > 0, m->d_box_raw + (size_t)first * MARS_MAX_DETS,
                                                 m->d_box_raw_cnt + first, MARS_MAX_DETS, HEAD_MAX_CAND);
         m->launches++;
         CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
@@ -600,14 +599,11 @@ static bool range_ok(Model *m, int first, int n) {
 }
 
 /* ---- decode + NMS on the device ----------------------------------------------- */
+/* reference src/mars/mars_yolo_test.c:84,92 -- host libm expf, one rounding per operation.  obj is the sigmoid table: :84 takes
+ * expf(-v * scale) and the table expf(-(v * scale)); negation commutes with the rounded product, so expf sees the same bits */
 static void build_decode_tables(float scale, DecodeTables *t) {
+    build_sigmoid_table(scale, t->obj);
     for (int v = -128; v < 128; v++) {
-        /* reference src/mars/mars_yolo_test.c:84,92 -- host libm expf, one rounding per operation */
-        volatile float a = -(float)v * scale;
-        volatile float e = expf(a);
-        volatile float den = 1.0f + e;
-        volatile float obj = 1.0f / den;
-        t->obj[v + 128] = obj;
         volatile float s = (float)v * scale;
         volatile float e2 = expf(-s);
         volatile float den2 = 1.0f + e2;
