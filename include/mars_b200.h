@@ -77,6 +77,18 @@ mars_error_t mars_b200_upload_inputs(mars_model_t *m, int first, int n, const vo
  * tensor 0 of slots [first, first+n): stbir_resize_uint8 (include/stb/stb_image_resize.h) semantics bit for bit, gray border
  * -17, px - 128, NCHW or NHWC as the tensor's format field says.  Replaces load_image + mars_b200_upload_inputs. */
 mars_error_t mars_b200_preprocess_batch(mars_model_t *m, int first, int n, const uint8_t *frames, size_t frame_stride, int w, int h);
+/* one RGB8 frame: h rows of w pixels, rows row_stride bytes apart (0 = w * 3) */
+typedef struct { const uint8_t *rgb; int32_t w, h; size_t row_stride; } mars_b200_frame_t;
+/* The same pre-processing for a batch of frames of any mix of sizes and row pitches, in one pass on the device; each slot's
+ * tensor is byte-identical to mars_b200_letterbox of its frame alone.  Host memory; synchronous like
+ * mars_b200_preprocess_batch; records each slot's frame size for the letterbox inverse (mars_b200_set_frame_size).
+ * Every frame is checked first -- rgb not NULL, w, h > 0, row_stride 0 or >= w * 3, a letterbox at least one pixel wide and
+ * tall -- and a rejected call writes no slot; mars_b200_last_error names the frame. */
+mars_error_t mars_b200_preprocess_frames(mars_model_t *m, int first, int n, const mars_b200_frame_t *frames);
+/* the same with rgb = device addresses on the model's device (e.g. a hardware decoder's output), read in place: enqueued on
+ * mars_b200_compute_stream(m) and returns.  The frames must be complete before that stream reaches the launches and stay
+ * valid until it has passed them; the table itself may be reused as soon as the call returns. */
+mars_error_t mars_b200_preprocess_frames_device(mars_model_t *m, int first, int n, const mars_b200_frame_t *frames);
 /* slots -> host: output tensor 0 of n images */
 mars_error_t mars_b200_download_outputs(mars_model_t *m, int first, int n, void *host, size_t stride);
 /* run all layers for slots [first, first+n) with inputs already resident in HBM */
@@ -126,7 +138,7 @@ int mars_b200_find_yolo_heads(const void *data, size_t size, uint32_t *tensor_id
  * drops captured graphs like mars_b200_set_opt_level. */
 mars_error_t mars_b200_set_yolo_heads(mars_model_t *m, const uint32_t *tensor_ids, int n, float conf_thresh);
 /* original frame size of slots [first, first+n) for the letterbox inverse (0 x 0: keep network coordinates, the default).
- * mars_b200_preprocess_batch records it as well. */
+ * mars_b200_preprocess_batch and the frames calls record it as well. */
 mars_error_t mars_b200_set_frame_size(mars_model_t *m, int first, int n, int w, int h);
 /* corner NMS + letterbox inverse on the candidates of the last pass of slots [first, first+n); results stay resident */
 mars_error_t mars_b200_detect_heads_resident(mars_model_t *m, int first, int n, float nms_thresh);
@@ -136,6 +148,14 @@ mars_error_t mars_b200_enqueue_step_heads_resident(mars_model_t *m, int first, i
 /* mars_b200_submit_batch with the heads decode: boxes[n][maxd], counts[n]; waited for with mars_b200_wait_batch */
 mars_error_t mars_b200_submit_heads_batch(mars_model_t *m, int pool, int n, const void *inputs, size_t in_stride, mars_box_t *boxes,
                                           int32_t *counts, int maxd, float nms_thresh);
+/* mars_b200_submit_heads_batch from n host frames (mars_b200_preprocess_frames): H2D of each frame on the copy stream, the
+ * letterbox, layers, heads, NMS and the letterbox inverse on the compute stream, D2H of the boxes -- in each frame's own
+ * coordinates.  The frames, boxes and counts must stay valid until mars_b200_wait_batch(pool) returns; the frames must be
+ * pinned (e.g. nna_malloc) for their upload to overlap the kernels.  Each pool keeps device staging for its frames and
+ * pinned staging for its descriptor table, sized by the largest batch so far: a batch that needs more grows it, which waits
+ * for the device once. */
+mars_error_t mars_b200_submit_frames_heads_batch(mars_model_t *m, int pool, int n, const mars_b200_frame_t *frames,
+                                                 mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh);
 /* kept boxes of slots [first, first+n): boxes[n][maxd] (maxd <= 1000), counts[n] */
 mars_error_t mars_b200_download_boxes(mars_model_t *m, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd);
 

@@ -73,6 +73,11 @@ BOX_DTYPE = np.dtype([("x0", "<f4"), ("y0", "<f4"), ("x1", "<f4"), ("y1", "<f4")
 
 PM = C.POINTER(Model)
 
+
+class FRAME(C.Structure):
+    """mars_b200_frame_t: one RGB8 frame, rows row_stride bytes apart (0 = w * 3)"""
+    _fields_ = [("rgb", C.c_void_p), ("w", C.c_int32), ("h", C.c_int32), ("row_stride", C.c_size_t)]
+
 # every symbol include/*.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     # include/mars_runtime.h
@@ -202,6 +207,10 @@ SIGNATURES = {
     "mars_b200_enqueue_step_heads_resident": (C.c_int, [PM, C.c_int, C.c_int, C.c_float]),
     "mars_b200_submit_heads_batch": (C.c_int, [PM, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_float]),
     "mars_b200_download_boxes": (C.c_int, [PM, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "mars_b200_preprocess_frames": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(FRAME)]),
+    "mars_b200_preprocess_frames_device": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(FRAME)]),
+    "mars_b200_submit_frames_heads_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(FRAME), C.c_void_p, C.c_void_p, C.c_int,
+                                                      C.c_float]),
 }
 
 _lib = None
@@ -235,6 +244,30 @@ def _addr(buf):
     raise TypeError(type(buf))
 
 
+def host_frames(frames):
+    """[h, w, 3] uint8 arrays -> (FRAME table, the arrays it points into).  A view whose rows are further apart than w * 3
+    (strides (pitch, 3, 1), e.g. a crop of a wider buffer) passes its pitch; any other layout is copied first."""
+    table = (FRAME * len(frames))()
+    keep = []
+    for i, f in enumerate(frames):
+        a = np.asarray(f)
+        h, w, c = a.shape
+        assert c == 3 and a.dtype == np.uint8
+        if not (a.strides[1:] == (3, 1) and a.strides[0] >= 3 * w):
+            a = np.ascontiguousarray(a)
+        keep.append(a)
+        table[i] = FRAME(a.ctypes.data, w, h, a.strides[0])
+    return table, keep
+
+
+def device_frames(frames):
+    """[(ptr, w, h, row_stride), ...] of frames in device memory -> FRAME table"""
+    table = (FRAME * len(frames))()
+    for i, (p, w, h, stride) in enumerate(frames):
+        table[i] = FRAME(p, w, h, stride)
+    return table
+
+
 def _numel(desc):
     n = 1
     for i in range(min(desc.ndims, 6)):
@@ -252,6 +285,7 @@ class MarsModel:
                 raise MarsError(-5, "mars_b200_set_device", L.mars_b200_last_error().decode())
         L.mars_b200_set_arena_bytes(arena_bytes)
         self.m = PM()
+        self._inflight = {}  # pool -> what a submitted batch reads until wait_batch
         if isinstance(model, (bytes, bytearray, memoryview)):
             self._blob = bytes(model)
             err = L.mars_load_memory(self._blob, len(self._blob), C.byref(self.m))
@@ -362,6 +396,18 @@ class MarsModel:
         self._check(lib().mars_b200_preprocess_batch(self.m, first, n, f.ctypes.data, h * w * 3, w, h), "preprocess_batch")
         return float(lib().mars_b200_last_gpu_ms(self.m))
 
+    def preprocess_frames(self, first, frames):
+        """frames: list of [h, w, 3] uint8 host arrays of any sizes -> letterboxed into input tensor 0 of slots
+        [first, first+len(frames)) in one pass; returns the GPU milliseconds of the copies + kernels"""
+        table, _keep = host_frames(frames)
+        self._check(lib().mars_b200_preprocess_frames(self.m, first, len(frames), table), "preprocess_frames")
+        return float(lib().mars_b200_last_gpu_ms(self.m))
+
+    def preprocess_frames_device(self, first, frames):
+        """frames: [(device ptr, w, h, row_stride), ...]; enqueued on compute_stream(), which the caller synchronises with"""
+        self._check(lib().mars_b200_preprocess_frames_device(self.m, first, len(frames), device_frames(frames)),
+                    "preprocess_frames_device")
+
     def download_outputs(self, first, n, host=None, stride=0):
         if host is None:
             host = np.zeros((n, self.out_bytes), dtype=np.uint8)
@@ -440,6 +486,14 @@ class MarsModel:
         self._check(lib().mars_b200_submit_heads_batch(self.m, pool, n, _addr(inputs), in_stride, _addr(boxes), _addr(counts), maxd, thresh),
                     "submit_heads_batch")
 
+    def submit_frames_heads_batch(self, pool, frames, boxes, counts, maxd=1000, thresh=0.45):
+        """submit_heads_batch from a list of [h, w, 3] uint8 host frames of any sizes; boxes in frame coordinates.  The
+        frames are kept alive until wait_batch(pool); boxes and counts must be kept alive by the caller"""
+        table, keep = host_frames(frames)
+        self._check(lib().mars_b200_submit_frames_heads_batch(self.m, pool, len(frames), table, _addr(boxes), _addr(counts), maxd, thresh),
+                    "submit_frames_heads_batch")
+        self._inflight[pool] = (table, keep)
+
     def download_boxes(self, first, n, maxd=1000):
         boxes = np.zeros((n, maxd), dtype=BOX_DTYPE)
         counts = np.zeros(n, dtype=np.int32)
@@ -447,7 +501,10 @@ class MarsModel:
         return boxes, counts
 
     def wait_batch(self, pool):
-        self._check(lib().mars_b200_wait_batch(self.m, pool), "wait_batch")
+        try:
+            self._check(lib().mars_b200_wait_batch(self.m, pool), "wait_batch")
+        finally:
+            self._inflight.pop(pool, None)
 
     def run_batch(self, n, inputs, in_stride, outputs, out_stride):
         self._check(lib().mars_b200_run_batch(self.m, n, _addr(inputs), in_stride, _addr(outputs), out_stride), "run_batch")

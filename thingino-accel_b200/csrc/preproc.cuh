@@ -13,12 +13,16 @@
  *     k_pre_horizontal    : H[f][r][x][c] = sum_t (u8 / 255.0f) * wh[t]            (stb :1243-1282, :1441-1652)
  *     k_pre_vertical_pack : v = sum_t H[f][src_t][x][c] * wv[t]; u8 = (int)((double)(sat(v) * 255.0f) + 0.5);
  *                           out = (int8)(u8 - 128), border -17  -- or RGBA u8, border 114 (stb :1692-1760, :1866-2061)
+ * Every frame of a launch has its own size, row pitch and tap lists (a table of PreFrame descriptors); the target size is
+ * shared.  A uniform batch is a table of identical descriptors.
  */
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
+#include <string.h>
 
+#include <algorithm>
 #include <vector>
 
 namespace marsb200 {
@@ -180,25 +184,50 @@ static inline LetterboxGeom letterbox_geom(int ow, int oh, int tw, int th) {
     return g;
 }
 
-/* frames: n x (oh x ow x 3) bytes, H: n x oh x nw x 3 floats.  grid (ceil(nw/128), oh, n) */
-__global__ void __launch_bounds__(128) k_pre_horizontal(const uint8_t *frames, size_t frame_stride, int ow, int oh, int nw,
-                                                        const int *hstart, const int *hsrc, const float *hw, float *H) {
+/* One frame of a ragged batch as the kernels see it.  A launch covers a run of frames that share the target size; each has
+ * its own source geometry, row pitch, tap lists and float rows.  Offsets are relative to the launch (chunk). */
+struct PreFrame {
+    const uint8_t *src;  /* row 0 of the RGB8 frame (device) */
+    size_t row_stride;   /* bytes from one row to the next (>= ow * 3) */
+    size_t hoff;         /* its first float in the H scratch: oh x nw x 3 floats */
+    int ow, oh, nw, nh, px, py;
+    int hs, vs;          /* its first entry in the start list of the horizontal / vertical taps */
+    int blk0;            /* its first block in the horizontal grid: blocks [blk0, blk0 + oh * ceil(nw / 128)) */
+};
+/* the concatenated tap lists of a batch: taps of output o of a list beginning at s are [start[s + o], start[s + o + 1]),
+ * indices straight into src / w */
+struct PreTaps {
+    const int *start, *src;
+    const float *w;
+};
+
+/* one thread per resized column of one source row.  The blocks of every frame follow each other (no grid sized to the
+ * largest frame); a block finds its frame by a binary search over the first blocks.  H[r][x][c] = sum_t (u8 / 255) * w[t] */
+__global__ void __launch_bounds__(128) k_pre_horizontal(const PreFrame *fr, int n, PreTaps t, float *H) {
     __shared__ float dec[256]; /* the decode step: (float)u8 / 255.0f, IEEE division */
     dec[threadIdx.x] = __fdiv_rn((float)threadIdx.x, 255.0f);
     dec[threadIdx.x + 128] = __fdiv_rn((float)(threadIdx.x + 128), 255.0f);
     __syncthreads();
-    const int x = blockIdx.x * 128 + threadIdx.x, r = blockIdx.y, f = blockIdx.z;
+    const int b = blockIdx.x;
+    int lo = 0, hi = n - 1; /* the last frame whose first block is <= b */
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (fr[mid].blk0 <= b) lo = mid;
+        else hi = mid - 1;
+    }
+    const PreFrame &d = fr[lo];
+    const int nw = d.nw, bx = (nw + 127) >> 7, local = b - d.blk0, r = local / bx, x = (local - r * bx) * 128 + threadIdx.x;
     if (x >= nw) return;
-    const uint8_t *row = frames + (size_t)f * frame_stride + (size_t)r * ow * 3;
+    const uint8_t *row = d.src + (size_t)r * d.row_stride;
     float a0 = 0.0f, a1 = 0.0f, a2 = 0.0f;
-    for (int t = hstart[x]; t < hstart[x + 1]; t++) {
-        const uint8_t *p = row + (size_t)hsrc[t] * 3;
-        const float c = hw[t];
+    for (int k = t.start[d.hs + x], ke = t.start[d.hs + x + 1]; k < ke; k++) {
+        const uint8_t *p = row + (size_t)t.src[k] * 3;
+        const float c = t.w[k];
         a0 = __fadd_rn(a0, __fmul_rn(dec[p[0]], c));
         a1 = __fadd_rn(a1, __fmul_rn(dec[p[1]], c));
         a2 = __fadd_rn(a2, __fmul_rn(dec[p[2]], c));
     }
-    float *o = H + (((size_t)f * oh + r) * nw + x) * 3;
+    float *o = H + d.hoff + ((size_t)r * nw + x) * 3;
     o[0] = a0; o[1] = a1; o[2] = a2;
 }
 
@@ -212,19 +241,23 @@ __device__ __forceinline__ int pre_encode_u8(float v) {
  * uint8 frame of examples/yolo_detect.cpp:104-124 (memset 114 -- alpha included -- then R, G, B, 0 inside the image) */
 enum { PRE_NCHW_I8 = 0, PRE_NHWC_I8 = 1, PRE_RGBA_U8 = 2 };
 
-/* one thread per target pixel: grid (ceil(tw/128), th, n); dst = target of frame 0 of the launch, frames slot_stride apart */
-__global__ void __launch_bounds__(128) k_pre_vertical_pack(const float *H, LetterboxGeom g, const int *vstart, const int *vsrc,
-                                                           const float *vw, int8_t *dst, size_t slot_stride, int mode) {
+/* one thread per target pixel: grid (ceil(tw/128), th, n); dst = target of frame 0 of the launch, frames slot_stride apart.
+ * frame_size (may be null) receives each frame's (ow, oh), for the letterbox inverse of the heads decode. */
+__global__ void __launch_bounds__(128) k_pre_vertical_pack(const float *H, const PreFrame *fr, int tw, int th, PreTaps t, int8_t *dst,
+                                                           size_t slot_stride, int mode, int2 *frame_size) {
     const int dx = blockIdx.x * 128 + threadIdx.x, dy = blockIdx.y, f = blockIdx.z;
-    if (dx >= g.tw) return;
-    const int x = dx - g.px, y = dy - g.py;
-    const bool inside = x >= 0 && x < g.nw && y >= 0 && y < g.nh;
+    const PreFrame &d = fr[f];
+    if (frame_size && dx == 0 && dy == 0) frame_size[f] = make_int2(d.ow, d.oh);
+    if (dx >= tw) return;
+    const int x = dx - d.px, y = dy - d.py, nw = d.nw;
+    const bool inside = x >= 0 && x < nw && y >= 0 && y < d.nh;
     int u0 = 0, u1 = 0, u2 = 0;
     if (inside) {
+        const float *Hf = H + d.hoff;
         float a0 = 0.0f, a1 = 0.0f, a2 = 0.0f;
-        for (int t = vstart[y]; t < vstart[y + 1]; t++) {
-            const float *p = H + (((size_t)f * g.oh + vsrc[t]) * g.nw + x) * 3;
-            const float c = vw[t];
+        for (int k = t.start[d.vs + y], ke = t.start[d.vs + y + 1]; k < ke; k++) {
+            const float *p = Hf + ((size_t)t.src[k] * nw + x) * 3;
+            const float c = t.w[k];
             a0 = __fadd_rn(a0, __fmul_rn(p[0], c));
             a1 = __fadd_rn(a1, __fmul_rn(p[1], c));
             a2 = __fadd_rn(a2, __fmul_rn(p[2], c));
@@ -234,63 +267,112 @@ __global__ void __launch_bounds__(128) k_pre_vertical_pack(const float *H, Lette
     int8_t *o = dst + (size_t)f * slot_stride;
     if (mode == PRE_RGBA_U8) {
         uchar4 px = inside ? make_uchar4((unsigned char)u0, (unsigned char)u1, (unsigned char)u2, 0) : make_uchar4(114, 114, 114, 114);
-        reinterpret_cast<uchar4 *>(o)[(size_t)dy * g.tw + dx] = px;
+        reinterpret_cast<uchar4 *>(o)[(size_t)dy * tw + dx] = px;
         return;
     }
     const int r0 = inside ? u0 - 128 : -17, r1 = inside ? u1 - 128 : -17, r2 = inside ? u2 - 128 : -17;
     if (mode == PRE_NHWC_I8) {
-        int8_t *q = o + ((size_t)dy * g.tw + dx) * 3;
+        int8_t *q = o + ((size_t)dy * tw + dx) * 3;
         q[0] = (int8_t)r0; q[1] = (int8_t)r1; q[2] = (int8_t)r2;
     } else {
-        const size_t ps = (size_t)g.tw * g.th, at = (size_t)dy * g.tw + dx;
+        const size_t ps = (size_t)tw * th, at = (size_t)dy * tw + dx;
         o[at] = (int8_t)r0; o[ps + at] = (int8_t)r1; o[2 * ps + at] = (int8_t)r2;
     }
 }
 
-/* device copies of the two tap lists of one geometry */
-struct LetterboxPlan {
-    LetterboxGeom g;
-    int *d_hstart = nullptr, *d_hsrc = nullptr, *d_vstart = nullptr, *d_vsrc = nullptr;
-    float *d_hw = nullptr, *d_vw = nullptr;
-    bool ok = false;
+/* the H scratch of one launch stays under this; a batch that needs more is split on frame boundaries */
+static const size_t PRE_H_CHUNK_BYTES = (size_t)256 << 20;
+
+/* Host side of a ragged batch: the descriptors, the concatenated tap lists (one copy per distinct (in, out) of an axis) and
+ * the launches.  Packed into one blob -- [PreFrame x n][start][src][w] -- that is copied to the device in one piece. */
+struct PreTable {
+    int tw = 0, th = 0;
+    std::vector<PreFrame> fr;
+    std::vector<size_t> stage; /* byte offset of each frame in a tightly packed staging buffer (rows ow * 3 apart) */
+    std::vector<int> start, src;
+    std::vector<float> w;
+    std::vector<int> first, blocks; /* launch k covers frames [first[k], first[k + 1]) with blocks[k] horizontal blocks */
+    size_t h_floats = 0;            /* H scratch of the largest launch */
+    size_t stage_bytes = 0;         /* staging of the largest launch (per_launch_staging) or of the whole batch */
+
+    size_t bytes() const { return fr.size() * sizeof(PreFrame) + (start.size() + src.size()) * sizeof(int) + w.size() * sizeof(float); }
+    void pack(void *out) const {
+        uint8_t *p = (uint8_t *)out;
+        memcpy(p, fr.data(), fr.size() * sizeof(PreFrame)); p += fr.size() * sizeof(PreFrame);
+        memcpy(p, start.data(), start.size() * sizeof(int)); p += start.size() * sizeof(int);
+        memcpy(p, src.data(), src.size() * sizeof(int)); p += src.size() * sizeof(int);
+        memcpy(p, w.data(), w.size() * sizeof(float));
+    }
+    /* where the tap lists sit in the device copy of the blob */
+    PreTaps taps(const void *dev) const {
+        const int *s = (const int *)((const uint8_t *)dev + fr.size() * sizeof(PreFrame));
+        return PreTaps{s, s + start.size(), (const float *)(s + start.size() + src.size())};
+    }
 };
 
-static inline void letterbox_plan_release(LetterboxPlan *p) {
-    cudaFree(p->d_hstart); cudaFree(p->d_hsrc); cudaFree(p->d_hw);
-    cudaFree(p->d_vstart); cudaFree(p->d_vsrc); cudaFree(p->d_vw);
-    *p = LetterboxPlan();
+/* Builds the table for n frames (geometry g[f] from letterbox_geom, all into the same target) whose source pointers and
+ * pitches the caller fills in afterwards.  taps_of(in, out) returns the ResizeTaps of one axis (the caller's cache).
+ * Launches split where the cumulative H bytes (oh * nw * 12 per frame) would pass PRE_H_CHUNK_BYTES; with
+ * per_launch_staging the staging offsets restart with every launch. */
+template <class TapsOf>
+static inline void pre_table_build(const LetterboxGeom *g, int n, TapsOf taps_of, bool per_launch_staging, PreTable *t) {
+    *t = PreTable();
+    if (n <= 0) return;
+    t->tw = g[0].tw; t->th = g[0].th;
+    t->fr.resize(n);
+    t->stage.resize(n);
+    std::vector<std::pair<std::pair<int, int>, int>> seen; /* (in, out) -> its first entry in start */
+    auto list = [&](int in, int out) {
+        for (auto &s : seen)
+            if (s.first.first == in && s.first.second == out) return s.second;
+        const ResizeTaps &rt = taps_of(in, out);
+        const int at = (int)t->start.size(), base = (int)t->src.size();
+        for (int o = 0; o <= out; o++) t->start.push_back(base + rt.start[o]);
+        t->src.insert(t->src.end(), rt.src.begin(), rt.src.end());
+        t->w.insert(t->w.end(), rt.w.begin(), rt.w.end());
+        seen.push_back({{in, out}, at});
+        return at;
+    };
+    size_t hbytes = 0, hfl = 0, soff = 0;
+    int blk = 0;
+    for (int f = 0; f < n; f++) {
+        const LetterboxGeom &q = g[f];
+        const size_t need = (size_t)q.oh * q.nw * 3 * sizeof(float);
+        if (f == 0 || (hbytes > 0 && hbytes + need > PRE_H_CHUNK_BYTES) || f - t->first.back() >= 65535) {
+            if (f > 0) t->blocks.push_back(blk);
+            t->first.push_back(f);
+            hbytes = 0; hfl = 0; blk = 0;
+            if (per_launch_staging) soff = 0;
+        }
+        PreFrame &d = t->fr[f];
+        d.src = nullptr; d.row_stride = 0;
+        d.hoff = hfl;
+        d.ow = q.ow; d.oh = q.oh; d.nw = q.nw; d.nh = q.nh; d.px = q.px; d.py = q.py;
+        d.hs = list(q.ow, q.nw);
+        d.vs = list(q.oh, q.nh);
+        d.blk0 = blk;
+        t->stage[f] = soff;
+        blk += q.oh * ((q.nw + 127) / 128);
+        hbytes += need;
+        hfl += need / sizeof(float);
+        soff += (size_t)q.ow * q.oh * 3;
+        t->h_floats = std::max(t->h_floats, hfl);
+        t->stage_bytes = std::max(t->stage_bytes, soff);
+    }
+    t->blocks.push_back(blk);
+    t->first.push_back(n);
 }
 
-static inline bool letterbox_plan_build(int ow, int oh, int tw, int th, LetterboxPlan *p) {
-    if (p->ok && p->g.ow == ow && p->g.oh == oh && p->g.tw == tw && p->g.th == th) return true;
-    letterbox_plan_release(p);
-    if (ow <= 0 || oh <= 0 || tw <= 0 || th <= 0) return false;
-    p->g = letterbox_geom(ow, oh, tw, th);
-    if (p->g.nw <= 0 || p->g.nh <= 0 || p->g.nw > tw || p->g.nh > th) return false;
-    ResizeTaps h, v;
-    build_resize_taps(ow, p->g.nw, &h);
-    build_resize_taps(oh, p->g.nh, &v);
-    auto up_i = [](const std::vector<int> &s, int **d) {
-        return cudaMalloc(d, (s.size() + 1) * sizeof(int)) == cudaSuccess &&
-               cudaMemcpy(*d, s.data(), s.size() * sizeof(int), cudaMemcpyHostToDevice) == cudaSuccess;
-    };
-    auto up_f = [](const std::vector<float> &s, float **d) {
-        return cudaMalloc(d, (s.size() + 1) * sizeof(float)) == cudaSuccess &&
-               cudaMemcpy(*d, s.data(), s.size() * sizeof(float), cudaMemcpyHostToDevice) == cudaSuccess;
-    };
-    p->ok = up_i(h.start, &p->d_hstart) && up_i(h.src, &p->d_hsrc) && up_f(h.w, &p->d_hw) && up_i(v.start, &p->d_vstart) &&
-            up_i(v.src, &p->d_vsrc) && up_f(v.w, &p->d_vw);
-    if (!p->ok) letterbox_plan_release(p);
-    return p->ok;
-}
-
-/* frames (device) -> int8 tensors at dst + f * slot_stride, f < n; H = scratch of n * oh * nw * 3 floats */
-static inline cudaError_t launch_letterbox(const LetterboxPlan &p, const uint8_t *d_frames, size_t frame_stride, int n, float *d_H,
-                                           int8_t *dst, size_t slot_stride, int mode, cudaStream_t s) {
-    const LetterboxGeom &g = p.g;
-    k_pre_horizontal<<<dim3((g.nw + 127) / 128, g.oh, n), 128, 0, s>>>(d_frames, frame_stride, g.ow, g.oh, g.nw, p.d_hstart, p.d_hsrc,
-                                                                       p.d_hw, d_H);
-    k_pre_vertical_pack<<<dim3((g.tw + 127) / 128, g.th, n), 128, 0, s>>>(d_H, g, p.d_vstart, p.d_vsrc, p.d_vw, dst, slot_stride, mode);
+/* launch k of a table whose blob was copied to dev: frames [first[k], first[k+1]) -> dst + f * slot_stride (dst = target of
+ * the table's frame 0), H = scratch of h_floats floats; frame_size (may be null) = that of the table's frame 0 */
+static inline cudaError_t launch_letterbox(const PreTable &t, int k, const void *dev, float *H, int8_t *dst, size_t slot_stride,
+                                           int mode, int2 *frame_size, cudaStream_t s) {
+    const int f0 = t.first[k], c = t.first[k + 1] - f0;
+    const PreFrame *fr = (const PreFrame *)dev + f0;
+    const PreTaps taps = t.taps(dev);
+    k_pre_horizontal<<<t.blocks[k], 128, 0, s>>>(fr, c, taps, H);
+    k_pre_vertical_pack<<<dim3((t.tw + 127) / 128, t.th, c), 128, 0, s>>>(H, fr, t.tw, t.th, taps, dst + (size_t)f0 * slot_stride,
+                                                                          slot_stride, mode, frame_size ? frame_size + f0 : nullptr);
     return cudaGetLastError();
 }
 

@@ -22,6 +22,7 @@
 #include <time.h>
 
 #include <algorithm>
+#include <map>
 #include <new>
 #include <string>
 #include <thread>
@@ -177,12 +178,17 @@ struct Model {
     uint64_t launches = 0;
     /* asynchronous batches (mars_b200_submit_batch / wait_batch): one in flight per half of the slot pool */
     struct Pending { bool active = false; int n = 0, maxd = 0; int32_t *counts = nullptr; } pending[2];
-    /* letterbox pre-processing (mars_b200_preprocess_batch): tap lists of the last geometry, frame staging, float rows */
-    LetterboxPlan pre_plan;
-    uint8_t *d_frames = nullptr;
-    size_t frames_cap = 0;
+    /* letterbox pre-processing (preproc.cuh): tap lists per (in, out) size of one axis -- camera sizes repeat, and the
+     * downscale taps cost O(in x out) on the host -- the float rows of one launch, and staging for frames and descriptor
+     * tables: one set per pool of the frames submit, one for the synchronous and device-frame calls (PRE_SYNC) */
+    std::map<std::pair<int, int>, ResizeTaps> pre_taps;
     float *d_preH = nullptr;
     size_t preH_cap = 0;
+    struct PreStage {
+        uint8_t *d_frames = nullptr, *d_tab = nullptr, *h_tab = nullptr; /* device frames, device table, pinned table */
+        size_t frames_cap = 0, tab_cap = 0, h_cap = 0;
+        cudaEvent_t ev = nullptr; /* the last upload from h_tab */
+    } pre_stage[3];
     /* captured steps (mars_b200_step_resident): one CUDA graph per (first, n, threshold, with_detect) seen twice */
     struct StepGraph { int first, n, with_detect; uint32_t thresh_bits; int seen; cudaGraphExec_t exec; uint64_t launches; };
     std::vector<StepGraph> graphs;
@@ -252,8 +258,12 @@ static void model_release(Model *m) {
         if (m->ev_done[i]) cudaEventDestroy(m->ev_done[i]);
         if (m->ev_out[i]) cudaEventDestroy(m->ev_out[i]);
     }
-    letterbox_plan_release(&m->pre_plan);
-    cudaFree(m->d_frames);
+    for (auto &st : m->pre_stage) {
+        if (st.ev) cudaEventSynchronize(st.ev);
+        if (st.ev) cudaEventDestroy(st.ev);
+        cudaFree(st.d_frames); cudaFree(st.d_tab);
+        if (st.h_tab) cudaFreeHost(st.h_tab);
+    }
     cudaFree(m->d_preH);
     if (m->stream) cudaStreamDestroy(m->stream);
     if (m->h2d_stream) cudaStreamDestroy(m->h2d_stream);
@@ -848,6 +858,7 @@ mars_error_t mars_load_memory(const void *data, size_t size, mars_model_t **out_
         cudaEventCreateWithFlags(&m->ev_done[i], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&m->ev_out[i], cudaEventDisableTiming);
     }
+    for (auto &st : m->pre_stage) cudaEventCreateWithFlags(&st.ev, cudaEventDisableTiming);
 
     uint32_t k = 0;
     for (uint32_t i = 0; i < h.num_tensors; i++) {
@@ -1211,63 +1222,206 @@ mars_error_t mars_b200_download_outputs(mars_model_t *model, int first, int n, v
     return MARS_OK;
 }
 
+/* ---- letterbox pre-processing of ragged batches (preproc.cuh) ------------------------------------------------------ */
+enum { PRE_SYNC = 2 }; /* pre_stage index of the synchronous and device-frame calls; 0 and 1 are the pools */
+enum PreSource { PRE_HOST_SYNC, PRE_DEVICE, PRE_HOST_POOL };
+
+/* the letterbox target: input tensor 0 of the slots, a 4-d int8 tensor (reference src/mars/mars_yolo_test.c:157-159) */
+static mars_error_t pre_target(Model *m, const char *what, uint32_t *ti, int *tw, int *th, int *nhwc) {
+    if (m->pub.header.num_inputs < 1) return MARS_ERR_INVALID_TENSOR;
+    *ti = m->pub.header.input_tensor_ids[0];
+    if (*ti >= m->pub.header.num_tensors || m->toff[*ti] < m->weights_size) return MARS_ERR_INVALID_TENSOR;
+    const mars_tensor_t &d = m->pub.tensors[*ti].desc;
+    if (d.dtype != MARS_DTYPE_INT8 || d.ndims < 4) {
+        set_last_error("%s: input 0 must be a 4-d int8 tensor (reference src/mars/mars_yolo_test.c:157-159)", what);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    *nhwc = d.format == MARS_FORMAT_NHWC;
+    *th = *nhwc ? d.shape[1] : d.shape[2];
+    *tw = *nhwc ? d.shape[2] : d.shape[3];
+    if (*th <= 0 || *tw <= 0 || (size_t)*tw * *th * 3 > m->buffer_size) return MARS_ERR_INVALID_TENSOR;
+    return MARS_OK;
+}
+
+/* every frame of a call is checked before any device work, so that a rejected call writes no slot */
+static mars_error_t pre_check_frames(Model *m, const char *what, int n, const mars_b200_frame_t *frames, int tw, int th, bool device,
+                                     std::vector<LetterboxGeom> *g) {
+    if (!frames) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
+    g->resize(n > 0 ? n : 0);
+    for (int f = 0; f < n; f++) {
+        const mars_b200_frame_t &fr = frames[f];
+        if (!fr.rgb) { set_last_error("%s: frame %d: rgb is NULL", what, f); return MARS_ERR_INVALID_FILE; }
+        if (fr.w <= 0 || fr.h <= 0) { set_last_error("%s: frame %d: %d x %d is not a frame size", what, f, fr.w, fr.h); return MARS_ERR_INVALID_TENSOR; }
+        if (fr.row_stride != 0 && fr.row_stride < (size_t)fr.w * 3) {
+            set_last_error("%s: frame %d: row_stride %zu < w * 3 = %zu", what, f, fr.row_stride, (size_t)fr.w * 3);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        const LetterboxGeom q = letterbox_geom(fr.w, fr.h, tw, th);
+        if (q.nw <= 0 || q.nh <= 0 || q.nw > tw || q.nh > th) {
+            set_last_error("%s: frame %d: cannot letterbox %dx%d into %dx%d", what, f, fr.w, fr.h, tw, th);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (device) {
+            cudaPointerAttributes at;
+            if (cudaPointerGetAttributes(&at, fr.rgb) != cudaSuccess ||
+                (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != m->device) {
+                cudaGetLastError();
+                set_last_error("%s: frame %d: rgb is not device memory of device %d", what, f, m->device);
+                return MARS_ERR_INVALID_FILE;
+            }
+        }
+        (*g)[f] = q;
+    }
+    return MARS_OK;
+}
+
+static const ResizeTaps &cached_taps(Model *m, int in, int out) {
+    const auto key = std::make_pair(in, out);
+    auto it = m->pre_taps.find(key);
+    if (it != m->pre_taps.end()) return it->second;
+    ResizeTaps &t = m->pre_taps[key];
+    build_resize_taps(in, out, &t);
+    return t;
+}
+
+/* a device buffer of at least `need` bytes; growing waits for the compute stream, whose launches may still read the old one */
+static bool pre_grow(Model *m, uint8_t **p, size_t *cap, size_t need) {
+    if (need <= *cap) return true;
+    cudaStreamSynchronize(m->stream);
+    cudaFree(*p);
+    *p = nullptr; *cap = 0;
+    if (cudaMalloc(p, need) != cudaSuccess) { *p = nullptr; return false; }
+    *cap = need;
+    return true;
+}
+
+/* host frames [f0, f1) of a table -> their staging offsets, rows ow * 3 apart.  Frames of one size with tight rows that sit
+ * equally spaced in host memory (mars_b200_preprocess_batch) go in one copy. */
+static cudaError_t pre_stage_frames(const PreTable &t, const mars_b200_frame_t *frames, int f0, int f1, uint8_t *d_stage, cudaStream_t s) {
+    for (int f = f0; f < f1;) {
+        const mars_b200_frame_t &a = frames[f];
+        const size_t row = (size_t)a.w * 3, pitch = a.row_stride ? a.row_stride : row, bytes = row * a.h;
+        int e = f + 1;
+        ptrdiff_t gap = 0;
+        if (pitch == row && e < f1) {
+            gap = frames[e].rgb - a.rgb;
+            while (e < f1 && gap >= (ptrdiff_t)bytes && frames[e].w == a.w && frames[e].h == a.h &&
+                   (frames[e].row_stride == 0 || frames[e].row_stride == row) && frames[e].rgb - a.rgb == gap * (e - f) &&
+                   t.stage[e] == t.stage[f] + bytes * (e - f))
+                e++;
+        }
+        const cudaError_t ce = e > f + 1 ? cudaMemcpy2DAsync(d_stage + t.stage[f], bytes, a.rgb, (size_t)gap, bytes, (size_t)(e - f), cudaMemcpyHostToDevice, s)
+                                         : cudaMemcpy2DAsync(d_stage + t.stage[f], row, a.rgb, pitch, row, (size_t)a.h, cudaMemcpyHostToDevice, s);
+        if (ce != cudaSuccess) return ce;
+        f = e;
+    }
+    return cudaSuccess;
+}
+
+/* Letterboxes n validated frames (geometry g) into input tensor ti of slots [first, first+n) and records each slot's frame
+ * size for the letterbox inverse; the launches go on the compute stream.
+ *   PRE_HOST_SYNC : host frames staged launch by launch on the compute stream (the caller synchronises);
+ *   PRE_DEVICE    : device frames read in place;
+ *   PRE_HOST_POOL : host frames and the table copied on the copy stream, then ev_in, which the compute stream waits for. */
+static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, const mars_b200_frame_t *frames,
+                                      const std::vector<LetterboxGeom> &g, uint32_t ti, int nhwc, PreSource how, cudaEvent_t ev_in) {
+    const int n = (int)g.size();
+    if (n == 0) return MARS_OK;
+    if (m->pre_taps.size() > 64) m->pre_taps.clear();
+    PreTable t;
+    pre_table_build(g.data(), n, [m](int in, int out) -> const ResizeTaps & { return cached_taps(m, in, out); }, how == PRE_HOST_SYNC, &t);
+    const size_t tab = t.bytes();
+    if ((how != PRE_DEVICE && !pre_grow(m, &st.d_frames, &st.frames_cap, t.stage_bytes)) || !pre_grow(m, &st.d_tab, &st.tab_cap, tab) ||
+        !pre_grow(m, (uint8_t **)&m->d_preH, &m->preH_cap, t.h_floats * sizeof(float))) {
+        set_last_error("preprocess: out of device memory for %d frames", n);
+        return MARS_ERR_ALLOC_FAILED;
+    }
+    for (int f = 0; f < n; f++) {
+        PreFrame &d = t.fr[f];
+        d.src = how == PRE_DEVICE ? frames[f].rgb : st.d_frames + t.stage[f];
+        d.row_stride = how == PRE_DEVICE && frames[f].row_stride ? frames[f].row_stride : (size_t)d.ow * 3;
+    }
+    /* the pinned table is rewritten only once the last upload from it has completed */
+    CU_OK(cudaEventSynchronize(st.ev), MARS_ERR_LAYER_FAILED);
+    if (tab > st.h_cap) {
+        if (st.h_tab) cudaFreeHost(st.h_tab);
+        st.h_tab = nullptr; st.h_cap = 0;
+        CU_OK(cudaHostAlloc((void **)&st.h_tab, tab, cudaHostAllocDefault), MARS_ERR_ALLOC_FAILED);
+        st.h_cap = tab;
+    }
+    t.pack(st.h_tab);
+    cudaStream_t cs = how == PRE_HOST_POOL ? m->h2d_stream : m->stream;
+    CU_OK(cudaMemcpyAsync(st.d_tab, st.h_tab, tab, cudaMemcpyHostToDevice, cs), MARS_ERR_LAYER_FAILED);
+    CU_OK(cudaEventRecord(st.ev, cs), MARS_ERR_LAYER_FAILED);
+    if (how == PRE_HOST_POOL) {
+        CU_OK(pre_stage_frames(t, frames, 0, n, st.d_frames, cs), MARS_ERR_LAYER_FAILED);
+        cudaEventRecord(ev_in, cs);
+        cudaStreamWaitEvent(m->stream, ev_in, 0);
+    }
+    int8_t *dst = reinterpret_cast<int8_t *>(dev_addr(m, m->toff[ti], first));
+    for (size_t k = 0; k + 1 < t.first.size(); k++) {
+        if (how == PRE_HOST_SYNC) CU_OK(pre_stage_frames(t, frames, t.first[k], t.first[k + 1], st.d_frames, m->stream), MARS_ERR_LAYER_FAILED);
+        CU_OK(launch_letterbox(t, (int)k, st.d_tab, m->d_preH, dst, m->slot_stride, nhwc, m->d_frame + first, m->stream), MARS_ERR_LAYER_FAILED);
+        m->launches += 2;
+    }
+    return MARS_OK;
+}
+
+/* the synchronous calls: validation, then copies + kernels as one device-timed region */
+static mars_error_t preprocess_sync(Model *m, const char *what, int first, int n, const mars_b200_frame_t *frames) {
+    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
+    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
+    uint32_t ti;
+    int tw, th, nhwc;
+    mars_error_t e = pre_target(m, what, &ti, &tw, &th, &nhwc);
+    std::vector<LetterboxGeom> g;
+    if (e == MARS_OK) e = pre_check_frames(m, what, n, frames, tw, th, false, &g);
+    if (e != MARS_OK) return e;
+    cudaEventRecord(m->ev0, m->stream);
+    e = enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, frames, g, ti, nhwc, PRE_HOST_SYNC, nullptr);
+    cudaEventRecord(m->ev1, m->stream);
+    const cudaError_t ce = cudaStreamSynchronize(m->stream);
+    if (e == MARS_OK && ce != cudaSuccess) {
+        set_last_error("%s: %s", what, cudaGetErrorString(ce));
+        e = MARS_ERR_LAYER_FAILED;
+    }
+    if (e == MARS_OK) cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1);
+    return e;
+}
+
 /* Pre-processing in front of mars_run, as the reference's caller does it on the CPU (src/mars/mars_yolo_test.c:40-77 and
  * :157-165): n RGB8 frames of w x h pixels (host memory, frame_stride bytes apart, >= w*h*3) are letterboxed into input
  * tensor 0 of slots [first, first+n) -- stbir_resize_uint8 semantics, gray border -17, px - 128, NCHW or NHWC as the
- * tensor's format field says.  Synchronous like mars_b200_upload_inputs. */
+ * tensor's format field says.  Synchronous like mars_b200_upload_inputs.  A table of identical frames on the ragged path. */
 mars_error_t mars_b200_preprocess_batch(mars_model_t *model, int first, int n, const uint8_t *frames, size_t frame_stride, int w, int h) {
     Model *m = as_model(model);
     if (!m || !frames) return MARS_ERR_INVALID_FILE;
+    if (w <= 0 || h <= 0) { set_last_error("preprocess: %d x %d is not a frame size", w, h); return MARS_ERR_INVALID_TENSOR; }
+    const size_t frame_bytes = (size_t)(w > 0 ? w : 0) * (h > 0 ? h : 0) * 3;
+    if (frame_stride < frame_bytes) frame_stride = frame_bytes;
+    std::vector<mars_b200_frame_t> fr((size_t)(n > 0 ? n : 0));
+    for (int f = 0; f < n; f++) fr[f] = mars_b200_frame_t{frames + (size_t)f * frame_stride, w, h, 0};
+    return preprocess_sync(m, "preprocess", first, n, fr.data());
+}
+
+mars_error_t mars_b200_preprocess_frames(mars_model_t *model, int first, int n, const mars_b200_frame_t *frames) {
+    Model *m = as_model(model);
+    if (!m) return MARS_ERR_INVALID_FILE;
+    return preprocess_sync(m, "preprocess_frames", first, n, frames);
+}
+
+mars_error_t mars_b200_preprocess_frames_device(mars_model_t *model, int first, int n, const mars_b200_frame_t *frames) {
+    Model *m = as_model(model);
+    if (!m) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    if (m->pub.header.num_inputs < 1) return MARS_ERR_INVALID_TENSOR;
-    const uint32_t ti = m->pub.header.input_tensor_ids[0];
-    if (ti >= m->pub.header.num_tensors || m->toff[ti] < m->weights_size) return MARS_ERR_INVALID_TENSOR;
-    const mars_tensor_t &d = m->pub.tensors[ti].desc;
-    if (d.dtype != MARS_DTYPE_INT8 || d.ndims < 4 || w <= 0 || h <= 0) {
-        set_last_error("preprocess: input 0 must be a 4-d int8 tensor (reference src/mars/mars_yolo_test.c:157-159)");
-        return MARS_ERR_INVALID_TENSOR;
-    }
-    const int nhwc = d.format == MARS_FORMAT_NHWC;
-    const int th = nhwc ? d.shape[1] : d.shape[2], tw = nhwc ? d.shape[2] : d.shape[3];
-    if (th <= 0 || tw <= 0 || (size_t)tw * th * 3 > m->buffer_size) return MARS_ERR_INVALID_TENSOR;
-    const size_t frame_bytes = (size_t)w * h * 3;
-    if (frame_stride < frame_bytes) frame_stride = frame_bytes;
-    if (!letterbox_plan_build(w, h, tw, th, &m->pre_plan)) {
-        set_last_error("preprocess: cannot letterbox %dx%d into %dx%d", w, h, tw, th);
-        return MARS_ERR_INVALID_TENSOR;
-    }
-    const size_t h_per = (size_t)h * m->pre_plan.g.nw * 3 * sizeof(float);
-    int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n, ((size_t)256 << 20) / std::max<size_t>(h_per, 1)));
-    if ((size_t)chunk * frame_bytes > m->frames_cap) {
-        cudaFree(m->d_frames);
-        m->d_frames = nullptr; m->frames_cap = 0;
-        CU_OK(cudaMalloc(&m->d_frames, (size_t)chunk * frame_bytes), MARS_ERR_ALLOC_FAILED);
-        m->frames_cap = (size_t)chunk * frame_bytes;
-    }
-    if ((size_t)chunk * h_per > m->preH_cap) {
-        cudaFree(m->d_preH);
-        m->d_preH = nullptr; m->preH_cap = 0;
-        CU_OK(cudaMalloc(&m->d_preH, (size_t)chunk * h_per), MARS_ERR_ALLOC_FAILED);
-        m->preH_cap = (size_t)chunk * h_per;
-    }
-    cudaEventRecord(m->ev0, m->stream);
-    for (int done = 0; done < n; done += chunk) {
-        const int c = std::min(chunk, n - done);
-        CU_OK(cudaMemcpy2DAsync(m->d_frames, frame_bytes, frames + (size_t)done * frame_stride, frame_stride, frame_bytes, (size_t)c,
-                                cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
-        CU_OK(launch_letterbox(m->pre_plan, m->d_frames, frame_bytes, c, m->d_preH,
-                               reinterpret_cast<int8_t *>(dev_addr(m, m->toff[ti], first + done)), m->slot_stride, nhwc, m->stream),
-              MARS_ERR_LAYER_FAILED);
-        m->launches += 2;
-    }
-    cudaEventRecord(m->ev1, m->stream);
-    /* the frame size of every slot, for the letterbox inverse of the heads decode (mars_b200_set_frame_size) */
-    std::vector<int2> fr((size_t)n, make_int2(w, h));
-    if (n > 0) CU_OK(cudaMemcpyAsync(m->d_frame + first, fr.data(), (size_t)n * sizeof(int2), cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
-    CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
-    cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1);
-    return MARS_OK;
+    uint32_t ti;
+    int tw, th, nhwc;
+    mars_error_t e = pre_target(m, "preprocess_frames_device", &ti, &tw, &th, &nhwc);
+    std::vector<LetterboxGeom> g;
+    if (e == MARS_OK) e = pre_check_frames(m, "preprocess_frames_device", n, frames, tw, th, true, &g);
+    if (e != MARS_OK) return e;
+    return enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, frames, g, ti, nhwc, PRE_DEVICE, nullptr);
 }
 
 mars_error_t mars_b200_run_resident(mars_model_t *model, int first, int n) {
@@ -1531,9 +1685,10 @@ mars_error_t mars_b200_run_batch(mars_model_t *model, int n, const void *inputs,
  * detection records on the read-back stream -- and the call returns.  While it runs the caller submits the next batch to the
  * other half, so the host->device copy of batch k+1 and the read-back of batch k-1 overlap the kernels of batch k.
  * inputs / dets / counts must stay valid (and should be pinned, e.g. nna_malloc) until mars_b200_wait_batch(pool) returns. */
+/* frames != NULL: inputs are letterboxed from those host frames instead (mars_b200_submit_frames_heads_batch) */
 static mars_error_t submit_batch(Model *m, int pool, int n, const void *inputs, size_t in_stride, void *dets, int32_t *counts, int maxd,
-                                 float nms_thresh, int flavour) {
-    if (!m || !inputs || !dets || !counts || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
+                                 float nms_thresh, int flavour, const mars_b200_frame_t *frames = nullptr) {
+    if (!m || !(inputs || frames) || !dets || !counts || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     const int half = m->capacity / 2;
     if (half < 1 || n < 0 || n > half) {
@@ -1549,14 +1704,27 @@ static mars_error_t submit_batch(Model *m, int pool, int n, const void *inputs, 
     const size_t in_bytes = io_bytes(&m->pub, 0);
     if (in_stride < in_bytes) in_stride = in_bytes;
     const int first = pool * half;
+    uint32_t ti = 0;
+    int tw = 0, th = 0, nhwc = 0;
+    std::vector<LetterboxGeom> g;
+    if (frames) {
+        mars_error_t e = pre_target(m, "submit_frames_heads_batch", &ti, &tw, &th, &nhwc);
+        if (e == MARS_OK) e = pre_check_frames(m, "submit_frames_heads_batch", n, frames, tw, th, false, &g);
+        if (e != MARS_OK) return e;
+    }
     mars_error_t e = compile_model(m); /* also drops captured graphs of an older program (set_opt_level, set_depthwise_mode) */
     if (e != MARS_OK) return e;
     if (n > 0) {
-        /* the half is free: its previous batch was waited for (read-back complete) before this call */
-        e = copy_io(m, first, n, const_cast<void *>(inputs), in_stride, 0, m->h2d_stream);
-        if (e != MARS_OK) return e;
-        cudaEventRecord(m->ev_in[pool], m->h2d_stream);
-        cudaStreamWaitEvent(m->stream, m->ev_in[pool], 0);
+        /* the half is free: its previous batch was waited for (read-back complete) before this call -- its staging too */
+        if (frames) {
+            e = enqueue_letterbox(m, m->pre_stage[pool], first, frames, g, ti, nhwc, PRE_HOST_POOL, m->ev_in[pool]);
+            if (e != MARS_OK) return e;
+        } else {
+            e = copy_io(m, first, n, const_cast<void *>(inputs), in_stride, 0, m->h2d_stream);
+            if (e != MARS_OK) return e;
+            cudaEventRecord(m->ev_in[pool], m->h2d_stream);
+            cudaStreamWaitEvent(m->stream, m->ev_in[pool], 0);
+        }
         e = enqueue_step_graphed(m, first, n, nms_thresh, flavour);
         if (e != MARS_OK) { cudaStreamSynchronize(m->stream); return e; }
         cudaEventRecord(m->ev_done[pool], m->stream);
@@ -1580,6 +1748,16 @@ mars_error_t mars_b200_submit_heads_batch(mars_model_t *model, int pool, int n, 
     Model *m = as_model(model);
     if (m && m->heads.empty()) { set_last_error("submit_heads_batch: no YOLO heads configured (mars_b200_set_yolo_heads)"); return MARS_ERR_INVALID_TENSOR; }
     return submit_batch(m, pool, n, inputs, in_stride, boxes, counts, maxd, nms_thresh, STEP_HEADS);
+}
+
+/* mars_b200_submit_heads_batch from RGB8 frames of any sizes and row pitches (host memory): H2D of each frame on the copy
+ * stream, the letterbox launches on the compute stream in front of the (graphed) step, frame coordinates for every slot */
+mars_error_t mars_b200_submit_frames_heads_batch(mars_model_t *model, int pool, int n, const mars_b200_frame_t *frames, mars_box_t *boxes,
+                                                 int32_t *counts, int maxd, float nms_thresh) {
+    Model *m = as_model(model);
+    if (m && m->heads.empty()) { set_last_error("submit_frames_heads_batch: no YOLO heads configured (mars_b200_set_yolo_heads)"); return MARS_ERR_INVALID_TENSOR; }
+    if (m && !frames) { set_last_error("submit_frames_heads_batch: no frame table"); return MARS_ERR_INVALID_FILE; }
+    return submit_batch(m, pool, n, nullptr, 0, boxes, counts, maxd, nms_thresh, STEP_HEADS, frames);
 }
 
 /* mars_b200_submit_batch without the YOLO post-process: the raw output tensor 0 of every image is read back instead
