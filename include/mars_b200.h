@@ -89,6 +89,26 @@ mars_error_t mars_b200_preprocess_frames(mars_model_t *m, int first, int n, cons
  * mars_b200_compute_stream(m) and returns.  The frames must be complete before that stream reaches the launches and stay
  * valid until it has passed them; the table itself may be reused as soon as the call returns. */
 mars_error_t mars_b200_preprocess_frames_device(mars_model_t *m, int first, int n, const mars_b200_frame_t *frames);
+/* YUV -> RGB conversion of an NV12 frame (16.16 fixed point, no chroma interpolation: the U,V pair of a 2 x 2 block serves
+ * all four pixels; mars_b200_yuv_coefficients), chosen per frame */
+enum { MARS_B200_YUV_BT601_LIMITED = 0, MARS_B200_YUV_BT709_LIMITED = 1, MARS_B200_YUV_BT601_FULL = 2, MARS_B200_YUV_BT709_FULL = 3 };
+/* one NV12 frame (a hardware video decoder's or a camera ISP's output): h rows of w luma bytes (y_stride apart, 0 = w), then
+ * ceil(h/2) rows of ceil(w/2) interleaved U,V pairs (uv_stride apart, 0 = 2 * ceil(w/2)); the planes may sit in one allocation
+ * (e.g. uv = y + pitch * aligned height) or two.  colour = MARS_B200_YUV_* */
+typedef struct { const uint8_t *y, *uv; int32_t w, h; size_t y_stride, uv_stride; int32_t colour; } mars_b200_nv12_frame_t;
+/* mars_b200_preprocess_frames from NV12 frames: each slot's tensor is byte-identical to that of the RGB8 frame the conversion
+ * gives, letterboxed by mars_b200_preprocess_frames.  The conversion happens where the resize reads each source pixel; no RGB
+ * copy is made.  Every frame is checked first -- y and uv not NULL, w, h > 0, y_stride 0 or >= w, uv_stride 0 or
+ * >= 2 * ceil(w/2), colour a MARS_B200_YUV_* value, a letterbox at least one pixel wide and tall -- and a rejected call writes
+ * no slot; mars_b200_last_error names the frame.  Host memory, synchronous; records each slot's frame size. */
+mars_error_t mars_b200_preprocess_frames_nv12(mars_model_t *m, int first, int n, const mars_b200_nv12_frame_t *frames);
+/* the same with both planes in device memory of the model's device (e.g. an NVDEC surface), read in place: enqueued on
+ * mars_b200_compute_stream(m), as mars_b200_preprocess_frames_device */
+mars_error_t mars_b200_preprocess_frames_nv12_device(mars_model_t *m, int first, int n, const mars_b200_nv12_frame_t *frames);
+/* host half, no GPU needed: out[6] = y0, cy, crv, cgu, cgv, cbu of a colour variant, with R = clamp((cy (Y - y0) + crv (V - 128)
+ * + 32768) >> 16), G = clamp((cy (Y - y0) - cgu (U - 128) - cgv (V - 128) + 32768) >> 16), B = clamp((cy (Y - y0) + cbu (U - 128)
+ * + 32768) >> 16).  Returns 0, or -1 for an unknown variant. */
+int mars_b200_yuv_coefficients(int colour, int32_t *out);
 /* slots -> host: output tensor 0 of n images */
 mars_error_t mars_b200_download_outputs(mars_model_t *m, int first, int n, void *host, size_t stride);
 /* run all layers for slots [first, first+n) with inputs already resident in HBM */
@@ -156,6 +176,10 @@ mars_error_t mars_b200_submit_heads_batch(mars_model_t *m, int pool, int n, cons
  * for the device once. */
 mars_error_t mars_b200_submit_frames_heads_batch(mars_model_t *m, int pool, int n, const mars_b200_frame_t *frames,
                                                  mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh);
+/* the same from n host NV12 frames (mars_b200_preprocess_frames_nv12): both planes of each frame are uploaded on the copy
+ * stream -- half the bytes of the RGB8 frame -- and converted inside the letterbox */
+mars_error_t mars_b200_submit_frames_nv12_heads_batch(mars_model_t *m, int pool, int n, const mars_b200_nv12_frame_t *frames,
+                                                      mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh);
 /* kept boxes of slots [first, first+n): boxes[n][maxd] (maxd <= 1000), counts[n] */
 mars_error_t mars_b200_download_boxes(mars_model_t *m, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd);
 

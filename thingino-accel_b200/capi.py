@@ -78,6 +78,18 @@ class FRAME(C.Structure):
     """mars_b200_frame_t: one RGB8 frame, rows row_stride bytes apart (0 = w * 3)"""
     _fields_ = [("rgb", C.c_void_p), ("w", C.c_int32), ("h", C.c_int32), ("row_stride", C.c_size_t)]
 
+
+# colour variants of an NV12 frame (MARS_B200_YUV_*)
+YUV_BT601_LIMITED, YUV_BT709_LIMITED, YUV_BT601_FULL, YUV_BT709_FULL = 0, 1, 2, 3
+
+
+class NV12_FRAME(C.Structure):
+    """mars_b200_nv12_frame_t: luma rows y_stride bytes apart (0 = w), ceil(h/2) rows of ceil(w/2) U,V pairs uv_stride bytes
+    apart (0 = 2 * ceil(w/2)), colour = YUV_*"""
+    _fields_ = [("y", C.c_void_p), ("uv", C.c_void_p), ("w", C.c_int32), ("h", C.c_int32), ("y_stride", C.c_size_t),
+                ("uv_stride", C.c_size_t), ("colour", C.c_int32)]
+
+
 # every symbol include/*.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     # include/mars_runtime.h
@@ -211,6 +223,11 @@ SIGNATURES = {
     "mars_b200_preprocess_frames_device": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(FRAME)]),
     "mars_b200_submit_frames_heads_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(FRAME), C.c_void_p, C.c_void_p, C.c_int,
                                                       C.c_float]),
+    "mars_b200_preprocess_frames_nv12": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME)]),
+    "mars_b200_preprocess_frames_nv12_device": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME)]),
+    "mars_b200_submit_frames_nv12_heads_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME), C.c_void_p, C.c_void_p,
+                                                           C.c_int, C.c_float]),
+    "mars_b200_yuv_coefficients": (C.c_int, [C.c_int, C.c_void_p]),
 }
 
 _lib = None
@@ -265,6 +282,33 @@ def device_frames(frames):
     table = (FRAME * len(frames))()
     for i, (p, w, h, stride) in enumerate(frames):
         table[i] = FRAME(p, w, h, stride)
+    return table
+
+
+def host_nv12_frames(frames):
+    """[(y, uv, colour), ...] with y a [h, w] uint8 array and uv a [ceil(h/2), ceil(w/2), 2] uint8 array -> (NV12_FRAME table,
+    the arrays it points into).  Views whose rows are further apart than their width (strides (pitch, 1) and (pitch, 2, 1))
+    pass their pitches; any other layout is copied first."""
+    table = (NV12_FRAME * len(frames))()
+    keep = []
+    for i, (y, uv, colour) in enumerate(frames):
+        y, uv = np.asarray(y), np.asarray(uv)
+        h, w = y.shape
+        assert y.dtype == np.uint8 and uv.dtype == np.uint8 and uv.shape == ((h + 1) // 2, (w + 1) // 2, 2), (y.shape, uv.shape)
+        if not (y.strides[1] == 1 and y.strides[0] >= w):
+            y = np.ascontiguousarray(y)
+        if not (uv.strides[1:] == (2, 1) and uv.strides[0] >= uv.shape[1] * 2):
+            uv = np.ascontiguousarray(uv)
+        keep += [y, uv]
+        table[i] = NV12_FRAME(y.ctypes.data, uv.ctypes.data, w, h, y.strides[0], uv.strides[0], colour)
+    return table, keep
+
+
+def device_nv12_frames(frames):
+    """[(y_ptr, uv_ptr, w, h, y_stride, uv_stride, colour), ...] of NV12 frames in device memory -> NV12_FRAME table"""
+    table = (NV12_FRAME * len(frames))()
+    for i, f in enumerate(frames):
+        table[i] = NV12_FRAME(*f)
     return table
 
 
@@ -408,6 +452,18 @@ class MarsModel:
         self._check(lib().mars_b200_preprocess_frames_device(self.m, first, len(frames), device_frames(frames)),
                     "preprocess_frames_device")
 
+    def preprocess_frames_nv12(self, first, frames):
+        """frames: list of (y, uv, colour) NV12 host frames of any sizes (host_nv12_frames) -> letterboxed into input tensor 0 of
+        slots [first, first+len(frames)) in one pass; returns the GPU milliseconds of the copies + kernels"""
+        table, _keep = host_nv12_frames(frames)
+        self._check(lib().mars_b200_preprocess_frames_nv12(self.m, first, len(frames), table), "preprocess_frames_nv12")
+        return float(lib().mars_b200_last_gpu_ms(self.m))
+
+    def preprocess_frames_nv12_device(self, first, frames):
+        """frames: [(y_ptr, uv_ptr, w, h, y_stride, uv_stride, colour), ...] in device memory; enqueued on compute_stream()"""
+        self._check(lib().mars_b200_preprocess_frames_nv12_device(self.m, first, len(frames), device_nv12_frames(frames)),
+                    "preprocess_frames_nv12_device")
+
     def download_outputs(self, first, n, host=None, stride=0):
         if host is None:
             host = np.zeros((n, self.out_bytes), dtype=np.uint8)
@@ -492,6 +548,14 @@ class MarsModel:
         table, keep = host_frames(frames)
         self._check(lib().mars_b200_submit_frames_heads_batch(self.m, pool, len(frames), table, _addr(boxes), _addr(counts), maxd, thresh),
                     "submit_frames_heads_batch")
+        self._inflight[pool] = (table, keep)
+
+    def submit_frames_nv12_heads_batch(self, pool, frames, boxes, counts, maxd=1000, thresh=0.45):
+        """submit_frames_heads_batch from a list of (y, uv, colour) NV12 host frames (host_nv12_frames).  The frames are kept
+        alive until wait_batch(pool); boxes and counts must be kept alive by the caller"""
+        table, keep = host_nv12_frames(frames)
+        self._check(lib().mars_b200_submit_frames_nv12_heads_batch(self.m, pool, len(frames), table, _addr(boxes), _addr(counts), maxd,
+                                                                   thresh), "submit_frames_nv12_heads_batch")
         self._inflight[pool] = (table, keep)
 
     def download_boxes(self, first, n, maxd=1000):
@@ -583,6 +647,14 @@ def resize_taps(in_size, out_size):
         if n <= cap:
             return start, src[:n].copy(), w[:n].copy()
         cap = n
+
+
+def yuv_coefficients(colour):
+    """host half of the NV12 conversion (no GPU): [y0, cy, crv, cgu, cgv, cbu] of a colour variant (YUV_*)"""
+    out = np.zeros(6, dtype=np.int32)
+    if lib().mars_b200_yuv_coefficients(colour, out.ctypes.data) != 0:
+        raise ValueError("yuv_coefficients(%d)" % colour)
+    return out
 
 
 def find_yolo_heads(blob):

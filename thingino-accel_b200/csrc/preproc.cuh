@@ -15,6 +15,9 @@
  *                           out = (int8)(u8 - 128), border -17  -- or RGBA u8, border 114 (stb :1692-1760, :1866-2061)
  * Every frame of a launch has its own size, row pitch and tap lists (a table of PreFrame descriptors); the target size is
  * shared.  A uniform batch is a table of identical descriptors.
+ *
+ * A frame is RGB8 or NV12.  An NV12 frame is converted to RGB8 where k_pre_horizontal reads its source bytes (pre_nv12_rgb),
+ * so it letterboxes to exactly the slot tensor of the RGB8 frame that conversion produces; no RGB copy is written.
  */
 #pragma once
 #include <cuda_runtime.h>
@@ -184,16 +187,52 @@ static inline LetterboxGeom letterbox_geom(int ow, int oh, int tw, int th) {
     return g;
 }
 
+/* source formats of a frame */
+enum { PRE_RGB8 = 0, PRE_NV12 = 1 };
+
+/* NV12 -> RGB8 in 16.16 fixed point, per colour variant (mars_b200.h MARS_B200_YUV_*): y0, cy, crv, cgu, cgv, cbu.  With
+ * Kg = 1 - Kr - Kb, each constant is floor(c * 65536 + 0.5) in double of cy = ys, crv = cs 2 (1 - Kr), cgu = cs 2 Kb (1 - Kb) / Kg,
+ * cgv = cs 2 Kr (1 - Kr) / Kg, cbu = cs 2 (1 - Kb); limited range ys = 255/219, cs = 255/224, y0 = 16; full range ys = cs = 1,
+ * y0 = 0.  BT.601 (Kr, Kb) = (0.299, 0.114), BT.709 (0.2126, 0.0722).  Every channel is within 0.5 + 2^-8 of the clamped
+ * exact matrix over all 2^24 (Y, U, V), and |accumulator| < 2^26. */
+#define PRE_YUV_COEF_INIT                                  \
+    {                                                      \
+        {16, 76309, 104597, 25675, 53279, 132201},  /* BT.601 limited */ \
+        {16, 76309, 117489, 13975, 34925, 138438},  /* BT.709 limited */ \
+        {0, 65536, 91881, 22553, 46802, 116130},    /* BT.601 full */    \
+        {0, 65536, 103206, 12276, 30679, 121609},   /* BT.709 full */    \
+    }
+enum { PRE_YUV_VARIANTS = 4 };
+static const int32_t PRE_YUV_COEF[PRE_YUV_VARIANTS][6] = PRE_YUV_COEF_INIT;
+static __constant__ int32_t pre_yuv_coef[PRE_YUV_VARIANTS][6] = PRE_YUV_COEF_INIT;
+
 /* One frame of a ragged batch as the kernels see it.  A launch covers a run of frames that share the target size; each has
- * its own source geometry, row pitch, tap lists and float rows.  Offsets are relative to the launch (chunk). */
+ * its own source format, geometry, row pitches, tap lists and float rows.  Offsets are relative to the launch (chunk). */
 struct PreFrame {
-    const uint8_t *src;  /* row 0 of the RGB8 frame (device) */
-    size_t row_stride;   /* bytes from one row to the next (>= ow * 3) */
+    const uint8_t *src;  /* row 0 of the RGB8 frame, or of the NV12 luma plane (device) */
+    const uint8_t *uv;   /* NV12: row 0 of the chroma plane, ceil(oh / 2) rows of ceil(ow / 2) U,V pairs (device) */
+    size_t row_stride;   /* bytes from one row of src to the next (>= ow * 3 for RGB8, >= ow for NV12) */
+    size_t uv_stride;    /* NV12: bytes from one chroma row to the next (>= 2 * ceil(ow / 2)) */
     size_t hoff;         /* its first float in the H scratch: oh x nw x 3 floats */
     int ow, oh, nw, nh, px, py;
     int hs, vs;          /* its first entry in the start list of the horizontal / vertical taps */
     int blk0;            /* its first block in the horizontal grid: blocks [blk0, blk0 + oh * ceil(nw / 128)) */
+    int fmt, colour;     /* PRE_RGB8 / PRE_NV12; the NV12 colour variant (row of pre_yuv_coef) */
 };
+
+/* bytes of a frame staged tightly on the device: RGB8 rows ow * 3 apart; NV12 the luma plane (rows ow apart), then the
+ * chroma plane (rows 2 * ceil(ow / 2) apart) */
+static inline size_t pre_frame_bytes(int fmt, int ow, int oh) {
+    return fmt == PRE_NV12 ? (size_t)ow * oh + (size_t)2 * ((ow + 1) / 2) * ((oh + 1) / 2) : (size_t)ow * oh * 3;
+}
+
+/* one NV12 sample -> R, G, B bytes; k = the variant's row of pre_yuv_coef.  Arithmetic shifts (floor), clamp to [0, 255]. */
+__device__ __forceinline__ void pre_nv12_rgb(int Y, int U, int V, int y0, int cy, int crv, int cgu, int cgv, int cbu, int *r, int *g, int *b) {
+    const int yy = cy * (Y - y0) + 32768, u = U - 128, v = V - 128;
+    *r = min(max((yy + crv * v) >> 16, 0), 255);
+    *g = min(max((yy - cgu * u - cgv * v) >> 16, 0), 255);
+    *b = min(max((yy + cbu * u) >> 16, 0), 255);
+}
 /* the concatenated tap lists of a batch: taps of output o of a list beginning at s are [start[s + o], start[s + o + 1]),
  * indices straight into src / w */
 struct PreTaps {
@@ -202,7 +241,9 @@ struct PreTaps {
 };
 
 /* one thread per resized column of one source row.  The blocks of every frame follow each other (no grid sized to the
- * largest frame); a block finds its frame by a binary search over the first blocks.  H[r][x][c] = sum_t (u8 / 255) * w[t] */
+ * largest frame); a block finds its frame by a binary search over the first blocks.  H[r][x][c] = sum_t (u8 / 255) * w[t],
+ * u8 read from the RGB8 frame or converted from the NV12 frame's luma byte and U,V pair at each tap (the branch is
+ * uniform over the block: a block belongs to one frame). */
 __global__ void __launch_bounds__(128) k_pre_horizontal(const PreFrame *fr, int n, PreTaps t, float *H) {
     __shared__ float dec[256]; /* the decode step: (float)u8 / 255.0f, IEEE division */
     dec[threadIdx.x] = __fdiv_rn((float)threadIdx.x, 255.0f);
@@ -220,12 +261,29 @@ __global__ void __launch_bounds__(128) k_pre_horizontal(const PreFrame *fr, int 
     if (x >= nw) return;
     const uint8_t *row = d.src + (size_t)r * d.row_stride;
     float a0 = 0.0f, a1 = 0.0f, a2 = 0.0f;
-    for (int k = t.start[d.hs + x], ke = t.start[d.hs + x + 1]; k < ke; k++) {
-        const uint8_t *p = row + (size_t)t.src[k] * 3;
-        const float c = t.w[k];
-        a0 = __fadd_rn(a0, __fmul_rn(dec[p[0]], c));
-        a1 = __fadd_rn(a1, __fmul_rn(dec[p[1]], c));
-        a2 = __fadd_rn(a2, __fmul_rn(dec[p[2]], c));
+    const int k0 = t.start[d.hs + x], ke = t.start[d.hs + x + 1];
+    if (d.fmt == PRE_NV12) {
+        const uint8_t *crow = d.uv + (size_t)(r >> 1) * d.uv_stride;
+        const int *q = pre_yuv_coef[d.colour];
+        const int y0 = q[0], cy = q[1], crv = q[2], cgu = q[3], cgv = q[4], cbu = q[5];
+        for (int k = k0; k < ke; k++) {
+            const int sx = t.src[k];
+            const uint8_t *p = crow + 2 * (sx >> 1);
+            int c0, c1, c2;
+            pre_nv12_rgb(row[sx], p[0], p[1], y0, cy, crv, cgu, cgv, cbu, &c0, &c1, &c2);
+            const float c = t.w[k];
+            a0 = __fadd_rn(a0, __fmul_rn(dec[c0], c));
+            a1 = __fadd_rn(a1, __fmul_rn(dec[c1], c));
+            a2 = __fadd_rn(a2, __fmul_rn(dec[c2], c));
+        }
+    } else {
+        for (int k = k0; k < ke; k++) {
+            const uint8_t *p = row + (size_t)t.src[k] * 3;
+            const float c = t.w[k];
+            a0 = __fadd_rn(a0, __fmul_rn(dec[p[0]], c));
+            a1 = __fadd_rn(a1, __fmul_rn(dec[p[1]], c));
+            a2 = __fadd_rn(a2, __fmul_rn(dec[p[2]], c));
+        }
     }
     float *o = H + d.hoff + ((size_t)r * nw + x) * 3;
     o[0] = a0; o[1] = a1; o[2] = a2;
@@ -288,7 +346,7 @@ static const size_t PRE_H_CHUNK_BYTES = (size_t)256 << 20;
 struct PreTable {
     int tw = 0, th = 0;
     std::vector<PreFrame> fr;
-    std::vector<size_t> stage; /* byte offset of each frame in a tightly packed staging buffer (rows ow * 3 apart) */
+    std::vector<size_t> stage; /* byte offset of each frame in a tightly packed staging buffer (pre_frame_bytes each) */
     std::vector<int> start, src;
     std::vector<float> w;
     std::vector<int> first, blocks; /* launch k covers frames [first[k], first[k + 1]) with blocks[k] horizontal blocks */
@@ -310,12 +368,12 @@ struct PreTable {
     }
 };
 
-/* Builds the table for n frames (geometry g[f] from letterbox_geom, all into the same target) whose source pointers and
- * pitches the caller fills in afterwards.  taps_of(in, out) returns the ResizeTaps of one axis (the caller's cache).
- * Launches split where the cumulative H bytes (oh * nw * 12 per frame) would pass PRE_H_CHUNK_BYTES; with
- * per_launch_staging the staging offsets restart with every launch. */
+/* Builds the table for n frames (geometry g[f] from letterbox_geom, all into the same target; source format fmt[f], or all
+ * RGB8 when fmt is null) whose source pointers, pitches and colour variants the caller fills in afterwards.  taps_of(in, out)
+ * returns the ResizeTaps of one axis (the caller's cache).  Launches split where the cumulative H bytes (oh * nw * 12 per
+ * frame) would pass PRE_H_CHUNK_BYTES; with per_launch_staging the staging offsets restart with every launch. */
 template <class TapsOf>
-static inline void pre_table_build(const LetterboxGeom *g, int n, TapsOf taps_of, bool per_launch_staging, PreTable *t) {
+static inline void pre_table_build(const LetterboxGeom *g, const int *fmt, int n, TapsOf taps_of, bool per_launch_staging, PreTable *t) {
     *t = PreTable();
     if (n <= 0) return;
     t->tw = g[0].tw; t->th = g[0].th;
@@ -345,7 +403,8 @@ static inline void pre_table_build(const LetterboxGeom *g, int n, TapsOf taps_of
             if (per_launch_staging) soff = 0;
         }
         PreFrame &d = t->fr[f];
-        d.src = nullptr; d.row_stride = 0;
+        d.src = nullptr; d.uv = nullptr; d.row_stride = 0; d.uv_stride = 0;
+        d.fmt = fmt ? fmt[f] : PRE_RGB8; d.colour = 0;
         d.hoff = hfl;
         d.ow = q.ow; d.oh = q.oh; d.nw = q.nw; d.nh = q.nh; d.px = q.px; d.py = q.py;
         d.hs = list(q.ow, q.nw);
@@ -355,7 +414,7 @@ static inline void pre_table_build(const LetterboxGeom *g, int n, TapsOf taps_of
         blk += q.oh * ((q.nw + 127) / 128);
         hbytes += need;
         hfl += need / sizeof(float);
-        soff += (size_t)q.ow * q.oh * 3;
+        soff += pre_frame_bytes(d.fmt, q.ow, q.oh);
         t->h_floats = std::max(t->h_floats, hfl);
         t->stage_bytes = std::max(t->stage_bytes, soff);
     }

@@ -1243,17 +1243,62 @@ static mars_error_t pre_target(Model *m, const char *what, uint32_t *ti, int *tw
     return MARS_OK;
 }
 
-/* every frame of a call is checked before any device work, so that a rejected call writes no slot */
-static mars_error_t pre_check_frames(Model *m, const char *what, int n, const mars_b200_frame_t *frames, int tw, int th, bool device,
-                                     std::vector<LetterboxGeom> *g) {
-    if (!frames) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
-    g->resize(n > 0 ? n : 0);
+/* One frame of a call, whichever public struct it arrived in: an RGB8 frame (p0) or the luma (p0) and chroma (p1) planes of
+ * an NV12 frame, with their row pitches (0 in the public struct = tight rows, resolved here), the size, the format and the
+ * NV12 colour variant.  Validation, staging and the letterbox launches see only this. */
+struct FrameSrc {
+    const uint8_t *p0, *p1;
+    size_t pitch0, pitch1;
+    int w, h, fmt, colour;
+};
+/* the public frame tables -> *s; null when there is no table */
+static const std::vector<FrameSrc> *rgb_sources(int n, const mars_b200_frame_t *frames, std::vector<FrameSrc> *s) {
+    if (!frames) return nullptr;
+    s->resize(n > 0 ? n : 0);
     for (int f = 0; f < n; f++) {
-        const mars_b200_frame_t &fr = frames[f];
-        if (!fr.rgb) { set_last_error("%s: frame %d: rgb is NULL", what, f); return MARS_ERR_INVALID_FILE; }
+        const mars_b200_frame_t &a = frames[f];
+        (*s)[f] = FrameSrc{a.rgb, nullptr, a.row_stride ? a.row_stride : (size_t)a.w * 3, 0, a.w, a.h, PRE_RGB8, 0};
+    }
+    return s;
+}
+static const std::vector<FrameSrc> *nv12_sources(int n, const mars_b200_nv12_frame_t *frames, std::vector<FrameSrc> *s) {
+    if (!frames) return nullptr;
+    s->resize(n > 0 ? n : 0);
+    for (int f = 0; f < n; f++) {
+        const mars_b200_nv12_frame_t &a = frames[f];
+        (*s)[f] = FrameSrc{a.y, a.uv, a.y_stride ? a.y_stride : (size_t)a.w, a.uv_stride ? a.uv_stride : (size_t)2 * ((a.w + 1) / 2),
+                           a.w, a.h, PRE_NV12, a.colour};
+    }
+    return s;
+}
+
+/* every frame of a call is checked before any device work, so that a rejected call writes no slot */
+static mars_error_t pre_check_frames(Model *m, const char *what, const std::vector<FrameSrc> *table, int tw, int th, bool device,
+                                     std::vector<LetterboxGeom> *g) {
+    if (!table) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
+    const std::vector<FrameSrc> &frames = *table;
+    const int n = (int)frames.size();
+    g->resize(n);
+    for (int f = 0; f < n; f++) {
+        const FrameSrc &fr = frames[f];
+        const bool nv12 = fr.fmt == PRE_NV12;
+        const char *plane[2] = {nv12 ? "y" : "rgb", "uv"};
+        const uint8_t *ptr[2] = {fr.p0, fr.p1};
+        const int planes = nv12 ? 2 : 1;
+        for (int p = 0; p < planes; p++)
+            if (!ptr[p]) { set_last_error("%s: frame %d: %s is NULL", what, f, plane[p]); return MARS_ERR_INVALID_FILE; }
         if (fr.w <= 0 || fr.h <= 0) { set_last_error("%s: frame %d: %d x %d is not a frame size", what, f, fr.w, fr.h); return MARS_ERR_INVALID_TENSOR; }
-        if (fr.row_stride != 0 && fr.row_stride < (size_t)fr.w * 3) {
-            set_last_error("%s: frame %d: row_stride %zu < w * 3 = %zu", what, f, fr.row_stride, (size_t)fr.w * 3);
+        const size_t row0 = (size_t)fr.w * (nv12 ? 1 : 3), row1 = (size_t)2 * ((fr.w + 1) / 2);
+        if (fr.pitch0 < row0) {
+            set_last_error("%s: frame %d: %s %zu < %s = %zu", what, f, nv12 ? "y_stride" : "row_stride", fr.pitch0, nv12 ? "w" : "w * 3", row0);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (nv12 && fr.pitch1 < row1) {
+            set_last_error("%s: frame %d: uv_stride %zu < 2 * ceil(w / 2) = %zu", what, f, fr.pitch1, row1);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (nv12 && (fr.colour < 0 || fr.colour >= PRE_YUV_VARIANTS)) {
+            set_last_error("%s: frame %d: colour %d is not a MARS_B200_YUV_* variant", what, f, fr.colour);
             return MARS_ERR_INVALID_TENSOR;
         }
         const LetterboxGeom q = letterbox_geom(fr.w, fr.h, tw, th);
@@ -1261,12 +1306,12 @@ static mars_error_t pre_check_frames(Model *m, const char *what, int n, const ma
             set_last_error("%s: frame %d: cannot letterbox %dx%d into %dx%d", what, f, fr.w, fr.h, tw, th);
             return MARS_ERR_INVALID_TENSOR;
         }
-        if (device) {
+        for (int p = 0; device && p < planes; p++) {
             cudaPointerAttributes at;
-            if (cudaPointerGetAttributes(&at, fr.rgb) != cudaSuccess ||
+            if (cudaPointerGetAttributes(&at, ptr[p]) != cudaSuccess ||
                 (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != m->device) {
                 cudaGetLastError();
-                set_last_error("%s: frame %d: rgb is not device memory of device %d", what, f, m->device);
+                set_last_error("%s: frame %d: %s is not device memory of device %d", what, f, plane[p], m->device);
                 return MARS_ERR_INVALID_FILE;
             }
         }
@@ -1295,23 +1340,33 @@ static bool pre_grow(Model *m, uint8_t **p, size_t *cap, size_t need) {
     return true;
 }
 
-/* host frames [f0, f1) of a table -> their staging offsets, rows ow * 3 apart.  Frames of one size with tight rows that sit
- * equally spaced in host memory (mars_b200_preprocess_batch) go in one copy. */
-static cudaError_t pre_stage_frames(const PreTable &t, const mars_b200_frame_t *frames, int f0, int f1, uint8_t *d_stage, cudaStream_t s) {
+/* host frames [f0, f1) of a table -> their staging offsets, tight rows (pre_frame_bytes): one copy per RGB8 frame, one per NV12
+ * plane.  RGB8 frames of one size with tight rows that sit equally spaced in host memory (mars_b200_preprocess_batch) go in
+ * one copy. */
+static cudaError_t pre_stage_frames(const PreTable &t, const FrameSrc *frames, int f0, int f1, uint8_t *d_stage, cudaStream_t s) {
     for (int f = f0; f < f1;) {
-        const mars_b200_frame_t &a = frames[f];
-        const size_t row = (size_t)a.w * 3, pitch = a.row_stride ? a.row_stride : row, bytes = row * a.h;
+        const FrameSrc &a = frames[f];
+        if (a.fmt == PRE_NV12) {
+            const size_t row1 = (size_t)2 * ((a.w + 1) / 2);
+            cudaError_t ce = cudaMemcpy2DAsync(d_stage + t.stage[f], (size_t)a.w, a.p0, a.pitch0, (size_t)a.w, (size_t)a.h, cudaMemcpyHostToDevice, s);
+            if (ce == cudaSuccess)
+                ce = cudaMemcpy2DAsync(d_stage + t.stage[f] + (size_t)a.w * a.h, row1, a.p1, a.pitch1, row1, (size_t)((a.h + 1) / 2),
+                                       cudaMemcpyHostToDevice, s);
+            if (ce != cudaSuccess) return ce;
+            f++;
+            continue;
+        }
+        const size_t row = (size_t)a.w * 3, pitch = a.pitch0, bytes = row * a.h;
         int e = f + 1;
         ptrdiff_t gap = 0;
         if (pitch == row && e < f1) {
-            gap = frames[e].rgb - a.rgb;
-            while (e < f1 && gap >= (ptrdiff_t)bytes && frames[e].w == a.w && frames[e].h == a.h &&
-                   (frames[e].row_stride == 0 || frames[e].row_stride == row) && frames[e].rgb - a.rgb == gap * (e - f) &&
-                   t.stage[e] == t.stage[f] + bytes * (e - f))
+            gap = frames[e].p0 - a.p0;
+            while (e < f1 && gap >= (ptrdiff_t)bytes && frames[e].fmt == PRE_RGB8 && frames[e].w == a.w && frames[e].h == a.h &&
+                   frames[e].pitch0 == row && frames[e].p0 - a.p0 == gap * (e - f) && t.stage[e] == t.stage[f] + bytes * (e - f))
                 e++;
         }
-        const cudaError_t ce = e > f + 1 ? cudaMemcpy2DAsync(d_stage + t.stage[f], bytes, a.rgb, (size_t)gap, bytes, (size_t)(e - f), cudaMemcpyHostToDevice, s)
-                                         : cudaMemcpy2DAsync(d_stage + t.stage[f], row, a.rgb, pitch, row, (size_t)a.h, cudaMemcpyHostToDevice, s);
+        const cudaError_t ce = e > f + 1 ? cudaMemcpy2DAsync(d_stage + t.stage[f], bytes, a.p0, (size_t)gap, bytes, (size_t)(e - f), cudaMemcpyHostToDevice, s)
+                                         : cudaMemcpy2DAsync(d_stage + t.stage[f], row, a.p0, pitch, row, (size_t)a.h, cudaMemcpyHostToDevice, s);
         if (ce != cudaSuccess) return ce;
         f = e;
     }
@@ -1323,13 +1378,15 @@ static cudaError_t pre_stage_frames(const PreTable &t, const mars_b200_frame_t *
  *   PRE_HOST_SYNC : host frames staged launch by launch on the compute stream (the caller synchronises);
  *   PRE_DEVICE    : device frames read in place;
  *   PRE_HOST_POOL : host frames and the table copied on the copy stream, then ev_in, which the compute stream waits for. */
-static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, const mars_b200_frame_t *frames,
+static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, const std::vector<FrameSrc> &frames,
                                       const std::vector<LetterboxGeom> &g, uint32_t ti, int nhwc, PreSource how, cudaEvent_t ev_in) {
     const int n = (int)g.size();
     if (n == 0) return MARS_OK;
     if (m->pre_taps.size() > 64) m->pre_taps.clear();
+    std::vector<int> fmt(n);
+    for (int f = 0; f < n; f++) fmt[f] = frames[f].fmt;
     PreTable t;
-    pre_table_build(g.data(), n, [m](int in, int out) -> const ResizeTaps & { return cached_taps(m, in, out); }, how == PRE_HOST_SYNC, &t);
+    pre_table_build(g.data(), fmt.data(), n, [m](int in, int out) -> const ResizeTaps & { return cached_taps(m, in, out); }, how == PRE_HOST_SYNC, &t);
     const size_t tab = t.bytes();
     if ((how != PRE_DEVICE && !pre_grow(m, &st.d_frames, &st.frames_cap, t.stage_bytes)) || !pre_grow(m, &st.d_tab, &st.tab_cap, tab) ||
         !pre_grow(m, (uint8_t **)&m->d_preH, &m->preH_cap, t.h_floats * sizeof(float))) {
@@ -1338,8 +1395,18 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
     }
     for (int f = 0; f < n; f++) {
         PreFrame &d = t.fr[f];
-        d.src = how == PRE_DEVICE ? frames[f].rgb : st.d_frames + t.stage[f];
-        d.row_stride = how == PRE_DEVICE && frames[f].row_stride ? frames[f].row_stride : (size_t)d.ow * 3;
+        const FrameSrc &a = frames[f];
+        const bool nv12 = a.fmt == PRE_NV12;
+        d.colour = a.colour;
+        if (how == PRE_DEVICE) {
+            d.src = a.p0; d.uv = a.p1;
+            d.row_stride = a.pitch0; d.uv_stride = a.pitch1;
+        } else { /* the tight staging layout of pre_stage_frames */
+            d.src = st.d_frames + t.stage[f];
+            d.row_stride = (size_t)d.ow * (nv12 ? 1 : 3);
+            d.uv = nv12 ? d.src + (size_t)d.ow * d.oh : nullptr;
+            d.uv_stride = nv12 ? (size_t)2 * ((d.ow + 1) / 2) : 0;
+        }
     }
     /* the pinned table is rewritten only once the last upload from it has completed */
     CU_OK(cudaEventSynchronize(st.ev), MARS_ERR_LAYER_FAILED);
@@ -1354,13 +1421,13 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
     CU_OK(cudaMemcpyAsync(st.d_tab, st.h_tab, tab, cudaMemcpyHostToDevice, cs), MARS_ERR_LAYER_FAILED);
     CU_OK(cudaEventRecord(st.ev, cs), MARS_ERR_LAYER_FAILED);
     if (how == PRE_HOST_POOL) {
-        CU_OK(pre_stage_frames(t, frames, 0, n, st.d_frames, cs), MARS_ERR_LAYER_FAILED);
+        CU_OK(pre_stage_frames(t, frames.data(), 0, n, st.d_frames, cs), MARS_ERR_LAYER_FAILED);
         cudaEventRecord(ev_in, cs);
         cudaStreamWaitEvent(m->stream, ev_in, 0);
     }
     int8_t *dst = reinterpret_cast<int8_t *>(dev_addr(m, m->toff[ti], first));
     for (size_t k = 0; k + 1 < t.first.size(); k++) {
-        if (how == PRE_HOST_SYNC) CU_OK(pre_stage_frames(t, frames, t.first[k], t.first[k + 1], st.d_frames, m->stream), MARS_ERR_LAYER_FAILED);
+        if (how == PRE_HOST_SYNC) CU_OK(pre_stage_frames(t, frames.data(), t.first[k], t.first[k + 1], st.d_frames, m->stream), MARS_ERR_LAYER_FAILED);
         CU_OK(launch_letterbox(t, (int)k, st.d_tab, m->d_preH, dst, m->slot_stride, nhwc, m->d_frame + first, m->stream), MARS_ERR_LAYER_FAILED);
         m->launches += 2;
     }
@@ -1368,17 +1435,18 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
 }
 
 /* the synchronous calls: validation, then copies + kernels as one device-timed region */
-static mars_error_t preprocess_sync(Model *m, const char *what, int first, int n, const mars_b200_frame_t *frames) {
+static mars_error_t preprocess_sync(Model *m, const char *what, int first, int n, const std::vector<FrameSrc> *frames) {
+    if (!m) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
     uint32_t ti;
     int tw, th, nhwc;
     mars_error_t e = pre_target(m, what, &ti, &tw, &th, &nhwc);
     std::vector<LetterboxGeom> g;
-    if (e == MARS_OK) e = pre_check_frames(m, what, n, frames, tw, th, false, &g);
+    if (e == MARS_OK) e = pre_check_frames(m, what, frames, tw, th, false, &g);
     if (e != MARS_OK) return e;
     cudaEventRecord(m->ev0, m->stream);
-    e = enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, frames, g, ti, nhwc, PRE_HOST_SYNC, nullptr);
+    e = enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, *frames, g, ti, nhwc, PRE_HOST_SYNC, nullptr);
     cudaEventRecord(m->ev1, m->stream);
     const cudaError_t ce = cudaStreamSynchronize(m->stream);
     if (e == MARS_OK && ce != cudaSuccess) {
@@ -1399,29 +1467,40 @@ mars_error_t mars_b200_preprocess_batch(mars_model_t *model, int first, int n, c
     if (w <= 0 || h <= 0) { set_last_error("preprocess: %d x %d is not a frame size", w, h); return MARS_ERR_INVALID_TENSOR; }
     const size_t frame_bytes = (size_t)(w > 0 ? w : 0) * (h > 0 ? h : 0) * 3;
     if (frame_stride < frame_bytes) frame_stride = frame_bytes;
-    std::vector<mars_b200_frame_t> fr((size_t)(n > 0 ? n : 0));
-    for (int f = 0; f < n; f++) fr[f] = mars_b200_frame_t{frames + (size_t)f * frame_stride, w, h, 0};
-    return preprocess_sync(m, "preprocess", first, n, fr.data());
+    std::vector<FrameSrc> fr((size_t)(n > 0 ? n : 0));
+    for (int f = 0; f < n; f++) fr[f] = FrameSrc{frames + (size_t)f * frame_stride, nullptr, (size_t)w * 3, 0, w, h, PRE_RGB8, 0};
+    return preprocess_sync(m, "preprocess", first, n, &fr);
 }
 
 mars_error_t mars_b200_preprocess_frames(mars_model_t *model, int first, int n, const mars_b200_frame_t *frames) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    return preprocess_sync(m, "preprocess_frames", first, n, frames);
+    std::vector<FrameSrc> s;
+    return preprocess_sync(as_model(model), "preprocess_frames", first, n, rgb_sources(n, frames, &s));
+}
+mars_error_t mars_b200_preprocess_frames_nv12(mars_model_t *model, int first, int n, const mars_b200_nv12_frame_t *frames) {
+    std::vector<FrameSrc> s;
+    return preprocess_sync(as_model(model), "preprocess_frames_nv12", first, n, nv12_sources(n, frames, &s));
 }
 
-mars_error_t mars_b200_preprocess_frames_device(mars_model_t *model, int first, int n, const mars_b200_frame_t *frames) {
-    Model *m = as_model(model);
+/* the device-frame calls: validation, then the launches on the compute stream */
+static mars_error_t preprocess_device(Model *m, const char *what, int first, int n, const std::vector<FrameSrc> *frames) {
     if (!m) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
     uint32_t ti;
     int tw, th, nhwc;
-    mars_error_t e = pre_target(m, "preprocess_frames_device", &ti, &tw, &th, &nhwc);
+    mars_error_t e = pre_target(m, what, &ti, &tw, &th, &nhwc);
     std::vector<LetterboxGeom> g;
-    if (e == MARS_OK) e = pre_check_frames(m, "preprocess_frames_device", n, frames, tw, th, true, &g);
+    if (e == MARS_OK) e = pre_check_frames(m, what, frames, tw, th, true, &g);
     if (e != MARS_OK) return e;
-    return enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, frames, g, ti, nhwc, PRE_DEVICE, nullptr);
+    return enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, *frames, g, ti, nhwc, PRE_DEVICE, nullptr);
+}
+mars_error_t mars_b200_preprocess_frames_device(mars_model_t *model, int first, int n, const mars_b200_frame_t *frames) {
+    std::vector<FrameSrc> s;
+    return preprocess_device(as_model(model), "preprocess_frames_device", first, n, rgb_sources(n, frames, &s));
+}
+mars_error_t mars_b200_preprocess_frames_nv12_device(mars_model_t *model, int first, int n, const mars_b200_nv12_frame_t *frames) {
+    std::vector<FrameSrc> s;
+    return preprocess_device(as_model(model), "preprocess_frames_nv12_device", first, n, nv12_sources(n, frames, &s));
 }
 
 mars_error_t mars_b200_run_resident(mars_model_t *model, int first, int n) {
@@ -1685,10 +1764,10 @@ mars_error_t mars_b200_run_batch(mars_model_t *model, int n, const void *inputs,
  * detection records on the read-back stream -- and the call returns.  While it runs the caller submits the next batch to the
  * other half, so the host->device copy of batch k+1 and the read-back of batch k-1 overlap the kernels of batch k.
  * inputs / dets / counts must stay valid (and should be pinned, e.g. nna_malloc) until mars_b200_wait_batch(pool) returns. */
-/* frames != NULL: inputs are letterboxed from those host frames instead (mars_b200_submit_frames_heads_batch) */
+/* what != NULL: inputs are letterboxed from the n host frames of `frames` instead (mars_b200_submit_frames_heads_batch) */
 static mars_error_t submit_batch(Model *m, int pool, int n, const void *inputs, size_t in_stride, void *dets, int32_t *counts, int maxd,
-                                 float nms_thresh, int flavour, const mars_b200_frame_t *frames = nullptr) {
-    if (!m || !(inputs || frames) || !dets || !counts || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
+                                 float nms_thresh, int flavour, const std::vector<FrameSrc> *frames = nullptr, const char *what = nullptr) {
+    if (!m || !(inputs || what) || !dets || !counts || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     const int half = m->capacity / 2;
     if (half < 1 || n < 0 || n > half) {
@@ -1707,17 +1786,17 @@ static mars_error_t submit_batch(Model *m, int pool, int n, const void *inputs, 
     uint32_t ti = 0;
     int tw = 0, th = 0, nhwc = 0;
     std::vector<LetterboxGeom> g;
-    if (frames) {
-        mars_error_t e = pre_target(m, "submit_frames_heads_batch", &ti, &tw, &th, &nhwc);
-        if (e == MARS_OK) e = pre_check_frames(m, "submit_frames_heads_batch", n, frames, tw, th, false, &g);
+    if (what) {
+        mars_error_t e = pre_target(m, what, &ti, &tw, &th, &nhwc);
+        if (e == MARS_OK) e = pre_check_frames(m, what, frames, tw, th, false, &g);
         if (e != MARS_OK) return e;
     }
     mars_error_t e = compile_model(m); /* also drops captured graphs of an older program (set_opt_level, set_depthwise_mode) */
     if (e != MARS_OK) return e;
     if (n > 0) {
         /* the half is free: its previous batch was waited for (read-back complete) before this call -- its staging too */
-        if (frames) {
-            e = enqueue_letterbox(m, m->pre_stage[pool], first, frames, g, ti, nhwc, PRE_HOST_POOL, m->ev_in[pool]);
+        if (what) {
+            e = enqueue_letterbox(m, m->pre_stage[pool], first, *frames, g, ti, nhwc, PRE_HOST_POOL, m->ev_in[pool]);
             if (e != MARS_OK) return e;
         } else {
             e = copy_io(m, first, n, const_cast<void *>(inputs), in_stride, 0, m->h2d_stream);
@@ -1750,14 +1829,26 @@ mars_error_t mars_b200_submit_heads_batch(mars_model_t *model, int pool, int n, 
     return submit_batch(m, pool, n, inputs, in_stride, boxes, counts, maxd, nms_thresh, STEP_HEADS);
 }
 
-/* mars_b200_submit_heads_batch from RGB8 frames of any sizes and row pitches (host memory): H2D of each frame on the copy
- * stream, the letterbox launches on the compute stream in front of the (graphed) step, frame coordinates for every slot */
+/* mars_b200_submit_heads_batch from RGB8 or NV12 frames of any sizes and row pitches (host memory): H2D of each frame (each
+ * NV12 plane) on the copy stream, the letterbox launches on the compute stream in front of the (graphed) step, frame
+ * coordinates for every slot */
+static mars_error_t submit_frames_heads(Model *m, const char *what, int pool, int n, const std::vector<FrameSrc> *frames, mars_box_t *boxes,
+                                        int32_t *counts, int maxd, float nms_thresh) {
+    if (m && m->heads.empty()) { set_last_error("%s: no YOLO heads configured (mars_b200_set_yolo_heads)", what); return MARS_ERR_INVALID_TENSOR; }
+    if (m && !frames) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
+    return submit_batch(m, pool, n, nullptr, 0, boxes, counts, maxd, nms_thresh, STEP_HEADS, frames, what);
+}
 mars_error_t mars_b200_submit_frames_heads_batch(mars_model_t *model, int pool, int n, const mars_b200_frame_t *frames, mars_box_t *boxes,
                                                  int32_t *counts, int maxd, float nms_thresh) {
-    Model *m = as_model(model);
-    if (m && m->heads.empty()) { set_last_error("submit_frames_heads_batch: no YOLO heads configured (mars_b200_set_yolo_heads)"); return MARS_ERR_INVALID_TENSOR; }
-    if (m && !frames) { set_last_error("submit_frames_heads_batch: no frame table"); return MARS_ERR_INVALID_FILE; }
-    return submit_batch(m, pool, n, nullptr, 0, boxes, counts, maxd, nms_thresh, STEP_HEADS, frames);
+    std::vector<FrameSrc> s;
+    return submit_frames_heads(as_model(model), "submit_frames_heads_batch", pool, n, rgb_sources(n, frames, &s), boxes, counts, maxd,
+                               nms_thresh);
+}
+mars_error_t mars_b200_submit_frames_nv12_heads_batch(mars_model_t *model, int pool, int n, const mars_b200_nv12_frame_t *frames,
+                                                      mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh) {
+    std::vector<FrameSrc> s;
+    return submit_frames_heads(as_model(model), "submit_frames_nv12_heads_batch", pool, n, nv12_sources(n, frames, &s), boxes, counts,
+                               maxd, nms_thresh);
 }
 
 /* mars_b200_submit_batch without the YOLO post-process: the raw output tensor 0 of every image is read back instead

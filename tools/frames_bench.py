@@ -4,9 +4,12 @@
                 mars_b200_preprocess_frames call, and grouped by size through three mars_b200_preprocess_batch calls
   (c) steady:   mars_b200_submit_frames_heads_batch on the yolov5s-shaped heads model, alternating pools, pinned frames:
                 frames/s and the latency from submit to boxes on the host (p50 / p99)
+  (d) nv12:     1920x1080 NV12 frames against RGB8 frames of the same size: 64 device-resident frames letterboxed in place
+                (mars_b200_preprocess_frames[_nv12]_device; ms by CUDA events, source bytes per frame, GB/s of source read), and
+                the steady-state submit of (c) from pinned NV12 frames (mars_b200_submit_frames_nv12_heads_batch)
 Frames live in pinned host memory (nna_malloc).  Device times are CUDA events around the copies + kernels; host times are
 wall clock around calls that end in a device synchronisation.
-usage: python tools/frames_bench.py [--part a|b|c|all] [--repeat N] [--batches N] [--pool N]"""
+usage: python tools/frames_bench.py [--part a|b|c|d|all] [--repeat N] [--batches N] [--pool N]"""
 import argparse
 import ctypes as C
 import json
@@ -34,19 +37,27 @@ def gpu_info():
     return q
 
 
-def pinned_frames(shapes, seed):
-    """one pinned buffer holding the frames back to back; returns (views, pointer)"""
-    total = sum(w * h * 3 for (w, h) in shapes)
+def frame_bytes(w, h, nv12=False):
+    return w * h + 2 * ((w + 1) // 2) * ((h + 1) // 2) if nv12 else w * h * 3
+
+
+def pinned_frames(shapes, seed, nv12=False):
+    """one pinned buffer holding the frames back to back -- RGB8 [h, w, 3] arrays, or NV12 (y, uv, BT.709 limited) tuples with
+    each frame's chroma plane right after its luma plane; returns (frames, pointer)"""
+    total = sum(frame_bytes(w, h, nv12) for (w, h) in shapes)
     ptr = L.nna_malloc(total)
     assert ptr, "nna_malloc(%d)" % total
     buf = np.ctypeslib.as_array((C.c_uint8 * total).from_address(ptr))
     rng = np.random.default_rng(seed)
+    buf[...] = rng.integers(0, 256, total, dtype=np.uint8)
     out, at = [], 0
     for (w, h) in shapes:
-        v = buf[at: at + w * h * 3].reshape(h, w, 3)
-        v[...] = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-        out.append(v)
-        at += w * h * 3
+        if nv12:
+            uv = buf[at + w * h: at + frame_bytes(w, h, True)].reshape((h + 1) // 2, (w + 1) // 2, 2)
+            out.append((buf[at: at + w * h].reshape(h, w), uv, pkg.capi.YUV_BT709_LIMITED))
+        else:
+            out.append(buf[at: at + w * h * 3].reshape(h, w, 3))
+        at += frame_bytes(w, h, nv12)
     return out, ptr
 
 
@@ -111,12 +122,13 @@ def part_b(repeat):
                                    frames_per_s=round(64 / wall2 * 1e3, 1)))
 
 
-def part_c(batches, pool_n, sizes):
+def part_c(batches, pool_n, sizes, nv12=False):
     gm = pkg.MarsModel(mf.build_yolov5(width=0.5, size=640, seed=5).to_bytes(), arena_bytes=mf.ARENA_YOLOV5S_INT8, device=0,
                        batch=2 * pool_n)
     gm.set_yolo_heads(None, 0.25)
     # two distinct sets of frames, one per pool
-    sets = [pinned_frames([sizes[i % len(sizes)] for i in range(pool_n)], 20 + p) for p in range(2)]
+    sets = [pinned_frames([sizes[i % len(sizes)] for i in range(pool_n)], 20 + p, nv12) for p in range(2)]
+    submit = gm.submit_frames_nv12_heads_batch if nv12 else gm.submit_frames_heads_batch
     out = [(np.zeros((pool_n, 100), dtype=pkg.capi.BOX_DTYPE), np.zeros(pool_n, dtype=np.int32)) for _ in range(2)]
     sub, lat = {}, []
 
@@ -127,7 +139,7 @@ def part_c(batches, pool_n, sizes):
                 gm.wait_batch(pool)
                 lat.append((time.perf_counter() - sub[i - 2]) * 1e3)
             sub[i] = time.perf_counter()
-            gm.submit_frames_heads_batch(pool, sets[pool][0], out[pool][0], out[pool][1], maxd=100)
+            submit(pool, sets[pool][0], out[pool][0], out[pool][1], maxd=100)
         for i in (k - 2, k - 1):
             gm.wait_batch(i % 2)
             lat.append((time.perf_counter() - sub[i]) * 1e3)
@@ -141,17 +153,58 @@ def part_c(batches, pool_n, sizes):
     gm.close()
     for _, ptr in sets:
         L.nna_free(ptr)
-    nbytes = sum(w * h * 3 for (w, h) in [sizes[i % len(sizes)] for i in range(pool_n)])
+    nbytes = sum(frame_bytes(w, h, nv12) for (w, h) in [sizes[i % len(sizes)] for i in range(pool_n)])
     fps = batches * pool_n / dt
-    return dict(part="c", model="yolov5s-shaped heads (width 0.5, 640)", pool_frames=pool_n, batches=batches,
+    return dict(part="d" if nv12 else "c", source="nv12" if nv12 else "rgb8", model="yolov5s-shaped heads (width 0.5, 640)",
+                pool_frames=pool_n, batches=batches,
                 sizes=sorted({"%dx%d" % s for s in sizes}), frames_per_s=round(fps, 1),
                 h2d_gb_per_s=round(fps * nbytes / pool_n / 1e9, 2),
                 latency_ms_p50=round(float(np.percentile(lat, 50)), 3), latency_ms_p99=round(float(np.percentile(lat, 99)), 3))
 
 
+def part_d_device(repeat, calls=5):
+    """64 device-resident 1920x1080 frames letterboxed in place: CUDA events on the compute stream around `calls` calls in a
+    row (the host work of one call -- validation, table upload -- overlaps the launches of the previous one), per call.
+    RGB8 and NV12 alternate within one model; 64 frames (199 MB NV12, 398 MB RGB8) exceed the 126 MB L2."""
+    import torch
+    n, w, h = 64, 1920, 1080
+    gm = letterbox_model(n)
+    g = torch.Generator(device="cuda").manual_seed(0)
+    rgb = torch.randint(0, 256, (n, h, w * 3), dtype=torch.uint8, device="cuda", generator=g)
+    luma = torch.randint(0, 256, (n, h, w), dtype=torch.uint8, device="cuda", generator=g)
+    chroma = torch.randint(0, 256, (n, h // 2, w), dtype=torch.uint8, device="cuda", generator=g)
+    torch.cuda.synchronize()
+    stream = torch.cuda.ExternalStream(gm.compute_stream())
+    t_rgb = pkg.capi.device_frames([(rgb[i].data_ptr(), w, h, 0) for i in range(n)])
+    t_nv12 = pkg.capi.device_nv12_frames([(luma[i].data_ptr(), chroma[i].data_ptr(), w, h, 0, 0, pkg.capi.YUV_BT709_LIMITED)
+                                          for i in range(n)])
+    runs = {"rgb8": lambda: L.mars_b200_preprocess_frames_device(gm.m, 0, n, t_rgb),
+            "nv12": lambda: L.mars_b200_preprocess_frames_nv12_device(gm.m, 0, n, t_nv12)}
+    ms = {k: [] for k in runs}
+    for it in range(repeat + 2):
+        for k, fn in runs.items():
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record(stream)
+            for _ in range(calls):
+                assert fn() == 0, L.mars_b200_last_error()
+            e1.record(stream)
+            e1.synchronize()
+            if it >= 2:
+                ms[k].append(e0.elapsed_time(e1) / calls)
+    gm.close()
+    out = dict(part="d", case="device-resident letterbox", frames=n, size="%dx%d" % (w, h))
+    for k, v in ms.items():
+        med = float(np.median(v))
+        fb = frame_bytes(w, h, k == "nv12")
+        out[k] = dict(ms=round(med, 3), ms_min=round(min(v), 3), ms_max=round(max(v), 3), source_bytes_per_frame=fb,
+                      source_gb_per_s=round(n * fb / med / 1e6, 1))
+    out["nv12_over_rgb8"] = round(out["nv12"]["ms"] / out["rgb8"]["ms"], 3)
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--part", default="all", choices=["a", "b", "c", "all"])
+    ap.add_argument("--part", default="all", choices=["a", "b", "c", "d", "all"])
     ap.add_argument("--repeat", type=int, default=20)
     ap.add_argument("--batches", type=int, default=60)
     ap.add_argument("--pool", type=int, default=32, help="frames per submit (half the slots)")
@@ -164,6 +217,10 @@ def main():
     if a.part in ("c", "all"):
         print(json.dumps(part_c(a.batches, a.pool, [(1920, 1080)])))
         print(json.dumps(part_c(a.batches, a.pool, [(1920, 1080), (1280, 720), (1920, 1080), (640, 360)])))
+    if a.part in ("d", "all"):
+        print(json.dumps(part_d_device(a.repeat)))
+        for nv12 in (False, True, False, True):  # alternated: RGB8 (part c) and NV12 on the same model and sizes
+            print(json.dumps(part_c(a.batches, a.pool, [(1920, 1080)], nv12)))
 
 
 if __name__ == "__main__":
