@@ -183,6 +183,55 @@ mars_error_t mars_b200_submit_frames_nv12_heads_batch(mars_model_t *m, int pool,
 /* kept boxes of slots [first, first+n): boxes[n][maxd] (maxd <= 1000), counts[n] */
 mars_error_t mars_b200_download_boxes(mars_model_t *m, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd);
 
+/* ---- tiled (sliced) detection on high-resolution frames --------------------------------------------------------------------
+ * A 3840x2160 frame fitted whole into a 640x640 input is shrunk 6 times; small objects vanish.  These calls letterbox regions of
+ * interest of the frames -- typically overlapping tiles, plus the whole frame -- into one slot each, run the heads step on the
+ * slots, shift each region's kept boxes back into its frame and merge them per frame with the corner NMS of
+ * examples/yolo_detect.cpp:152-173.  Tiling and the merge are this library's additions (the reference has neither); the merge's
+ * NMS is the reference's nms.  Regions of one frame are contiguous in the region table; their order fixes the order in which
+ * their boxes are concatenated for the merge. */
+/* one region of interest of frame `frame` (an index into the call's frame table): the w x h pixels at (x, y) */
+typedef struct { int32_t frame, x, y, w, h; } mars_b200_roi_t;
+/* host only, no GPU: the tile grid of a w x h frame.  Along x the step is tile_w - overlap_w; there is one column when
+ * w <= tile_w, else ceil((w - tile_w) / step) + 1; column i starts at min(i * step, w - tile_w) (the last is flush with the right
+ * edge) and is min(tile_w, w) wide.  The same along y.  Tiles in row-major order; with_full and more than one tile: the whole
+ * frame comes first as one more region.  Returns the count (when it exceeds cap nothing is written), or -1 for non-positive
+ * sizes, a negative overlap or an overlap not smaller than its tile.  3840x2160, 640x640 tiles, overlap 128: 8 x 4 = 32 tiles. */
+int mars_b200_tile_rois(int frame, int w, int h, int tile_w, int tile_h, int overlap_w, int overlap_h, int with_full,
+                        mars_b200_roi_t *out, int cap);
+/* Letterboxes region r of rois into input tensor 0 of slot first + r: byte-identical to mars_b200_letterbox of the cropped frame
+ * frame[y:y+h, x:x+w] (for NV12, of the same crop of the RGB8 frame the conversion gives; chroma comes from the frame's own 2 x 2
+ * blocks, so odd origins are exact).  Each slot records the region's size as its frame size, so the letterbox inverse gives
+ * boxes in region coordinates.  Each frame is uploaded once, however many regions it has.  Every frame and region is checked
+ * first -- the frame checks of mars_b200_preprocess_frames, frame in [0, n_frames) and not decreasing, x, y >= 0, w, h > 0,
+ * inside its frame, a letterbox at least one pixel wide and tall, n_rois slots in range -- and a rejected call writes no slot;
+ * mars_b200_last_error names the frame or region.  Host RGB8 frames, synchronous. */
+mars_error_t mars_b200_preprocess_rois(mars_model_t *m, int first, int n_frames, const mars_b200_frame_t *frames, int n_rois,
+                                       const mars_b200_roi_t *rois);
+/* the same from NV12 frames in device memory of the model's device, read in place: enqueued on mars_b200_compute_stream(m) */
+mars_error_t mars_b200_preprocess_rois_nv12_device(mars_model_t *m, int first, int n_frames, const mars_b200_nv12_frame_t *frames,
+                                                   int n_rois, const mars_b200_roi_t *rois);
+/* After a heads step on slots [first, first+n_rois) (mars_b200_step_heads_resident or the enqueue form): for each frame f the
+ * kept boxes of its regions' slots, in region order and each slot's kept order, shifted into frame coordinates (x + (float)roi.x,
+ * y + (float)roi.y), capped at the first 1000 by descending confidence (ties in that order), then the corner NMS (same class,
+ * IoU > merge_thresh) -> frame record first + f (mars_b200_download_frame_boxes).  The slots' own boxes stay as they are.
+ * Enqueued on mars_b200_compute_stream(m). */
+mars_error_t mars_b200_merge_rois_resident(mars_model_t *m, int first, int n_frames, int n_rois, const mars_b200_roi_t *rois,
+                                           float merge_thresh);
+/* merged boxes of frame records [first, first+n): boxes[n][maxd] (maxd <= 1000), counts[n] */
+mars_error_t mars_b200_download_frame_boxes(mars_model_t *m, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd);
+/* The whole flow on one pool: the n_frames host frames uploaded once each and the region and merge tables in one pinned upload,
+ * on the copy stream; then on the compute stream the letterbox of n_rois slots, the (graphed) heads step on them and the merge;
+ * then the D2H of the n_frames frame records.  boxes[n_frames][maxd], counts[n_frames], in frame coordinates; waited for with
+ * mars_b200_wait_batch.  n_rois and n_frames must fit half the slot pool.  Nothing returns to the host in between. */
+mars_error_t mars_b200_submit_rois_heads_batch(mars_model_t *m, int pool, int n_frames, const mars_b200_frame_t *frames, int n_rois,
+                                               const mars_b200_roi_t *rois, mars_box_t *boxes, int32_t *counts, int maxd,
+                                               float nms_thresh, float merge_thresh);
+/* the same from host NV12 frames (both planes uploaded, converted inside the letterbox) */
+mars_error_t mars_b200_submit_rois_nv12_heads_batch(mars_model_t *m, int pool, int n_frames, const mars_b200_nv12_frame_t *frames,
+                                                    int n_rois, const mars_b200_roi_t *rois, mars_box_t *boxes, int32_t *counts,
+                                                    int maxd, float nms_thresh, float merge_thresh);
+
 /* ---- several GPUs of one box behind one call (batch sharded over the devices, no inter-GPU traffic on the path) ---------- */
 typedef struct mars_b200_group mars_b200_group_t;
 /* one replica of the model per device (devices = NULL: ordinals 0 .. n_devices-1), `per_gpu_batch` image slots each */

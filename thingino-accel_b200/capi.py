@@ -90,6 +90,14 @@ class NV12_FRAME(C.Structure):
                 ("uv_stride", C.c_size_t), ("colour", C.c_int32)]
 
 
+class ROI(C.Structure):
+    """mars_b200_roi_t: the w x h pixels at (x, y) of frame `frame` (an index into the call's frame table)"""
+    _fields_ = [("frame", C.c_int32), ("x", C.c_int32), ("y", C.c_int32), ("w", C.c_int32), ("h", C.c_int32)]
+
+
+ROI_DTYPE = np.dtype([("frame", "<i4"), ("x", "<i4"), ("y", "<i4"), ("w", "<i4"), ("h", "<i4")])
+
+
 # every symbol include/*.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     # include/mars_runtime.h
@@ -228,6 +236,15 @@ SIGNATURES = {
     "mars_b200_submit_frames_nv12_heads_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME), C.c_void_p, C.c_void_p,
                                                            C.c_int, C.c_float]),
     "mars_b200_yuv_coefficients": (C.c_int, [C.c_int, C.c_void_p]),
+    "mars_b200_tile_rois": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int]),
+    "mars_b200_preprocess_rois": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(FRAME), C.c_int, C.c_void_p]),
+    "mars_b200_preprocess_rois_nv12_device": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME), C.c_int, C.c_void_p]),
+    "mars_b200_merge_rois_resident": (C.c_int, [PM, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_float]),
+    "mars_b200_download_frame_boxes": (C.c_int, [PM, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "mars_b200_submit_rois_heads_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(FRAME), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                    C.c_int, C.c_float, C.c_float]),
+    "mars_b200_submit_rois_nv12_heads_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME), C.c_int, C.c_void_p, C.c_void_p,
+                                                         C.c_void_p, C.c_int, C.c_float, C.c_float]),
 }
 
 _lib = None
@@ -310,6 +327,13 @@ def device_nv12_frames(frames):
     for i, f in enumerate(frames):
         table[i] = NV12_FRAME(*f)
     return table
+
+
+def roi_table(rois):
+    """[(frame, x, y, w, h), ...] or a ROI_DTYPE array -> contiguous ROI_DTYPE array (the layout of mars_b200_roi_t)"""
+    if isinstance(rois, np.ndarray) and rois.dtype == ROI_DTYPE:
+        return np.ascontiguousarray(rois)
+    return np.array([tuple(int(v) for v in r) for r in rois], dtype=ROI_DTYPE)
 
 
 def _numel(desc):
@@ -463,6 +487,50 @@ class MarsModel:
         """frames: [(y_ptr, uv_ptr, w, h, y_stride, uv_stride, colour), ...] in device memory; enqueued on compute_stream()"""
         self._check(lib().mars_b200_preprocess_frames_nv12_device(self.m, first, len(frames), device_nv12_frames(frames)),
                     "preprocess_frames_nv12_device")
+
+    # ---- tiled detection: regions of frames, merged per frame (include/mars_b200.h) -------------
+    def preprocess_rois(self, first, frames, rois):
+        """frames: list of [h, w, 3] uint8 host arrays (row-strided views pass their pitch); rois: (frame, x, y, w, h) per region
+        (tile_rois) -> region r letterboxed into slot first + r; returns the GPU milliseconds of the copies + kernels"""
+        table, _keep = host_frames(frames)
+        r = roi_table(rois)
+        self._check(lib().mars_b200_preprocess_rois(self.m, first, len(frames), table, len(r), r.ctypes.data), "preprocess_rois")
+        return float(lib().mars_b200_last_gpu_ms(self.m))
+
+    def preprocess_rois_nv12_device(self, first, frames, rois):
+        """frames: [(y_ptr, uv_ptr, w, h, y_stride, uv_stride, colour), ...] in device memory; enqueued on compute_stream()"""
+        r = roi_table(rois)
+        self._check(lib().mars_b200_preprocess_rois_nv12_device(self.m, first, len(frames), device_nv12_frames(frames), len(r), r.ctypes.data),
+                    "preprocess_rois_nv12_device")
+
+    def merge_rois_resident(self, first, n_frames, rois, merge_thresh=0.45):
+        """after a heads step on slots [first, first + len(rois)): boxes of each frame's regions shifted into the frame and merged
+        by the corner NMS into frame records [first, first + n_frames); enqueued on compute_stream()"""
+        r = roi_table(rois)
+        self._check(lib().mars_b200_merge_rois_resident(self.m, first, n_frames, len(r), r.ctypes.data, merge_thresh), "merge_rois_resident")
+
+    def download_frame_boxes(self, first, n, maxd=1000):
+        boxes = np.zeros((n, maxd), dtype=BOX_DTYPE)
+        counts = np.zeros(n, dtype=np.int32)
+        self._check(lib().mars_b200_download_frame_boxes(self.m, first, n, boxes.ctypes.data, counts.ctypes.data, maxd), "download_frame_boxes")
+        return boxes, counts
+
+    def submit_rois_heads_batch(self, pool, frames, rois, boxes, counts, maxd=1000, thresh=0.45, merge_thresh=0.45):
+        """the tiled flow on one pool from [h, w, 3] uint8 host frames: boxes [len(frames), maxd] in frame coordinates.  The frames
+        and regions are kept alive until wait_batch(pool); boxes and counts must be kept alive by the caller"""
+        table, keep = host_frames(frames)
+        r = roi_table(rois)
+        self._check(lib().mars_b200_submit_rois_heads_batch(self.m, pool, len(frames), table, len(r), r.ctypes.data, _addr(boxes), _addr(counts),
+                                                            maxd, thresh, merge_thresh), "submit_rois_heads_batch")
+        self._inflight[pool] = (table, keep, r)
+
+    def submit_rois_nv12_heads_batch(self, pool, frames, rois, boxes, counts, maxd=1000, thresh=0.45, merge_thresh=0.45):
+        """submit_rois_heads_batch from (y, uv, colour) NV12 host frames (host_nv12_frames)"""
+        table, keep = host_nv12_frames(frames)
+        r = roi_table(rois)
+        self._check(lib().mars_b200_submit_rois_nv12_heads_batch(self.m, pool, len(frames), table, len(r), r.ctypes.data, _addr(boxes),
+                                                                 _addr(counts), maxd, thresh, merge_thresh), "submit_rois_nv12_heads_batch")
+        self._inflight[pool] = (table, keep, r)
 
     def download_outputs(self, first, n, host=None, stride=0):
         if host is None:
@@ -647,6 +715,16 @@ def resize_taps(in_size, out_size):
         if n <= cap:
             return start, src[:n].copy(), w[:n].copy()
         cap = n
+
+
+def tile_rois(w, h, tile_w=640, tile_h=640, overlap_w=128, overlap_h=128, with_full=False, frame=0):
+    """host only (no GPU): the tile grid of a w x h frame (mars_b200_tile_rois) as a ROI_DTYPE array"""
+    n = lib().mars_b200_tile_rois(frame, w, h, tile_w, tile_h, overlap_w, overlap_h, 1 if with_full else 0, None, 0)
+    if n < 0:
+        raise ValueError("tile_rois(%d, %d, %d, %d, %d, %d)" % (w, h, tile_w, tile_h, overlap_w, overlap_h))
+    out = np.zeros(n, dtype=ROI_DTYPE)
+    assert lib().mars_b200_tile_rois(frame, w, h, tile_w, tile_h, overlap_w, overlap_h, 1 if with_full else 0, out.ctypes.data, n) == n
+    return out
 
 
 def yuv_coefficients(colour):

@@ -13,6 +13,8 @@
  *  k_head_decode  : anchor-grid decode (mgk-decompiler/test_yolo_inference.py:136-202) of one head level, reading the raw
  *                   head convolution where the program leaves it (OP_YOLO_HEAD, mars_b200_set_yolo_heads);
  *  k_nms_corner_batch : nms() of reference examples/yolo_detect.cpp:152-173 (corner boxes), with the letterbox inverse;
+ *  k_merge_rois   : the boxes of a frame's regions (tiled detection; ours, the reference does not tile) shifted into the frame and
+ *                   merged by the same corner NMS (nms_corner_image, shared with k_nms_corner_batch);
  *  k_scale_detections : the letterbox inverse alone (reference examples/yolo_detect.cpp:208-227).
  * The host-pointer entry points (seam.inc) run these kernels on a batch of one image.
  * One thread block per image; blocks are independent (images shard with no exchange).
@@ -642,28 +644,27 @@ struct NmsBatchShared {
     int removed_before[32];
 };
 
-__global__ void __launch_bounds__(NMSB_THREADS) k_nms_corner_batch(const mars_box_t *in_all, const int32_t *counts_in, mars_box_t *out_all,
-                                                                  int32_t *counts_out, int box_stride, float thresh, unsigned *scratch,
-                                                                  const int2 *frames, int net_w, int net_h) {
-    __shared__ NmsBatchShared sh;
-    const mars_box_t *in = in_all + (size_t)blockIdx.x * box_stride;
-    mars_box_t *out = out_all + (size_t)blockIdx.x * box_stride;
-    unsigned *const mask = scratch + (size_t)blockIdx.x * NMS_SCRATCH_WORDS;
-    const int n = min(counts_in[blockIdx.x], MARS_MAX_DETS);
+/* the 32-bit sort key of a confidence: ascending key = descending confidence, -0 == +0 (a tie, as the comparison sort sees it),
+ * NaN last */
+__device__ __forceinline__ unsigned nms_conf_key(float c) {
+    if (c != c) return 0xFFFFFFFFu;
+    const unsigned b = __float_as_uint(__fadd_rn(c, 0.0f));
+    const unsigned asc = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+    return ~asc;
+}
+
+/* The corner NMS of one image by one NMSB_THREADS block, shared by k_nms_corner_batch and k_merge_rois: input element j < n
+ * (n <= MARS_MAX_DETS) is load(j), a mars_box_t; kept element r (sorted order) goes out as emit(r, box); the kept count to
+ * *count_out.  mask = the image's NMS_SCRATCH_WORDS of global scratch. */
+template <class Load, class Emit>
+__device__ __forceinline__ void nms_corner_image(NmsBatchShared &sh, int n, float thresh, unsigned *mask, int32_t *count_out, Load load,
+                                                 Emit emit) {
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     unsigned long long key[NMSB_ITEMS];
 #pragma unroll
     for (int k = 0; k < NMSB_ITEMS; k++) {
         const int j = tid * NMSB_ITEMS + k;
-        unsigned u = 0xFFFFFFFFu; /* NaN and padding sort last */
-        if (j < n) {
-            const float c = in[j].confidence;
-            if (c == c) {
-                const unsigned b = __float_as_uint(__fadd_rn(c, 0.0f)); /* -0 == +0: a tie, as the comparison sort sees it */
-                const unsigned asc = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-                u = ~asc;
-            }
-        }
+        const unsigned u = j < n ? nms_conf_key(load(j).confidence) : 0xFFFFFFFFu; /* padding sorts last */
         key[k] = ((unsigned long long)u << 10) | (unsigned)j;
     }
     cub::BlockRadixSort<unsigned long long, NMSB_THREADS, NMSB_ITEMS>(sh.sort).Sort(key, 0, 42);
@@ -671,7 +672,7 @@ __global__ void __launch_bounds__(NMSB_THREADS) k_nms_corner_batch(const mars_bo
     for (int k = 0; k < NMSB_ITEMS; k++) sh.order[tid * NMSB_ITEMS + k] = (uint16_t)(key[k] & 1023u);
     __syncthreads(); /* the sort's storage is reused for the sorted boxes */
     for (int j = tid; j < n; j += NMSB_THREADS) {
-        const mars_box_t b = in[sh.order[j]];
+        const mars_box_t b = load(sh.order[j]);
         sh.box.x0[j] = b.x0; sh.box.y0[j] = b.y0; sh.box.x1[j] = b.x1; sh.box.y1[j] = b.y1;
         sh.cls[j] = b.class_id;
     }
@@ -694,18 +695,116 @@ __global__ void __launch_bounds__(NMSB_THREADS) k_nms_corner_batch(const mars_bo
         }
     }
     __syncthreads();
-    if (wid == 0) nms_publish_removed(nms_walk<8>(mask, n, lane), n, lane, sh.removed, sh.removed_before, &counts_out[blockIdx.x]);
+    if (wid == 0) nms_publish_removed(nms_walk<8>(mask, n, lane), n, lane, sh.removed, sh.removed_before, count_out);
     __syncthreads();
-    const int2 fr = frames[blockIdx.x];
-    const bool inv = fr.x > 0 && fr.y > 0;
-    const Letterbox lb = inv ? letterbox_params(fr.x, fr.y, net_w, net_h) : Letterbox{1.0f, 0.0f, 0.0f, 0.0f, 0.0f};
     for (int j = tid; j < n; j += NMSB_THREADS) {
         const unsigned word = sh.removed[j >> 5];
         if ((word >> (j & 31)) & 1u) continue;
-        mars_box_t b = in[sh.order[j]];
-        if (inv) b = letterbox_inverse(b, lb);
-        out[j - sh.removed_before[j >> 5] - __popc(word & ((1u << (j & 31)) - 1u))] = b;
+        emit(j - sh.removed_before[j >> 5] - __popc(word & ((1u << (j & 31)) - 1u)), load(sh.order[j]));
     }
+}
+
+__global__ void __launch_bounds__(NMSB_THREADS) k_nms_corner_batch(const mars_box_t *in_all, const int32_t *counts_in, mars_box_t *out_all,
+                                                                  int32_t *counts_out, int box_stride, float thresh, unsigned *scratch,
+                                                                  const int2 *frames, int net_w, int net_h) {
+    __shared__ NmsBatchShared sh;
+    const mars_box_t *in = in_all + (size_t)blockIdx.x * box_stride;
+    mars_box_t *out = out_all + (size_t)blockIdx.x * box_stride;
+    const int n = min(counts_in[blockIdx.x], MARS_MAX_DETS);
+    const int2 fr = frames[blockIdx.x];
+    const bool inv = fr.x > 0 && fr.y > 0;
+    const Letterbox lb = inv ? letterbox_params(fr.x, fr.y, net_w, net_h) : Letterbox{1.0f, 0.0f, 0.0f, 0.0f, 0.0f};
+    nms_corner_image(sh, n, thresh, scratch + (size_t)blockIdx.x * NMS_SCRATCH_WORDS, &counts_out[blockIdx.x],
+                     [in](int j) { return in[j]; },
+                     [out, inv, &lb](int r, mars_box_t b) { out[r] = inv ? letterbox_inverse(b, lb) : b; });
+}
+
+/* ---- merge of the regions of a frame (mars_b200_merge_rois_resident) ----------------------------------------------------
+ * The candidates of frame f are the kept boxes of its regions' slots, concatenated in region order, each shifted into frame
+ * coordinates by its region's origin (one float add per coordinate).  The first MERGE_CAP of them by (confidence key, position
+ * in the concatenation) are selected without materialising the union: a radix select over the 32-bit key, 8 bits per pass,
+ * finds the key T of the MERGE_CAP-th; every candidate with a smaller key and the first ones equal to T (in concatenation order)
+ * are compacted in concatenation order.  Compaction keeps that order, so the (key, position) sort of nms_corner_image over the
+ * selection orders ties exactly as a stable sort of the whole union would.  One block per frame.
+ *   tab: [n_frames + 1] region starts (frame f has regions [tab[f], tab[f + 1]) of the call), then (x, y) per region;
+ *   boxes / counts: the kept boxes of the call's slots (region r in slot r), box_stride apart. */
+#define MERGE_CAP HEAD_MAX_CAND
+struct MergeShared {
+    NmsBatchShared nms;
+    int cand[MARS_MAX_DETS]; /* selected candidate: region << 10 | index in the region's slot */
+    int warp_sums[32];
+    unsigned hist[256];
+    unsigned prefix;
+    int need;
+};
+
+__global__ void __launch_bounds__(NMSB_THREADS) k_merge_rois(const mars_box_t *boxes, const int32_t *counts, int box_stride, const int *tab,
+                                                            int n_frames, mars_box_t *out_all, int32_t *counts_out, float thresh, unsigned *scratch) {
+    __shared__ MergeShared sh;
+    const int f = blockIdx.x, tid = threadIdx.x;
+    const int r0 = tab[f], r1 = tab[f + 1];
+    const int *org = tab + n_frames + 1; /* (x, y) of region r at org[2r], org[2r + 1]: 4-byte aligned only */
+    auto key_of = [&](int r, int k) { return nms_conf_key(boxes[(size_t)r * box_stride + k].confidence); };
+    int total = 0;
+    for (int r = r0; r < r1; r++) total += min(counts[r], MARS_MAX_DETS);
+    /* select: candidates with key < thr, then the first `need` with key == thr */
+    unsigned thr = 0xFFFFFFFFu;
+    int need = 0x7FFFFFFF;
+    if (total > MERGE_CAP) {
+        unsigned prefix = 0u;
+        need = MERGE_CAP;
+        for (int shift = 24; shift >= 0; shift -= 8) {
+            const unsigned hi = shift == 24 ? 0u : 0xFFFFFFFFu << (shift + 8);
+            sh.hist[tid] = 0u;
+            __syncthreads();
+            for (int r = r0; r < r1; r++) {
+                const int c = min(counts[r], MARS_MAX_DETS);
+                for (int k = tid; k < c; k += NMSB_THREADS) {
+                    const unsigned u = key_of(r, k);
+                    if ((u & hi) == prefix) atomicAdd(&sh.hist[(u >> shift) & 255u], 1u);
+                }
+            }
+            __syncthreads();
+            const int h = (int)sh.hist[tid];
+            int sum;
+            const int before = block_excl_scan(h, &sum, sh.warp_sums);
+            if (before < need && before + h >= need) { sh.prefix = prefix | ((unsigned)tid << shift); sh.need = need - before; }
+            __syncthreads();
+            prefix = sh.prefix;
+            need = sh.need;
+        }
+        thr = prefix;
+    }
+    /* ordered compaction of the selection */
+    int eq_seen = 0, taken = 0;
+    for (int r = r0; r < r1; r++) {
+        const int c = min(counts[r], MARS_MAX_DETS);
+        for (int base = 0; base < c; base += NMSB_THREADS) {
+            const int k = base + tid;
+            const unsigned u = k < c ? key_of(r, k) : 0xFFFFFFFFu;
+            const bool eq = k < c && u == thr;
+            int n_eq, n_take;
+            const int eq_rank = eq_seen + block_excl_scan(eq ? 1 : 0, &n_eq, sh.warp_sums);
+            const bool take = k < c && (u < thr || (eq && eq_rank < need));
+            const int pos = taken + block_excl_scan(take ? 1 : 0, &n_take, sh.warp_sums);
+            if (take) sh.cand[pos] = (r << 10) | k;
+            eq_seen += n_eq;
+            taken += n_take;
+        }
+    }
+    __syncthreads();
+    mars_box_t *out = out_all + (size_t)f * MARS_MAX_DETS;
+    nms_corner_image(
+        sh.nms, taken, thresh, scratch + (size_t)f * NMS_SCRATCH_WORDS, &counts_out[f],
+        [&](int j) {
+            const int c = sh.cand[j], r = c >> 10;
+            mars_box_t b = boxes[(size_t)r * box_stride + (c & 1023)];
+            const float ox = (float)org[2 * r], oy = (float)org[2 * r + 1];
+            b.x0 = __fadd_rn(b.x0, ox); b.y0 = __fadd_rn(b.y0, oy);
+            b.x1 = __fadd_rn(b.x1, ox); b.y1 = __fadd_rn(b.y1, oy);
+            return b;
+        },
+        [out](int r, mars_box_t b) { out[r] = b; });
 }
 
 } // namespace marsb200

@@ -207,13 +207,16 @@ static const int32_t PRE_YUV_COEF[PRE_YUV_VARIANTS][6] = PRE_YUV_COEF_INIT;
 static __constant__ int32_t pre_yuv_coef[PRE_YUV_VARIANTS][6] = PRE_YUV_COEF_INIT;
 
 /* One frame of a ragged batch as the kernels see it.  A launch covers a run of frames that share the target size; each has
- * its own source format, geometry, row pitches, tap lists and float rows.  Offsets are relative to the launch (chunk). */
+ * its own source format, geometry, row pitches, tap lists and float rows.  Offsets are relative to the launch (chunk).
+ * A region of a larger frame is the ow x oh pixels at (ox, oy) of the frame that src / uv point at: the kernels read row
+ * oy + r and column ox + c of the full planes, so an NV12 region at an odd origin keeps the chroma of the frame's 2 x 2 blocks. */
 struct PreFrame {
     const uint8_t *src;  /* row 0 of the RGB8 frame, or of the NV12 luma plane (device) */
-    const uint8_t *uv;   /* NV12: row 0 of the chroma plane, ceil(oh / 2) rows of ceil(ow / 2) U,V pairs (device) */
-    size_t row_stride;   /* bytes from one row of src to the next (>= ow * 3 for RGB8, >= ow for NV12) */
-    size_t uv_stride;    /* NV12: bytes from one chroma row to the next (>= 2 * ceil(ow / 2)) */
+    const uint8_t *uv;   /* NV12: row 0 of the chroma plane, ceil(h / 2) rows of ceil(w / 2) U,V pairs of the w x h frame (device) */
+    size_t row_stride;   /* bytes from one row of src to the next (>= w * 3 for RGB8, >= w for NV12) */
+    size_t uv_stride;    /* NV12: bytes from one chroma row to the next (>= 2 * ceil(w / 2)) */
     size_t hoff;         /* its first float in the H scratch: oh x nw x 3 floats */
+    int ox, oy;          /* the region's origin in the frame (0, 0 for a whole frame) */
     int ow, oh, nw, nh, px, py;
     int hs, vs;          /* its first entry in the start list of the horizontal / vertical taps */
     int blk0;            /* its first block in the horizontal grid: blocks [blk0, blk0 + oh * ceil(nw / 128)) */
@@ -259,15 +262,17 @@ __global__ void __launch_bounds__(128) k_pre_horizontal(const PreFrame *fr, int 
     const PreFrame &d = fr[lo];
     const int nw = d.nw, bx = (nw + 127) >> 7, local = b - d.blk0, r = local / bx, x = (local - r * bx) * 128 + threadIdx.x;
     if (x >= nw) return;
-    const uint8_t *row = d.src + (size_t)r * d.row_stride;
+    const int sy = d.oy + r;
+    const uint8_t *row = d.src + (size_t)sy * d.row_stride;
     float a0 = 0.0f, a1 = 0.0f, a2 = 0.0f;
     const int k0 = t.start[d.hs + x], ke = t.start[d.hs + x + 1];
     if (d.fmt == PRE_NV12) {
-        const uint8_t *crow = d.uv + (size_t)(r >> 1) * d.uv_stride;
+        const uint8_t *crow = d.uv + (size_t)(sy >> 1) * d.uv_stride;
         const int *q = pre_yuv_coef[d.colour];
         const int y0 = q[0], cy = q[1], crv = q[2], cgu = q[3], cgv = q[4], cbu = q[5];
+        const int ox = d.ox;
         for (int k = k0; k < ke; k++) {
-            const int sx = t.src[k];
+            const int sx = ox + t.src[k];
             const uint8_t *p = crow + 2 * (sx >> 1);
             int c0, c1, c2;
             pre_nv12_rgb(row[sx], p[0], p[1], y0, cy, crv, cgu, cgv, cbu, &c0, &c1, &c2);
@@ -277,6 +282,7 @@ __global__ void __launch_bounds__(128) k_pre_horizontal(const PreFrame *fr, int 
             a2 = __fadd_rn(a2, __fmul_rn(dec[c2], c));
         }
     } else {
+        row += (size_t)d.ox * 3;
         for (int k = k0; k < ke; k++) {
             const uint8_t *p = row + (size_t)t.src[k] * 3;
             const float c = t.w[k];
@@ -342,24 +348,28 @@ __global__ void __launch_bounds__(128) k_pre_vertical_pack(const float *H, const
 static const size_t PRE_H_CHUNK_BYTES = (size_t)256 << 20;
 
 /* Host side of a ragged batch: the descriptors, the concatenated tap lists (one copy per distinct (in, out) of an axis) and
- * the launches.  Packed into one blob -- [PreFrame x n][start][src][w] -- that is copied to the device in one piece. */
+ * the launches.  Packed into one blob -- [PreFrame x n][start][src][w][merge] -- that is copied to the device in one piece.
+ * The entries of a table are frames, or regions of frames (then several entries read one staged frame). */
 struct PreTable {
     int tw = 0, th = 0;
     std::vector<PreFrame> fr;
-    std::vector<size_t> stage; /* byte offset of each frame in a tightly packed staging buffer (pre_frame_bytes each) */
+    std::vector<size_t> stage; /* byte offset of each source frame in a tightly packed staging buffer (pre_frame_bytes each) */
     std::vector<int> start, src;
     std::vector<float> w;
-    std::vector<int> first, blocks; /* launch k covers frames [first[k], first[k + 1]) with blocks[k] horizontal blocks */
+    std::vector<int> merge;         /* optional trailer: the region merge table of k_merge_rois, carried in the same upload */
+    std::vector<int> first, blocks; /* launch k covers entries [first[k], first[k + 1]) with blocks[k] horizontal blocks */
     size_t h_floats = 0;            /* H scratch of the largest launch */
-    size_t stage_bytes = 0;         /* staging of the largest launch (per_launch_staging) or of the whole batch */
+    size_t stage_bytes = 0;         /* staging of the largest launch (per_launch staging) or of every frame */
 
-    size_t bytes() const { return fr.size() * sizeof(PreFrame) + (start.size() + src.size()) * sizeof(int) + w.size() * sizeof(float); }
+    size_t merge_offset() const { return fr.size() * sizeof(PreFrame) + (start.size() + src.size()) * sizeof(int) + w.size() * sizeof(float); }
+    size_t bytes() const { return merge_offset() + merge.size() * sizeof(int); }
     void pack(void *out) const {
         uint8_t *p = (uint8_t *)out;
         memcpy(p, fr.data(), fr.size() * sizeof(PreFrame)); p += fr.size() * sizeof(PreFrame);
         memcpy(p, start.data(), start.size() * sizeof(int)); p += start.size() * sizeof(int);
         memcpy(p, src.data(), src.size() * sizeof(int)); p += src.size() * sizeof(int);
-        memcpy(p, w.data(), w.size() * sizeof(float));
+        memcpy(p, w.data(), w.size() * sizeof(float)); p += w.size() * sizeof(float);
+        memcpy(p, merge.data(), merge.size() * sizeof(int));
     }
     /* where the tap lists sit in the device copy of the blob */
     PreTaps taps(const void *dev) const {
@@ -368,17 +378,16 @@ struct PreTable {
     }
 };
 
-/* Builds the table for n frames (geometry g[f] from letterbox_geom, all into the same target; source format fmt[f], or all
- * RGB8 when fmt is null) whose source pointers, pitches and colour variants the caller fills in afterwards.  taps_of(in, out)
- * returns the ResizeTaps of one axis (the caller's cache).  Launches split where the cumulative H bytes (oh * nw * 12 per
- * frame) would pass PRE_H_CHUNK_BYTES; with per_launch_staging the staging offsets restart with every launch. */
+/* Builds the table for n entries (geometry g[f] from letterbox_geom, all into the same target; source format fmt[f], or all
+ * RGB8 when fmt is null) whose source pointers, pitches, origins and colour variants the caller fills in afterwards.
+ * taps_of(in, out) returns the ResizeTaps of one axis (the caller's cache).  Launches split where the cumulative H bytes
+ * (oh * nw * 12 per entry) would pass PRE_H_CHUNK_BYTES. */
 template <class TapsOf>
-static inline void pre_table_build(const LetterboxGeom *g, const int *fmt, int n, TapsOf taps_of, bool per_launch_staging, PreTable *t) {
+static inline void pre_table_build(const LetterboxGeom *g, const int *fmt, int n, TapsOf taps_of, PreTable *t) {
     *t = PreTable();
     if (n <= 0) return;
     t->tw = g[0].tw; t->th = g[0].th;
     t->fr.resize(n);
-    t->stage.resize(n);
     std::vector<std::pair<std::pair<int, int>, int>> seen; /* (in, out) -> its first entry in start */
     auto list = [&](int in, int out) {
         for (auto &s : seen)
@@ -391,7 +400,7 @@ static inline void pre_table_build(const LetterboxGeom *g, const int *fmt, int n
         seen.push_back({{in, out}, at});
         return at;
     };
-    size_t hbytes = 0, hfl = 0, soff = 0;
+    size_t hbytes = 0, hfl = 0;
     int blk = 0;
     for (int f = 0; f < n; f++) {
         const LetterboxGeom &q = g[f];
@@ -400,26 +409,37 @@ static inline void pre_table_build(const LetterboxGeom *g, const int *fmt, int n
             if (f > 0) t->blocks.push_back(blk);
             t->first.push_back(f);
             hbytes = 0; hfl = 0; blk = 0;
-            if (per_launch_staging) soff = 0;
         }
         PreFrame &d = t->fr[f];
         d.src = nullptr; d.uv = nullptr; d.row_stride = 0; d.uv_stride = 0;
         d.fmt = fmt ? fmt[f] : PRE_RGB8; d.colour = 0;
         d.hoff = hfl;
+        d.ox = 0; d.oy = 0;
         d.ow = q.ow; d.oh = q.oh; d.nw = q.nw; d.nh = q.nh; d.px = q.px; d.py = q.py;
         d.hs = list(q.ow, q.nw);
         d.vs = list(q.oh, q.nh);
         d.blk0 = blk;
-        t->stage[f] = soff;
         blk += q.oh * ((q.nw + 127) / 128);
         hbytes += need;
         hfl += need / sizeof(float);
-        soff += pre_frame_bytes(d.fmt, q.ow, q.oh);
         t->h_floats = std::max(t->h_floats, hfl);
-        t->stage_bytes = std::max(t->stage_bytes, soff);
     }
     t->blocks.push_back(blk);
     t->first.push_back(n);
+}
+
+/* staging offsets of the n_frames source frames (frame_bytes[f] = pre_frame_bytes each), packed back to back.  per_launch: the
+ * entries are the frames themselves and each launch stages its own frames, so the offsets restart with every launch. */
+static inline void pre_table_stage(PreTable *t, const size_t *frame_bytes, int n_frames, bool per_launch) {
+    t->stage.assign(n_frames, 0);
+    t->stage_bytes = 0;
+    size_t soff = 0;
+    for (int f = 0, k = 0; f < n_frames; f++) {
+        if (per_launch && k + 1 < (int)t->first.size() && f == t->first[k]) { soff = 0; k++; }
+        t->stage[f] = soff;
+        soff += frame_bytes[f];
+        t->stage_bytes = std::max(t->stage_bytes, soff);
+    }
 }
 
 /* launch k of a table whose blob was copied to dev: frames [first[k], first[k+1]) -> dst + f * slot_stride (dst = target of

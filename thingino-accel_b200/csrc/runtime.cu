@@ -203,6 +203,9 @@ struct Model {
     mars_box_t *d_box_raw = nullptr, *d_box = nullptr;
     int32_t *d_box_raw_cnt = nullptr, *d_box_cnt = nullptr;
     int2 *d_frame = nullptr;
+    /* frame records of the region merge (mars_b200_merge_rois_resident): capacity x MARS_MAX_DETS boxes, counts */
+    mars_box_t *d_fbox = nullptr;
+    int32_t *d_fbox_cnt = nullptr;
     DecodeTables *d_tab = nullptr;
     float tab_scale = 0.0f;
     bool tab_valid = false;
@@ -250,6 +253,7 @@ static void model_release(Model *m) {
     cudaFree(m->d_weights); cudaFree(m->d_slots); cudaFree(m->d_scratch); cudaFree(m->d_cpool); cudaFree(m->d_tc_scratch); cudaFree(m->d_linked);
     cudaFree(m->d_raw); cudaFree(m->d_det); cudaFree(m->d_raw_cnt); cudaFree(m->d_det_cnt); cudaFree(m->d_tab); cudaFree(m->d_nms_mask);
     cudaFree(m->d_box_raw); cudaFree(m->d_box); cudaFree(m->d_box_raw_cnt); cudaFree(m->d_box_cnt); cudaFree(m->d_frame);
+    cudaFree(m->d_fbox); cudaFree(m->d_fbox_cnt);
     if (m->h_arena) cudaFreeHost(m->h_arena);
     if (m->ev0) cudaEventDestroy(m->ev0);
     if (m->ev1) cudaEventDestroy(m->ev1);
@@ -309,6 +313,11 @@ static mars_error_t set_capacity(Model *m, int capacity) {
     CU_OK(cudaMalloc(&nbrc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaMalloc(&nbc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaMalloc(&nfr, (size_t)capacity * sizeof(int2)), MARS_ERR_ALLOC_FAILED);
+    mars_box_t *nfbox = nullptr;
+    int32_t *nfbc = nullptr;
+    CU_OK(cudaMalloc(&nfbox, (size_t)capacity * MARS_MAX_DETS * sizeof(mars_box_t)), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMalloc(&nfbc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMemsetAsync(nfbc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaMemsetAsync(nbrc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaMemsetAsync(nbc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaMemsetAsync(nfr, 0, (size_t)capacity * sizeof(int2), m->stream), MARS_ERR_ALLOC_FAILED);
@@ -318,6 +327,8 @@ static mars_error_t set_capacity(Model *m, int capacity) {
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     cudaFree(m->d_box_raw); cudaFree(m->d_box); cudaFree(m->d_box_raw_cnt); cudaFree(m->d_box_cnt); cudaFree(m->d_frame);
     m->d_box_raw = nbraw; m->d_box = nbox; m->d_box_raw_cnt = nbrc; m->d_box_cnt = nbc; m->d_frame = nfr;
+    cudaFree(m->d_fbox); cudaFree(m->d_fbox_cnt);
+    m->d_fbox = nfbox; m->d_fbox_cnt = nfbc;
     cudaFree(m->d_slots); cudaFree(m->d_scratch); cudaFree(m->d_raw); cudaFree(m->d_det);
     cudaFree(m->d_raw_cnt); cudaFree(m->d_det_cnt); cudaFree(m->d_nms_mask);
     m->d_nms_mask = nmask;
@@ -1320,6 +1331,73 @@ static mars_error_t pre_check_frames(Model *m, const char *what, const std::vect
     return MARS_OK;
 }
 
+/* the region table of a call (mars_b200_roi_t) */
+struct RoiList {
+    int n;
+    const mars_b200_roi_t *p;
+};
+
+/* Every region of a call is checked before any device work: frame in [0, n_frames) and not decreasing (the regions of a frame
+ * are contiguous: that fixes the concatenation order of the merge), x, y >= 0, w, h > 0, inside its frame (when there is a frame
+ * table), a letterbox at least one pixel wide and tall (when g is given: *g receives each region's geometry), and region r in
+ * slot first + r within the batch capacity. */
+static mars_error_t pre_check_rois(Model *m, const char *what, int first, int n_frames, const std::vector<FrameSrc> *frames, const RoiList &rois,
+                                   int tw, int th, std::vector<LetterboxGeom> *g) {
+    if (rois.n < 0 || (rois.n > 0 && !rois.p)) { set_last_error("%s: no region table for %d regions", what, rois.n); return MARS_ERR_INVALID_FILE; }
+    if (first < 0 || first + rois.n > m->capacity) {
+        const int r = first < 0 ? 0 : m->capacity - first;
+        set_last_error("%s: region %d: slot %d outside the batch capacity %d (mars_b200_set_batch)", what, r, first + r, m->capacity);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    if (g) g->resize(rois.n);
+    for (int r = 0; r < rois.n; r++) {
+        const mars_b200_roi_t &q = rois.p[r];
+        if (q.frame < 0 || q.frame >= n_frames) {
+            set_last_error("%s: region %d: frame %d outside [0, %d)", what, r, q.frame, n_frames);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (r > 0 && q.frame < rois.p[r - 1].frame) {
+            set_last_error("%s: region %d: frame %d after frame %d (the regions of a frame must be contiguous, frames ascending)", what, r,
+                           q.frame, rois.p[r - 1].frame);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (q.x < 0 || q.y < 0 || q.w <= 0 || q.h <= 0) {
+            set_last_error("%s: region %d: %d x %d at (%d, %d) is not a region", what, r, q.w, q.h, q.x, q.y);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (frames) {
+            const FrameSrc &a = (*frames)[q.frame];
+            if ((long long)q.x + q.w > a.w || (long long)q.y + q.h > a.h) {
+                set_last_error("%s: region %d: %d x %d at (%d, %d) reaches past frame %d (%d x %d)", what, r, q.w, q.h, q.x, q.y, q.frame, a.w, a.h);
+                return MARS_ERR_INVALID_TENSOR;
+            }
+        }
+        if (g) {
+            const LetterboxGeom lg = letterbox_geom(q.w, q.h, tw, th);
+            if (lg.nw <= 0 || lg.nh <= 0 || lg.nw > tw || lg.nh > th) {
+                set_last_error("%s: region %d: cannot letterbox %dx%d into %dx%d", what, r, q.w, q.h, tw, th);
+                return MARS_ERR_INVALID_TENSOR;
+            }
+            (*g)[r] = lg;
+        }
+    }
+    return MARS_OK;
+}
+
+/* the merge table of k_merge_rois for validated regions: the first region of each frame (n_frames + 1 entries), then (x, y) of
+ * each region */
+static void merge_table(int n_frames, const RoiList &rois, std::vector<int> *tab) {
+    tab->assign((size_t)n_frames + 1 + 2 * (size_t)rois.n, 0);
+    for (int f = 0, r = 0; f <= n_frames; f++) {
+        while (r < rois.n && rois.p[r].frame < f) r++;
+        (*tab)[f] = r;
+    }
+    for (int r = 0; r < rois.n; r++) {
+        (*tab)[n_frames + 1 + 2 * r] = rois.p[r].x;
+        (*tab)[n_frames + 2 + 2 * r] = rois.p[r].y;
+    }
+}
+
 static const ResizeTaps &cached_taps(Model *m, int in, int out) {
     const auto key = std::make_pair(in, out);
     auto it = m->pre_taps.find(key);
@@ -1373,42 +1451,14 @@ static cudaError_t pre_stage_frames(const PreTable &t, const FrameSrc *frames, i
     return cudaSuccess;
 }
 
-/* Letterboxes n validated frames (geometry g) into input tensor ti of slots [first, first+n) and records each slot's frame
- * size for the letterbox inverse; the launches go on the compute stream.
- *   PRE_HOST_SYNC : host frames staged launch by launch on the compute stream (the caller synchronises);
- *   PRE_DEVICE    : device frames read in place;
- *   PRE_HOST_POOL : host frames and the table copied on the copy stream, then ev_in, which the compute stream waits for. */
-static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, const std::vector<FrameSrc> &frames,
-                                      const std::vector<LetterboxGeom> &g, uint32_t ti, int nhwc, PreSource how, cudaEvent_t ev_in) {
-    const int n = (int)g.size();
-    if (n == 0) return MARS_OK;
-    if (m->pre_taps.size() > 64) m->pre_taps.clear();
-    std::vector<int> fmt(n);
-    for (int f = 0; f < n; f++) fmt[f] = frames[f].fmt;
-    PreTable t;
-    pre_table_build(g.data(), fmt.data(), n, [m](int in, int out) -> const ResizeTaps & { return cached_taps(m, in, out); }, how == PRE_HOST_SYNC, &t);
+/* the blob of t -> the stage's device table on stream s.  The pinned copy is rewritten only once the last upload from it has
+ * completed; growing the device table waits for the compute stream (pre_grow). */
+static mars_error_t pre_upload(Model *m, Model::PreStage &st, const PreTable &t, cudaStream_t s) {
     const size_t tab = t.bytes();
-    if ((how != PRE_DEVICE && !pre_grow(m, &st.d_frames, &st.frames_cap, t.stage_bytes)) || !pre_grow(m, &st.d_tab, &st.tab_cap, tab) ||
-        !pre_grow(m, (uint8_t **)&m->d_preH, &m->preH_cap, t.h_floats * sizeof(float))) {
-        set_last_error("preprocess: out of device memory for %d frames", n);
+    if (!pre_grow(m, &st.d_tab, &st.tab_cap, tab)) {
+        set_last_error("preprocess: out of device memory for a %zu-byte table", tab);
         return MARS_ERR_ALLOC_FAILED;
     }
-    for (int f = 0; f < n; f++) {
-        PreFrame &d = t.fr[f];
-        const FrameSrc &a = frames[f];
-        const bool nv12 = a.fmt == PRE_NV12;
-        d.colour = a.colour;
-        if (how == PRE_DEVICE) {
-            d.src = a.p0; d.uv = a.p1;
-            d.row_stride = a.pitch0; d.uv_stride = a.pitch1;
-        } else { /* the tight staging layout of pre_stage_frames */
-            d.src = st.d_frames + t.stage[f];
-            d.row_stride = (size_t)d.ow * (nv12 ? 1 : 3);
-            d.uv = nv12 ? d.src + (size_t)d.ow * d.oh : nullptr;
-            d.uv_stride = nv12 ? (size_t)2 * ((d.ow + 1) / 2) : 0;
-        }
-    }
-    /* the pinned table is rewritten only once the last upload from it has completed */
     CU_OK(cudaEventSynchronize(st.ev), MARS_ERR_LAYER_FAILED);
     if (tab > st.h_cap) {
         if (st.h_tab) cudaFreeHost(st.h_tab);
@@ -1417,17 +1467,70 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
         st.h_cap = tab;
     }
     t.pack(st.h_tab);
+    CU_OK(cudaMemcpyAsync(st.d_tab, st.h_tab, tab, cudaMemcpyHostToDevice, s), MARS_ERR_LAYER_FAILED);
+    CU_OK(cudaEventRecord(st.ev, s), MARS_ERR_LAYER_FAILED);
+    return MARS_OK;
+}
+
+/* Letterboxes validated frames into input tensor ti of slots first, first+1, ... and records each slot's source size for the
+ * letterbox inverse; the launches go on the compute stream.  Without rois slot first + f gets frame f (geometry g[f]); with
+ * rois slot first + r gets region r (geometry g[r]) of frame rois[r].frame -- each frame staged once, whatever its number of
+ * regions.  merge_tab (with rois): receives the device address of the merge table (merge_table), carried in the same upload.
+ *   PRE_HOST_SYNC : host frames staged on the compute stream, launch by launch without regions (the caller synchronises);
+ *   PRE_DEVICE    : device frames read in place;
+ *   PRE_HOST_POOL : host frames and the table copied on the copy stream, then ev_in, which the compute stream waits for. */
+static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, const std::vector<FrameSrc> &frames,
+                                      const std::vector<LetterboxGeom> &g, uint32_t ti, int nhwc, PreSource how, cudaEvent_t ev_in,
+                                      const RoiList *rois = nullptr, const int **merge_tab = nullptr) {
+    const int n = (int)g.size(), nfr = (int)frames.size();
+    if (n == 0) return MARS_OK;
+    if (m->pre_taps.size() > 64) m->pre_taps.clear();
+    auto frame_of = [rois](int e) { return rois ? rois->p[e].frame : e; };
+    std::vector<int> fmt(n);
+    for (int e = 0; e < n; e++) fmt[e] = frames[frame_of(e)].fmt;
+    PreTable t;
+    pre_table_build(g.data(), fmt.data(), n, [m](int in, int out) -> const ResizeTaps & { return cached_taps(m, in, out); }, &t);
+    std::vector<size_t> fbytes(nfr);
+    for (int f = 0; f < nfr; f++) fbytes[f] = pre_frame_bytes(frames[f].fmt, frames[f].w, frames[f].h);
+    const bool per_launch = how == PRE_HOST_SYNC && !rois;
+    pre_table_stage(&t, fbytes.data(), nfr, per_launch);
+    if (rois && merge_tab) merge_table(nfr, *rois, &t.merge);
+    if ((how != PRE_DEVICE && !pre_grow(m, &st.d_frames, &st.frames_cap, t.stage_bytes)) ||
+        !pre_grow(m, (uint8_t **)&m->d_preH, &m->preH_cap, t.h_floats * sizeof(float))) {
+        set_last_error("preprocess: out of device memory for %d frames", n);
+        return MARS_ERR_ALLOC_FAILED;
+    }
+    for (int e = 0; e < n; e++) {
+        PreFrame &d = t.fr[e];
+        const int f = frame_of(e);
+        const FrameSrc &a = frames[f];
+        const bool nv12 = a.fmt == PRE_NV12;
+        d.colour = a.colour;
+        if (rois) { d.ox = rois->p[e].x; d.oy = rois->p[e].y; }
+        if (how == PRE_DEVICE) {
+            d.src = a.p0; d.uv = a.p1;
+            d.row_stride = a.pitch0; d.uv_stride = a.pitch1;
+        } else { /* the tight staging layout of pre_stage_frames */
+            d.src = st.d_frames + t.stage[f];
+            d.row_stride = (size_t)a.w * (nv12 ? 1 : 3);
+            d.uv = nv12 ? d.src + (size_t)a.w * a.h : nullptr;
+            d.uv_stride = nv12 ? (size_t)2 * ((a.w + 1) / 2) : 0;
+        }
+    }
     cudaStream_t cs = how == PRE_HOST_POOL ? m->h2d_stream : m->stream;
-    CU_OK(cudaMemcpyAsync(st.d_tab, st.h_tab, tab, cudaMemcpyHostToDevice, cs), MARS_ERR_LAYER_FAILED);
-    CU_OK(cudaEventRecord(st.ev, cs), MARS_ERR_LAYER_FAILED);
-    if (how == PRE_HOST_POOL) {
-        CU_OK(pre_stage_frames(t, frames.data(), 0, n, st.d_frames, cs), MARS_ERR_LAYER_FAILED);
-        cudaEventRecord(ev_in, cs);
-        cudaStreamWaitEvent(m->stream, ev_in, 0);
+    mars_error_t e = pre_upload(m, st, t, cs);
+    if (e != MARS_OK) return e;
+    if (merge_tab) *merge_tab = reinterpret_cast<const int *>(st.d_tab + t.merge_offset());
+    if (how == PRE_HOST_POOL || (how == PRE_HOST_SYNC && !per_launch)) {
+        CU_OK(pre_stage_frames(t, frames.data(), 0, nfr, st.d_frames, cs), MARS_ERR_LAYER_FAILED);
+        if (how == PRE_HOST_POOL) {
+            cudaEventRecord(ev_in, cs);
+            cudaStreamWaitEvent(m->stream, ev_in, 0);
+        }
     }
     int8_t *dst = reinterpret_cast<int8_t *>(dev_addr(m, m->toff[ti], first));
     for (size_t k = 0; k + 1 < t.first.size(); k++) {
-        if (how == PRE_HOST_SYNC) CU_OK(pre_stage_frames(t, frames.data(), t.first[k], t.first[k + 1], st.d_frames, m->stream), MARS_ERR_LAYER_FAILED);
+        if (per_launch) CU_OK(pre_stage_frames(t, frames.data(), t.first[k], t.first[k + 1], st.d_frames, m->stream), MARS_ERR_LAYER_FAILED);
         CU_OK(launch_letterbox(t, (int)k, st.d_tab, m->d_preH, dst, m->slot_stride, nhwc, m->d_frame + first, m->stream), MARS_ERR_LAYER_FAILED);
         m->launches += 2;
     }
@@ -1435,18 +1538,29 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
 }
 
 /* the synchronous calls: validation, then copies + kernels as one device-timed region */
-static mars_error_t preprocess_sync(Model *m, const char *what, int first, int n, const std::vector<FrameSrc> *frames) {
+/* the checks of a letterbox call after its slot range: the target, the frames and (with rois) the regions; *g receives the
+ * geometry of each slot's source, frame or region */
+static mars_error_t pre_validate(Model *m, const char *what, int first, const std::vector<FrameSrc> *frames, const RoiList *rois, bool device,
+                                 uint32_t *ti, int *nhwc, std::vector<LetterboxGeom> *g) {
+    int tw, th;
+    mars_error_t e = pre_target(m, what, ti, &tw, &th, nhwc);
+    if (e == MARS_OK) e = pre_check_frames(m, what, frames, tw, th, device, g);
+    if (e == MARS_OK && rois) e = pre_check_rois(m, what, first, (int)frames->size(), frames, *rois, tw, th, g);
+    return e;
+}
+
+/* rois: slot first + r gets region r of the n frames (the regions check their own slot range) */
+static mars_error_t preprocess_sync(Model *m, const char *what, int first, int n, const std::vector<FrameSrc> *frames, const RoiList *rois = nullptr) {
     if (!m) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
+    if (!rois && !range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
     uint32_t ti;
-    int tw, th, nhwc;
-    mars_error_t e = pre_target(m, what, &ti, &tw, &th, &nhwc);
+    int nhwc;
     std::vector<LetterboxGeom> g;
-    if (e == MARS_OK) e = pre_check_frames(m, what, frames, tw, th, false, &g);
+    mars_error_t e = pre_validate(m, what, first, frames, rois, false, &ti, &nhwc, &g);
     if (e != MARS_OK) return e;
     cudaEventRecord(m->ev0, m->stream);
-    e = enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, *frames, g, ti, nhwc, PRE_HOST_SYNC, nullptr);
+    e = enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, *frames, g, ti, nhwc, PRE_HOST_SYNC, nullptr, rois);
     cudaEventRecord(m->ev1, m->stream);
     const cudaError_t ce = cudaStreamSynchronize(m->stream);
     if (e == MARS_OK && ce != cudaSuccess) {
@@ -1482,17 +1596,16 @@ mars_error_t mars_b200_preprocess_frames_nv12(mars_model_t *model, int first, in
 }
 
 /* the device-frame calls: validation, then the launches on the compute stream */
-static mars_error_t preprocess_device(Model *m, const char *what, int first, int n, const std::vector<FrameSrc> *frames) {
+static mars_error_t preprocess_device(Model *m, const char *what, int first, int n, const std::vector<FrameSrc> *frames, const RoiList *rois = nullptr) {
     if (!m) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
+    if (!rois && !range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
     uint32_t ti;
-    int tw, th, nhwc;
-    mars_error_t e = pre_target(m, what, &ti, &tw, &th, &nhwc);
+    int nhwc;
     std::vector<LetterboxGeom> g;
-    if (e == MARS_OK) e = pre_check_frames(m, what, frames, tw, th, true, &g);
+    mars_error_t e = pre_validate(m, what, first, frames, rois, true, &ti, &nhwc, &g);
     if (e != MARS_OK) return e;
-    return enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, *frames, g, ti, nhwc, PRE_DEVICE, nullptr);
+    return enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, *frames, g, ti, nhwc, PRE_DEVICE, nullptr, rois);
 }
 mars_error_t mars_b200_preprocess_frames_device(mars_model_t *model, int first, int n, const mars_b200_frame_t *frames) {
     std::vector<FrameSrc> s;
@@ -1501,6 +1614,50 @@ mars_error_t mars_b200_preprocess_frames_device(mars_model_t *model, int first, 
 mars_error_t mars_b200_preprocess_frames_nv12_device(mars_model_t *model, int first, int n, const mars_b200_nv12_frame_t *frames) {
     std::vector<FrameSrc> s;
     return preprocess_device(as_model(model), "preprocess_frames_nv12_device", first, n, nv12_sources(n, frames, &s));
+}
+
+/* regions of frames (mars_b200_tile_rois) -> one slot each */
+mars_error_t mars_b200_preprocess_rois(mars_model_t *model, int first, int n_frames, const mars_b200_frame_t *frames, int n_rois,
+                                       const mars_b200_roi_t *rois) {
+    std::vector<FrameSrc> s;
+    const RoiList rl{n_rois, rois};
+    return preprocess_sync(as_model(model), "preprocess_rois", first, n_frames, rgb_sources(n_frames, frames, &s), &rl);
+}
+mars_error_t mars_b200_preprocess_rois_nv12_device(mars_model_t *model, int first, int n_frames, const mars_b200_nv12_frame_t *frames,
+                                                   int n_rois, const mars_b200_roi_t *rois) {
+    std::vector<FrameSrc> s;
+    const RoiList rl{n_rois, rois};
+    return preprocess_device(as_model(model), "preprocess_rois_nv12_device", first, n_frames, nv12_sources(n_frames, frames, &s), &rl);
+}
+
+/* the region merge of frames [0, n_frames) of a call whose regions occupy slots [first, first + n_rois): tab = the merge table
+ * on the device; the kept boxes of the step's corner NMS in, frame records first + f out */
+static mars_error_t enqueue_merge(Model *m, int first, int n_frames, const int *tab, float thresh) {
+    if (n_frames <= 0) return MARS_OK;
+    k_merge_rois<<<n_frames, NMSB_THREADS, 0, m->stream>>>(m->d_box + (size_t)first * MARS_MAX_DETS, m->d_box_cnt + first, MARS_MAX_DETS, tab,
+                                                          n_frames, m->d_fbox + (size_t)first * MARS_MAX_DETS, m->d_fbox_cnt + first, thresh,
+                                                          m->d_nms_mask + (size_t)first * NMS_SCRATCH_WORDS);
+    m->launches++;
+    CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
+    return MARS_OK;
+}
+
+/* The merge reads the step's kept boxes and uses the suppression scratch rows of frame records [first, first + n_frames), free
+ * once the step's own NMS has run (stream order).  Enqueued on the compute stream. */
+mars_error_t mars_b200_merge_rois_resident(mars_model_t *model, int first, int n_frames, int n_rois, const mars_b200_roi_t *rois, float merge_thresh) {
+    Model *m = as_model(model);
+    if (!m) return MARS_ERR_INVALID_FILE;
+    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
+    if (!range_ok(m, first, n_frames)) return MARS_ERR_INVALID_TENSOR;
+    const RoiList rl{n_rois, rois};
+    mars_error_t e = pre_check_rois(m, "merge_rois_resident", first, n_frames, nullptr, rl, 0, 0, nullptr);
+    if (e != MARS_OK || n_frames == 0) return e;
+    PreTable t;
+    merge_table(n_frames, rl, &t.merge);
+    Model::PreStage &st = m->pre_stage[PRE_SYNC];
+    e = pre_upload(m, st, t, m->stream);
+    if (e != MARS_OK) return e;
+    return enqueue_merge(m, first, n_frames, reinterpret_cast<const int *>(st.d_tab), merge_thresh);
 }
 
 mars_error_t mars_b200_run_resident(mars_model_t *model, int first, int n) {
@@ -1667,12 +1824,15 @@ mars_error_t mars_b200_detect_heads_resident(mars_model_t *model, int first, int
 }
 
 /* kept records of slots [first, first+n): mars_det_t of the output0 path, or (boxes) mars_box_t of the heads path (both 24 bytes) */
-static mars_error_t copy_dets(Model *m, int first, int n, void *dets, int32_t *counts, int maxd, cudaStream_t s, bool boxes = false) {
+enum Records { REC_DETS, REC_BOXES, REC_FRAME_BOXES };
+static mars_error_t copy_dets(Model *m, int first, int n, void *dets, int32_t *counts, int maxd, cudaStream_t s, Records rec = REC_DETS) {
     static_assert(sizeof(mars_det_t) == sizeof(mars_box_t), "one record size");
     if (maxd > 1000) maxd = 1000;
     if (maxd < 0) maxd = 0;
-    const int32_t *dcnt = boxes ? m->d_box_cnt : m->d_det_cnt;
-    const void *drec = boxes ? (const void *)(m->d_box + (size_t)first * MARS_MAX_DETS) : (const void *)(m->d_det + (size_t)first * MARS_MAX_DETS);
+    const int32_t *dcnt = rec == REC_BOXES ? m->d_box_cnt : (rec == REC_FRAME_BOXES ? m->d_fbox_cnt : m->d_det_cnt);
+    const void *drec = rec == REC_BOXES ? (const void *)(m->d_box + (size_t)first * MARS_MAX_DETS)
+                     : rec == REC_FRAME_BOXES ? (const void *)(m->d_fbox + (size_t)first * MARS_MAX_DETS)
+                                              : (const void *)(m->d_det + (size_t)first * MARS_MAX_DETS);
     CU_OK(cudaMemcpyAsync(counts, dcnt + first, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
     if (maxd > 0)
         CU_OK(cudaMemcpy2DAsync(dets, (size_t)maxd * sizeof(mars_det_t), drec,
@@ -1681,22 +1841,25 @@ static mars_error_t copy_dets(Model *m, int first, int n, void *dets, int32_t *c
     return MARS_OK;
 }
 
-static mars_error_t download_records(mars_model_t *model, int first, int n, void *dets, int32_t *counts, int maxd, bool boxes) {
+static mars_error_t download_records(mars_model_t *model, int first, int n, void *dets, int32_t *counts, int maxd, Records rec) {
     Model *m = as_model(model);
     if (!m || !dets || !counts) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    mars_error_t e = copy_dets(m, first, n, dets, counts, maxd, m->stream, boxes);
+    mars_error_t e = copy_dets(m, first, n, dets, counts, maxd, m->stream, rec);
     if (e != MARS_OK) return e;
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     for (int i = 0; i < n; i++) if (counts[i] > maxd) counts[i] = maxd;
     return MARS_OK;
 }
 mars_error_t mars_b200_download_detections(mars_model_t *model, int first, int n, mars_det_t *dets, int32_t *counts, int maxd) {
-    return download_records(model, first, n, dets, counts, maxd, false);
+    return download_records(model, first, n, dets, counts, maxd, REC_DETS);
 }
 mars_error_t mars_b200_download_boxes(mars_model_t *model, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd) {
-    return download_records(model, first, n, boxes, counts, maxd, true);
+    return download_records(model, first, n, boxes, counts, maxd, REC_BOXES);
+}
+mars_error_t mars_b200_download_frame_boxes(mars_model_t *model, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd) {
+    return download_records(model, first, n, boxes, counts, maxd, REC_FRAME_BOXES);
 }
 
 /* end to end from host buffers, double-buffered over the two halves of the slot pool:
@@ -1764,14 +1927,23 @@ mars_error_t mars_b200_run_batch(mars_model_t *model, int n, const void *inputs,
  * detection records on the read-back stream -- and the call returns.  While it runs the caller submits the next batch to the
  * other half, so the host->device copy of batch k+1 and the read-back of batch k-1 overlap the kernels of batch k.
  * inputs / dets / counts must stay valid (and should be pinned, e.g. nna_malloc) until mars_b200_wait_batch(pool) returns. */
-/* what != NULL: inputs are letterboxed from the n host frames of `frames` instead (mars_b200_submit_frames_heads_batch) */
+/* what != NULL: inputs are letterboxed from the n host frames of `frames` instead (mars_b200_submit_frames_heads_batch); with rois
+ * from the n = rois->n regions of those frames, whose boxes are merged per frame after the step (k_merge_rois, merge_thresh) and
+ * read back as frames->size() frame records (mars_b200_submit_rois_heads_batch) */
 static mars_error_t submit_batch(Model *m, int pool, int n, const void *inputs, size_t in_stride, void *dets, int32_t *counts, int maxd,
-                                 float nms_thresh, int flavour, const std::vector<FrameSrc> *frames = nullptr, const char *what = nullptr) {
+                                 float nms_thresh, int flavour, const std::vector<FrameSrc> *frames = nullptr, const char *what = nullptr,
+                                 const RoiList *rois = nullptr, float merge_thresh = 0.0f) {
     if (!m || !(inputs || what) || !dets || !counts || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
     CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
     const int half = m->capacity / 2;
     if (half < 1 || n < 0 || n > half) {
-        set_last_error("submit_batch: %d images do not fit half of the slot pool (capacity %d; mars_b200_set_batch)", n, m->capacity);
+        set_last_error("submit_batch: %d %s do not fit half of the slot pool (capacity %d; mars_b200_set_batch)", n, rois ? "regions" : "images",
+                       m->capacity);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    const int nrec = rois ? (int)frames->size() : n; /* records read back */
+    if (rois && nrec > half) {
+        set_last_error("%s: %d frames do not fit half of the slot pool (capacity %d; mars_b200_set_batch)", what, nrec, m->capacity);
         return MARS_ERR_INVALID_TENSOR;
     }
     if (m->pending[pool].active) {
@@ -1784,19 +1956,19 @@ static mars_error_t submit_batch(Model *m, int pool, int n, const void *inputs, 
     if (in_stride < in_bytes) in_stride = in_bytes;
     const int first = pool * half;
     uint32_t ti = 0;
-    int tw = 0, th = 0, nhwc = 0;
+    int nhwc = 0;
     std::vector<LetterboxGeom> g;
     if (what) {
-        mars_error_t e = pre_target(m, what, &ti, &tw, &th, &nhwc);
-        if (e == MARS_OK) e = pre_check_frames(m, what, frames, tw, th, false, &g);
+        mars_error_t e = pre_validate(m, what, first, frames, rois, false, &ti, &nhwc, &g);
         if (e != MARS_OK) return e;
     }
     mars_error_t e = compile_model(m); /* also drops captured graphs of an older program (set_opt_level, set_depthwise_mode) */
     if (e != MARS_OK) return e;
     if (n > 0) {
         /* the half is free: its previous batch was waited for (read-back complete) before this call -- its staging too */
+        const int *merge_tab = nullptr;
         if (what) {
-            e = enqueue_letterbox(m, m->pre_stage[pool], first, *frames, g, ti, nhwc, PRE_HOST_POOL, m->ev_in[pool]);
+            e = enqueue_letterbox(m, m->pre_stage[pool], first, *frames, g, ti, nhwc, PRE_HOST_POOL, m->ev_in[pool], rois, rois ? &merge_tab : nullptr);
             if (e != MARS_OK) return e;
         } else {
             e = copy_io(m, first, n, const_cast<void *>(inputs), in_stride, 0, m->h2d_stream);
@@ -1805,15 +1977,18 @@ static mars_error_t submit_batch(Model *m, int pool, int n, const void *inputs, 
             cudaStreamWaitEvent(m->stream, m->ev_in[pool], 0);
         }
         e = enqueue_step_graphed(m, first, n, nms_thresh, flavour);
+        if (e == MARS_OK && rois) e = enqueue_merge(m, first, nrec, merge_tab, merge_thresh);
         if (e != MARS_OK) { cudaStreamSynchronize(m->stream); return e; }
         cudaEventRecord(m->ev_done[pool], m->stream);
         cudaStreamWaitEvent(m->d2h_stream, m->ev_done[pool], 0);
-        e = copy_dets(m, first, n, dets, counts, maxd, m->d2h_stream, flavour == STEP_HEADS);
+        e = copy_dets(m, first, nrec, dets, counts, maxd, m->d2h_stream, rois ? REC_FRAME_BOXES : (flavour == STEP_HEADS ? REC_BOXES : REC_DETS));
         if (e != MARS_OK) return e;
+    } else {
+        for (int i = 0; i < nrec; i++) counts[i] = 0; /* frames without regions */
     }
     cudaEventRecord(m->ev_out[pool], m->d2h_stream);
     m->pending[pool].active = true;
-    m->pending[pool].n = n; m->pending[pool].maxd = maxd; m->pending[pool].counts = counts;
+    m->pending[pool].n = nrec; m->pending[pool].maxd = maxd; m->pending[pool].counts = counts;
     return MARS_OK;
 }
 mars_error_t mars_b200_submit_batch(mars_model_t *model, int pool, int n, const void *inputs, size_t in_stride, mars_det_t *dets,
@@ -1849,6 +2024,30 @@ mars_error_t mars_b200_submit_frames_nv12_heads_batch(mars_model_t *model, int p
     std::vector<FrameSrc> s;
     return submit_frames_heads(as_model(model), "submit_frames_nv12_heads_batch", pool, n, nv12_sources(n, frames, &s), boxes, counts,
                                maxd, nms_thresh);
+}
+
+/* the tiled flow of mars_b200_submit_frames_heads_batch: regions of the frames letterboxed into the pool's slots, their boxes
+ * merged per frame (k_merge_rois) and read back per frame */
+static mars_error_t submit_rois_heads(Model *m, const char *what, int pool, const std::vector<FrameSrc> *frames, int n_rois, const mars_b200_roi_t *rois,
+                                      mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh, float merge_thresh) {
+    if (m && m->heads.empty()) { set_last_error("%s: no YOLO heads configured (mars_b200_set_yolo_heads)", what); return MARS_ERR_INVALID_TENSOR; }
+    if (m && !frames) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
+    const RoiList rl{n_rois, rois};
+    return submit_batch(m, pool, n_rois, nullptr, 0, boxes, counts, maxd, nms_thresh, STEP_HEADS, frames, what, &rl, merge_thresh);
+}
+mars_error_t mars_b200_submit_rois_heads_batch(mars_model_t *model, int pool, int n_frames, const mars_b200_frame_t *frames, int n_rois,
+                                               const mars_b200_roi_t *rois, mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh,
+                                               float merge_thresh) {
+    std::vector<FrameSrc> s;
+    return submit_rois_heads(as_model(model), "submit_rois_heads_batch", pool, rgb_sources(n_frames, frames, &s), n_rois, rois, boxes, counts,
+                             maxd, nms_thresh, merge_thresh);
+}
+mars_error_t mars_b200_submit_rois_nv12_heads_batch(mars_model_t *model, int pool, int n_frames, const mars_b200_nv12_frame_t *frames,
+                                                    int n_rois, const mars_b200_roi_t *rois, mars_box_t *boxes, int32_t *counts, int maxd,
+                                                    float nms_thresh, float merge_thresh) {
+    std::vector<FrameSrc> s;
+    return submit_rois_heads(as_model(model), "submit_rois_nv12_heads_batch", pool, nv12_sources(n_frames, frames, &s), n_rois, rois, boxes,
+                             counts, maxd, nms_thresh, merge_thresh);
 }
 
 /* mars_b200_submit_batch without the YOLO post-process: the raw output tensor 0 of every image is read back instead
