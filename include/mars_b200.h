@@ -157,6 +157,29 @@ int mars_b200_find_yolo_heads(const void *data, size_t size, uint32_t *tensor_id
  * conv output, has the wrong channel count or grid, a scale <= 0, or the heads are not produced in level order.  Recompiles and
  * drops captured graphs like mars_b200_set_opt_level. */
 mars_error_t mars_b200_set_yolo_heads(mars_model_t *m, const uint32_t *tensor_ids, int n, float conf_thresh);
+/* NanoDet GFL heads (this library's decode; the reference has no NanoDet code).  A GFL head is the int8 output of the 1x1 conv
+ * NanoDet shares between classification and regression, NCHW [1,C,gh,gw] or NHWC [1,gh,gw,C] with C = nc + 4 (reg_max + 1): nc
+ * class logits, then the distributions of the left, top, right and bottom distances, reg_max + 1 bins each.  Level k has stride
+ * 8 << k; 3 levels (NanoDet-m) or 4 (NanoDet-Plus).  Per cell: score = max over classes of sigmoid (label = the first class with
+ * that score), a candidate when score > conf_thresh; each distance is the expectation of the softmax of its bins, times the
+ * stride; the box is (cx - l, cy - t, cx + r, cy + b) clipped to the input, cx = (x + 0.5) * stride with
+ * MARS_B200_GFL_CENTRE_HALF (NanoDet-m), x * stride with MARS_B200_GFL_CENTRE_CORNER (NanoDet-Plus).  Every operation is one
+ * float32 rounding, exponentials come from host-built tables: the result is bit-exact to the C statement.  Candidates (at most
+ * 1000 per image, in (level, y, x) order) then go through the same corner NMS and letterbox inverse as the YOLOv5 heads, so
+ * every heads entry point below serves a model with GFL heads set. */
+#define MARS_B200_GFL_CENTRE_HALF 0
+#define MARS_B200_GFL_CENTRE_CORNER 1
+/* host only: tensor ids of the GFL head convs in stride order: per stride 8 / 16 / 32 / 64 the last 1x1 CONV2D without activation
+ * and without a compute reader that has nc + 4 (reg_max + 1) channels.  Returns 3 or 4, or 0 when the strides are not 8, 16, 32
+ * (, 64) */
+int mars_b200_find_gfl_heads(const void *data, size_t size, int nc, int reg_max, uint32_t *tensor_ids, int cap);
+/* decode these heads (n = 3 or 4, level k = stride 8 << k) inside every run, replacing YOLO heads if set; tensor_ids = NULL (n != 0):
+ * mars_b200_find_gfl_heads; n = 0: off.  MARS_ERR_INVALID_TENSOR (mars_b200_last_error) when a tensor is not an int8 4-D conv
+ * output, has the wrong channel count or grid, a scale <= 0 or not finite, lives in the weight blob, or the heads are not produced
+ * in level order; when nc < 1, reg_max is outside 1..16, centre is unknown or conf_thresh is not finite.  Recompiles and drops
+ * captured graphs only when something changed. */
+mars_error_t mars_b200_set_gfl_heads(mars_model_t *m, const uint32_t *tensor_ids, int n, int nc, int reg_max, int centre,
+                                     float conf_thresh);
 /* original frame size of slots [first, first+n) for the letterbox inverse (0 x 0: keep network coordinates, the default).
  * mars_b200_preprocess_batch and the frames calls record it as well. */
 mars_error_t mars_b200_set_frame_size(mars_model_t *m, int first, int n, int w, int h);
@@ -325,6 +348,10 @@ void mars_yolo_scale_detections(mars_box_t *dets, int n, int orig_w, int orig_h,
  * examples/yolo_detect.cpp:176-181).  head = int8 [3,gh,gw,85]; appends after `cnt`. */
 int mars_yolo_decode_anchor_grid(const int8_t *head, int gh, int gw, float scale, int level,
                                  float conf_thresh, mars_box_t *dets, int cnt, int maxd);
+/* the GFL decode of mars_b200_set_gfl_heads on one head: head = int8 [gh][gw][nc + 4 (reg_max + 1)] dequantised with `scale`,
+ * level stride `stride`, boxes clipped to net_w x net_h; appends after `cnt`, at most maxd in all.  Returns the new count */
+int mars_b200_decode_gfl(const int8_t *head, int gh, int gw, int nc, int reg_max, float scale, int stride, int centre, int net_w,
+                         int net_h, float conf_thresh, mars_box_t *dets, int cnt, int maxd);
 
 #ifdef __cplusplus
 }

@@ -221,6 +221,10 @@ SIGNATURES = {
     "mars_yolo_decode_anchor_grid": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_int, C.c_float, C.c_void_p, C.c_int, C.c_int]),
     "mars_b200_find_yolo_heads": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int]),
     "mars_b200_set_yolo_heads": (C.c_int, [PM, C.c_void_p, C.c_int, C.c_float]),
+    "mars_b200_find_gfl_heads": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_int]),
+    "mars_b200_set_gfl_heads": (C.c_int, [PM, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float]),
+    "mars_b200_decode_gfl": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int, C.c_int,
+                                       C.c_float, C.c_void_p, C.c_int, C.c_int]),
     "mars_b200_set_frame_size": (C.c_int, [PM, C.c_int, C.c_int, C.c_int, C.c_int]),
     "mars_b200_detect_heads_resident": (C.c_int, [PM, C.c_int, C.c_int, C.c_float]),
     "mars_b200_step_heads_resident": (C.c_int, [PM, C.c_int, C.c_int, C.c_float]),
@@ -590,6 +594,20 @@ class MarsModel:
             n = ids.size
         self._check(lib().mars_b200_set_yolo_heads(self.m, None if ids is None else ids.ctypes.data, n, conf_thresh), "set_yolo_heads")
 
+    def set_gfl_heads(self, tensor_ids=None, nc=80, reg_max=7, centre="half", conf_thresh=0.25, enable=True):
+        """decode NanoDet GFL head convs (3 or 4 levels, nc + 4 (reg_max + 1) channels) inside every run, replacing YOLO heads if set;
+        tensor_ids None: find them; centre "half" (NanoDet-m) or "corner" (NanoDet-Plus); enable=False switches decoding off"""
+        if not enable:
+            ids, n = None, 0
+        elif tensor_ids is None:
+            ids, n = None, 3
+        else:
+            ids = np.ascontiguousarray(tensor_ids, dtype=np.uint32)
+            n = ids.size
+        code = GFL_CENTRE[centre] if isinstance(centre, str) else int(centre)
+        self._check(lib().mars_b200_set_gfl_heads(self.m, None if ids is None else ids.ctypes.data, n, nc, reg_max, code, conf_thresh),
+                    "set_gfl_heads")
+
     def set_frame_size(self, first, n, w, h):
         """original frame size of slots [first, first+n) for the letterbox inverse (0, 0: network coordinates)"""
         self._check(lib().mars_b200_set_frame_size(self.m, first, n, w, h), "set_frame_size")
@@ -743,6 +761,17 @@ def find_yolo_heads(blob):
     return [int(v) for v in ids[:n]]
 
 
+GFL_CENTRE = {"half": 0, "corner": 1}  # MARS_B200_GFL_CENTRE_HALF / _CORNER
+
+
+def find_gfl_heads(blob, nc=80, reg_max=7):
+    """tensor ids of the NanoDet GFL head convs of a .mars blob in stride order 8 / 16 / 32 (/ 64), or [] (host only, no GPU)"""
+    b = bytes(blob)
+    ids = (C.c_uint32 * 4)()
+    n = lib().mars_b200_find_gfl_heads(b, len(b), nc, reg_max, ids, 4)
+    return [int(v) for v in ids[:n]]
+
+
 # ---- post-process on host arrays (runs on the device) ---------------------------------
 def parse_output(out_i8, npred, scale, maxd=1000):
     dets = np.zeros(max(maxd, 1), dtype=DET_DTYPE)
@@ -755,6 +784,20 @@ def nms(dets, thresh=0.45):
     d = np.ascontiguousarray(dets.copy())
     n = lib().mars_yolo_nms(d.ctypes.data, len(d), thresh)
     return d[:max(n, 0)].copy()
+
+
+def decode_gfl(head, nc, reg_max, scale, stride, net_w, net_h, conf_thresh=0.25, centre="half", dets=None, cnt=0, maxd=1000):
+    """GFL decode of one int8 [gh, gw, nc + 4 (reg_max + 1)] head on the device (k_gfl_decode): boxes appended after dets[:cnt]
+    (dets: BOX_DTYPE [>= maxd] or None), returns dets[:count]"""
+    h = np.ascontiguousarray(head, dtype=np.int8)
+    gh, gw, _ = h.shape
+    out = np.zeros(maxd, dtype=BOX_DTYPE)
+    if dets is not None and cnt:
+        out[:cnt] = dets[:cnt]
+    code = GFL_CENTRE[centre] if isinstance(centre, str) else int(centre)
+    n = lib().mars_b200_decode_gfl(h.ctypes.data, gh, gw, nc, reg_max, scale, stride, code, net_w, net_h, conf_thresh, out.ctypes.data,
+                                   cnt, maxd)
+    return out[:n].copy()
 
 
 def nms_boxes(boxes, thresh=0.45):

@@ -42,6 +42,7 @@ enum OpKind : int {
     OP_UPSAMPLE,       /* :1003-1044 */
     OP_LUT_I8,         /* fused chain of int8 unary layers as one table */
     OP_YOLO_HEAD,      /* anchor-grid decode of one YOLO head conv output (mars_b200_set_yolo_heads), right after the conv */
+    OP_GFL_HEAD,       /* GFL decode of one NanoDet head conv output (mars_b200_set_gfl_heads), right after the conv */
     OP_KIND_COUNT
 };
 
@@ -101,21 +102,32 @@ struct Op {
     int fwd_stream = -1;
     /* write/read extents for hazard analysis and bounds checks */
     int64_t wlo = 0, whi = 0;
-    /* OP_YOLO_HEAD: the head tensor is [in0, in0 + n) with grid oh x ow, `lut` = const-pool offset of its 256-float sigmoid table,
-     * f0 = confidence threshold, sh = stride (8 << head_level) */
-    int head_level = -1, head_nc = 0;
+    /* OP_YOLO_HEAD / OP_GFL_HEAD: the head tensor is [in0, in0 + n) with grid oh x ow, `lut` = const-pool offset of its 256-float
+     * sigmoid table (OP_GFL_HEAD: followed by the 256-float table E[d] = expf(-(d * scale))), f0 = confidence threshold,
+     * sh = stride (8 << head_level).  OP_GFL_HEAD: f2 = cell centre offset (0.5 or 0), iw x ih = network input size */
+    int head_level = -1, head_nc = 0, head_reg_max = 0;
     bool head_nhwc = false;
     std::string note;
 };
 
-/* one YOLOv5 Detect head as the layer table describes it */
-struct YoloHead {
+/* one detection head conv (YOLOv5 Detect or NanoDet GFL) as the layer table describes it */
+struct HeadTensor {
     uint32_t id = 0;   /* tensor id (mars_tensor_t.id) of the head conv's output */
     int tensor = -1;   /* its tensor table index */
     int layer = -1;    /* the CONV2D layer that writes it */
-    int nc = 0, gh = 0, gw = 0, stride = 0;
+    int channels = 0, nc = 0, gh = 0, gw = 0, stride = 0;
     bool nhwc = false;
     float scale = 0.0f;
+};
+
+/* the detection heads a model decodes inside its program: one kind or none (each setter replaces what is set) */
+enum HeadKind : int { HEADS_NONE = 0, HEADS_YOLO, HEADS_GFL };
+struct HeadSet {
+    int kind = HEADS_NONE;
+    std::vector<HeadTensor> heads; /* in level order */
+    float conf = 0.25f;
+    int reg_max = 0, centre = 0;   /* HEADS_GFL (centre: MARS_B200_GFL_CENTRE_*) */
+    bool empty() const { return heads.empty(); }
 };
 
 /* the three YOLOv5 Detect levels of reference examples/yolo_detect.cpp:176-181: stride and (w, h) of each of the level's anchors */
@@ -162,13 +174,25 @@ void build_sigmoid_table(float scale, float sig[256]);
 mars_error_t compile_program(const mars_header_t &h, const mars_runtime_tensor_t *tensors,
                              const mars_runtime_layer_t *layers, const std::vector<size_t> &toff,
                              size_t weights_size, size_t arena_size, int opt_level, int depthwise_mode,
-                             Program *out, int f32_mode = 0, const std::vector<YoloHead> *heads = nullptr, float head_conf = 0.25f);
+                             Program *out, int f32_mode = 0, const HeadSet *heads = nullptr);
 std::string describe_program(const Program &p);
 /* the outputs of the three CONV2D layers of a YOLOv5 Detect block in stride order 8 / 16 / 32 (host only); 0 when there are none */
 int find_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers, uint32_t *ids, int cap);
 /* checks n head tensor ids for mars_b200_set_yolo_heads: MARS_ERR_INVALID_TENSOR (with mars_b200_last_error) or MARS_OK + *out */
 mars_error_t resolve_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers,
-                                const std::vector<size_t> &toff, size_t weights_size, const uint32_t *ids, int n, std::vector<YoloHead> *out);
+                                const std::vector<size_t> &toff, size_t weights_size, const uint32_t *ids, int n, std::vector<HeadTensor> *out);
+/* the last 1x1 CONV2D per stride 8 / 16 / 32 (/ 64) with nc + 4 (reg_max + 1) channels, no activation and no compute reader, in
+ * stride order (host only); returns 3 or 4, or 0 when the strides found are not 8, 16, 32 (, 64) */
+int find_gfl_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers, int nc, int reg_max,
+                   uint32_t *ids, int cap);
+/* the parameters of mars_b200_set_gfl_heads: MARS_ERR_INVALID_TENSOR (with mars_b200_last_error) or MARS_OK */
+mars_error_t check_gfl_params(int nc, int reg_max, int centre, float conf);
+/* checks n GFL head tensor ids and the parameters for mars_b200_set_gfl_heads, like resolve_yolo_heads */
+mars_error_t resolve_gfl_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers,
+                               const std::vector<size_t> &toff, size_t weights_size, const uint32_t *ids, int n, int nc, int reg_max,
+                               int centre, float conf, std::vector<HeadTensor> *out);
+/* E[d] = expf(-(d * scale)) for d = 0..255: the host libm's expf, one rounding per operation (the GFL softmax) */
+void build_gfl_exp_table(float scale, float e[256]);
 
 } // namespace marsb200
 

@@ -12,6 +12,7 @@
  *                   threads per image for large batches, 1024 for small ones);
  *  k_head_decode  : anchor-grid decode (mgk-decompiler/test_yolo_inference.py:136-202) of one head level, reading the raw
  *                   head convolution where the program leaves it (OP_YOLO_HEAD, mars_b200_set_yolo_heads);
+ *  k_gfl_decode   : GFL decode of one NanoDet head level (ours; OP_GFL_HEAD, mars_b200_set_gfl_heads), the same placement;
  *  k_nms_corner_batch : nms() of reference examples/yolo_detect.cpp:152-173 (corner boxes), with the letterbox inverse;
  *  k_merge_rois   : the boxes of a frame's regions (tiled detection; ours, the reference does not tile) shifted into the frame and
  *                   merged by the same corner NMS (nms_corner_image, shared with k_nms_corner_batch);
@@ -618,6 +619,74 @@ __global__ void __launch_bounds__(256) k_head_decode(const int8_t *head, size_t 
             d.x0 = __fsub_rn(cx, hw); d.y0 = __fsub_rn(cy, hh); d.x1 = __fadd_rn(cx, hw); d.y1 = __fadd_rn(cy, hh);
             d.confidence = conf; d.class_id = best;
             out[rank] = d;
+        }
+        cnt += total;
+    }
+    if (threadIdx.x == 0) counts[blockIdx.x] = min(cnt, maxd);
+}
+
+/* ---- NanoDet GFL heads (ours: the reference has no NanoDet code) --------------------------------------------------------
+ * GFL decode of one level for every image of the launch: the head of image b is at head + b * img_stride, element (channel c, cell
+ * p = y * gw + x) at c * cstride + p * pstride (NCHW: cstride = gh * gw, pstride = 1, so a warp reads each class plane across
+ * adjacent x; NHWC: cstride = 1, pstride = C).  tab = sig[256] (sig[v+128] = 1/(1+expf(-(v*scale)))) then E[256] (E[d] =
+ * expf(-(d*scale))), both from the host.  Per cell, every operation one float32 rounding:
+ *   score = max_c sig[v_c], label = the first c with that score (floats compared: the table saturates); candidate when score >
+ *   conf_thresh;
+ *   side s (left, top, right, bottom): bins v_j (j = 0..R), e_j = E[vmax - v_j] (the softmax numerators), den = sum e_j and
+ *   dist = sum j * (e_j / den), both in j order; distance = dist * stride;
+ *   cx = (x + off) * stride; box (max(cx - l, 0), max(cy - t, 0), min(cx + r, net_w), min(cy + b, net_h)).
+ * The distribution bins are read only for candidates.  Candidates go to boxes[b][...] in (y, x) order, ordered compaction after
+ * the image's running count when `append` is set (else from 0), capped at maxd. */
+/* one side's distance: the expectation of the softmax of its nb bins q[j * cstride], times the stride */
+__device__ __forceinline__ float gfl_distance(const int8_t *q, int nb, int cstride, const float *E, float stride) {
+    int vmax = q[0];
+    for (int j = 1; j < nb; j++) vmax = max(vmax, (int)q[(size_t)j * cstride]);
+    float den = E[vmax - q[0]];
+    for (int j = 1; j < nb; j++) den = __fadd_rn(den, E[vmax - q[(size_t)j * cstride]]);
+    float dist = 0.0f;
+    for (int j = 0; j < nb; j++) dist = __fadd_rn(dist, __fmul_rn((float)j, __fdiv_rn(E[vmax - q[(size_t)j * cstride]], den)));
+    return __fmul_rn(dist, stride);
+}
+
+__global__ void __launch_bounds__(256) k_gfl_decode(const int8_t *head, size_t img_stride, int gh, int gw, int nc, int reg_max, int cstride,
+                                                    int pstride, const float *tab, float stride, float off, float net_w, float net_h,
+                                                    float conf_thresh, int append, mars_box_t *boxes, int32_t *counts, int box_stride,
+                                                    int maxd) {
+    __shared__ int warp_sums[32];
+    __shared__ float sig[256], E[256];
+    const int8_t *hb = head + (size_t)blockIdx.x * img_stride;
+    mars_box_t *out = boxes + (size_t)blockIdx.x * box_stride;
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) { sig[i] = tab[i]; E[i] = tab[256 + i]; }
+    const int P = gh * gw, nb = reg_max + 1;
+    int cnt = append ? min(counts[blockIdx.x], maxd) : 0;
+    __syncthreads(); /* the tables are in place and every thread has read the count before thread 0 rewrites it */
+    for (int base = 0; base < P && cnt < maxd; base += blockDim.x) {
+        const int cell = base + threadIdx.x;
+        int pass = 0, label = 0;
+        float score = 0.0f;
+        const int8_t *p = hb + (size_t)cell * pstride;
+        if (cell < P) {
+            score = sig[(int)p[0] + 128];
+            for (int c = 1; c < nc; c++) {
+                const float s = sig[(int)p[(size_t)c * cstride] + 128];
+                if (s > score) { score = s; label = c; }
+            }
+            pass = score > conf_thresh;
+        }
+        int total;
+        const int rank = cnt + block_excl_scan(pass, &total, warp_sums);
+        if (pass && rank < maxd) {
+            const int8_t *q = p + (size_t)nc * cstride;
+            const size_t side = (size_t)nb * cstride;
+            const float dl = gfl_distance(q, nb, cstride, E, stride), dt = gfl_distance(q + side, nb, cstride, E, stride);
+            const float dr = gfl_distance(q + 2 * side, nb, cstride, E, stride), db = gfl_distance(q + 3 * side, nb, cstride, E, stride);
+            const int y = cell / gw, x = cell - y * gw;
+            const float cx = __fmul_rn(__fadd_rn((float)x, off), stride), cy = __fmul_rn(__fadd_rn((float)y, off), stride);
+            mars_box_t b;
+            b.x0 = fmaxf(__fsub_rn(cx, dl), 0.0f); b.y0 = fmaxf(__fsub_rn(cy, dt), 0.0f);
+            b.x1 = fminf(__fadd_rn(cx, dr), net_w); b.y1 = fminf(__fadd_rn(cy, db), net_h);
+            b.confidence = score; b.class_id = label;
+            out[rank] = b;
         }
         cnt += total;
     }

@@ -55,6 +55,14 @@ void build_sigmoid_table(float scale, float sig[256]) {
     }
 }
 
+void build_gfl_exp_table(float scale, float e[256]) {
+    for (int d = 0; d < 256; d++) {
+        volatile float x = (float)d * scale;
+        volatile float r = expf(-x);
+        e[d] = r;
+    }
+}
+
 /* reference src/mars/mars_runtime.c:752-768 tabulated over the 256 possible inputs */
 static void build_sigmoid_lut(float in_scale, float out_scale_raw, int8_t lut[256]) {
     float os = out_scale_raw > 0 ? out_scale_raw : 1.0f;
@@ -521,25 +529,30 @@ static mars_error_t compile_concat(Ctx &c, int li, const mars_layer_t &L) {
 }
 
 
-/* ---- YOLOv5 Detect heads (mars_b200_set_yolo_heads) ------------------------------------------------------------------
+/* ---- detection heads (mars_b200_set_yolo_heads, mars_b200_set_gfl_heads) -------------------------------------------------
  * The compiler drops the Split / Pow / Constant nodes of the Detect block, so everything after the three head convolutions runs
  * over zero elements and output0 holds stale bytes (SURVEY Appendix B.2).  The detections are in the raw head convolutions
- * [1, 3 (5 + nc), gh, gw] (or [1, gh, gw, 3 (5 + nc)] with --nhwc).  The planner's round-robin buffers let later layers overwrite a
- * head, so each head is decoded by an op placed right after the op that completes it. */
+ * [1, 3 (5 + nc), gh, gw] (or [1, gh, gw, 3 (5 + nc)] with --nhwc).  A NanoDet graph keeps its GFL heads the same way:
+ * [1, nc + 4 (reg_max + 1), gh, gw] per level, of which at most one is a model output.  The planner's round-robin buffers let later
+ * layers overwrite a head, so each head is decoded by an op placed right after the op that completes it. */
+static const int YOLO_STRIDES[3] = {8, 16, 32};
+static const int GFL_STRIDES[4] = {8, 16, 32, 64};
 
-/* geometry of a head candidate: int8 [1,C,gh,gw] / [1,gh,gw,C] whose grid divides the network input by 8, 16 or 32.  Returns false
- * when the tensor does not have that shape; *why (optional) says what is wrong */
-static bool head_geometry(const mars_header_t &h, const mars_runtime_tensor_t *tensors, int ti, YoloHead *hd, const char **why) {
+/* geometry of a head candidate: int8 [1,C,gh,gw] / [1,gh,gw,C] whose channel count C passes `channels_ok(C, hd, why)` (which sets
+ * hd->nc) and whose grid divides the network input by one of strides[0..ns).  Returns false when the tensor does not have that
+ * shape; *why (optional) says what is wrong */
+template <class ChannelRule>
+static bool head_geometry(const mars_header_t &h, const mars_runtime_tensor_t *tensors, int ti, HeadTensor *hd, const char **why,
+                          const int *strides, int ns, const char *grid_why, ChannelRule channels_ok) {
     static const char *dummy;
     const char *&w = why ? *why : dummy;
     const mars_tensor_t &d = tensors[ti].desc;
     if (d.dtype != MARS_DTYPE_INT8 || d.ndims != 4 || d.shape[0] != 1) { w = "is not an int8 [1,C,gh,gw] / [1,gh,gw,C] tensor"; return false; }
     hd->nhwc = d.format == MARS_FORMAT_NHWC;
-    const int C = hd->nhwc ? d.shape[3] : d.shape[1];
+    hd->channels = hd->nhwc ? d.shape[3] : d.shape[1];
     hd->gh = hd->nhwc ? d.shape[1] : d.shape[2];
     hd->gw = hd->nhwc ? d.shape[2] : d.shape[3];
-    if (C < 18 || C % 3) { w = "does not have 3 * (5 + nc) channels (nc >= 1)"; return false; }
-    hd->nc = C / 3 - 5;
+    if (!channels_ok(hd->channels, hd, &w)) return false;
     hd->scale = d.scale;
     const uint32_t ii = h.num_inputs ? h.input_tensor_ids[0] : 0xFFFFFFFFu;
     if (ii >= h.num_tensors) { w = "belongs to a model without an input tensor"; return false; }
@@ -548,9 +561,28 @@ static bool head_geometry(const mars_header_t &h, const mars_runtime_tensor_t *t
     const int H = in_nhwc ? in.shape[1] : in.shape[2], W = in_nhwc ? in.shape[2] : in.shape[3];
     hd->stride = 0;
     if (hd->gh > 0 && hd->gw > 0 && H % hd->gh == 0 && W % hd->gw == 0 && H / hd->gh == W / hd->gw)
-        for (const YoloLevel &l : YOLO_LEVELS) if (H / hd->gh == l.stride) hd->stride = l.stride;
-    if (!hd->stride) { w = "has a grid that is not the input size divided by 8, 16 or 32"; return false; }
+        for (int k = 0; k < ns; k++) if (H / hd->gh == strides[k]) hd->stride = strides[k];
+    if (!hd->stride) { w = grid_why; return false; }
     return true;
+}
+
+static bool yolo_geometry(const mars_header_t &h, const mars_runtime_tensor_t *tensors, int ti, HeadTensor *hd, const char **why) {
+    return head_geometry(h, tensors, ti, hd, why, YOLO_STRIDES, 3, "has a grid that is not the input size divided by 8, 16 or 32",
+                         [](int C, HeadTensor *t, const char **w) {
+                             if (C < 18 || C % 3) { *w = "does not have 3 * (5 + nc) channels (nc >= 1)"; return false; }
+                             t->nc = C / 3 - 5;
+                             return true;
+                         });
+}
+
+static bool gfl_geometry(const mars_header_t &h, const mars_runtime_tensor_t *tensors, int ti, HeadTensor *hd, const char **why, int nc,
+                         int reg_max) {
+    return head_geometry(h, tensors, ti, hd, why, GFL_STRIDES, 4, "has a grid that is not the input size divided by 8, 16, 32 or 64",
+                         [nc, reg_max](int C, HeadTensor *t, const char **w) {
+                             if (C != nc + 4 * (reg_max + 1)) { *w = "does not have nc + 4 * (reg_max + 1) channels"; return false; }
+                             t->nc = nc;
+                             return true;
+                         });
 }
 
 /* the last CONV2D layer that writes tensor `id`, or -1 */
@@ -572,18 +604,23 @@ static bool read_by_compute(const mars_header_t &h, const mars_runtime_layer_t *
     return false;
 }
 
+/* true for a 1x1 CONV2D without activation whose output no compute layer reads: what a detection head conv looks like */
+static bool head_conv(const mars_header_t &h, const mars_runtime_layer_t *layers, const mars_layer_t &L) {
+    if ((int)L.type != MARS_LAYER_CONV2D || L.num_outputs < 1) return false;
+    const mars_conv_params_t &p = L.params.conv;
+    return p.kernel_h == 1 && p.kernel_w == 1 && p.activation == MARS_ACT_NONE && !read_by_compute(h, layers, L.output_tensor_ids[0]);
+}
+
 int find_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers, uint32_t *ids, int cap) {
     /* A Detect head is a 1x1 conv without activation whose output only the dropped decode layers read.  The last such conv fixes
      * nc; each stride then takes its last conv of that channel count. */
     int nc = -1, found[3] = {-1, -1, -1};
     for (uint32_t i = h.num_layers; i-- > 0;) {
         const mars_layer_t &L = layers[i].desc;
-        if ((int)L.type != MARS_LAYER_CONV2D || L.num_outputs < 1) continue;
-        const mars_conv_params_t &p = L.params.conv;
-        if (p.kernel_h != 1 || p.kernel_w != 1 || p.activation != MARS_ACT_NONE || read_by_compute(h, layers, L.output_tensor_ids[0])) continue;
+        if (!head_conv(h, layers, L)) continue;
         const int ti = find_tensor(h, tensors, L.output_tensor_ids[0]);
-        YoloHead hd;
-        if (ti < 0 || !head_geometry(h, tensors, ti, &hd, nullptr)) continue;
+        HeadTensor hd;
+        if (ti < 0 || !yolo_geometry(h, tensors, ti, &hd, nullptr)) continue;
         if (nc < 0) nc = hd.nc;
         if (hd.nc != nc) continue;
         for (int k = 0; k < 3; k++)
@@ -594,86 +631,158 @@ int find_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors
     return 3;
 }
 
-mars_error_t resolve_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers,
-                                const std::vector<size_t> &toff, size_t weights_size, const uint32_t *ids, int n, std::vector<YoloHead> *out) {
-    out->clear();
-    if (n != 3) {
-        set_last_error("set_yolo_heads: %d heads given; a YOLOv5 Detect block has 3 (n = 0 switches the decode off)", n);
-        return MARS_ERR_INVALID_TENSOR;
+int find_gfl_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers, int nc, int reg_max,
+                   uint32_t *ids, int cap) {
+    if (nc < 1 || reg_max < 1 || reg_max > 16) return 0;
+    int found[4] = {-1, -1, -1, -1};
+    for (uint32_t i = h.num_layers; i-- > 0;) {
+        const mars_layer_t &L = layers[i].desc;
+        if (!head_conv(h, layers, L)) continue;
+        const int ti = find_tensor(h, tensors, L.output_tensor_ids[0]);
+        HeadTensor hd;
+        if (ti < 0 || !gfl_geometry(h, tensors, ti, &hd, nullptr, nc, reg_max)) continue;
+        for (int k = 0; k < 4; k++)
+            if (hd.stride == GFL_STRIDES[k] && found[k] < 0) found[k] = (int)i;
     }
+    if (found[0] < 0 || found[1] < 0 || found[2] < 0) return 0;
+    const int n = found[3] < 0 ? 3 : 4;
+    for (int k = 0; k < n && k < cap; k++) if (ids) ids[k] = layers[found[k]].desc.output_tensor_ids[0];
+    return n;
+}
+
+/* the checks both setters make on n resolved heads: conv output, geometry (`geometry(ti, hd, why)`), scale, arena placement, level
+ * order and each level's stride (strides[k]) */
+template <class Geometry>
+static mars_error_t resolve_heads(const char *what, const mars_header_t &h, const mars_runtime_tensor_t *tensors,
+                                  const mars_runtime_layer_t *layers, const std::vector<size_t> &toff, size_t weights_size,
+                                  const uint32_t *ids, int n, const int *strides, Geometry geometry, std::vector<HeadTensor> *out) {
     for (int k = 0; k < n; k++) {
-        YoloHead hd;
+        HeadTensor hd;
         hd.id = ids[k];
         hd.tensor = find_tensor(h, tensors, ids[k]);
         hd.layer = hd.tensor < 0 ? -1 : producing_conv(h, layers, ids[k]);
         const char *why = "";
         if (hd.layer < 0) {
-            set_last_error("set_yolo_heads: head %d (tensor id %u) is not the output of a CONV2D layer", k, ids[k]);
+            set_last_error("%s: head %d (tensor id %u) is not the output of a CONV2D layer", what, k, ids[k]);
             return MARS_ERR_INVALID_TENSOR;
         }
-        if (!head_geometry(h, tensors, hd.tensor, &hd, &why)) {
-            set_last_error("set_yolo_heads: head %d (tensor id %u) %s", k, ids[k], why);
+        if (!geometry(hd.tensor, &hd, &why)) {
+            set_last_error("%s: head %d (tensor id %u) %s", what, k, ids[k], why);
             return MARS_ERR_INVALID_TENSOR;
         }
-        if (k > 0 && hd.nc != (*out)[0].nc) {
-            set_last_error("set_yolo_heads: head %d (tensor id %u) has %d channels, head 0 has %d: the channel count must be the same 3 * (5 + nc)",
-                           k, ids[k], 3 * (5 + hd.nc), 3 * (5 + (*out)[0].nc));
+        if (k > 0 && hd.channels != (*out)[0].channels) {
+            set_last_error("%s: head %d (tensor id %u) has %d channels, head 0 has %d: the channel count must be the same", what, k, ids[k],
+                           hd.channels, (*out)[0].channels);
             return MARS_ERR_INVALID_TENSOR;
         }
-        if (!(hd.scale > 0.0f) || !std::isfinite(hd.scale)) { /* the class argmax runs on raw bytes: it needs a monotone dequantisation */
-            set_last_error("set_yolo_heads: head %d (tensor id %u) has scale %g; the decode needs a finite scale > 0", k, ids[k], (double)hd.scale);
+        if (!(hd.scale > 0.0f) || !std::isfinite(hd.scale)) { /* the decodes need a monotone dequantisation */
+            set_last_error("%s: head %d (tensor id %u) has scale %g; the decode needs a finite scale > 0", what, k, ids[k], (double)hd.scale);
             return MARS_ERR_INVALID_TENSOR;
         }
         if (toff[hd.tensor] < weights_size) {
-            set_last_error("set_yolo_heads: head %d (tensor id %u) lives in the weight blob", k, ids[k]);
+            set_last_error("%s: head %d (tensor id %u) lives in the weight blob", what, k, ids[k]);
             return MARS_ERR_INVALID_TENSOR;
         }
         out->push_back(hd);
     }
-    const std::vector<YoloHead> &v = *out;
+    const std::vector<HeadTensor> &v = *out;
     for (int k = 1; k < n; k++)
         if (v[k].layer <= v[k - 1].layer) {
-            set_last_error("set_yolo_heads: head %d (layer %d) is not produced after head %d (layer %d): heads are decoded in level order",
+            set_last_error("%s: head %d (layer %d) is not produced after head %d (layer %d): heads are decoded in level order", what,
                            k, v[k].layer, k - 1, v[k - 1].layer);
             return MARS_ERR_INVALID_TENSOR;
         }
     for (int k = 0; k < n; k++)
-        if (v[k].stride != YOLO_LEVELS[k].stride) {
-            set_last_error("set_yolo_heads: head %d (tensor id %u) has stride %d; level %d needs stride %d", k, ids[k], v[k].stride, k, YOLO_LEVELS[k].stride);
+        if (v[k].stride != strides[k]) {
+            set_last_error("%s: head %d (tensor id %u) has stride %d; level %d needs stride %d", what, k, ids[k], v[k].stride, k, strides[k]);
             return MARS_ERR_INVALID_TENSOR;
         }
     return MARS_OK;
 }
 
-/* one OP_YOLO_HEAD behind the last op of each head's layer (its conv, or the byte-ReLU that follows it), with the head's sigmoid
- * table */
-static mars_error_t insert_yolo_heads(Ctx &c, const std::vector<YoloHead> &heads, float conf) {
+mars_error_t resolve_yolo_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers,
+                                const std::vector<size_t> &toff, size_t weights_size, const uint32_t *ids, int n, std::vector<HeadTensor> *out) {
+    out->clear();
+    if (n != 3) {
+        set_last_error("set_yolo_heads: %d heads given; a YOLOv5 Detect block has 3 (n = 0 switches the decode off)", n);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    return resolve_heads("set_yolo_heads", h, tensors, layers, toff, weights_size, ids, n, YOLO_STRIDES,
+                         [&](int ti, HeadTensor *hd, const char **why) { return yolo_geometry(h, tensors, ti, hd, why); }, out);
+}
+
+mars_error_t check_gfl_params(int nc, int reg_max, int centre, float conf) {
+    if (nc < 1) { set_last_error("set_gfl_heads: nc = %d; a GFL head has at least one class", nc); return MARS_ERR_INVALID_TENSOR; }
+    if (reg_max < 1 || reg_max > 16) {
+        set_last_error("set_gfl_heads: reg_max = %d is outside 1..16", reg_max);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    if (centre != MARS_B200_GFL_CENTRE_HALF && centre != MARS_B200_GFL_CENTRE_CORNER) {
+        set_last_error("set_gfl_heads: centre = %d is not MARS_B200_GFL_CENTRE_HALF or MARS_B200_GFL_CENTRE_CORNER", centre);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    if (!std::isfinite(conf)) { set_last_error("set_gfl_heads: conf_thresh %g is not finite", (double)conf); return MARS_ERR_INVALID_TENSOR; }
+    return MARS_OK;
+}
+
+mars_error_t resolve_gfl_heads(const mars_header_t &h, const mars_runtime_tensor_t *tensors, const mars_runtime_layer_t *layers,
+                               const std::vector<size_t> &toff, size_t weights_size, const uint32_t *ids, int n, int nc, int reg_max,
+                               int centre, float conf, std::vector<HeadTensor> *out) {
+    out->clear();
+    mars_error_t e = check_gfl_params(nc, reg_max, centre, conf);
+    if (e != MARS_OK) return e;
+    if (n != 3 && n != 4) {
+        set_last_error("set_gfl_heads: %d heads given; a GFL head has 3 or 4 levels (n = 0 switches the decode off)", n);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    return resolve_heads("set_gfl_heads", h, tensors, layers, toff, weights_size, ids, n, GFL_STRIDES,
+                         [&](int ti, HeadTensor *hd, const char **why) { return gfl_geometry(h, tensors, ti, hd, why, nc, reg_max); }, out);
+}
+
+/* one OP_YOLO_HEAD / OP_GFL_HEAD behind the last op of each head's layer (its conv, or the byte-ReLU that follows it), with the
+ * head's tables */
+static mars_error_t insert_heads(Ctx &c, const HeadSet &hs) {
     std::vector<Op> &ops = c.prog->ops;
-    for (size_t k = heads.size(); k-- > 0;) {
-        const YoloHead &hd = heads[k];
+    const bool gfl = hs.kind == HEADS_GFL;
+    const mars_tensor_t &in = c.tensors[c.h.input_tensor_ids[0]].desc; /* checked by the setters */
+    const bool in_nhwc = in.format == MARS_FORMAT_NHWC;
+    for (size_t k = hs.heads.size(); k-- > 0;) {
+        const HeadTensor &hd = hs.heads[k];
         size_t at = 0;
         for (size_t i = ops.size(); i-- > 0;)
             if (ops[i].layer == hd.layer) { at = i + 1; break; }
-        if (!at) { set_last_error("YOLO head %zu: layer %d compiled to no device op", k, hd.layer); return MARS_ERR_INVALID_TENSOR; }
+        if (!at) { set_last_error("detection head %zu: layer %d compiled to no device op", k, hd.layer); return MARS_ERR_INVALID_TENSOR; }
         Op o;
-        o.kind = OP_YOLO_HEAD;
+        o.kind = gfl ? OP_GFL_HEAD : OP_YOLO_HEAD;
         o.layer = hd.layer;
         o.in0 = c.off(hd.tensor);
-        o.oc = 3 * (5 + hd.nc); o.oh = hd.gh; o.ow = hd.gw;
+        o.oc = hd.channels; o.oh = hd.gh; o.ow = hd.gw;
         o.sh = o.sw = hd.stride;
         o.n = (uint64_t)o.oc * hd.gh * hd.gw;
-        o.f0 = conf; o.f1 = hd.scale;
+        o.f0 = hs.conf; o.f1 = hd.scale;
         o.head_level = (int)k; o.head_nc = hd.nc; o.head_nhwc = hd.nhwc;
         mars_error_t e;
         if ((e = check_read(c, hd.layer, o.in0, o.in0 + (int64_t)o.n))) return e;
-        float sig[256];
-        build_sigmoid_table(hd.scale, sig);
-        o.lut = (int)c.prog->const_pool.size(); /* four 256-byte units, float-aligned */
-        c.prog->const_pool.resize(c.prog->const_pool.size() + sizeof sig);
-        memcpy(&c.prog->const_pool[o.lut], sig, sizeof sig);
-        char note[160];
-        snprintf(note, sizeof note, "level %zu stride %d nc %d %s conf %g: decodes [in, in+n), the head store is kept", k, hd.stride, hd.nc,
-                 hd.nhwc ? "nhwc" : "nchw", (double)conf);
+        float tab[512];
+        build_sigmoid_table(hd.scale, tab);
+        if (gfl) build_gfl_exp_table(hd.scale, tab + 256);
+        const size_t bytes = (gfl ? 512 : 256) * sizeof(float);
+        o.lut = (int)c.prog->const_pool.size(); /* 256-byte units, float-aligned */
+        c.prog->const_pool.resize(c.prog->const_pool.size() + bytes);
+        memcpy(&c.prog->const_pool[o.lut], tab, bytes);
+        char note[192];
+        if (gfl) {
+            o.head_reg_max = hs.reg_max;
+            o.f2 = hs.centre == MARS_B200_GFL_CENTRE_HALF ? 0.5f : 0.0f;
+            o.ih = in_nhwc ? in.shape[1] : in.shape[2];
+            o.iw = in_nhwc ? in.shape[2] : in.shape[3];
+            snprintf(note, sizeof note, "level %zu stride %d nc %d reg_max %d %s centre %s conf %g: decodes [in, in+n), the head store is kept",
+                     k, hd.stride, hd.nc, hs.reg_max, hd.nhwc ? "nhwc" : "nchw", hs.centre == MARS_B200_GFL_CENTRE_HALF ? "half" : "corner",
+                     (double)hs.conf);
+        } else {
+            snprintf(note, sizeof note, "level %zu stride %d nc %d %s conf %g: decodes [in, in+n), the head store is kept", k, hd.stride, hd.nc,
+                     hd.nhwc ? "nhwc" : "nchw", (double)hs.conf);
+        }
         o.note = note;
         ops.insert(ops.begin() + (ptrdiff_t)at, o);
     }
@@ -908,7 +1017,7 @@ static void op_access(const Op &o, Access *a) {
             if (o.ic == o.oc) K(o.out + o.coff, (int64_t)o.n); /* strided writes kill nothing (conservative) */
             break;
         case OP_CONCAT_PERIODIC: R(o.out, o.coff); K(o.out + o.coff, (int64_t)o.n); break;
-        case OP_YOLO_HEAD: R(o.in0, (int64_t)o.n); break; /* keeps the head conv's store alive through dead-store elision */
+        case OP_YOLO_HEAD: case OP_GFL_HEAD: R(o.in0, (int64_t)o.n); break; /* keeps the head conv's store alive through dead-store elision */
         default: break;
     }
 }
@@ -1005,7 +1114,7 @@ static void elide_dead_stores(Program *p, const IvSet &observed, const IvSet &ho
 mars_error_t compile_program(const mars_header_t &h, const mars_runtime_tensor_t *tensors,
                              const mars_runtime_layer_t *layers, const std::vector<size_t> &toff,
                              size_t weights_size, size_t arena_size, int opt_level, int depthwise_mode,
-                             Program *out, int f32_mode, const std::vector<YoloHead> *heads, float head_conf) {
+                             Program *out, int f32_mode, const HeadSet *heads) {
     out->ops.clear();
     out->const_pool.clear();
     out->scratch_bytes = 0;
@@ -1036,7 +1145,7 @@ mars_error_t compile_program(const mars_header_t &h, const mars_runtime_tensor_t
         if (e != MARS_OK) return e;
     }
     if (heads && !heads->empty()) {
-        mars_error_t e = insert_yolo_heads(c, *heads, head_conf);
+        mars_error_t e = insert_heads(c, *heads);
         if (e != MARS_OK) return e;
     }
     if (opt_level >= 1) select_tensor_core_convs(out, f32_mode);
@@ -1068,7 +1177,7 @@ static const char *kind_name(int k) {
     static const char *n[] = {"nop", "conv_i8_nchw", "conv_i8_nhwc", "conv_f32_nchw", "dw_i8", "byte_relu",
                               "sigmoid_i8", "sigmoid_f32", "mul_i8", "add_i8", "mul_f32", "add_f32", "relu_i8",
                               "relu_f32", "bn_i8", "bn_f32", "maxpool", "concat", "concat_periodic", "upsample", "lut_i8",
-                              "yolo_head"};
+                              "yolo_head", "gfl_head"};
     return (k >= 0 && k < OP_KIND_COUNT) ? n[k] : "?";
 }
 static const char *mode_name(int m) {

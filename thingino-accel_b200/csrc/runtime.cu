@@ -197,9 +197,9 @@ struct Model {
     mars_det_t *d_raw = nullptr, *d_det = nullptr;
     int32_t *d_raw_cnt = nullptr, *d_det_cnt = nullptr;
     unsigned *d_nms_mask = nullptr; /* capacity x 1024 x 32 words: suppression bit matrices */
-    /* YOLO heads (mars_b200_set_yolo_heads): decoded candidates, kept boxes, and the original frame size per slot (0 = none) */
-    std::vector<YoloHead> heads;
-    float head_conf = 0.25f;
+    /* detection heads (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads): decoded candidates, kept boxes, and the original frame
+     * size per slot (0 = none) */
+    HeadSet heads;
     mars_box_t *d_box_raw = nullptr, *d_box = nullptr;
     int32_t *d_box_raw_cnt = nullptr, *d_box_cnt = nullptr;
     int2 *d_frame = nullptr;
@@ -353,7 +353,7 @@ static mars_error_t compile_model(Model *m) {
     release_graphs(m); /* kernel parameters (slot addresses, tensor maps, tables) are about to change */
     Program p;
     mars_error_t e = compile_program(m->pub.header, m->pub.tensors, m->pub.layers, m->toff, m->weights_size,
-                                     m->arena_size, m->opt_level, m->depthwise_mode, &p, m->f32_mode, &m->heads, m->head_conf);
+                                     m->arena_size, m->opt_level, m->depthwise_mode, &p, m->f32_mode, &m->heads);
     if (e != MARS_OK) return e;
     m->prog = std::move(p);
     cudaFree(m->d_cpool);
@@ -474,6 +474,16 @@ static mars_error_t launch_op(Model *m, size_t op_index, int first, int n, bool 
                                                 o.head_nhwc ? C : 1, reinterpret_cast<const float *>(m->d_cpool + o.lut), (float)o.sh,
                                                 YOLO_LEVELS[o.head_level].anchors, o.f0, o.head_level > 0, m->d_box_raw + (size_t)first * MARS_MAX_DETS,
                                                 m->d_box_raw_cnt + first, MARS_MAX_DETS, HEAD_MAX_CAND);
+        m->launches++;
+        CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
+        return MARS_OK;
+    }
+    if (o.kind == OP_GFL_HEAD) {
+        k_gfl_decode<<<n, 256, 0, m->stream>>>(reinterpret_cast<const int8_t *>(dev_addr(m, (size_t)o.in0, first)), m->slot_stride, o.oh, o.ow,
+                                               o.head_nc, o.head_reg_max, o.head_nhwc ? 1 : o.oh * o.ow, o.head_nhwc ? o.oc : 1,
+                                               reinterpret_cast<const float *>(m->d_cpool + o.lut), (float)o.sh, o.f2, (float)o.iw, (float)o.ih,
+                                               o.f0, o.head_level > 0, m->d_box_raw + (size_t)first * MARS_MAX_DETS, m->d_box_raw_cnt + first,
+                                               MARS_MAX_DETS, HEAD_MAX_CAND);
         m->launches++;
         CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
         return MARS_OK;
@@ -669,13 +679,13 @@ static mars_error_t enqueue_detect(Model *m, int first, int n, float thresh) {
     return MARS_OK;
 }
 
-/* corner NMS + letterbox inverse over the candidates the program's OP_YOLO_HEAD ops left for slots [first, first+n) */
+/* corner NMS + letterbox inverse over the candidates the program's OP_YOLO_HEAD / OP_GFL_HEAD ops left for slots [first, first+n) */
 static mars_error_t enqueue_heads_nms(Model *m, int first, int n, float thresh) {
     if (m->heads.empty()) {
-        set_last_error("no YOLO heads configured (mars_b200_set_yolo_heads)");
+        set_last_error("no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)");
         return MARS_ERR_INVALID_TENSOR;
     }
-    const mars_tensor_t &in = m->pub.tensors[m->pub.header.input_tensor_ids[0]].desc; /* checked by set_yolo_heads */
+    const mars_tensor_t &in = m->pub.tensors[m->pub.header.input_tensor_ids[0]].desc; /* checked by the heads setters */
     const bool nhwc = in.format == MARS_FORMAT_NHWC;
     const int net_h = nhwc ? in.shape[1] : in.shape[2], net_w = nhwc ? in.shape[2] : in.shape[3];
     k_nms_corner_batch<<<n, NMSB_THREADS, 0, m->stream>>>(m->d_box_raw + (size_t)first * MARS_MAX_DETS, m->d_box_raw_cnt + first,
@@ -754,22 +764,40 @@ size_t mars_b200_plan_describe(const void *data, size_t size, size_t arena_bytes
     return s.size();
 }
 
+/* the header, tensor and layer tables of a .mars blob, without touching a device; false when it is not one */
+static bool parse_tables(const void *data, size_t size, mars_header_t *h, std::vector<mars_runtime_tensor_t> *tensors,
+                         std::vector<mars_runtime_layer_t> *layers) {
+    if (!data || size < sizeof(mars_header_t)) return false;
+    memcpy(h, data, sizeof *h);
+    if (h->magic != MARS_MAGIC || h->version_major != MARS_VERSION_MAJOR) return false;
+    const size_t tables = sizeof *h + (size_t)h->num_tensors * sizeof(mars_tensor_t) + (size_t)h->num_layers * sizeof(mars_layer_t);
+    if (size < tables) return false;
+    tensors->assign(h->num_tensors ? h->num_tensors : 1, mars_runtime_tensor_t());
+    layers->assign(h->num_layers ? h->num_layers : 1, mars_runtime_layer_t());
+    memset(tensors->data(), 0, tensors->size() * sizeof(mars_runtime_tensor_t));
+    memset(layers->data(), 0, layers->size() * sizeof(mars_runtime_layer_t));
+    const uint8_t *p = (const uint8_t *)data + sizeof *h;
+    for (uint32_t i = 0; i < h->num_tensors; i++, p += sizeof(mars_tensor_t)) memcpy(&(*tensors)[i].desc, p, sizeof(mars_tensor_t));
+    for (uint32_t i = 0; i < h->num_layers; i++, p += sizeof(mars_layer_t)) memcpy(&(*layers)[i].desc, p, sizeof(mars_layer_t));
+    return true;
+}
+
 /* The outputs of the three CONV2D layers of a YOLOv5 Detect block, stride 8 / 16 / 32, without touching a device */
 int mars_b200_find_yolo_heads(const void *data, size_t size, uint32_t *tensor_ids, int cap) {
-    if (!data || size < sizeof(mars_header_t)) return 0;
     mars_header_t h;
-    memcpy(&h, data, sizeof h);
-    if (h.magic != MARS_MAGIC || h.version_major != MARS_VERSION_MAJOR) return 0;
-    const size_t tables = sizeof h + (size_t)h.num_tensors * sizeof(mars_tensor_t) + (size_t)h.num_layers * sizeof(mars_layer_t);
-    if (size < tables) return 0;
-    std::vector<mars_runtime_tensor_t> tensors(h.num_tensors ? h.num_tensors : 1);
-    std::vector<mars_runtime_layer_t> layers(h.num_layers ? h.num_layers : 1);
-    memset(tensors.data(), 0, tensors.size() * sizeof(mars_runtime_tensor_t));
-    memset(layers.data(), 0, layers.size() * sizeof(mars_runtime_layer_t));
-    const uint8_t *p = (const uint8_t *)data + sizeof h;
-    for (uint32_t i = 0; i < h.num_tensors; i++, p += sizeof(mars_tensor_t)) memcpy(&tensors[i].desc, p, sizeof(mars_tensor_t));
-    for (uint32_t i = 0; i < h.num_layers; i++, p += sizeof(mars_layer_t)) memcpy(&layers[i].desc, p, sizeof(mars_layer_t));
+    std::vector<mars_runtime_tensor_t> tensors;
+    std::vector<mars_runtime_layer_t> layers;
+    if (!parse_tables(data, size, &h, &tensors, &layers)) return 0;
     return find_yolo_heads(h, tensors.data(), layers.data(), tensor_ids, cap);
+}
+
+/* The NanoDet GFL head convs, stride 8 / 16 / 32 (/ 64), without touching a device */
+int mars_b200_find_gfl_heads(const void *data, size_t size, int nc, int reg_max, uint32_t *tensor_ids, int cap) {
+    mars_header_t h;
+    std::vector<mars_runtime_tensor_t> tensors;
+    std::vector<mars_runtime_layer_t> layers;
+    if (!parse_tables(data, size, &h, &tensors, &layers)) return 0;
+    return find_gfl_heads(h, tensors.data(), layers.data(), nc, reg_max, tensor_ids, cap);
 }
 
 mars_error_t mars_load_memory(const void *data, size_t size, mars_model_t **out_model) {
@@ -1115,10 +1143,24 @@ void mars_b200_set_opt_level(mars_model_t *model, int level) {
 }
 void mars_b200_set_strict(int on) { g_strict = on ? 1 : 0; }
 
+/* make `hs` the model's detection heads; recompiles (and drops the captured graphs) only when something changed */
+static mars_error_t replace_heads(Model *m, HeadSet hs) {
+    const HeadSet &o = m->heads;
+    bool same = hs.kind == o.kind && hs.heads.size() == o.heads.size() &&
+                (hs.empty() || (memcmp(&hs.conf, &o.conf, 4) == 0 && hs.reg_max == o.reg_max && hs.centre == o.centre));
+    for (size_t k = 0; same && k < hs.heads.size(); k++) same = hs.heads[k].id == o.heads[k].id && hs.heads[k].nc == o.heads[k].nc;
+    if (same) return MARS_OK;
+    cudaSetDevice(m->device);
+    cudaStreamSynchronize(m->stream);
+    m->heads = std::move(hs);
+    m->compiled = false; /* the next call recompiles and drops the captured graphs */
+    return MARS_OK;
+}
+
 mars_error_t mars_b200_set_yolo_heads(mars_model_t *model, const uint32_t *tensor_ids, int n, float conf_thresh) {
     Model *m = as_model(model);
     if (!m) return MARS_ERR_INVALID_FILE;
-    std::vector<YoloHead> heads;
+    HeadSet hs;
     if (n != 0) {
         uint32_t found[3];
         if (!tensor_ids) {
@@ -1126,18 +1168,39 @@ mars_error_t mars_b200_set_yolo_heads(mars_model_t *model, const uint32_t *tenso
             if (n == 0) { set_last_error("set_yolo_heads: the model has no YOLOv5 Detect head convolutions"); return MARS_ERR_INVALID_TENSOR; }
             tensor_ids = found;
         }
-        mars_error_t e = resolve_yolo_heads(m->pub.header, m->pub.tensors, m->pub.layers, m->toff, m->weights_size, tensor_ids, n, &heads);
+        mars_error_t e = resolve_yolo_heads(m->pub.header, m->pub.tensors, m->pub.layers, m->toff, m->weights_size, tensor_ids, n, &hs.heads);
         if (e != MARS_OK) return e;
+        hs.kind = HEADS_YOLO;
+        hs.conf = conf_thresh;
     }
-    bool same = heads.size() == m->heads.size() && (heads.empty() || memcmp(&conf_thresh, &m->head_conf, 4) == 0);
-    for (size_t k = 0; same && k < heads.size(); k++) same = heads[k].id == m->heads[k].id;
-    if (same) return MARS_OK;
-    cudaSetDevice(m->device);
-    cudaStreamSynchronize(m->stream);
-    m->heads = std::move(heads);
-    m->head_conf = conf_thresh;
-    m->compiled = false; /* the next call recompiles and drops the captured graphs */
-    return MARS_OK;
+    return replace_heads(m, std::move(hs));
+}
+
+mars_error_t mars_b200_set_gfl_heads(mars_model_t *model, const uint32_t *tensor_ids, int n, int nc, int reg_max, int centre, float conf_thresh) {
+    Model *m = as_model(model);
+    if (!m) return MARS_ERR_INVALID_FILE;
+    HeadSet hs;
+    if (n != 0) {
+        mars_error_t e = check_gfl_params(nc, reg_max, centre, conf_thresh);
+        if (e != MARS_OK) return e;
+        uint32_t found[4];
+        if (!tensor_ids) {
+            n = find_gfl_heads(m->pub.header, m->pub.tensors, m->pub.layers, nc, reg_max, found, 4);
+            if (n == 0) {
+                set_last_error("set_gfl_heads: the model has no GFL head convolutions with %d + 4 * (%d + 1) channels at strides 8, 16, 32", nc, reg_max);
+                return MARS_ERR_INVALID_TENSOR;
+            }
+            tensor_ids = found;
+        }
+        e = resolve_gfl_heads(m->pub.header, m->pub.tensors, m->pub.layers, m->toff, m->weights_size, tensor_ids, n, nc, reg_max, centre,
+                              conf_thresh, &hs.heads);
+        if (e != MARS_OK) return e;
+        hs.kind = HEADS_GFL;
+        hs.conf = conf_thresh;
+        hs.reg_max = reg_max;
+        hs.centre = centre;
+    }
+    return replace_heads(m, std::move(hs));
 }
 
 mars_error_t mars_b200_set_frame_size(mars_model_t *model, int first, int n, int w, int h) {
@@ -1795,12 +1858,12 @@ mars_error_t mars_b200_enqueue_step_resident(mars_model_t *model, int first, int
 /* all layers (with the head decodes the program holds), corner NMS and the letterbox inverse as one timed region */
 mars_error_t mars_b200_step_heads_resident(mars_model_t *model, int first, int n, float nms_thresh) {
     Model *m = as_model(model);
-    if (m && m->heads.empty()) { set_last_error("step_heads_resident: no YOLO heads configured (mars_b200_set_yolo_heads)"); return MARS_ERR_INVALID_TENSOR; }
+    if (m && m->heads.empty()) { set_last_error("step_heads_resident: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)"); return MARS_ERR_INVALID_TENSOR; }
     return step_resident(m, first, n, nms_thresh, STEP_HEADS);
 }
 mars_error_t mars_b200_enqueue_step_heads_resident(mars_model_t *model, int first, int n, float nms_thresh) {
     Model *m = as_model(model);
-    if (m && m->heads.empty()) { set_last_error("enqueue_step_heads_resident: no YOLO heads configured (mars_b200_set_yolo_heads)"); return MARS_ERR_INVALID_TENSOR; }
+    if (m && m->heads.empty()) { set_last_error("enqueue_step_heads_resident: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)"); return MARS_ERR_INVALID_TENSOR; }
     return enqueue_step_resident(m, first, n, nms_thresh, STEP_HEADS);
 }
 
@@ -2000,7 +2063,7 @@ mars_error_t mars_b200_submit_batch(mars_model_t *model, int pool, int n, const 
 mars_error_t mars_b200_submit_heads_batch(mars_model_t *model, int pool, int n, const void *inputs, size_t in_stride, mars_box_t *boxes,
                                           int32_t *counts, int maxd, float nms_thresh) {
     Model *m = as_model(model);
-    if (m && m->heads.empty()) { set_last_error("submit_heads_batch: no YOLO heads configured (mars_b200_set_yolo_heads)"); return MARS_ERR_INVALID_TENSOR; }
+    if (m && m->heads.empty()) { set_last_error("submit_heads_batch: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)"); return MARS_ERR_INVALID_TENSOR; }
     return submit_batch(m, pool, n, inputs, in_stride, boxes, counts, maxd, nms_thresh, STEP_HEADS);
 }
 
@@ -2009,7 +2072,7 @@ mars_error_t mars_b200_submit_heads_batch(mars_model_t *model, int pool, int n, 
  * coordinates for every slot */
 static mars_error_t submit_frames_heads(Model *m, const char *what, int pool, int n, const std::vector<FrameSrc> *frames, mars_box_t *boxes,
                                         int32_t *counts, int maxd, float nms_thresh) {
-    if (m && m->heads.empty()) { set_last_error("%s: no YOLO heads configured (mars_b200_set_yolo_heads)", what); return MARS_ERR_INVALID_TENSOR; }
+    if (m && m->heads.empty()) { set_last_error("%s: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)", what); return MARS_ERR_INVALID_TENSOR; }
     if (m && !frames) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
     return submit_batch(m, pool, n, nullptr, 0, boxes, counts, maxd, nms_thresh, STEP_HEADS, frames, what);
 }
@@ -2030,7 +2093,7 @@ mars_error_t mars_b200_submit_frames_nv12_heads_batch(mars_model_t *model, int p
  * merged per frame (k_merge_rois) and read back per frame */
 static mars_error_t submit_rois_heads(Model *m, const char *what, int pool, const std::vector<FrameSrc> *frames, int n_rois, const mars_b200_roi_t *rois,
                                       mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh, float merge_thresh) {
-    if (m && m->heads.empty()) { set_last_error("%s: no YOLO heads configured (mars_b200_set_yolo_heads)", what); return MARS_ERR_INVALID_TENSOR; }
+    if (m && m->heads.empty()) { set_last_error("%s: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)", what); return MARS_ERR_INVALID_TENSOR; }
     if (m && !frames) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
     const RoiList rl{n_rois, rois};
     return submit_batch(m, pool, n_rois, nullptr, 0, boxes, counts, maxd, nms_thresh, STEP_HEADS, frames, what, &rl, merge_thresh);

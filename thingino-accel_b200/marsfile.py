@@ -422,12 +422,18 @@ def build_tiny(size=160, seed=11, f32=False, relu_layers=True, chans=(16, 32, 64
     return m
 
 
-def build_nanodet_like(size=320, seed=7, width=1.0):
+def build_nanodet_like(size=320, seed=7, width=1.0, nhwc=False, nc=80, reg_max=7, levels=3):
     """NanoDet-m-shaped graph (ShuffleNetV2-style stem, depthwise 3x3 + pointwise 1x1 blocks,
     concat, 2x nearest upsample, 1x1 heads).  The reference has no NanoDet file or code; its
     DEPTHWISE_CONV2D layer is a no-op (src/mars/mars_runtime.c:1168-1170), which this library
-    reproduces by default (mars_b200_set_depthwise_mode(1) = restated depthwise)."""
-    b = _Builder(seed)
+    reproduces by default (mars_b200_set_depthwise_mode(1) = restated depthwise).
+    Each head "/head{k}.out/Conv_output_0" is the shared classification + regression conv of a GFL
+    head: nc + 4 (reg_max + 1) channels at stride 8 << k.  levels=4 adds a stride-64 level
+    (NanoDet-Plus) behind the other three, fed by a stride-2 depthwise block on the last head's
+    features.  nhwc=True lays every activation out as [1, h, w, c] (the depthwise weights as OHWI
+    [c, 3, 3, 1], the same bytes)."""
+    assert levels in (3, 4)
+    b = _Builder(seed, nhwc=nhwc)
     m = b.m
     c = lambda v: int(v * width)
     x = m.add_tensor("data", b.adt, b.afmt, b.ashape(3, size, size), 1.0)
@@ -443,7 +449,8 @@ def build_nanodet_like(size=320, seed=7, width=1.0):
         ci, h, w = b.shape[xin]
         wt = b.rng.integers(-127, 128, size=(ci, 1, 3, 3), dtype=np.int8)
         bs = b.rng.integers(-500, 501, size=ci).astype(np.int32)
-        wid = m.add_tensor(name + ".weight", DT_I8, FMT_OIHW, [ci, 1, 3, 3], float(np.float32(28.0 / (3 * 73.6 * 24.0))), wt.tobytes())
+        wfmt, wshape = (FMT_OHWI, [ci, 3, 3, 1]) if nhwc else (FMT_OIHW, [ci, 1, 3, 3])
+        wid = m.add_tensor(name + ".weight", DT_I8, wfmt, wshape, float(np.float32(28.0 / (3 * 73.6 * 24.0))), wt.tobytes())
         bid = m.add_tensor(name + ".bias", DT_F32, FMT_NCHW, [ci], 1.0, bs.tobytes())
         y = b.rt(name + "_out", ci, (h + 2 - 3) // s + 1, (w + 2 - 3) // s + 1)
         m.add_layer(L_DW, [xin], [y], _conv_params(3, s, 1, wid, bid, padding=PAD_EXPLICIT, groups=ci))
@@ -472,10 +479,14 @@ def build_nanodet_like(size=320, seed=7, width=1.0):
     u0 = b.upsample(102, t1)
     t0 = b.rt("/fpn/add0", *b.shape[f[0]])
     m.add_layer(L_ADD, [u0, f[0]], [t0])
-    outs = []
+    outs, chans = [], nc + 4 * (reg_max + 1)
     for i, t in enumerate((t0, t1, f[2])):
         h1 = pw("head%d.pw" % i, dw("head%d.dw" % i, t, 1), c(96))
-        outs.append(b.conv("head%d.out" % i, "/head%d.out" % i, h1, 80 + 32, 1, 1))
+        outs.append(b.conv("head%d.out" % i, "/head%d.out" % i, h1, chans, 1, 1))
+    if levels == 4:
+        t3 = pw("fpn.extra.pw", dw("fpn.extra.dw", h1, 2), c(96))
+        h1 = pw("head3.pw", dw("head3.dw", t3, 1), c(96))
+        outs.append(b.conv("head3.out", "/head3.out", h1, chans, 1, 1))
     m.outputs = [outs[0]]
     return m
 
