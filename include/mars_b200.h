@@ -313,6 +313,10 @@ size_t mars_b200_plan_describe(const void *data, size_t size, size_t arena_bytes
 int mars_b200_requant_fit(float scale, long long tmax, int *m, int *s, long long *c);
 /* the reference's requantisation of one value, restated (what the fit is checked against) */
 int mars_b200_requant_ref(int t, float scale);
+/* the requantisation variant the tcgen05 conv epilogue takes for conv scale `scale` and bound = max over output channels of
+ * 128 * sum |w| + |bias| (read as int32): 3 integer form, 2 float half-up, 1 float with a fast conversion, 0 general float with the
+ * x86 overflow rule.  A compiled model reports the variant of each such layer as " rq=N" in mars_b200_describe. */
+int mars_b200_requant_variant(float scale, long long bound);
 
 /* ---- NNA-native tensor layouts (SURVEY 8f4) -------------------------------- */
 /* The layouts behind the format tags MARS_FORMAT_NMHWSOIB2 / MARS_FORMAT_NDHWC32 (reference include/mars.h:46-56), which the

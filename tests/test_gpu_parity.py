@@ -109,13 +109,16 @@ def micro(pkg, kind, **kw):
     return pkg.marsfile.build_single_layer(kind, **kw).to_bytes()
 
 
-from util import MICRO  # noqa: E402  (shared with the CPU pin of the restatement against the reference, tests/test_oracle.py)
+from util import MICRO, MICRO_TC  # noqa: E402  (shared with the CPU pin of the restatement against the reference, tests/test_oracle.py)
 
 
 @pytest.mark.parametrize("kind,kw", MICRO)
 def test_micro_models(pkg, ob, kind, kw):
     blob = micro(pkg, kind, **kw)
     gm = pkg.MarsModel(blob)
+    if (kind, kw) in MICRO_TC:  # a failed tensor-core plan would silently recompile on the direct kernels
+        desc = gm.describe()
+        assert " impl=1 rq=" in desc, "%r did not take the tensor-core path:\n%s" % (kw, desc)
     om = ob.OracleModel(blob)
     rng = np.random.default_rng(2)
     W = om.weights_size

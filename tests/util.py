@@ -81,6 +81,9 @@ MICRO = [
     ("maxpool", dict(k=5, s=1, h=20, w=20, c=20)), ("maxpool", dict(k=3, s=2, h=9, w=11)), ("upsample", dict(scale=2)),
     ("upsample", dict(scale=3, ratio_fallback=True)), ("concat", dict(n=4)), ("concat", dict(n=2)), ("batchnorm", {}),
     ("batchnorm", dict(f32=True)), ("depthwise", {}),
+]
+# int8 convs that take the tcgen05 path (tests/test_gpu_parity.py asserts impl=1 for each)
+MICRO_TC = [
     # shapes that take the tcgen05 path (Ci % 32 == 0)
     ("conv", dict(k=1, s=1, c=32, co=64, h=20, w=20)), ("conv", dict(k=1, s=1, c=64, co=32, h=16, w=24)),
     ("conv", dict(k=1, s=1, c=128, co=512, h=8, w=8)), ("conv", dict(k=1, s=1, c=256, co=255, h=20, w=20)),
@@ -116,3 +119,4 @@ MICRO = [
     ("conv", dict(k=6, s=2, nhwc=True, c=3, co=32, h=128, w=128, pad=2)), ("conv", dict(k=6, s=2, nhwc=True, c=4, co=48, h=128, w=160, pad=2, padding=1)),
     ("conv", dict(k=3, s=1, nhwc=True, c=256, co=512, h=20, w=20)),
 ]
+MICRO = MICRO + MICRO_TC

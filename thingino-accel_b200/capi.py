@@ -206,6 +206,7 @@ SIGNATURES = {
     "mars_b200_plan_describe": (C.c_size_t, [C.c_void_p, C.c_size_t, C.c_size_t, C.c_int, C.c_char_p, C.c_size_t]),
     "mars_b200_requant_fit": (C.c_int, [C.c_float, C.c_longlong, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_longlong)]),
     "mars_b200_requant_ref": (C.c_int, [C.c_int, C.c_float]),
+    "mars_b200_requant_variant": (C.c_int, [C.c_float, C.c_longlong]),
     "mars_b200_nmhwsoib2_size": (C.c_size_t, [C.c_int] * 4),
     "mars_b200_ndhwc32_size": (C.c_size_t, [C.c_int] * 4),
     "mars_b200_pack_weights_nmhwsoib2": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),

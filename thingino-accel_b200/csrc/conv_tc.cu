@@ -119,10 +119,13 @@ struct TcParams {
  * avoided the conversion with five integer-pipe instructions; the integer pipe (16 lanes per scheduler) is what limits
  * the epilogue.  The +-0.5 add stays a scalar FADD: ptxas contracts mul.rn.f32x2 + add.rn.f32x2 into FFMA2 (one
  * rounding), which is not the reference's arithmetic. */
-/* RQ = 0: general (I2F, x86 overflow rule); 1: FAST, sign-exact, F2I; 2: FAST, round-half-up without conversion instructions.
+/* RQ = 0: general (I2F, x86 overflow rule); 1: FAST, sign-exact, F2I; 2: FAST, round-half-up without conversion instructions;
+ * 3: the integer form (requant_int).  select_requant picks one per layer.
  *
- * RQ 2 (the common case).  ncu on the F2I variant showed the XU pipe (conversions, 16 lanes per SM) 87 % busy: one F2I per
- * output element is what limited the epilogue.  floor(fl(sc + 0.5f)) needs none: a round-down add of 1.5 * 2^23 leaves
+ * RQ 2 is chosen when the integer form does not fit (scales <= 0 or >= 0.49, or the rare positive scale whose thresholds no
+ * integer triple reproduces), max |acc + bias| < 2^22, |cs| < 512 and no accumulator value in range lands on a negative tie.
+ * Most builder scales fit the integer form, so RQ 2 is now the exception.  ncu on the F2I variant showed the XU pipe
+ * (conversions, 16 lanes per SM) 87 % busy: one F2I per output element is what limited the epilogue.  floor(fl(sc + 0.5f)) needs none: a round-down add of 1.5 * 2^23 leaves
  * floor(h) in the low mantissa bits, and one VIADDMNMX.RELU (DPX) subtracts the exponent pattern and clamps to [0, 255]
  * = r + 128.  Round-half-up differs from the reference's round-half-away only when sc is a NEGATIVE exact tie -(n + 0.5)
  * (or -pred(0.5), where fl(sc - 0.5f) rounds to -1): the host enumerates those few floats per layer and selects RQ 2 only
@@ -1155,24 +1158,6 @@ static void build_lutw(const Op &o, const uint8_t *h_cpool, const int stream_byt
     }
 }
 
-/* may the layer use the magic-number int -> float conversion (FAST)?  max |acc + bias| over all output channels, from the real
- * weights; returns that bound, or -1 when it does not fit */
-static long long fast_requant_bound(const Op &o, const ArenaGeom &ag) {
-    if (!(fabsf(o.f0) < 512.0f)) return -1; /* also rejects NaN */
-    const int8_t *w = reinterpret_cast<const int8_t *>(ag.h_weights + o.w);
-    const long long K = (long long)o.ic * o.kh * o.kw;
-    long long bound = 0;
-    for (int co = 0; co < o.oc; co++) {
-        long long sum = 0;
-        for (long long k = 0; k < K; k++) sum += std::abs((int)w[co * K + k]);
-        long long b = 0;
-        if (o.bias >= 0) { int32_t bv; memcpy(&bv, ag.h_weights + o.bias + 4 * (size_t)co, 4); b = std::llabs((long long)bv); }
-        if (sum * 128 + b >= (1ll << 22)) return -1;
-        bound = std::max(bound, sum * 128 + b);
-    }
-    return bound;
-}
-
 /* Is floor(fl(sc + 0.5f)) the reference's (int32)(sc + (sc >= 0 ? 0.5f : -0.5f)) (src/mars/mxu_conv.c:663-666) for every
  * t = acc + bias with |t| <= bound, sc = fl((float)t * cs)?  For sc >= 0 both are floor(fl(sc + 0.5f)).  For sc < 0 the sum
  * sc + 0.5f is exact, and the two differ exactly when sc is a tie -(n + 0.5) (half-away gives -(n + 1), half-up -n; equal after
@@ -1284,6 +1269,19 @@ static bool int_requant_fit(float cs, long long tmax, int *m_out, int *s_out, lo
     if (g(-tmax) != lo_r || g(tmax) != hi_r) return false;
     *m_out = (int)m; *s_out = sh; *c_out = (long long)c;
     return true;
+}
+
+/* requantisation variant of the epilogue (requant_pair / requant_int) for conv scale cs and bound = max |acc + bias| over all
+ * output channels (acc_bound):
+ *   3  the integer form reproduces the reference on |t| <= bound (int_requant_fit fills m / s / c);
+ *   2  else, when |cs| < 512 and bound < 2^22 (the magic-number int -> float conversion is exact and |sc| < 2^31) and no t in range
+ *      lands on a negative tie (halfup_requant_ok);
+ *   1  else, under the same two limits;
+ *   0  otherwise: huge, infinite or NaN scales, accumulators from 2^22 up (int32 wrap-around of acc + bias included). */
+static int select_requant(float cs, long long bound, int *m, int *s, long long *c) {
+    if (int_requant_fit(cs, std::max(1ll, bound), m, s, c)) return 3;
+    if (!(fabsf(cs) < 512.0f) || bound >= (1ll << 22)) return 0; /* also rejects NaN */
+    return halfup_requant_ok(cs, bound) ? 2 : 1;
 }
 
 /* kernel variants: requantisation x GATHER producer x word table x number of stored streams x output mode (0 NCHW planes,
@@ -1400,11 +1398,7 @@ bool tc_plan(const Op &o, const ArenaGeom &ag, uint8_t *scratch, size_t scratch_
     for (int k = 0; k < t->nst; k++) if (p.out_off[k] % 16) t->tst = false;
     const int epi_warps = (!gather && t->ctas_per_sm == 1) ? 16 : 8;
     const int stg_bytes = t->tst ? (epi_warps / 4) * 2 * t->nst * 2048 : 0;
-    { /* requantisation variant of the epilogue (requant_pair / requant_int) */
-        const long long bound = fast_requant_bound(o, ag);
-        t->rq = bound < 0 ? 0 : (halfup_requant_ok(o.f0, bound) ? 2 : 1);
-        if (int_requant_fit(o.f0, std::max(1ll, acc_bound(o, ag)), &p.q_m, &p.q_s, &p.q_c)) t->rq = 3;
-    }
+    t->rq = select_requant(o.f0, acc_bound(o, ag), &p.q_m, &p.q_s, &p.q_c);
     const int cm64_bytes = t->rq == 3 ? 8 * p.n_tiles * p.n_tile : 0; /* RQ 3: per-channel int64 addends behind the table */
     const int nsteps = g.ntaps * p.ksteps_per_tap;
     int grp0 = p.grp, acc0 = p.acc_bufs;
@@ -1670,6 +1664,8 @@ bool tc_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, bool u
     return cudaGetLastError() == cudaSuccess;
 }
 
+int tc_rq(const TcPlan &plan) { return plan.i8 ? plan.i8->rq : -1; }
+
 void tc_release(std::vector<TcPlan> &plans) {
     for (auto &pl : plans) {
         if (TcPlanImpl *t = pl.i8) { cudaFree(t->d_wr); cudaFree(t->d_lutw); delete t; }
@@ -1690,4 +1686,8 @@ int mars_b200_requant_fit(float scale, long long tmax, int *m, int *s, long long
     return 1;
 }
 int mars_b200_requant_ref(int t, float scale) { return marsb200::ref_requant((int32_t)t, scale); }
+int mars_b200_requant_variant(float scale, long long bound) {
+    int m = 0, s = 0; long long c = 0;
+    return marsb200::select_requant(scale, bound, &m, &s, &c);
+}
 }

@@ -88,6 +88,8 @@ bool tc_plan(const Op &o, const ArenaGeom &g, uint8_t *scratch, size_t scratch_s
 /* pre-pass (if any) + conv kernel for image slots [first, first+n) */
 /* use_linked: read the producer-written copy (full passes) instead of running the layout pre-pass on the arena tensor */
 bool tc_launch(const TcPlan &plan, uint8_t *slots_base, int first, int n, bool use_linked, cudaStream_t s, uint64_t *launches);
+/* the requantisation variant (0..3, see select_requant) of an int8 plan, or -1 when the op has none */
+int tc_rq(const TcPlan &plan);
 void tc_release(std::vector<TcPlan> &plans);
 
 } // namespace marsb200

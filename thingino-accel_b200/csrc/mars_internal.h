@@ -107,6 +107,7 @@ struct Op {
      * sh = stride (8 << head_level).  OP_GFL_HEAD: f2 = cell centre offset (0.5 or 0), iw x ih = network input size */
     int head_level = -1, head_nc = 0, head_reg_max = 0;
     bool head_nhwc = false;
+    int rq = -1; /* int8 tensor-core conv: requantisation variant of its planned epilogue (tc_rq), set when the model compiles */
     std::string note;
 };
 

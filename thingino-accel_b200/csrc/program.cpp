@@ -1196,9 +1196,11 @@ std::string describe_program(const Program &p) {
     char line[512];
     for (size_t i = 0; i < p.ops.size(); i++) {
         const Op &o = p.ops[i];
+        char rq[16] = ""; /* int8 tensor-core convs of a compiled model: the epilogue's requantisation variant */
+        if (o.rq >= 0) snprintf(rq, sizeof rq, " rq=%d", o.rq);
         snprintf(line, sizeof line,
-                 "op %3zu layer %3d %-16s %-18s impl=%d in=%lld out=%lld ic=%d ih=%d iw=%d oc=%d oh=%d ow=%d k=%dx%d s=%d,%d p=%d,%d n=%llu fused=%d%s %s\n",
-                 i, o.layer, kind_name(o.kind), mode_name(o.mode), o.impl, (long long)o.in0, (long long)o.out, o.ic,
+                 "op %3zu layer %3d %-16s %-18s impl=%d%s in=%lld out=%lld ic=%d ih=%d iw=%d oc=%d oh=%d ow=%d k=%dx%d s=%d,%d p=%d,%d n=%llu fused=%d%s %s\n",
+                 i, o.layer, kind_name(o.kind), mode_name(o.mode), o.impl, rq, (long long)o.in0, (long long)o.out, o.ic,
                  o.ih, o.iw, o.oc, o.oh, o.ow, o.kh, o.kw, o.sh, o.sw, o.pt, o.pl, (unsigned long long)o.n,
                  o.fused_layers, o.xlat ? " xlat" : "", o.note.c_str());
         s += line;

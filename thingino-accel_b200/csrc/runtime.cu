@@ -422,6 +422,7 @@ static mars_error_t compile_model(Model *m) {
             m->opt_level = 0;
             return compile_model(m);
         }
+        o.rq = tc_rq(m->tc[i]);
     }
     m->prof_ms.assign(m->prog.ops.size(), 0.0);
     m->prof_calls.assign(m->prog.ops.size(), 0);
