@@ -46,6 +46,15 @@ def test_find_gfl_heads_without_gfl_heads(pkg):
         assert pkg.capi.find_yolo_heads(mf.build_nanodet_like(**kw).to_bytes()) == [], kw
 
 
+def test_find_heads_in_a_blob_cut_short(pkg):
+    """the finders parse a blob as mars_load_memory does: weights that run past its end make it no model"""
+    mf = pkg.marsfile
+    for blob, find in ((mf.build_nanodet_like().to_bytes(), pkg.capi.find_gfl_heads),
+                       (mf.build_yolov5(width=0.25, size=320).to_bytes(), pkg.capi.find_yolo_heads)):
+        assert len(find(blob)) == 3
+        assert find(blob[:-1]) == []
+
+
 def test_default_nanodet_blobs_unchanged(pkg):
     for size, want in ((320, "35fba38eaf8c246645f270ffdabeb2ff1501326f4332c2fbe6e44bfb39476676"),
                        (416, "79d2667b2ac239e664d9d6fd13dac7b5321ea8c1891d902e41d69864db09b54f")):

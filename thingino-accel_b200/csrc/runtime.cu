@@ -62,6 +62,31 @@ void set_last_error(const char *fmt, ...) {
         }                                                                                      \
     } while (0)
 
+/* an owned device array of T; moves, never copies, and frees itself */
+template <typename T = uint8_t> struct DevBuf {
+    T *p = nullptr;
+    DevBuf() = default;
+    explicit DevBuf(size_t n) { alloc(n); }
+    ~DevBuf() { cudaFree(p); }
+    DevBuf(DevBuf &&o) noexcept : p(o.p) { o.p = nullptr; }
+    DevBuf &operator=(DevBuf &&o) noexcept {
+        if (this != &o) { cudaFree(p); p = o.p; o.p = nullptr; }
+        return *this;
+    }
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    void reset() { cudaFree(p); p = nullptr; }
+    /* replaces the array by n (at least one) fresh elements; false, empty and the reason in the last error when that fails */
+    bool alloc(size_t n) {
+        reset();
+        const cudaError_t e = cudaMalloc(&p, (n ? n : 1) * sizeof(T));
+        if (e == cudaSuccess) return true;
+        p = nullptr;
+        set_last_error("cudaMalloc of %zu bytes failed: %s", (n ? n : 1) * sizeof(T), cudaGetErrorString(e));
+        return false;
+    }
+};
+
 bool first_time_on_device(unsigned long long *mask) {
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev > 63) return true;
@@ -150,6 +175,23 @@ int find_tensor(const mars_header_t &h, const mars_runtime_tensor_t *tensors, ui
 /* ---- the private model object ------------------------------------------------ */
 static const uint32_t MODEL_TAG = 0x4232304Du; /* "M02B" */
 
+/* MARS_MAX_DETS records and one count per image slot */
+template <typename R> struct RecordSet {
+    DevBuf<R> rec;
+    DevBuf<int32_t> cnt;
+    bool alloc(int slots) { return rec.alloc((size_t)slots * MARS_MAX_DETS) && cnt.alloc((size_t)slots); }
+    R *at(int slot) const { return rec.p + (size_t)slot * MARS_MAX_DETS; }
+};
+
+/* the per-slot device state besides the slots themselves, (re)allocated together by set_capacity */
+struct SlotRecords {
+    RecordSet<mars_det_t> raw, det;      /* the output0 path: parsed candidates, kept detections */
+    RecordSet<mars_box_t> box_raw, box;  /* the heads path: decoded candidates, kept corner boxes */
+    RecordSet<mars_box_t> fbox;          /* frame records of the region merge (mars_b200_merge_rois_resident) */
+    DevBuf<unsigned> nms_mask;           /* NMS_SCRATCH_WORDS per slot: suppression bit matrices */
+    DevBuf<int2> frame;                  /* original frame size per slot (0 = none), for the letterbox inverse */
+};
+
 struct Model {
     mars_model_t pub; /* must stay first: applications hold &pub */
     uint32_t tag = MODEL_TAG;
@@ -158,15 +200,15 @@ struct Model {
     int num_buffers = 0;
     std::vector<size_t> toff;
     uint8_t *h_arena = nullptr;  /* pinned host mirror of [weights | buf0 | buf1 | (buf2)] */
-    uint8_t *d_weights = nullptr;
-    uint8_t *d_slots = nullptr;
+    DevBuf<> weights;
+    DevBuf<> slots;
     int capacity = 0;
-    uint8_t *d_scratch = nullptr;
+    DevBuf<> scratch;
     size_t scratch_stride = 0;
-    uint8_t *d_cpool = nullptr;
-    uint8_t *d_tc_scratch = nullptr; /* padded / phase-split conv inputs, one region per image slot */
+    DevBuf<> cpool;
+    DevBuf<> tc_scratch;         /* padded / phase-split conv inputs, one region per image slot */
     size_t tc_scratch_stride = 0;
-    uint8_t *d_linked = nullptr;     /* producer-written conv input copies (Program::linked_bytes per image), pads stay zero */
+    DevBuf<> linked;             /* producer-written conv input copies (Program::linked_bytes per image), pads stay zero */
     size_t linked_stride = 0;
     Program prog;
     int opt_level = 3, depthwise_mode = 0;
@@ -182,10 +224,11 @@ struct Model {
      * downscale taps cost O(in x out) on the host -- the float rows of one launch, and staging for frames and descriptor
      * tables: one set per pool of the frames submit, one for the synchronous and device-frame calls (PRE_SYNC) */
     std::map<std::pair<int, int>, ResizeTaps> pre_taps;
-    float *d_preH = nullptr;
+    DevBuf<float> preH;
     size_t preH_cap = 0;
     struct PreStage {
-        uint8_t *d_frames = nullptr, *d_tab = nullptr, *h_tab = nullptr; /* device frames, device table, pinned table */
+        DevBuf<> frames, tab;    /* device frames, device table */
+        uint8_t *h_tab = nullptr; /* pinned table */
         size_t frames_cap = 0, tab_cap = 0, h_cap = 0;
         cudaEvent_t ev = nullptr; /* the last upload from h_tab */
     } pre_stage[3];
@@ -193,20 +236,10 @@ struct Model {
     struct StepGraph { int first, n, with_detect; uint32_t thresh_bits; int seen; cudaGraphExec_t exec; uint64_t launches; };
     std::vector<StepGraph> graphs;
     bool graphs_broken = false;
-    /* device-resident detections */
-    mars_det_t *d_raw = nullptr, *d_det = nullptr;
-    int32_t *d_raw_cnt = nullptr, *d_det_cnt = nullptr;
-    unsigned *d_nms_mask = nullptr; /* capacity x 1024 x 32 words: suppression bit matrices */
-    /* detection heads (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads): decoded candidates, kept boxes, and the original frame
-     * size per slot (0 = none) */
+    SlotRecords rec; /* device-resident detections, boxes and frame sizes */
+    /* detection heads (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads) */
     HeadSet heads;
-    mars_box_t *d_box_raw = nullptr, *d_box = nullptr;
-    int32_t *d_box_raw_cnt = nullptr, *d_box_cnt = nullptr;
-    int2 *d_frame = nullptr;
-    /* frame records of the region merge (mars_b200_merge_rois_resident): capacity x MARS_MAX_DETS boxes, counts */
-    mars_box_t *d_fbox = nullptr;
-    int32_t *d_fbox_cnt = nullptr;
-    DecodeTables *d_tab = nullptr;
+    DevBuf<DecodeTables> tab;
     float tab_scale = 0.0f;
     bool tab_valid = false;
     /* per-op profile (CUDA events around every op when enabled) */
@@ -228,7 +261,7 @@ static Model *as_model(mars_model_t *p) {
 }
 
 static inline uint8_t *dev_addr(const Model *m, size_t off, int slot) {
-    return off < m->weights_size ? m->d_weights + off : m->d_slots + (size_t)slot * m->slot_stride + (off - m->weights_size);
+    return off < m->weights_size ? m->weights.p + off : m->slots.p + (size_t)slot * m->slot_stride + (off - m->weights_size);
 }
 
 static uint64_t fnv1a(const uint8_t *p, size_t n) {
@@ -250,10 +283,6 @@ static void model_release(Model *m) {
     release_graphs(m);
     tc_release(m->tc);
     for (auto e : m->prof_ev) cudaEventDestroy(e);
-    cudaFree(m->d_weights); cudaFree(m->d_slots); cudaFree(m->d_scratch); cudaFree(m->d_cpool); cudaFree(m->d_tc_scratch); cudaFree(m->d_linked);
-    cudaFree(m->d_raw); cudaFree(m->d_det); cudaFree(m->d_raw_cnt); cudaFree(m->d_det_cnt); cudaFree(m->d_tab); cudaFree(m->d_nms_mask);
-    cudaFree(m->d_box_raw); cudaFree(m->d_box); cudaFree(m->d_box_raw_cnt); cudaFree(m->d_box_cnt); cudaFree(m->d_frame);
-    cudaFree(m->d_fbox); cudaFree(m->d_fbox_cnt);
     if (m->h_arena) cudaFreeHost(m->h_arena);
     if (m->ev0) cudaEventDestroy(m->ev0);
     if (m->ev1) cudaEventDestroy(m->ev1);
@@ -265,10 +294,8 @@ static void model_release(Model *m) {
     for (auto &st : m->pre_stage) {
         if (st.ev) cudaEventSynchronize(st.ev);
         if (st.ev) cudaEventDestroy(st.ev);
-        cudaFree(st.d_frames); cudaFree(st.d_tab);
         if (st.h_tab) cudaFreeHost(st.h_tab);
     }
-    cudaFree(m->d_preH);
     if (m->stream) cudaStreamDestroy(m->stream);
     if (m->h2d_stream) cudaStreamDestroy(m->h2d_stream);
     if (m->d2h_stream) cudaStreamDestroy(m->d2h_stream);
@@ -276,73 +303,42 @@ static void model_release(Model *m) {
     free(m->pub.layers);
     if (g_last_model == m) g_last_model = nullptr;
     m->tag = 0;
-    delete m;
+    delete m; /* frees the device buffers */
 }
 
-/* (re)allocate `capacity` image slots; slot 0 keeps its contents */
+/* (re)allocate `capacity` image slots; the slots both capacities share keep their contents and frame sizes.  The new set is
+ * complete before it replaces the old one: on failure the model keeps its slots */
 static mars_error_t set_capacity(Model *m, int capacity) {
     if (capacity < 1) capacity = 1;
     if (capacity == m->capacity) return MARS_OK;
-    uint8_t *ns = nullptr, *nscr = nullptr;
-    mars_det_t *nraw = nullptr, *ndet = nullptr;
-    int32_t *nrc = nullptr, *ndc = nullptr;
-    size_t bytes = (size_t)capacity * m->slot_stride;
+    const size_t c = (size_t)capacity, keep = (size_t)std::min(capacity, m->capacity);
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
-    CU_OK(cudaMalloc(&ns, bytes), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMemsetAsync(ns, 0, bytes, m->stream), MARS_ERR_ALLOC_FAILED);
-    if (m->d_slots) {
-        size_t keep = (size_t)std::min(capacity, m->capacity) * m->slot_stride;
-        CU_OK(cudaMemcpyAsync(ns, m->d_slots, keep, cudaMemcpyDeviceToDevice, m->stream), MARS_ERR_ALLOC_FAILED);
+    DevBuf<> slots, scratch;
+    SlotRecords r;
+    if (!slots.alloc(c * m->slot_stride) || (m->scratch_stride && !scratch.alloc(c * m->scratch_stride)) || !r.raw.alloc(capacity) ||
+        !r.det.alloc(capacity) || !r.box_raw.alloc(capacity) || !r.box.alloc(capacity) || !r.fbox.alloc(capacity) ||
+        !r.nms_mask.alloc(c * NMS_SCRATCH_WORDS) || !r.frame.alloc(c))
+        return MARS_ERR_ALLOC_FAILED;
+    CU_OK(cudaMemsetAsync(slots.p, 0, c * m->slot_stride, m->stream), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMemsetAsync(r.frame.p, 0, c * sizeof(int2), m->stream), MARS_ERR_ALLOC_FAILED);
+    for (int32_t *cnt : {r.raw.cnt.p, r.det.cnt.p, r.box_raw.cnt.p, r.box.cnt.p, r.fbox.cnt.p})
+        CU_OK(cudaMemsetAsync(cnt, 0, c * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
+    if (m->slots.p) {
+        CU_OK(cudaMemcpyAsync(slots.p, m->slots.p, keep * m->slot_stride, cudaMemcpyDeviceToDevice, m->stream), MARS_ERR_ALLOC_FAILED);
+        CU_OK(cudaMemcpyAsync(r.frame.p, m->rec.frame.p, keep * sizeof(int2), cudaMemcpyDeviceToDevice, m->stream), MARS_ERR_ALLOC_FAILED);
     }
-    if (m->scratch_stride) {
-        CU_OK(cudaMalloc(&nscr, (size_t)capacity * m->scratch_stride), MARS_ERR_ALLOC_FAILED);
-    }
-    CU_OK(cudaMalloc(&nraw, (size_t)capacity * MARS_MAX_DETS * sizeof(mars_det_t)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMalloc(&ndet, (size_t)capacity * MARS_MAX_DETS * sizeof(mars_det_t)), MARS_ERR_ALLOC_FAILED);
-    unsigned *nmask = nullptr;
-    CU_OK(cudaMalloc(&nmask, (size_t)capacity * NMS_SCRATCH_WORDS * sizeof(unsigned)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMalloc(&nrc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMalloc(&ndc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMemsetAsync(nrc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMemsetAsync(ndc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
-    mars_box_t *nbraw = nullptr, *nbox = nullptr;
-    int32_t *nbrc = nullptr, *nbc = nullptr;
-    int2 *nfr = nullptr;
-    CU_OK(cudaMalloc(&nbraw, (size_t)capacity * MARS_MAX_DETS * sizeof(mars_box_t)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMalloc(&nbox, (size_t)capacity * MARS_MAX_DETS * sizeof(mars_box_t)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMalloc(&nbrc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMalloc(&nbc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMalloc(&nfr, (size_t)capacity * sizeof(int2)), MARS_ERR_ALLOC_FAILED);
-    mars_box_t *nfbox = nullptr;
-    int32_t *nfbc = nullptr;
-    CU_OK(cudaMalloc(&nfbox, (size_t)capacity * MARS_MAX_DETS * sizeof(mars_box_t)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMalloc(&nfbc, (size_t)capacity * sizeof(int32_t)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMemsetAsync(nfbc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMemsetAsync(nbrc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMemsetAsync(nbc, 0, (size_t)capacity * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMemsetAsync(nfr, 0, (size_t)capacity * sizeof(int2), m->stream), MARS_ERR_ALLOC_FAILED);
-    if (m->d_frame)
-        CU_OK(cudaMemcpyAsync(nfr, m->d_frame, (size_t)std::min(capacity, m->capacity) * sizeof(int2), cudaMemcpyDeviceToDevice, m->stream),
-              MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
-    cudaFree(m->d_box_raw); cudaFree(m->d_box); cudaFree(m->d_box_raw_cnt); cudaFree(m->d_box_cnt); cudaFree(m->d_frame);
-    m->d_box_raw = nbraw; m->d_box = nbox; m->d_box_raw_cnt = nbrc; m->d_box_cnt = nbc; m->d_frame = nfr;
-    cudaFree(m->d_fbox); cudaFree(m->d_fbox_cnt);
-    m->d_fbox = nfbox; m->d_fbox_cnt = nfbc;
-    cudaFree(m->d_slots); cudaFree(m->d_scratch); cudaFree(m->d_raw); cudaFree(m->d_det);
-    cudaFree(m->d_raw_cnt); cudaFree(m->d_det_cnt); cudaFree(m->d_nms_mask);
-    m->d_nms_mask = nmask;
-    m->d_slots = ns; m->d_scratch = nscr; m->d_raw = nraw; m->d_det = ndet; m->d_raw_cnt = nrc; m->d_det_cnt = ndc;
+    m->slots = std::move(slots);
+    m->scratch = std::move(scratch);
+    m->rec = std::move(r);
     m->capacity = capacity;
-    m->pub.ddr_paddr = m->d_slots;
+    m->pub.ddr_paddr = m->slots.p;
     for (uint32_t i = 0; i < m->pub.header.num_tensors; i++) m->pub.tensors[i].paddr = dev_addr(m, m->toff[i], 0);
     /* tensor maps embed slot addresses and the slot count */
     tc_release(m->tc);
-    cudaFree(m->d_tc_scratch);
-    m->d_tc_scratch = nullptr;
+    m->tc_scratch.reset();
     m->tc_scratch_stride = 0;
-    cudaFree(m->d_linked);
-    m->d_linked = nullptr;
+    m->linked.reset();
     m->linked_stride = 0;
     m->compiled = false;
     return MARS_OK;
@@ -356,16 +352,12 @@ static mars_error_t compile_model(Model *m) {
                                      m->arena_size, m->opt_level, m->depthwise_mode, &p, m->f32_mode, &m->heads);
     if (e != MARS_OK) return e;
     m->prog = std::move(p);
-    cudaFree(m->d_cpool);
-    m->d_cpool = nullptr;
-    CU_OK(cudaMalloc(&m->d_cpool, m->prog.const_pool.size()), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMemcpy(m->d_cpool, m->prog.const_pool.data(), m->prog.const_pool.size(), cudaMemcpyHostToDevice),
+    if (!m->cpool.alloc(m->prog.const_pool.size())) return MARS_ERR_ALLOC_FAILED;
+    CU_OK(cudaMemcpy(m->cpool.p, m->prog.const_pool.data(), m->prog.const_pool.size(), cudaMemcpyHostToDevice),
           MARS_ERR_ALLOC_FAILED);
     if (m->prog.scratch_bytes > m->scratch_stride) {
         m->scratch_stride = (m->prog.scratch_bytes + 255) & ~(size_t)255;
-        cudaFree(m->d_scratch);
-        m->d_scratch = nullptr;
-        CU_OK(cudaMalloc(&m->d_scratch, (size_t)m->capacity * m->scratch_stride), MARS_ERR_ALLOC_FAILED);
+        if (!m->scratch.alloc((size_t)m->capacity * m->scratch_stride)) return MARS_ERR_ALLOC_FAILED;
     }
     tc_release(m->tc);
     m->tc.assign(m->prog.ops.size(), TcPlan());
@@ -375,25 +367,22 @@ static mars_error_t compile_model(Model *m) {
         if (o.impl == CONV_TC_F32) need = std::max(need, tf32_scratch_need(o, m->f32_mode));
     }
     need = (need + 1023) & ~(size_t)1023;
-    if (need > m->tc_scratch_stride || (need && !m->d_tc_scratch)) {
-        cudaFree(m->d_tc_scratch);
-        m->d_tc_scratch = nullptr;
+    if (need > m->tc_scratch_stride || (need && !m->tc_scratch.p)) {
         m->tc_scratch_stride = need;
-        CU_OK(cudaMalloc(&m->d_tc_scratch, (size_t)m->capacity * need), MARS_ERR_ALLOC_FAILED);
+        if (!m->tc_scratch.alloc((size_t)m->capacity * need)) return MARS_ERR_ALLOC_FAILED;
     }
     /* the link area is private to one compiled program: pads must be zero, so (re)allocate it zeroed every time */
-    cudaFree(m->d_linked);
-    m->d_linked = nullptr;
+    m->linked.reset();
     m->linked_stride = (m->prog.linked_bytes + 1023) & ~(size_t)1023;
     if (m->linked_stride) {
-        CU_OK(cudaMalloc(&m->d_linked, (size_t)m->capacity * m->linked_stride), MARS_ERR_ALLOC_FAILED);
-        CU_OK(cudaMemset(m->d_linked, 0, (size_t)m->capacity * m->linked_stride), MARS_ERR_ALLOC_FAILED);
+        if (!m->linked.alloc((size_t)m->capacity * m->linked_stride)) return MARS_ERR_ALLOC_FAILED;
+        CU_OK(cudaMemset(m->linked.p, 0, (size_t)m->capacity * m->linked_stride), MARS_ERR_ALLOC_FAILED);
     }
-    ArenaGeom g{m->d_weights, m->d_slots, m->weights_size, m->slot_stride, m->capacity, m->h_arena, m->prog.const_pool.data()};
+    ArenaGeom g{m->weights.p, m->slots.p, m->weights_size, m->slot_stride, m->capacity, m->h_arena, m->prog.const_pool.data()};
     for (size_t i = 0; i < m->prog.ops.size(); i++) {
         Op &o = m->prog.ops[i];
         if (o.impl == CONV_TC_F32) { /* float32 layer on the tf32 tensor path; a failed plan simply stays on the exact kernel */
-            if (!tf32_plan(o, g, m->f32_mode, m->d_tc_scratch, m->tc_scratch_stride, &m->tc[i])) {
+            if (!tf32_plan(o, g, m->f32_mode, m->tc_scratch.p, m->tc_scratch_stride, &m->tc[i])) {
                 if (strict_mode()) {
                     char why[600];
                     snprintf(why, sizeof why, "%s", g_err);
@@ -407,7 +396,7 @@ static mars_error_t compile_model(Model *m) {
         }
         if (o.impl != CONV_TC_NCHW) continue;
         const Op *consumer = o.nhwc_consumer >= 0 ? &m->prog.ops[o.nhwc_consumer] : nullptr;
-        if (!tc_plan(o, g, m->d_tc_scratch, m->tc_scratch_stride, m->d_linked, m->linked_stride, consumer, &m->tc[i])) {
+        if (!tc_plan(o, g, m->tc_scratch.p, m->tc_scratch_stride, m->linked.p, m->linked_stride, consumer, &m->tc[i])) {
             /* a fused op cannot simply fall back (its followers were folded): recompile exact -- unless the caller asked
              * to be told (mars_b200_set_strict / MARS_STRICT=1): the direct kernels are ~100x slower */
             if (strict_mode()) {
@@ -472,9 +461,9 @@ static mars_error_t launch_op(Model *m, size_t op_index, int first, int n, bool 
         const int C = o.oc, P = o.oh * o.ow;
         k_head_decode<<<n, 256, 0, m->stream>>>(reinterpret_cast<const int8_t *>(dev_addr(m, (size_t)o.in0, first)), m->slot_stride, o.oh, o.ow,
                                                 o.head_nc, o.head_nhwc ? 5 + o.head_nc : (5 + o.head_nc) * P, o.head_nhwc ? 1 : P,
-                                                o.head_nhwc ? C : 1, reinterpret_cast<const float *>(m->d_cpool + o.lut), (float)o.sh,
-                                                YOLO_LEVELS[o.head_level].anchors, o.f0, o.head_level > 0, m->d_box_raw + (size_t)first * MARS_MAX_DETS,
-                                                m->d_box_raw_cnt + first, MARS_MAX_DETS, HEAD_MAX_CAND);
+                                                o.head_nhwc ? C : 1, reinterpret_cast<const float *>(m->cpool.p + o.lut), (float)o.sh,
+                                                YOLO_LEVELS[o.head_level].anchors, o.f0, o.head_level > 0, m->rec.box_raw.at(first),
+                                                m->rec.box_raw.cnt.p + first, MARS_MAX_DETS, HEAD_MAX_CAND);
         m->launches++;
         CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
         return MARS_OK;
@@ -482,20 +471,20 @@ static mars_error_t launch_op(Model *m, size_t op_index, int first, int n, bool 
     if (o.kind == OP_GFL_HEAD) {
         k_gfl_decode<<<n, 256, 0, m->stream>>>(reinterpret_cast<const int8_t *>(dev_addr(m, (size_t)o.in0, first)), m->slot_stride, o.oh, o.ow,
                                                o.head_nc, o.head_reg_max, o.head_nhwc ? 1 : o.oh * o.ow, o.head_nhwc ? o.oc : 1,
-                                               reinterpret_cast<const float *>(m->d_cpool + o.lut), (float)o.sh, o.f2, (float)o.iw, (float)o.ih,
-                                               o.f0, o.head_level > 0, m->d_box_raw + (size_t)first * MARS_MAX_DETS, m->d_box_raw_cnt + first,
+                                               reinterpret_cast<const float *>(m->cpool.p + o.lut), (float)o.sh, o.f2, (float)o.iw, (float)o.ih,
+                                               o.f0, o.head_level > 0, m->rec.box_raw.at(first), m->rec.box_raw.cnt.p + first,
                                                MARS_MAX_DETS, HEAD_MAX_CAND);
         m->launches++;
         CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
         return MARS_OK;
     }
     ArenaView v;
-    v.wbase = m->d_weights;
-    v.sbase = m->d_slots + (size_t)first * m->slot_stride;
+    v.wbase = m->weights.p;
+    v.sbase = m->slots.p + (size_t)first * m->slot_stride;
     v.W = m->weights_size;
     v.slot_stride = m->slot_stride;
-    v.cpool = m->d_cpool;
-    v.scratch = m->d_scratch ? m->d_scratch + (size_t)first * m->scratch_stride : nullptr;
+    v.cpool = m->cpool.p;
+    v.scratch = m->scratch.p ? m->scratch.p + (size_t)first * m->scratch_stride : nullptr;
     v.scratch_stride = m->scratch_stride;
     KOp k = to_kop(o);
     cudaStream_t s = m->stream;
@@ -508,9 +497,9 @@ static mars_error_t launch_op(Model *m, size_t op_index, int first, int n, bool 
         const uint64_t P = (uint64_t)o.oh * o.ow;
         const int es = o.kind == OP_CONV_F32_NCHW ? 4 : 1;
         if (o.impl == CONV_TC_F32 && m->tc[op_index].f32) {
-            if (!tf32_launch(m->tc[op_index], m->d_slots, first, n, s, &m->launches)) return MARS_ERR_LAYER_FAILED;
+            if (!tf32_launch(m->tc[op_index], m->slots.p, first, n, s, &m->launches)) return MARS_ERR_LAYER_FAILED;
         } else if (o.impl == CONV_TC_NCHW && m->tc[op_index].i8) {
-            if (!tc_launch(m->tc[op_index], m->d_slots, first, n, full_pass, s, &m->launches)) return MARS_ERR_LAYER_FAILED;
+            if (!tc_launch(m->tc[op_index], m->slots.p, first, n, full_pass, s, &m->launches)) return MARS_ERR_LAYER_FAILED;
         } else if (o.mode == EXEC_PARALLEL) {
             if (o.kind == OP_CONV_I8_NCHW && !xl && fast_conv_nchw_ok(k)) {
                 launch_fast_conv_nchw(v, k, n, s);
@@ -622,12 +611,50 @@ static void profile_collect(Model *m) {
     }
 }
 
-static bool range_ok(Model *m, int first, int n) {
-    if (first < 0 || n < 0 || first + n > m->capacity) {
-        set_last_error("slots [%d,%d) outside the batch capacity %d (mars_b200_set_batch)", first, first + n, m->capacity);
-        return false;
+/* the start of every model entry point: *m = the model behind the handle, made the current device */
+static mars_error_t enter(mars_model_t *model, Model **m) {
+    *m = as_model(model);
+    if (!*m) return MARS_ERR_INVALID_FILE;
+    CU_OK(cudaSetDevice((*m)->device), MARS_ERR_NNA_INIT_FAILED);
+    return MARS_OK;
+}
+/* ... of an entry point that works on slots [first, first+n) */
+static mars_error_t enter(mars_model_t *model, Model **m, int first, int n) {
+    mars_error_t e = enter(model, m);
+    if (e == MARS_OK && (first < 0 || n < 0 || first + n > (*m)->capacity)) {
+        set_last_error("slots [%d,%d) outside the batch capacity %d (mars_b200_set_batch)", first, first + n, (*m)->capacity);
+        e = MARS_ERR_INVALID_TENSOR;
     }
-    return true;
+    return e;
+}
+
+static mars_error_t need_heads(Model *m, const char *what) {
+    if (!m->heads.empty()) return MARS_OK;
+    set_last_error("%s: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)", what);
+    return MARS_ERR_INVALID_TENSOR;
+}
+
+/* a setting the compiled program depends on is about to change: wait for the work that uses it; the next call recompiles (and
+ * drops the captured graphs) */
+static void invalidate_program(Model *m) {
+    cudaSetDevice(m->device);
+    cudaStreamSynchronize(m->stream);
+    m->compiled = false;
+}
+
+/* a synchronous call: enqueue() on the compute stream between ev0 and ev1, wait for it, and keep its device time as last_ms.
+ * The stream is idle afterwards, so a pending per-op profile pass is complete and folded in. */
+template <typename F> static mars_error_t timed_call(Model *m, const char *what, F enqueue) {
+    cudaEventRecord(m->ev0, m->stream);
+    mars_error_t e = enqueue();
+    cudaEventRecord(m->ev1, m->stream);
+    const cudaError_t ce = cudaStreamSynchronize(m->stream);
+    if (e == MARS_OK && ce != cudaSuccess) {
+        set_last_error("%s: %s", what, cudaGetErrorString(ce));
+        e = MARS_ERR_LAYER_FAILED;
+    }
+    if (e == MARS_OK) { cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1); profile_collect(m); }
+    return e;
 }
 
 /* ---- decode + NMS on the device ----------------------------------------------- */
@@ -650,8 +677,8 @@ static mars_error_t ensure_tables(Model *m, float scale) {
     if (m->tab_valid && memcmp(&m->tab_scale, &scale, 4) == 0) return MARS_OK;
     DecodeTables t;
     build_decode_tables(scale, &t);
-    if (!m->d_tab) CU_OK(cudaMalloc(&m->d_tab, sizeof(DecodeTables)), MARS_ERR_ALLOC_FAILED);
-    CU_OK(cudaMemcpyAsync(m->d_tab, &t, sizeof t, cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
+    if (!m->tab.p && !m->tab.alloc(1)) return MARS_ERR_ALLOC_FAILED;
+    CU_OK(cudaMemcpyAsync(m->tab.p, &t, sizeof t, cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED); /* t is a stack object */
     m->tab_scale = scale;
     m->tab_valid = true;
@@ -670,10 +697,10 @@ static mars_error_t enqueue_detect(Model *m, int first, int n, float thresh) {
     mars_error_t e = ensure_tables(m, d.scale);
     if (e != MARS_OK) return e;
     const int8_t *data = reinterpret_cast<const int8_t *>(dev_addr(m, m->toff[oi], first));
-    k_parse_output<<<n, 256, 0, m->stream>>>(data, m->slot_stride, d.shape[1], d.scale, m->d_tab, m->d_raw + (size_t)first * MARS_MAX_DETS,
-                                             m->d_raw_cnt + first, 1000, MARS_MAX_DETS);
-    CU_OK(launch_nms_center(m->d_raw + (size_t)first * MARS_MAX_DETS, m->d_raw_cnt + first, m->d_det + (size_t)first * MARS_MAX_DETS,
-                            m->d_det_cnt + first, MARS_MAX_DETS, thresh, n, m->d_nms_mask + (size_t)first * NMS_SCRATCH_WORDS, m->stream),
+    k_parse_output<<<n, 256, 0, m->stream>>>(data, m->slot_stride, d.shape[1], d.scale, m->tab.p, m->rec.raw.at(first),
+                                             m->rec.raw.cnt.p + first, 1000, MARS_MAX_DETS);
+    CU_OK(launch_nms_center(m->rec.raw.at(first), m->rec.raw.cnt.p + first, m->rec.det.at(first),
+                            m->rec.det.cnt.p + first, MARS_MAX_DETS, thresh, n, m->rec.nms_mask.p + (size_t)first * NMS_SCRATCH_WORDS, m->stream),
           MARS_ERR_LAYER_FAILED);
     m->launches += 3; /* parse, NMS sort, NMS suppression */
     CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
@@ -682,16 +709,12 @@ static mars_error_t enqueue_detect(Model *m, int first, int n, float thresh) {
 
 /* corner NMS + letterbox inverse over the candidates the program's OP_YOLO_HEAD / OP_GFL_HEAD ops left for slots [first, first+n) */
 static mars_error_t enqueue_heads_nms(Model *m, int first, int n, float thresh) {
-    if (m->heads.empty()) {
-        set_last_error("no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)");
-        return MARS_ERR_INVALID_TENSOR;
-    }
     const mars_tensor_t &in = m->pub.tensors[m->pub.header.input_tensor_ids[0]].desc; /* checked by the heads setters */
     const bool nhwc = in.format == MARS_FORMAT_NHWC;
     const int net_h = nhwc ? in.shape[1] : in.shape[2], net_w = nhwc ? in.shape[2] : in.shape[3];
-    k_nms_corner_batch<<<n, NMSB_THREADS, 0, m->stream>>>(m->d_box_raw + (size_t)first * MARS_MAX_DETS, m->d_box_raw_cnt + first,
-                                                         m->d_box + (size_t)first * MARS_MAX_DETS, m->d_box_cnt + first, MARS_MAX_DETS, thresh,
-                                                         m->d_nms_mask + (size_t)first * NMS_SCRATCH_WORDS, m->d_frame + first, net_w, net_h);
+    k_nms_corner_batch<<<n, NMSB_THREADS, 0, m->stream>>>(m->rec.box_raw.at(first), m->rec.box_raw.cnt.p + first,
+                                                         m->rec.box.at(first), m->rec.box.cnt.p + first, MARS_MAX_DETS, thresh,
+                                                         m->rec.nms_mask.p + (size_t)first * NMS_SCRATCH_WORDS, m->rec.frame.p + first, net_w, net_h);
     m->launches++;
     CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
@@ -703,6 +726,38 @@ static inline double now_us() {
     return ts.tv_sec * 1e6 + ts.tv_nsec * 1e-3;
 }
 
+/* a device buffer of at least `need` elements; growing waits for the compute stream, whose launches may still read the old one */
+template <typename T> static bool pre_grow(Model *m, DevBuf<T> &b, size_t *cap, size_t need) {
+    if (need <= *cap) return true;
+    cudaStreamSynchronize(m->stream);
+    *cap = 0;
+    if (!b.alloc(need)) return false;
+    *cap = need;
+    return true;
+}
+
+/* kept records of slots [first, first+n) of a record set -> dets[n][maxd], counts[n] on stream s */
+template <typename R>
+static mars_error_t copy_dets(const RecordSet<R> &rs, int first, int n, void *dets, int32_t *counts, int maxd, cudaStream_t s) {
+    if (maxd > 1000) maxd = 1000;
+    if (maxd < 0) maxd = 0;
+    CU_OK(cudaMemcpyAsync(counts, rs.cnt.p + first, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
+    if (maxd > 0)
+        CU_OK(cudaMemcpy2DAsync(dets, (size_t)maxd * sizeof(R), rs.at(first), (size_t)MARS_MAX_DETS * sizeof(R), (size_t)maxd * sizeof(R),
+                                (size_t)n, cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
+    return MARS_OK;
+}
+
+template <typename R>
+static mars_error_t download_records(mars_model_t *model, RecordSet<R> SlotRecords::*set, int first, int n, R *dets, int32_t *counts, int maxd) {
+    Model *m;
+    mars_error_t e = dets && counts ? enter(model, &m, first, n) : MARS_ERR_INVALID_FILE;
+    if (e == MARS_OK) e = copy_dets(m->rec.*set, first, n, dets, counts, maxd, m->stream);
+    if (e != MARS_OK) return e;
+    CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
+    for (int i = 0; i < n; i++) if (counts[i] > maxd) counts[i] = maxd;
+    return MARS_OK;
+}
 } // namespace marsb200
 
 using namespace marsb200;
@@ -721,42 +776,65 @@ const char *mars_get_error_string(mars_error_t err) {
     return (i >= 0 && i < 9) ? s[i] : "Unknown error";
 }
 
-/* reference src/mars/mars_runtime.c:126-349 */
-/* The planner's decisions for a .mars blob without touching a device: parses the tables, lays the tensors out as mars_load_memory
- * does (reference src/mars/mars_runtime.c:248-337), compiles the layer table at `opt_level` and writes the op list (one line per
- * op: kind, mode, kernel choice, fused / linked / forwarded / elided streams) to dst.  Returns the length of the description
- * (0 on error).  Host logic only -- the CPU test suite checks fusion, concat trimming and forwarding through it. */
-size_t mars_b200_plan_describe(const void *data, size_t size, size_t arena_bytes, int opt_level, char *dst, size_t cap) {
-    if (!data || size < sizeof(mars_header_t)) return 0;
-    mars_header_t h;
-    memcpy(&h, data, sizeof h);
-    if (h.magic != MARS_MAGIC || h.version_major != MARS_VERSION_MAJOR) return 0;
-    const size_t tables = sizeof h + (size_t)h.num_tensors * sizeof(mars_tensor_t) + (size_t)h.num_layers * sizeof(mars_layer_t);
-    if (size < tables || h.weights_offset > size || h.weights_size > size - h.weights_offset) return 0;
-    std::vector<mars_runtime_tensor_t> tensors(h.num_tensors ? h.num_tensors : 1);
-    std::vector<mars_runtime_layer_t> layers(h.num_layers ? h.num_layers : 1);
-    memset(tensors.data(), 0, tensors.size() * sizeof(mars_runtime_tensor_t));
-    memset(layers.data(), 0, layers.size() * sizeof(mars_runtime_layer_t));
-    const uint8_t *p = (const uint8_t *)data + sizeof h;
-    for (uint32_t i = 0; i < h.num_tensors; i++, p += sizeof(mars_tensor_t)) memcpy(&tensors[i].desc, p, sizeof(mars_tensor_t));
-    for (uint32_t i = 0; i < h.num_layers; i++, p += sizeof(mars_layer_t)) memcpy(&layers[i].desc, p, sizeof(mars_layer_t));
-    const size_t arena = arena_bytes ? arena_bytes : (size_t)8 << 20, W = (size_t)h.weights_size;
-    if (W > arena) return 0;
-    size_t remaining = arena - W, maxsz = 0;
+/* The header, tensor and layer tables of a .mars blob, without touching a device.  MARS_ERR_INVALID_MAGIC,
+ * MARS_ERR_VERSION_MISMATCH (*h holds the header), or MARS_ERR_INVALID_FILE when the blob is shorter than its header, its tables
+ * or its weights: the reference would read past the buffer there. */
+static mars_error_t parse_tables(const void *data, size_t size, mars_header_t *h, std::vector<mars_runtime_tensor_t> *tensors,
+                                 std::vector<mars_runtime_layer_t> *layers) {
+    if (!data || size < sizeof(mars_header_t)) return MARS_ERR_INVALID_FILE;
+    memcpy(h, data, sizeof *h);
+    if (h->magic != MARS_MAGIC) return MARS_ERR_INVALID_MAGIC;
+    if (h->version_major != MARS_VERSION_MAJOR) return MARS_ERR_VERSION_MISMATCH;
+    const size_t tables = sizeof *h + (size_t)h->num_tensors * sizeof(mars_tensor_t) + (size_t)h->num_layers * sizeof(mars_layer_t);
+    if (size < tables || h->weights_offset > size || h->weights_size > size - h->weights_offset) {
+        set_last_error("file truncated: %zu bytes, tables need %zu, weights [%llu,+%llu)", size, tables,
+                       (unsigned long long)h->weights_offset, (unsigned long long)h->weights_size);
+        return MARS_ERR_INVALID_FILE;
+    }
+    tensors->assign(h->num_tensors ? h->num_tensors : 1, mars_runtime_tensor_t());
+    layers->assign(h->num_layers ? h->num_layers : 1, mars_runtime_layer_t());
+    memset(tensors->data(), 0, tensors->size() * sizeof(mars_runtime_tensor_t));
+    memset(layers->data(), 0, layers->size() * sizeof(mars_runtime_layer_t));
+    const uint8_t *p = (const uint8_t *)data + sizeof *h;
+    for (uint32_t i = 0; i < h->num_tensors; i++, p += sizeof(mars_tensor_t)) memcpy(&(*tensors)[i].desc, p, sizeof(mars_tensor_t));
+    for (uint32_t i = 0; i < h->num_layers; i++, p += sizeof(mars_layer_t)) memcpy(&(*layers)[i].desc, p, sizeof(mars_layer_t));
+    return MARS_OK;
+}
+
+/* The work-buffer planner of reference src/mars/mars_runtime.c:248-337 (SURVEY Appendix C.1) behind weights of
+ * h.weights_size <= arena bytes, producing arena offsets: weight tensors point into the blob (:321-326), runtime tensors go
+ * round-robin into *num_buffers work buffers of *buffer_size bytes (:316-334).  False when the buffers do not fit the arena. */
+static bool plan_work_buffers(const mars_header_t &h, mars_runtime_tensor_t *tensors, size_t arena, size_t *num_buffers,
+                              size_t *buffer_size, std::vector<size_t> *toff) {
+    const size_t W = (size_t)h.weights_size, remaining = arena - W;
+    size_t maxsz = 0;
     for (uint32_t i = 0; i < h.num_tensors; i++)
         if (tensors[i].desc.data_size == 0) maxsz = std::max(maxsz, (tensor_byte_size(&tensors[i].desc) + 63) & ~(size_t)63);
     size_t nb = 3, bs = maxsz;
     if (bs * nb > remaining) nb = 2;
-    if (bs * nb > remaining) { bs = (remaining / 2) & ~(size_t)63; if (bs < 65536) return 0; }
-    std::vector<size_t> toff(h.num_tensors ? h.num_tensors : 1);
-    uint32_t k = 0;
-    for (uint32_t i = 0; i < h.num_tensors; i++) {
-        if (tensors[i].desc.data_size > 0) { toff[i] = (size_t)tensors[i].desc.data_offset; tensors[i].alloc_size = (size_t)tensors[i].desc.data_size; }
-        else { toff[i] = W + (size_t)(k % nb) * bs; tensors[i].alloc_size = bs; k++; }
+    if (bs * nb > remaining) {
+        bs = (remaining / 2) & ~(size_t)63;
+        if (bs < 65536) return false;
     }
-    Program prog;
-    if (compile_program(h, tensors.data(), layers.data(), toff, W, arena, opt_level, 0, &prog, 2 /* the library's default float32 mode: tf32x3 */) != MARS_OK) return 0;
-    const std::string s = describe_program(prog);
+    toff->assign(h.num_tensors ? h.num_tensors : 1, 0);
+    for (uint32_t i = 0, k = 0; i < h.num_tensors; i++) {
+        mars_runtime_tensor_t &t = tensors[i];
+        if (t.desc.data_size > 0) {
+            (*toff)[i] = (size_t)t.desc.data_offset;
+            t.alloc_size = (size_t)t.desc.data_size;
+        } else {
+            (*toff)[i] = W + (size_t)(k % nb) * bs;
+            t.alloc_size = bs;
+            k++;
+        }
+    }
+    *num_buffers = nb;
+    *buffer_size = bs;
+    return true;
+}
+
+/* s -> dst, cut to cap - 1 bytes and NUL-terminated; returns the length of s */
+static size_t copy_out(const std::string &s, char *dst, size_t cap) {
     if (dst && cap) {
         const size_t n = std::min(cap - 1, s.size());
         memcpy(dst, s.data(), n);
@@ -765,22 +843,24 @@ size_t mars_b200_plan_describe(const void *data, size_t size, size_t arena_bytes
     return s.size();
 }
 
-/* the header, tensor and layer tables of a .mars blob, without touching a device; false when it is not one */
-static bool parse_tables(const void *data, size_t size, mars_header_t *h, std::vector<mars_runtime_tensor_t> *tensors,
-                         std::vector<mars_runtime_layer_t> *layers) {
-    if (!data || size < sizeof(mars_header_t)) return false;
-    memcpy(h, data, sizeof *h);
-    if (h->magic != MARS_MAGIC || h->version_major != MARS_VERSION_MAJOR) return false;
-    const size_t tables = sizeof *h + (size_t)h->num_tensors * sizeof(mars_tensor_t) + (size_t)h->num_layers * sizeof(mars_layer_t);
-    if (size < tables) return false;
-    tensors->assign(h->num_tensors ? h->num_tensors : 1, mars_runtime_tensor_t());
-    layers->assign(h->num_layers ? h->num_layers : 1, mars_runtime_layer_t());
-    memset(tensors->data(), 0, tensors->size() * sizeof(mars_runtime_tensor_t));
-    memset(layers->data(), 0, layers->size() * sizeof(mars_runtime_layer_t));
-    const uint8_t *p = (const uint8_t *)data + sizeof *h;
-    for (uint32_t i = 0; i < h->num_tensors; i++, p += sizeof(mars_tensor_t)) memcpy(&(*tensors)[i].desc, p, sizeof(mars_tensor_t));
-    for (uint32_t i = 0; i < h->num_layers; i++, p += sizeof(mars_layer_t)) memcpy(&(*layers)[i].desc, p, sizeof(mars_layer_t));
-    return true;
+/* The planner's decisions for a .mars blob without touching a device: parses the tables, lays the tensors out as mars_load_memory
+ * does, compiles the layer table at `opt_level` and writes the op list (one line per op: kind, mode, kernel choice, fused /
+ * linked / forwarded / elided streams) to dst.  Returns the length of the description (0 on error).  Host logic only -- the CPU
+ * test suite checks fusion, concat trimming and forwarding through it. */
+size_t mars_b200_plan_describe(const void *data, size_t size, size_t arena_bytes, int opt_level, char *dst, size_t cap) {
+    mars_header_t h;
+    std::vector<mars_runtime_tensor_t> tensors;
+    std::vector<mars_runtime_layer_t> layers;
+    if (parse_tables(data, size, &h, &tensors, &layers) != MARS_OK) return 0;
+    const size_t arena = arena_bytes ? arena_bytes : (size_t)8 << 20;
+    size_t nb, bs;
+    std::vector<size_t> toff;
+    if (h.weights_size > arena || !plan_work_buffers(h, tensors.data(), arena, &nb, &bs, &toff)) return 0;
+    Program prog;
+    if (compile_program(h, tensors.data(), layers.data(), toff, (size_t)h.weights_size, arena, opt_level, 0, &prog,
+                        2 /* the library's default float32 mode: tf32x3 */) != MARS_OK)
+        return 0;
+    return copy_out(describe_program(prog), dst, cap);
 }
 
 /* The outputs of the three CONV2D layers of a YOLOv5 Detect block, stride 8 / 16 / 32, without touching a device */
@@ -788,7 +868,7 @@ int mars_b200_find_yolo_heads(const void *data, size_t size, uint32_t *tensor_id
     mars_header_t h;
     std::vector<mars_runtime_tensor_t> tensors;
     std::vector<mars_runtime_layer_t> layers;
-    if (!parse_tables(data, size, &h, &tensors, &layers)) return 0;
+    if (parse_tables(data, size, &h, &tensors, &layers) != MARS_OK) return 0;
     return find_yolo_heads(h, tensors.data(), layers.data(), tensor_ids, cap);
 }
 
@@ -797,28 +877,21 @@ int mars_b200_find_gfl_heads(const void *data, size_t size, int nc, int reg_max,
     mars_header_t h;
     std::vector<mars_runtime_tensor_t> tensors;
     std::vector<mars_runtime_layer_t> layers;
-    if (!parse_tables(data, size, &h, &tensors, &layers)) return 0;
+    if (parse_tables(data, size, &h, &tensors, &layers) != MARS_OK) return 0;
     return find_gfl_heads(h, tensors.data(), layers.data(), nc, reg_max, tensor_ids, cap);
 }
 
+/* reference src/mars/mars_runtime.c:126-349 */
 mars_error_t mars_load_memory(const void *data, size_t size, mars_model_t **out_model) {
-    if (!data || !out_model || size < sizeof(mars_header_t)) return MARS_ERR_INVALID_FILE;
+    if (!out_model) return MARS_ERR_INVALID_FILE;
     mars_header_t h;
-    memcpy(&h, data, sizeof h);
-    if (h.magic != MARS_MAGIC) {
-        fprintf(stderr, "Mars: Invalid magic 0x%08x (expected 0x%08x)\n", h.magic, MARS_MAGIC);
-        return MARS_ERR_INVALID_MAGIC;
-    }
-    if (h.version_major != MARS_VERSION_MAJOR) {
+    std::vector<mars_runtime_tensor_t> tensors;
+    std::vector<mars_runtime_layer_t> layers;
+    const mars_error_t pe = parse_tables(data, size, &h, &tensors, &layers);
+    if (pe == MARS_ERR_INVALID_MAGIC) fprintf(stderr, "Mars: Invalid magic 0x%08x (expected 0x%08x)\n", h.magic, MARS_MAGIC);
+    if (pe == MARS_ERR_VERSION_MISMATCH)
         fprintf(stderr, "Mars: Version mismatch %d.%d (expected %d.x)\n", h.version_major, h.version_minor, MARS_VERSION_MAJOR);
-        return MARS_ERR_VERSION_MISMATCH;
-    }
-    const size_t tables = sizeof h + (size_t)h.num_tensors * sizeof(mars_tensor_t) + (size_t)h.num_layers * sizeof(mars_layer_t);
-    if (size < tables || h.weights_offset > size || h.weights_size > size - h.weights_offset) {
-        set_last_error("file truncated: %zu bytes, tables need %zu, weights [%llu,+%llu)", size, tables,
-                       (unsigned long long)h.weights_offset, (unsigned long long)h.weights_size);
-        return MARS_ERR_INVALID_FILE; /* the reference would read past the buffer here */
-    }
+    if (pe != MARS_OK) return pe;
     if (!g_ready && device_up() != NNA_SUCCESS) return MARS_ERR_NNA_INIT_FAILED;
     CU_OK(cudaSetDevice(g_device), MARS_ERR_NNA_INIT_FAILED);
 
@@ -828,12 +901,11 @@ mars_error_t mars_load_memory(const void *data, size_t size, mars_model_t **out_
     m->device = g_device;
     { const char *e = getenv("MARS_F32_MODE"); if (e && *e) m->f32_mode = std::max(0, std::min(2, atoi(e))); }
     m->pub.header = h;
-    m->pub.tensors = (mars_runtime_tensor_t *)calloc(h.num_tensors ? h.num_tensors : 1, sizeof(mars_runtime_tensor_t));
-    m->pub.layers = (mars_runtime_layer_t *)calloc(h.num_layers ? h.num_layers : 1, sizeof(mars_runtime_layer_t));
+    m->pub.tensors = (mars_runtime_tensor_t *)calloc(tensors.size(), sizeof(mars_runtime_tensor_t));
+    m->pub.layers = (mars_runtime_layer_t *)calloc(layers.size(), sizeof(mars_runtime_layer_t));
     if (!m->pub.tensors || !m->pub.layers) { model_release(m); return MARS_ERR_ALLOC_FAILED; }
-    const uint8_t *p = (const uint8_t *)data + sizeof h;
-    for (uint32_t i = 0; i < h.num_tensors; i++, p += sizeof(mars_tensor_t)) memcpy(&m->pub.tensors[i].desc, p, sizeof(mars_tensor_t));
-    for (uint32_t i = 0; i < h.num_layers; i++, p += sizeof(mars_layer_t)) memcpy(&m->pub.layers[i].desc, p, sizeof(mars_layer_t));
+    memcpy(m->pub.tensors, tensors.data(), tensors.size() * sizeof(mars_runtime_tensor_t));
+    memcpy(m->pub.layers, layers.data(), layers.size() * sizeof(mars_runtime_layer_t));
 
     /* arena size: the reference's literal 8 MiB (:209) unless the application asked for more */
     size_t arena = g_arena_bytes;
@@ -849,30 +921,17 @@ mars_error_t mars_load_memory(const void *data, size_t size, mars_model_t **out_
         model_release(m);
         return MARS_ERR_ALLOC_FAILED;
     }
-
-    /* the planner of reference :248-337 (SURVEY Appendix C.1), producing arena offsets */
-    size_t remaining = arena - m->weights_size, maxsz = 0;
-    for (uint32_t i = 0; i < h.num_tensors; i++)
-        if (m->pub.tensors[i].desc.data_size == 0) {
-            size_t sz = (tensor_byte_size(&m->pub.tensors[i].desc) + 63) & ~(size_t)63;
-            maxsz = std::max(maxsz, sz);
-        }
-    size_t nb = 3, bs = maxsz;
-    if (bs * nb > remaining) nb = 2;
-    if (bs * nb > remaining) {
-        bs = (remaining / 2) & ~(size_t)63;
-        if (bs < 65536) {
-            fprintf(stderr, "Mars: Not enough DDR for work buffers (set MARS_ARENA_BYTES / mars_b200_set_arena_bytes)\n");
-            model_release(m);
-            return MARS_ERR_ALLOC_FAILED;
-        }
+    size_t nb, bs;
+    if (!plan_work_buffers(h, m->pub.tensors, arena, &nb, &bs, &m->toff)) {
+        fprintf(stderr, "Mars: Not enough DDR for work buffers (set MARS_ARENA_BYTES / mars_b200_set_arena_bytes)\n");
+        model_release(m);
+        return MARS_ERR_ALLOC_FAILED;
     }
     m->num_buffers = (int)nb;
     m->buffer_size = bs;
     m->slot_bytes = nb * bs;
     m->slot_stride = (m->slot_bytes + 1023) & ~(size_t)1023;
     if (m->slot_stride == 0) m->slot_stride = 1024;
-    m->toff.resize(h.num_tensors ? h.num_tensors : 1);
 
     if (cudaHostAlloc((void **)&m->h_arena, arena + 4096, cudaHostAllocDefault) != cudaSuccess) {
         set_last_error("pinned host mirror of %zu bytes: %s", arena, cudaGetErrorString(cudaGetLastError()));
@@ -882,9 +941,9 @@ mars_error_t mars_load_memory(const void *data, size_t size, mars_model_t **out_
     memset(m->h_arena, 0, arena + 4096);
     memcpy(m->h_arena, (const uint8_t *)data + h.weights_offset, m->weights_size);
     /* 64 KiB of zeroed slack behind the weights keeps stray device reads mapped */
-    if (cudaMalloc(&m->d_weights, m->weights_size + 65536) != cudaSuccess ||
-        cudaMemset(m->d_weights, 0, m->weights_size + 65536) != cudaSuccess ||
-        cudaMemcpy(m->d_weights, m->h_arena, m->weights_size, cudaMemcpyHostToDevice) != cudaSuccess ||
+    if (!m->weights.alloc(m->weights_size + 65536) ||
+        cudaMemset(m->weights.p, 0, m->weights_size + 65536) != cudaSuccess ||
+        cudaMemcpy(m->weights.p, m->h_arena, m->weights_size, cudaMemcpyHostToDevice) != cudaSuccess ||
         cudaStreamCreateWithFlags(&m->stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaStreamCreateWithFlags(&m->h2d_stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaStreamCreateWithFlags(&m->d2h_stream, cudaStreamNonBlocking) != cudaSuccess ||
@@ -900,19 +959,9 @@ mars_error_t mars_load_memory(const void *data, size_t size, mars_model_t **out_
     }
     for (auto &st : m->pre_stage) cudaEventCreateWithFlags(&st.ev, cudaEventDisableTiming);
 
-    uint32_t k = 0;
     for (uint32_t i = 0; i < h.num_tensors; i++) {
-        mars_runtime_tensor_t &t = m->pub.tensors[i];
-        if (t.desc.data_size > 0) { /* weight tensor: points into the blob (:321-326) */
-            m->toff[i] = (size_t)t.desc.data_offset;
-            t.alloc_size = (size_t)t.desc.data_size;
-        } else { /* runtime tensor: round-robin work buffer (:316-334) */
-            m->toff[i] = m->weights_size + (size_t)(k % nb) * bs;
-            t.alloc_size = bs;
-            k++;
-        }
-        t.vaddr = m->toff[i] <= arena ? m->h_arena + m->toff[i] : nullptr;
-        t.is_external = false;
+        m->pub.tensors[i].vaddr = m->toff[i] <= arena ? m->h_arena + m->toff[i] : nullptr;
+        m->pub.tensors[i].is_external = false;
     }
     m->pub.ddr_base = m->h_arena;
     m->pub.ddr_size = arena;
@@ -996,47 +1045,44 @@ void mars_print_summary(mars_model_t *model) {
                   m->num_buffers, m->buffer_size, m->capacity, m->prog.ops.size());
 }
 
-/* reference src/mars/mars_runtime.c:439-459: synchronous, one image */
-mars_error_t mars_run(mars_model_t *model) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    double t0 = now_us();
+/* the host mirror's work buffers <-> slot 0 on the compute stream: those holding the model's inputs (or outputs), each once,
+ * or with MARS_MIRROR=full the whole slot */
+static mars_error_t mirror_work_buffers(Model *m, bool outputs) {
     static int full_mirror = -1;
     if (full_mirror < 0) { const char *e = getenv("MARS_MIRROR"); full_mirror = (e && !strcmp(e, "full")) ? 1 : 0; }
-    const size_t W = m->weights_size;
+    const mars_header_t &h = m->pub.header;
+    const cudaMemcpyKind kind = outputs ? cudaMemcpyDeviceToHost : cudaMemcpyHostToDevice;
+    uint8_t *host = m->h_arena + m->weights_size, *dev = m->slots.p;
     if (full_mirror) {
-        CU_OK(cudaMemcpyAsync(m->d_slots, m->h_arena + W, m->slot_bytes, cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
-    } else {
-        bool done[3] = {false, false, false};
-        for (uint32_t i = 0; i < model->header.num_inputs && i < 4; i++) {
-            uint32_t ti = model->header.input_tensor_ids[i];
-            if (ti >= model->header.num_tensors || m->toff[ti] < W) continue;
-            size_t b = (m->toff[ti] - W) / m->buffer_size;
-            if (b < 3 && !done[b]) {
-                done[b] = true;
-                CU_OK(cudaMemcpyAsync(m->d_slots + b * m->buffer_size, m->h_arena + W + b * m->buffer_size, m->buffer_size,
-                                      cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
-            }
+        CU_OK(cudaMemcpyAsync(outputs ? host : dev, outputs ? dev : host, m->slot_bytes, kind, m->stream), MARS_ERR_LAYER_FAILED);
+        return MARS_OK;
+    }
+    bool done[3] = {false, false, false};
+    for (uint32_t i = 0; i < (outputs ? h.num_outputs : h.num_inputs) && i < 4; i++) {
+        const uint32_t ti = outputs ? h.output_tensor_ids[i] : h.input_tensor_ids[i];
+        if (ti >= h.num_tensors || m->toff[ti] < m->weights_size) continue;
+        const size_t b = (m->toff[ti] - m->weights_size) / m->buffer_size, off = b * m->buffer_size;
+        if (b < 3 && !done[b]) {
+            done[b] = true;
+            CU_OK(cudaMemcpyAsync(outputs ? host + off : dev + off, outputs ? dev + off : host + off, m->buffer_size, kind, m->stream),
+                  MARS_ERR_LAYER_FAILED);
         }
     }
-    mars_error_t e = enqueue_ops(m, 0, 1, -1);
+    return MARS_OK;
+}
+
+/* reference src/mars/mars_runtime.c:439-459: synchronous, one image */
+mars_error_t mars_run(mars_model_t *model) {
+    Model *m;
+    mars_error_t e = enter(model, &m);
+    if (e != MARS_OK) return e;
+    double t0 = now_us();
+    e = mirror_work_buffers(m, false);
+    if (e != MARS_OK) return e;
+    e = enqueue_ops(m, 0, 1, -1);
     if (e != MARS_OK) { cudaStreamSynchronize(m->stream); return e; }
-    if (full_mirror) {
-        CU_OK(cudaMemcpyAsync(m->h_arena + W, m->d_slots, m->slot_bytes, cudaMemcpyDeviceToHost, m->stream), MARS_ERR_LAYER_FAILED);
-    } else {
-        bool done[3] = {false, false, false};
-        for (uint32_t i = 0; i < model->header.num_outputs && i < 4; i++) {
-            uint32_t ti = model->header.output_tensor_ids[i];
-            if (ti >= model->header.num_tensors || m->toff[ti] < W) continue;
-            size_t b = (m->toff[ti] - W) / m->buffer_size;
-            if (b < 3 && !done[b]) {
-                done[b] = true;
-                CU_OK(cudaMemcpyAsync(m->h_arena + W + b * m->buffer_size, m->d_slots + b * m->buffer_size, m->buffer_size,
-                                      cudaMemcpyDeviceToHost, m->stream), MARS_ERR_LAYER_FAILED);
-            }
-        }
-    }
+    e = mirror_work_buffers(m, true);
+    if (e != MARS_OK) return e;
     cudaError_t ce = cudaStreamSynchronize(m->stream);
     if (ce != cudaSuccess) {
         set_last_error("mars_run: %s", cudaGetErrorString(ce));
@@ -1066,53 +1112,51 @@ void mars_b200_set_arena_bytes(size_t bytes) { g_arena_bytes = bytes; }
 const char *mars_b200_last_error(void) { return g_err; }
 
 mars_error_t mars_b200_arena_upload(mars_model_t *model, int slot) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, slot, 1)) return MARS_ERR_INVALID_TENSOR;
+    Model *m;
+    mars_error_t e = enter(model, &m, slot, 1);
+    if (e != MARS_OK) return e;
     /* the host mirror of the weights is writable (model->weights, tensor->vaddr, as in the reference): the tensor-core plans
      * hold a repacked copy and requantisation bounds derived from the blob, so an edit invalidates the compiled program */
-    if (m->compiled && fnv1a(m->h_arena, m->weights_size) != m->weights_hash) { cudaStreamSynchronize(m->stream); m->compiled = false; }
-    CU_OK(cudaMemcpyAsync(m->d_weights, m->h_arena, m->weights_size, cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
+    if (m->compiled && fnv1a(m->h_arena, m->weights_size) != m->weights_hash) invalidate_program(m);
+    CU_OK(cudaMemcpyAsync(m->weights.p, m->h_arena, m->weights_size, cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
     size_t nbytes = std::min(m->slot_bytes, m->arena_size - m->weights_size);
-    CU_OK(cudaMemcpyAsync(m->d_slots + (size_t)slot * m->slot_stride, m->h_arena + m->weights_size, nbytes,
+    CU_OK(cudaMemcpyAsync(m->slots.p + (size_t)slot * m->slot_stride, m->h_arena + m->weights_size, nbytes,
                           cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     return compile_model(m);
 }
 
 mars_error_t mars_b200_arena_download(mars_model_t *model, int slot, void *host_dst, size_t bytes) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, slot, 1)) return MARS_ERR_INVALID_TENSOR;
+    Model *m;
+    mars_error_t e = enter(model, &m, slot, 1);
+    if (e != MARS_OK) return e;
     uint8_t *dst = host_dst ? (uint8_t *)host_dst : m->h_arena;
     if (!host_dst || bytes > m->weights_size + m->slot_bytes) bytes = std::min(m->arena_size, m->weights_size + m->slot_bytes);
     size_t wb = std::min(bytes, m->weights_size);
-    CU_OK(cudaMemcpyAsync(dst, m->d_weights, wb, cudaMemcpyDeviceToHost, m->stream), MARS_ERR_LAYER_FAILED);
+    CU_OK(cudaMemcpyAsync(dst, m->weights.p, wb, cudaMemcpyDeviceToHost, m->stream), MARS_ERR_LAYER_FAILED);
     if (bytes > wb)
-        CU_OK(cudaMemcpyAsync(dst + wb, m->d_slots + (size_t)slot * m->slot_stride, bytes - wb, cudaMemcpyDeviceToHost,
+        CU_OK(cudaMemcpyAsync(dst + wb, m->slots.p + (size_t)slot * m->slot_stride, bytes - wb, cudaMemcpyDeviceToHost,
                               m->stream), MARS_ERR_LAYER_FAILED);
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
 }
 
 mars_error_t mars_b200_arena_clear(mars_model_t *model) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    CU_OK(cudaMemsetAsync(m->d_slots, 0, (size_t)m->capacity * m->slot_stride, m->stream), MARS_ERR_LAYER_FAILED);
+    Model *m;
+    mars_error_t e = enter(model, &m);
+    if (e != MARS_OK) return e;
+    CU_OK(cudaMemsetAsync(m->slots.p, 0, (size_t)m->capacity * m->slot_stride, m->stream), MARS_ERR_LAYER_FAILED);
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     memset(m->h_arena + m->weights_size, 0, m->arena_size - m->weights_size);
     return MARS_OK;
 }
 
 mars_error_t mars_b200_run_layer(mars_model_t *model, uint32_t layer) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
+    Model *m;
+    mars_error_t e = enter(model, &m);
+    if (e != MARS_OK) return e;
     if (layer >= model->header.num_layers) return MARS_ERR_INVALID_LAYER;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    mars_error_t e = enqueue_ops(m, 0, 1, (int)layer);
+    e = enqueue_ops(m, 0, 1, (int)layer);
     cudaError_t ce = cudaStreamSynchronize(m->stream);
     if (e == MARS_OK && ce != cudaSuccess) {
         set_last_error("run_layer %u: %s", layer, cudaGetErrorString(ce));
@@ -1125,22 +1169,14 @@ size_t mars_b200_describe(mars_model_t *model, char *dst, size_t cap) {
     Model *m = as_model(model);
     if (!m) return 0;
     if (compile_model(m) != MARS_OK) return 0;
-    std::string s = describe_program(m->prog);
-    if (dst && cap) {
-        size_t n = std::min(cap - 1, s.size());
-        memcpy(dst, s.data(), n);
-        dst[n] = 0;
-    }
-    return s.size();
+    return copy_out(describe_program(m->prog), dst, cap);
 }
 
 void mars_b200_set_opt_level(mars_model_t *model, int level) {
     Model *m = as_model(model);
     if (!m || m->opt_level == level) return;
-    cudaSetDevice(m->device);
-    cudaStreamSynchronize(m->stream);
+    invalidate_program(m);
     m->opt_level = level;
-    m->compiled = false;
 }
 void mars_b200_set_strict(int on) { g_strict = on ? 1 : 0; }
 
@@ -1151,10 +1187,8 @@ static mars_error_t replace_heads(Model *m, HeadSet hs) {
                 (hs.empty() || (memcmp(&hs.conf, &o.conf, 4) == 0 && hs.reg_max == o.reg_max && hs.centre == o.centre));
     for (size_t k = 0; same && k < hs.heads.size(); k++) same = hs.heads[k].id == o.heads[k].id && hs.heads[k].nc == o.heads[k].nc;
     if (same) return MARS_OK;
-    cudaSetDevice(m->device);
-    cudaStreamSynchronize(m->stream);
+    invalidate_program(m);
     m->heads = std::move(hs);
-    m->compiled = false; /* the next call recompiles and drops the captured graphs */
     return MARS_OK;
 }
 
@@ -1205,41 +1239,35 @@ mars_error_t mars_b200_set_gfl_heads(mars_model_t *model, const uint32_t *tensor
 }
 
 mars_error_t mars_b200_set_frame_size(mars_model_t *model, int first, int n, int w, int h) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
+    Model *m;
+    mars_error_t e = enter(model, &m, first, n);
+    if (e != MARS_OK) return e;
     if (w < 0 || h < 0 || (w == 0) != (h == 0)) {
         set_last_error("set_frame_size: %d x %d is not a frame size (0 x 0 clears it)", w, h);
         return MARS_ERR_INVALID_TENSOR;
     }
     std::vector<int2> fr((size_t)n, make_int2(w, h));
-    if (n > 0) CU_OK(cudaMemcpyAsync(m->d_frame + first, fr.data(), (size_t)n * sizeof(int2), cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
+    if (n > 0) CU_OK(cudaMemcpyAsync(m->rec.frame.p + first, fr.data(), (size_t)n * sizeof(int2), cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
 }
 void mars_b200_set_f32_mode(mars_model_t *model, int mode) {
     Model *m = as_model(model);
     if (!m || m->f32_mode == mode) return;
-    cudaSetDevice(m->device);
-    cudaStreamSynchronize(m->stream);
+    invalidate_program(m);
     m->f32_mode = mode < 0 ? 0 : (mode > 2 ? 2 : mode);
-    m->compiled = false;
 }
 void mars_b200_set_depthwise_mode(mars_model_t *model, int mode) {
     Model *m = as_model(model);
     if (!m || m->depthwise_mode == mode) return;
-    cudaSetDevice(m->device);
-    cudaStreamSynchronize(m->stream);
+    invalidate_program(m);
     m->depthwise_mode = mode;
-    m->compiled = false;
 }
 
 mars_error_t mars_b200_set_batch(mars_model_t *model, int capacity) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    mars_error_t e = set_capacity(m, capacity);
+    Model *m;
+    mars_error_t e = enter(model, &m);
+    if (e == MARS_OK) e = set_capacity(m, capacity);
     if (e == MARS_OK) e = compile_model(m);
     return e;
 }
@@ -1261,7 +1289,6 @@ size_t mars_b200_output_bytes(mars_model_t *model) { return io_bytes(model, 1); 
 
 static mars_error_t copy_io(Model *m, int first, int n, void *host, size_t stride, int output, cudaStream_t s) {
     mars_model_t *model = &m->pub;
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
     uint32_t ti = output ? model->header.output_tensor_ids[0] : model->header.input_tensor_ids[0];
     if ((output ? model->header.num_outputs : model->header.num_inputs) < 1 || ti >= model->header.num_tensors ||
         m->toff[ti] < m->weights_size)
@@ -1279,19 +1306,17 @@ static mars_error_t copy_io(Model *m, int first, int n, void *host, size_t strid
 }
 
 mars_error_t mars_b200_upload_inputs(mars_model_t *model, int first, int n, const void *host, size_t stride) {
-    Model *m = as_model(model);
-    if (!m || !host) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    mars_error_t e = copy_io(m, first, n, const_cast<void *>(host), stride, 0, m->stream);
+    Model *m;
+    mars_error_t e = host ? enter(model, &m, first, n) : MARS_ERR_INVALID_FILE;
+    if (e == MARS_OK) e = copy_io(m, first, n, const_cast<void *>(host), stride, 0, m->stream);
     if (e != MARS_OK) return e;
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
 }
 mars_error_t mars_b200_download_outputs(mars_model_t *model, int first, int n, void *host, size_t stride) {
-    Model *m = as_model(model);
-    if (!m || !host) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    mars_error_t e = copy_io(m, first, n, host, stride, 1, m->stream);
+    Model *m;
+    mars_error_t e = host ? enter(model, &m, first, n) : MARS_ERR_INVALID_FILE;
+    if (e == MARS_OK) e = copy_io(m, first, n, host, stride, 1, m->stream);
     if (e != MARS_OK) return e;
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
@@ -1471,17 +1496,6 @@ static const ResizeTaps &cached_taps(Model *m, int in, int out) {
     return t;
 }
 
-/* a device buffer of at least `need` bytes; growing waits for the compute stream, whose launches may still read the old one */
-static bool pre_grow(Model *m, uint8_t **p, size_t *cap, size_t need) {
-    if (need <= *cap) return true;
-    cudaStreamSynchronize(m->stream);
-    cudaFree(*p);
-    *p = nullptr; *cap = 0;
-    if (cudaMalloc(p, need) != cudaSuccess) { *p = nullptr; return false; }
-    *cap = need;
-    return true;
-}
-
 /* host frames [f0, f1) of a table -> their staging offsets, tight rows (pre_frame_bytes): one copy per RGB8 frame, one per NV12
  * plane.  RGB8 frames of one size with tight rows that sit equally spaced in host memory (mars_b200_preprocess_batch) go in
  * one copy. */
@@ -1519,7 +1533,7 @@ static cudaError_t pre_stage_frames(const PreTable &t, const FrameSrc *frames, i
  * completed; growing the device table waits for the compute stream (pre_grow). */
 static mars_error_t pre_upload(Model *m, Model::PreStage &st, const PreTable &t, cudaStream_t s) {
     const size_t tab = t.bytes();
-    if (!pre_grow(m, &st.d_tab, &st.tab_cap, tab)) {
+    if (!pre_grow(m, st.tab, &st.tab_cap, tab)) {
         set_last_error("preprocess: out of device memory for a %zu-byte table", tab);
         return MARS_ERR_ALLOC_FAILED;
     }
@@ -1531,7 +1545,7 @@ static mars_error_t pre_upload(Model *m, Model::PreStage &st, const PreTable &t,
         st.h_cap = tab;
     }
     t.pack(st.h_tab);
-    CU_OK(cudaMemcpyAsync(st.d_tab, st.h_tab, tab, cudaMemcpyHostToDevice, s), MARS_ERR_LAYER_FAILED);
+    CU_OK(cudaMemcpyAsync(st.tab.p, st.h_tab, tab, cudaMemcpyHostToDevice, s), MARS_ERR_LAYER_FAILED);
     CU_OK(cudaEventRecord(st.ev, s), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
 }
@@ -1559,8 +1573,7 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
     const bool per_launch = how == PRE_HOST_SYNC && !rois;
     pre_table_stage(&t, fbytes.data(), nfr, per_launch);
     if (rois && merge_tab) merge_table(nfr, *rois, &t.merge);
-    if ((how != PRE_DEVICE && !pre_grow(m, &st.d_frames, &st.frames_cap, t.stage_bytes)) ||
-        !pre_grow(m, (uint8_t **)&m->d_preH, &m->preH_cap, t.h_floats * sizeof(float))) {
+    if ((how != PRE_DEVICE && !pre_grow(m, st.frames, &st.frames_cap, t.stage_bytes)) || !pre_grow(m, m->preH, &m->preH_cap, t.h_floats)) {
         set_last_error("preprocess: out of device memory for %d frames", n);
         return MARS_ERR_ALLOC_FAILED;
     }
@@ -1575,7 +1588,7 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
             d.src = a.p0; d.uv = a.p1;
             d.row_stride = a.pitch0; d.uv_stride = a.pitch1;
         } else { /* the tight staging layout of pre_stage_frames */
-            d.src = st.d_frames + t.stage[f];
+            d.src = st.frames.p + t.stage[f];
             d.row_stride = (size_t)a.w * (nv12 ? 1 : 3);
             d.uv = nv12 ? d.src + (size_t)a.w * a.h : nullptr;
             d.uv_stride = nv12 ? (size_t)2 * ((a.w + 1) / 2) : 0;
@@ -1584,9 +1597,9 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
     cudaStream_t cs = how == PRE_HOST_POOL ? m->h2d_stream : m->stream;
     mars_error_t e = pre_upload(m, st, t, cs);
     if (e != MARS_OK) return e;
-    if (merge_tab) *merge_tab = reinterpret_cast<const int *>(st.d_tab + t.merge_offset());
+    if (merge_tab) *merge_tab = reinterpret_cast<const int *>(st.tab.p + t.merge_offset());
     if (how == PRE_HOST_POOL || (how == PRE_HOST_SYNC && !per_launch)) {
-        CU_OK(pre_stage_frames(t, frames.data(), 0, nfr, st.d_frames, cs), MARS_ERR_LAYER_FAILED);
+        CU_OK(pre_stage_frames(t, frames.data(), 0, nfr, st.frames.p, cs), MARS_ERR_LAYER_FAILED);
         if (how == PRE_HOST_POOL) {
             cudaEventRecord(ev_in, cs);
             cudaStreamWaitEvent(m->stream, ev_in, 0);
@@ -1594,14 +1607,13 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
     }
     int8_t *dst = reinterpret_cast<int8_t *>(dev_addr(m, m->toff[ti], first));
     for (size_t k = 0; k + 1 < t.first.size(); k++) {
-        if (per_launch) CU_OK(pre_stage_frames(t, frames.data(), t.first[k], t.first[k + 1], st.d_frames, m->stream), MARS_ERR_LAYER_FAILED);
-        CU_OK(launch_letterbox(t, (int)k, st.d_tab, m->d_preH, dst, m->slot_stride, nhwc, m->d_frame + first, m->stream), MARS_ERR_LAYER_FAILED);
+        if (per_launch) CU_OK(pre_stage_frames(t, frames.data(), t.first[k], t.first[k + 1], st.frames.p, m->stream), MARS_ERR_LAYER_FAILED);
+        CU_OK(launch_letterbox(t, (int)k, st.tab.p, m->preH.p, dst, m->slot_stride, nhwc, m->rec.frame.p + first, m->stream), MARS_ERR_LAYER_FAILED);
         m->launches += 2;
     }
     return MARS_OK;
 }
 
-/* the synchronous calls: validation, then copies + kernels as one device-timed region */
 /* the checks of a letterbox call after its slot range: the target, the frames and (with rois) the regions; *g receives the
  * geometry of each slot's source, frame or region */
 static mars_error_t pre_validate(Model *m, const char *what, int first, const std::vector<FrameSrc> *frames, const RoiList *rois, bool device,
@@ -1613,26 +1625,21 @@ static mars_error_t pre_validate(Model *m, const char *what, int first, const st
     return e;
 }
 
-/* rois: slot first + r gets region r of the n frames (the regions check their own slot range) */
-static mars_error_t preprocess_sync(Model *m, const char *what, int first, int n, const std::vector<FrameSrc> *frames, const RoiList *rois = nullptr) {
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!rois && !range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
+/* The letterbox calls on the compute stream: host frames staged and letterboxed as one timed call (synchronous), or device
+ * frames read in place (enqueued only).  rois: slot first + r gets region r of the n frames (the regions check their own slot
+ * range). */
+static mars_error_t preprocess(mars_model_t *model, const char *what, int first, int n, const std::vector<FrameSrc> *frames, PreSource how,
+                               const RoiList *rois = nullptr) {
+    Model *m;
+    mars_error_t e = rois ? enter(model, &m) : enter(model, &m, first, n);
+    if (e != MARS_OK) return e;
     uint32_t ti;
     int nhwc;
     std::vector<LetterboxGeom> g;
-    mars_error_t e = pre_validate(m, what, first, frames, rois, false, &ti, &nhwc, &g);
+    e = pre_validate(m, what, first, frames, rois, how == PRE_DEVICE, &ti, &nhwc, &g);
     if (e != MARS_OK) return e;
-    cudaEventRecord(m->ev0, m->stream);
-    e = enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, *frames, g, ti, nhwc, PRE_HOST_SYNC, nullptr, rois);
-    cudaEventRecord(m->ev1, m->stream);
-    const cudaError_t ce = cudaStreamSynchronize(m->stream);
-    if (e == MARS_OK && ce != cudaSuccess) {
-        set_last_error("%s: %s", what, cudaGetErrorString(ce));
-        e = MARS_ERR_LAYER_FAILED;
-    }
-    if (e == MARS_OK) cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1);
-    return e;
+    auto enqueue = [&] { return enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, *frames, g, ti, nhwc, how, nullptr, rois); };
+    return how == PRE_DEVICE ? enqueue() : timed_call(m, what, enqueue);
 }
 
 /* Pre-processing in front of mars_run, as the reference's caller does it on the CPU (src/mars/mars_yolo_test.c:40-77 and
@@ -1647,37 +1654,25 @@ mars_error_t mars_b200_preprocess_batch(mars_model_t *model, int first, int n, c
     if (frame_stride < frame_bytes) frame_stride = frame_bytes;
     std::vector<FrameSrc> fr((size_t)(n > 0 ? n : 0));
     for (int f = 0; f < n; f++) fr[f] = FrameSrc{frames + (size_t)f * frame_stride, nullptr, (size_t)w * 3, 0, w, h, PRE_RGB8, 0};
-    return preprocess_sync(m, "preprocess", first, n, &fr);
+    return preprocess(model, "preprocess", first, n, &fr, PRE_HOST_SYNC);
 }
 
 mars_error_t mars_b200_preprocess_frames(mars_model_t *model, int first, int n, const mars_b200_frame_t *frames) {
     std::vector<FrameSrc> s;
-    return preprocess_sync(as_model(model), "preprocess_frames", first, n, rgb_sources(n, frames, &s));
+    return preprocess(model, "preprocess_frames", first, n, rgb_sources(n, frames, &s), PRE_HOST_SYNC);
 }
 mars_error_t mars_b200_preprocess_frames_nv12(mars_model_t *model, int first, int n, const mars_b200_nv12_frame_t *frames) {
     std::vector<FrameSrc> s;
-    return preprocess_sync(as_model(model), "preprocess_frames_nv12", first, n, nv12_sources(n, frames, &s));
+    return preprocess(model, "preprocess_frames_nv12", first, n, nv12_sources(n, frames, &s), PRE_HOST_SYNC);
 }
 
-/* the device-frame calls: validation, then the launches on the compute stream */
-static mars_error_t preprocess_device(Model *m, const char *what, int first, int n, const std::vector<FrameSrc> *frames, const RoiList *rois = nullptr) {
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!rois && !range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    uint32_t ti;
-    int nhwc;
-    std::vector<LetterboxGeom> g;
-    mars_error_t e = pre_validate(m, what, first, frames, rois, true, &ti, &nhwc, &g);
-    if (e != MARS_OK) return e;
-    return enqueue_letterbox(m, m->pre_stage[PRE_SYNC], first, *frames, g, ti, nhwc, PRE_DEVICE, nullptr, rois);
-}
 mars_error_t mars_b200_preprocess_frames_device(mars_model_t *model, int first, int n, const mars_b200_frame_t *frames) {
     std::vector<FrameSrc> s;
-    return preprocess_device(as_model(model), "preprocess_frames_device", first, n, rgb_sources(n, frames, &s));
+    return preprocess(model, "preprocess_frames_device", first, n, rgb_sources(n, frames, &s), PRE_DEVICE);
 }
 mars_error_t mars_b200_preprocess_frames_nv12_device(mars_model_t *model, int first, int n, const mars_b200_nv12_frame_t *frames) {
     std::vector<FrameSrc> s;
-    return preprocess_device(as_model(model), "preprocess_frames_nv12_device", first, n, nv12_sources(n, frames, &s));
+    return preprocess(model, "preprocess_frames_nv12_device", first, n, nv12_sources(n, frames, &s), PRE_DEVICE);
 }
 
 /* regions of frames (mars_b200_tile_rois) -> one slot each */
@@ -1685,22 +1680,22 @@ mars_error_t mars_b200_preprocess_rois(mars_model_t *model, int first, int n_fra
                                        const mars_b200_roi_t *rois) {
     std::vector<FrameSrc> s;
     const RoiList rl{n_rois, rois};
-    return preprocess_sync(as_model(model), "preprocess_rois", first, n_frames, rgb_sources(n_frames, frames, &s), &rl);
+    return preprocess(model, "preprocess_rois", first, n_frames, rgb_sources(n_frames, frames, &s), PRE_HOST_SYNC, &rl);
 }
 mars_error_t mars_b200_preprocess_rois_nv12_device(mars_model_t *model, int first, int n_frames, const mars_b200_nv12_frame_t *frames,
                                                    int n_rois, const mars_b200_roi_t *rois) {
     std::vector<FrameSrc> s;
     const RoiList rl{n_rois, rois};
-    return preprocess_device(as_model(model), "preprocess_rois_nv12_device", first, n_frames, nv12_sources(n_frames, frames, &s), &rl);
+    return preprocess(model, "preprocess_rois_nv12_device", first, n_frames, nv12_sources(n_frames, frames, &s), PRE_DEVICE, &rl);
 }
 
 /* the region merge of frames [0, n_frames) of a call whose regions occupy slots [first, first + n_rois): tab = the merge table
  * on the device; the kept boxes of the step's corner NMS in, frame records first + f out */
 static mars_error_t enqueue_merge(Model *m, int first, int n_frames, const int *tab, float thresh) {
     if (n_frames <= 0) return MARS_OK;
-    k_merge_rois<<<n_frames, NMSB_THREADS, 0, m->stream>>>(m->d_box + (size_t)first * MARS_MAX_DETS, m->d_box_cnt + first, MARS_MAX_DETS, tab,
-                                                          n_frames, m->d_fbox + (size_t)first * MARS_MAX_DETS, m->d_fbox_cnt + first, thresh,
-                                                          m->d_nms_mask + (size_t)first * NMS_SCRATCH_WORDS);
+    k_merge_rois<<<n_frames, NMSB_THREADS, 0, m->stream>>>(m->rec.box.at(first), m->rec.box.cnt.p + first, MARS_MAX_DETS, tab,
+                                                          n_frames, m->rec.fbox.at(first), m->rec.fbox.cnt.p + first, thresh,
+                                                          m->rec.nms_mask.p + (size_t)first * NMS_SCRATCH_WORDS);
     m->launches++;
     CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
@@ -1709,53 +1704,32 @@ static mars_error_t enqueue_merge(Model *m, int first, int n_frames, const int *
 /* The merge reads the step's kept boxes and uses the suppression scratch rows of frame records [first, first + n_frames), free
  * once the step's own NMS has run (stream order).  Enqueued on the compute stream. */
 mars_error_t mars_b200_merge_rois_resident(mars_model_t *model, int first, int n_frames, int n_rois, const mars_b200_roi_t *rois, float merge_thresh) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n_frames)) return MARS_ERR_INVALID_TENSOR;
+    Model *m;
+    mars_error_t e = enter(model, &m, first, n_frames);
+    if (e != MARS_OK) return e;
     const RoiList rl{n_rois, rois};
-    mars_error_t e = pre_check_rois(m, "merge_rois_resident", first, n_frames, nullptr, rl, 0, 0, nullptr);
+    e = pre_check_rois(m, "merge_rois_resident", first, n_frames, nullptr, rl, 0, 0, nullptr);
     if (e != MARS_OK || n_frames == 0) return e;
     PreTable t;
     merge_table(n_frames, rl, &t.merge);
     Model::PreStage &st = m->pre_stage[PRE_SYNC];
     e = pre_upload(m, st, t, m->stream);
     if (e != MARS_OK) return e;
-    return enqueue_merge(m, first, n_frames, reinterpret_cast<const int *>(st.d_tab), merge_thresh);
+    return enqueue_merge(m, first, n_frames, reinterpret_cast<const int *>(st.tab.p), merge_thresh);
 }
 
 mars_error_t mars_b200_run_resident(mars_model_t *model, int first, int n) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    cudaEventRecord(m->ev0, m->stream);
-    mars_error_t e = enqueue_ops(m, first, n, -1);
-    cudaEventRecord(m->ev1, m->stream);
-    cudaError_t ce = cudaStreamSynchronize(m->stream);
-    if (e == MARS_OK && ce != cudaSuccess) {
-        set_last_error("run_resident: %s", cudaGetErrorString(ce));
-        e = MARS_ERR_LAYER_FAILED;
-    }
-    if (e == MARS_OK) { cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1); profile_collect(m); }
-    return e;
+    Model *m;
+    mars_error_t e = enter(model, &m, first, n);
+    if (e != MARS_OK) return e;
+    return timed_call(m, "run_resident", [&] { return enqueue_ops(m, first, n, -1); });
 }
 
 mars_error_t mars_b200_detect_resident(mars_model_t *model, int first, int n, float nms_thresh) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    cudaEventRecord(m->ev0, m->stream);
-    mars_error_t e = enqueue_detect(m, first, n, nms_thresh);
-    cudaEventRecord(m->ev1, m->stream);
-    cudaError_t ce = cudaStreamSynchronize(m->stream);
-    if (e == MARS_OK && ce != cudaSuccess) {
-        set_last_error("detect_resident: %s", cudaGetErrorString(ce));
-        e = MARS_ERR_LAYER_FAILED;
-    }
-    if (e == MARS_OK) { cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1); profile_collect(m); }
-    return e;
+    Model *m;
+    mars_error_t e = enter(model, &m, first, n);
+    if (e != MARS_OK) return e;
+    return timed_call(m, "detect_resident", [&] { return enqueue_detect(m, first, n, nms_thresh); });
 }
 
 /* The ~110 launches of a step replayed as one CUDA graph: the second time a (first, n, threshold) combination is seen the
@@ -1818,112 +1792,53 @@ static mars_error_t enqueue_step_graphed(Model *m, int first, int n, float nms_t
     return MARS_OK;
 }
 
-static mars_error_t step_resident(Model *m, int first, int n, float nms_thresh, int flavour) {
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    mars_error_t e = compile_model(m);
+/* the step of slots [first, first+n), as one timed call (timed) or enqueued only */
+static mars_error_t step_resident(mars_model_t *model, const char *what, int first, int n, float nms_thresh, int flavour, bool timed) {
+    Model *m;
+    mars_error_t e = enter(model, &m, first, n);
+    if (e == MARS_OK && flavour == STEP_HEADS) e = need_heads(m, what);
+    if (e == MARS_OK) e = compile_model(m);
     if (e != MARS_OK) return e;
-    cudaEventRecord(m->ev0, m->stream);
-    e = enqueue_step_graphed(m, first, n, nms_thresh, flavour);
-    cudaEventRecord(m->ev1, m->stream);
-    cudaError_t ce = cudaStreamSynchronize(m->stream);
-    if (e == MARS_OK && ce != cudaSuccess) {
-        set_last_error("step_resident: %s", cudaGetErrorString(ce));
-        e = MARS_ERR_LAYER_FAILED;
-    }
-    if (e == MARS_OK) { cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1); profile_collect(m); }
-    return e;
-}
-
-static mars_error_t enqueue_step_resident(Model *m, int first, int n, float nms_thresh, int flavour) {
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    mars_error_t e = compile_model(m);
-    if (e != MARS_OK) return e;
-    return enqueue_step_graphed(m, first, n, nms_thresh, flavour);
+    auto enqueue = [&] { return enqueue_step_graphed(m, first, n, nms_thresh, flavour); };
+    return timed ? timed_call(m, what, enqueue) : enqueue();
 }
 
 /* run + detect as one timed region (the bench's resident step) */
 mars_error_t mars_b200_step_resident(mars_model_t *model, int first, int n, float nms_thresh, int with_detect) {
-    return step_resident(as_model(model), first, n, nms_thresh, with_detect ? STEP_DETECT : STEP_LAYERS);
+    return step_resident(model, "step_resident", first, n, nms_thresh, with_detect ? STEP_DETECT : STEP_LAYERS, true);
 }
 
 /* the same step, enqueued only: the call returns as soon as the launches (one CUDA-graph replay from the second time on) are on the
  * model's compute stream; the caller orders its own work behind them there (mars_b200_compute_stream) and synchronises itself */
 mars_error_t mars_b200_enqueue_step_resident(mars_model_t *model, int first, int n, float nms_thresh, int with_detect) {
-    return enqueue_step_resident(as_model(model), first, n, nms_thresh, with_detect ? STEP_DETECT : STEP_LAYERS);
+    return step_resident(model, "enqueue_step_resident", first, n, nms_thresh, with_detect ? STEP_DETECT : STEP_LAYERS, false);
 }
 
 /* all layers (with the head decodes the program holds), corner NMS and the letterbox inverse as one timed region */
 mars_error_t mars_b200_step_heads_resident(mars_model_t *model, int first, int n, float nms_thresh) {
-    Model *m = as_model(model);
-    if (m && m->heads.empty()) { set_last_error("step_heads_resident: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)"); return MARS_ERR_INVALID_TENSOR; }
-    return step_resident(m, first, n, nms_thresh, STEP_HEADS);
+    return step_resident(model, "step_heads_resident", first, n, nms_thresh, STEP_HEADS, true);
 }
 mars_error_t mars_b200_enqueue_step_heads_resident(mars_model_t *model, int first, int n, float nms_thresh) {
-    Model *m = as_model(model);
-    if (m && m->heads.empty()) { set_last_error("enqueue_step_heads_resident: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)"); return MARS_ERR_INVALID_TENSOR; }
-    return enqueue_step_resident(m, first, n, nms_thresh, STEP_HEADS);
+    return step_resident(model, "enqueue_step_heads_resident", first, n, nms_thresh, STEP_HEADS, false);
 }
 
 mars_error_t mars_b200_detect_heads_resident(mars_model_t *model, int first, int n, float nms_thresh) {
-    Model *m = as_model(model);
-    if (!m) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    mars_error_t e = compile_model(m);
+    Model *m;
+    mars_error_t e = enter(model, &m, first, n);
+    if (e == MARS_OK) e = need_heads(m, "detect_heads_resident");
+    if (e == MARS_OK) e = compile_model(m);
     if (e != MARS_OK) return e;
-    cudaEventRecord(m->ev0, m->stream);
-    e = enqueue_heads_nms(m, first, n, nms_thresh);
-    cudaEventRecord(m->ev1, m->stream);
-    cudaError_t ce = cudaStreamSynchronize(m->stream);
-    if (e == MARS_OK && ce != cudaSuccess) {
-        set_last_error("detect_heads_resident: %s", cudaGetErrorString(ce));
-        e = MARS_ERR_LAYER_FAILED;
-    }
-    if (e == MARS_OK) cudaEventElapsedTime(&m->last_ms, m->ev0, m->ev1);
-    return e;
+    return timed_call(m, "detect_heads_resident", [&] { return enqueue_heads_nms(m, first, n, nms_thresh); });
 }
 
-/* kept records of slots [first, first+n): mars_det_t of the output0 path, or (boxes) mars_box_t of the heads path (both 24 bytes) */
-enum Records { REC_DETS, REC_BOXES, REC_FRAME_BOXES };
-static mars_error_t copy_dets(Model *m, int first, int n, void *dets, int32_t *counts, int maxd, cudaStream_t s, Records rec = REC_DETS) {
-    static_assert(sizeof(mars_det_t) == sizeof(mars_box_t), "one record size");
-    if (maxd > 1000) maxd = 1000;
-    if (maxd < 0) maxd = 0;
-    const int32_t *dcnt = rec == REC_BOXES ? m->d_box_cnt : (rec == REC_FRAME_BOXES ? m->d_fbox_cnt : m->d_det_cnt);
-    const void *drec = rec == REC_BOXES ? (const void *)(m->d_box + (size_t)first * MARS_MAX_DETS)
-                     : rec == REC_FRAME_BOXES ? (const void *)(m->d_fbox + (size_t)first * MARS_MAX_DETS)
-                                              : (const void *)(m->d_det + (size_t)first * MARS_MAX_DETS);
-    CU_OK(cudaMemcpyAsync(counts, dcnt + first, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
-    if (maxd > 0)
-        CU_OK(cudaMemcpy2DAsync(dets, (size_t)maxd * sizeof(mars_det_t), drec,
-                                (size_t)MARS_MAX_DETS * sizeof(mars_det_t), (size_t)maxd * sizeof(mars_det_t), (size_t)n,
-                                cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
-    return MARS_OK;
-}
-
-static mars_error_t download_records(mars_model_t *model, int first, int n, void *dets, int32_t *counts, int maxd, Records rec) {
-    Model *m = as_model(model);
-    if (!m || !dets || !counts) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    if (!range_ok(m, first, n)) return MARS_ERR_INVALID_TENSOR;
-    mars_error_t e = copy_dets(m, first, n, dets, counts, maxd, m->stream, rec);
-    if (e != MARS_OK) return e;
-    CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
-    for (int i = 0; i < n; i++) if (counts[i] > maxd) counts[i] = maxd;
-    return MARS_OK;
-}
 mars_error_t mars_b200_download_detections(mars_model_t *model, int first, int n, mars_det_t *dets, int32_t *counts, int maxd) {
-    return download_records(model, first, n, dets, counts, maxd, REC_DETS);
+    return download_records(model, &SlotRecords::det, first, n, dets, counts, maxd);
 }
 mars_error_t mars_b200_download_boxes(mars_model_t *model, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd) {
-    return download_records(model, first, n, boxes, counts, maxd, REC_BOXES);
+    return download_records(model, &SlotRecords::box, first, n, boxes, counts, maxd);
 }
 mars_error_t mars_b200_download_frame_boxes(mars_model_t *model, int first, int n, mars_box_t *boxes, int32_t *counts, int maxd) {
-    return download_records(model, first, n, boxes, counts, maxd, REC_FRAME_BOXES);
+    return download_records(model, &SlotRecords::fbox, first, n, boxes, counts, maxd);
 }
 
 /* end to end from host buffers, double-buffered over the two halves of the slot pool:
@@ -1954,7 +1869,7 @@ static mars_error_t batch_pipeline(Model *m, int n, const void *inputs, size_t i
         if (e != MARS_OK) break;
         cudaEventRecord(m->ev_done[h], m->stream);
         cudaStreamWaitEvent(m->d2h_stream, m->ev_done[h], 0);
-        if (dets) e = copy_dets(m, first, cnt, dets + (size_t)done * maxd, counts + done, maxd, m->d2h_stream);
+        if (dets) e = copy_dets(m->rec.det, first, cnt, dets + (size_t)done * maxd, counts + done, maxd, m->d2h_stream);
         if (e == MARS_OK && outputs) e = copy_io(m, first, cnt, (uint8_t *)outputs + (size_t)done * out_stride, out_stride, 1, m->d2h_stream);
         cudaEventRecord(m->ev_out[h], m->d2h_stream);
     }
@@ -1973,191 +1888,178 @@ static mars_error_t batch_pipeline(Model *m, int n, const void *inputs, size_t i
 
 mars_error_t mars_b200_detect_batch(mars_model_t *model, int n, const void *inputs, size_t in_stride, mars_det_t *dets,
                                     int32_t *counts, int maxd, float nms_thresh) {
-    Model *m = as_model(model);
-    if (!m || !inputs || !dets || !counts) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    return batch_pipeline(m, n, inputs, in_stride, nullptr, 0, dets, counts, maxd, nms_thresh);
+    Model *m;
+    mars_error_t e = inputs && dets && counts ? enter(model, &m) : MARS_ERR_INVALID_FILE;
+    return e == MARS_OK ? batch_pipeline(m, n, inputs, in_stride, nullptr, 0, dets, counts, maxd, nms_thresh) : e;
 }
 
 mars_error_t mars_b200_run_batch(mars_model_t *model, int n, const void *inputs, size_t in_stride, void *outputs, size_t out_stride) {
-    Model *m = as_model(model);
-    if (!m || !inputs || !outputs) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    return batch_pipeline(m, n, inputs, in_stride, outputs, out_stride, nullptr, nullptr, 0, 0.0f);
+    Model *m;
+    mars_error_t e = inputs && outputs ? enter(model, &m) : MARS_ERR_INVALID_FILE;
+    return e == MARS_OK ? batch_pipeline(m, n, inputs, in_stride, outputs, out_stride, nullptr, nullptr, 0, 0.0f) : e;
 }
+
+/* where the images of a pooled submit come from: host input tensors 0, `stride` bytes apart, or (from_frames) host frames
+ * letterboxed into the slots -- one frame per slot, or with rois one region of them per slot (frames is null when the caller
+ * passed no table) */
+struct SubmitIn {
+    const void *tensors;
+    size_t stride;
+    bool from_frames;
+    const std::vector<FrameSrc> *frames;
+    const RoiList *rois;
+};
+/* what a pooled submit reads back, which also picks the step: the kept detections of output0 (decode + centre NMS), the kept
+ * corner boxes of the heads, the frame records of the region merge (rois), or the raw output tensor 0 (the layers alone) */
+struct SubmitOut {
+    enum Kind { DETS, BOXES, FRAME_BOXES, TENSOR } kind;
+    void *dst; /* records [records][maxd], or output tensors `stride` bytes apart */
+    int32_t *counts;
+    int maxd;
+    size_t stride;
+};
 
 /* Asynchronous form of mars_b200_detect_batch: the slot pool is split into two halves ("pools" 0 and 1); a batch of up to
  * capacity/2 images is queued on one half -- H2D on the copy stream, layers + decode + NMS on the compute stream, D2H of the
  * detection records on the read-back stream -- and the call returns.  While it runs the caller submits the next batch to the
  * other half, so the host->device copy of batch k+1 and the read-back of batch k-1 overlap the kernels of batch k.
- * inputs / dets / counts must stay valid (and should be pinned, e.g. nna_malloc) until mars_b200_wait_batch(pool) returns. */
-/* what != NULL: inputs are letterboxed from the n host frames of `frames` instead (mars_b200_submit_frames_heads_batch); with rois
- * from the n = rois->n regions of those frames, whose boxes are merged per frame after the step (k_merge_rois, merge_thresh) and
- * read back as frames->size() frame records (mars_b200_submit_rois_heads_batch) */
-static mars_error_t submit_batch(Model *m, int pool, int n, const void *inputs, size_t in_stride, void *dets, int32_t *counts, int maxd,
-                                 float nms_thresh, int flavour, const std::vector<FrameSrc> *frames = nullptr, const char *what = nullptr,
-                                 const RoiList *rois = nullptr, float merge_thresh = 0.0f) {
-    if (!m || !(inputs || what) || !dets || !counts || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
+ * Inputs and outputs must stay valid (and should be pinned, e.g. nna_malloc) until mars_b200_wait_batch(pool) returns.
+ * With frames the letterbox launches go on the compute stream in front of the (graphed) step; with rois the boxes of the
+ * n = rois->n regions are merged per frame after the step (k_merge_rois, merge_thresh) and read back as frames->size() frame
+ * records. */
+static mars_error_t submit_batch(mars_model_t *model, const char *what, int pool, int n, const SubmitIn &in, SubmitOut out,
+                                 float nms_thresh, float merge_thresh = 0.0f) {
+    const bool records = out.kind != SubmitOut::TENSOR;
+    const int flavour = out.kind == SubmitOut::DETS ? STEP_DETECT : records ? STEP_HEADS : STEP_LAYERS;
+    Model *m = as_model(model);
+    if (m && flavour == STEP_HEADS && need_heads(m, what) != MARS_OK) return MARS_ERR_INVALID_TENSOR;
+    if (m && in.from_frames && !in.frames) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
+    if (!(in.from_frames || in.tensors) || !out.dst || (records && !out.counts) || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
+    mars_error_t e = enter(model, &m);
+    if (e != MARS_OK) return e;
     const int half = m->capacity / 2;
     if (half < 1 || n < 0 || n > half) {
-        set_last_error("submit_batch: %d %s do not fit half of the slot pool (capacity %d; mars_b200_set_batch)", n, rois ? "regions" : "images",
+        set_last_error("%s: %d %s do not fit half of the slot pool (capacity %d; mars_b200_set_batch)", what, n, in.rois ? "regions" : "images",
                        m->capacity);
         return MARS_ERR_INVALID_TENSOR;
     }
-    const int nrec = rois ? (int)frames->size() : n; /* records read back */
-    if (rois && nrec > half) {
+    const int nrec = in.rois ? (int)in.frames->size() : n; /* records read back */
+    if (in.rois && nrec > half) {
         set_last_error("%s: %d frames do not fit half of the slot pool (capacity %d; mars_b200_set_batch)", what, nrec, m->capacity);
         return MARS_ERR_INVALID_TENSOR;
     }
     if (m->pending[pool].active) {
-        set_last_error("submit_batch: pool %d still has a batch in flight (mars_b200_wait_batch first)", pool);
+        set_last_error("%s: pool %d still has a batch in flight (mars_b200_wait_batch first)", what, pool);
         return MARS_ERR_LAYER_FAILED;
     }
-    if (maxd > 1000) maxd = 1000;
-    if (maxd < 0) maxd = 0;
-    const size_t in_bytes = io_bytes(&m->pub, 0);
-    if (in_stride < in_bytes) in_stride = in_bytes;
+    if (out.maxd > 1000) out.maxd = 1000;
+    if (out.maxd < 0) out.maxd = 0;
+    const size_t in_stride = std::max(in.stride, io_bytes(&m->pub, 0)), out_stride = std::max(out.stride, io_bytes(&m->pub, 1));
     const int first = pool * half;
     uint32_t ti = 0;
     int nhwc = 0;
     std::vector<LetterboxGeom> g;
-    if (what) {
-        mars_error_t e = pre_validate(m, what, first, frames, rois, false, &ti, &nhwc, &g);
+    if (in.from_frames) {
+        e = pre_validate(m, what, first, in.frames, in.rois, false, &ti, &nhwc, &g);
         if (e != MARS_OK) return e;
     }
-    mars_error_t e = compile_model(m); /* also drops captured graphs of an older program (set_opt_level, set_depthwise_mode) */
+    e = compile_model(m); /* also drops captured graphs of an older program (set_opt_level, set_depthwise_mode) */
     if (e != MARS_OK) return e;
     if (n > 0) {
         /* the half is free: its previous batch was waited for (read-back complete) before this call -- its staging too */
         const int *merge_tab = nullptr;
-        if (what) {
-            e = enqueue_letterbox(m, m->pre_stage[pool], first, *frames, g, ti, nhwc, PRE_HOST_POOL, m->ev_in[pool], rois, rois ? &merge_tab : nullptr);
+        if (in.from_frames) {
+            e = enqueue_letterbox(m, m->pre_stage[pool], first, *in.frames, g, ti, nhwc, PRE_HOST_POOL, m->ev_in[pool], in.rois,
+                                  in.rois ? &merge_tab : nullptr);
             if (e != MARS_OK) return e;
         } else {
-            e = copy_io(m, first, n, const_cast<void *>(inputs), in_stride, 0, m->h2d_stream);
+            e = copy_io(m, first, n, const_cast<void *>(in.tensors), in_stride, 0, m->h2d_stream);
             if (e != MARS_OK) return e;
             cudaEventRecord(m->ev_in[pool], m->h2d_stream);
             cudaStreamWaitEvent(m->stream, m->ev_in[pool], 0);
         }
         e = enqueue_step_graphed(m, first, n, nms_thresh, flavour);
-        if (e == MARS_OK && rois) e = enqueue_merge(m, first, nrec, merge_tab, merge_thresh);
+        if (e == MARS_OK && in.rois) e = enqueue_merge(m, first, nrec, merge_tab, merge_thresh);
         if (e != MARS_OK) { cudaStreamSynchronize(m->stream); return e; }
         cudaEventRecord(m->ev_done[pool], m->stream);
         cudaStreamWaitEvent(m->d2h_stream, m->ev_done[pool], 0);
-        e = copy_dets(m, first, nrec, dets, counts, maxd, m->d2h_stream, rois ? REC_FRAME_BOXES : (flavour == STEP_HEADS ? REC_BOXES : REC_DETS));
+        switch (out.kind) {
+            case SubmitOut::DETS: e = copy_dets(m->rec.det, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
+            case SubmitOut::BOXES: e = copy_dets(m->rec.box, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
+            case SubmitOut::FRAME_BOXES: e = copy_dets(m->rec.fbox, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
+            case SubmitOut::TENSOR: e = copy_io(m, first, n, out.dst, out_stride, 1, m->d2h_stream); break;
+        }
         if (e != MARS_OK) return e;
     } else {
-        for (int i = 0; i < nrec; i++) counts[i] = 0; /* frames without regions */
+        for (int i = 0; i < nrec; i++) out.counts[i] = 0; /* frames without regions */
     }
     cudaEventRecord(m->ev_out[pool], m->d2h_stream);
-    m->pending[pool].active = true;
-    m->pending[pool].n = nrec; m->pending[pool].maxd = maxd; m->pending[pool].counts = counts;
+    Model::Pending &pd = m->pending[pool];
+    pd.active = true;
+    pd.n = records ? nrec : 0; pd.maxd = out.maxd; pd.counts = out.counts;
     return MARS_OK;
 }
 mars_error_t mars_b200_submit_batch(mars_model_t *model, int pool, int n, const void *inputs, size_t in_stride, mars_det_t *dets,
                                     int32_t *counts, int maxd, float nms_thresh) {
-    return submit_batch(as_model(model), pool, n, inputs, in_stride, dets, counts, maxd, nms_thresh, STEP_DETECT);
+    return submit_batch(model, "submit_batch", pool, n, SubmitIn{inputs, in_stride, false, nullptr, nullptr},
+                        SubmitOut{SubmitOut::DETS, dets, counts, maxd, 0}, nms_thresh);
 }
 /* mars_b200_submit_batch with the YOLO heads decode (mars_b200_set_yolo_heads): boxes[n][maxd] corner boxes, frame coordinates for
  * slots with a frame size */
 mars_error_t mars_b200_submit_heads_batch(mars_model_t *model, int pool, int n, const void *inputs, size_t in_stride, mars_box_t *boxes,
                                           int32_t *counts, int maxd, float nms_thresh) {
-    Model *m = as_model(model);
-    if (m && m->heads.empty()) { set_last_error("submit_heads_batch: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)"); return MARS_ERR_INVALID_TENSOR; }
-    return submit_batch(m, pool, n, inputs, in_stride, boxes, counts, maxd, nms_thresh, STEP_HEADS);
+    return submit_batch(model, "submit_heads_batch", pool, n, SubmitIn{inputs, in_stride, false, nullptr, nullptr},
+                        SubmitOut{SubmitOut::BOXES, boxes, counts, maxd, 0}, nms_thresh);
 }
 
 /* mars_b200_submit_heads_batch from RGB8 or NV12 frames of any sizes and row pitches (host memory): H2D of each frame (each
  * NV12 plane) on the copy stream, the letterbox launches on the compute stream in front of the (graphed) step, frame
  * coordinates for every slot */
-static mars_error_t submit_frames_heads(Model *m, const char *what, int pool, int n, const std::vector<FrameSrc> *frames, mars_box_t *boxes,
-                                        int32_t *counts, int maxd, float nms_thresh) {
-    if (m && m->heads.empty()) { set_last_error("%s: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)", what); return MARS_ERR_INVALID_TENSOR; }
-    if (m && !frames) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
-    return submit_batch(m, pool, n, nullptr, 0, boxes, counts, maxd, nms_thresh, STEP_HEADS, frames, what);
-}
 mars_error_t mars_b200_submit_frames_heads_batch(mars_model_t *model, int pool, int n, const mars_b200_frame_t *frames, mars_box_t *boxes,
                                                  int32_t *counts, int maxd, float nms_thresh) {
     std::vector<FrameSrc> s;
-    return submit_frames_heads(as_model(model), "submit_frames_heads_batch", pool, n, rgb_sources(n, frames, &s), boxes, counts, maxd,
-                               nms_thresh);
+    return submit_batch(model, "submit_frames_heads_batch", pool, n, SubmitIn{nullptr, 0, true, rgb_sources(n, frames, &s), nullptr},
+                        SubmitOut{SubmitOut::BOXES, boxes, counts, maxd, 0}, nms_thresh);
 }
 mars_error_t mars_b200_submit_frames_nv12_heads_batch(mars_model_t *model, int pool, int n, const mars_b200_nv12_frame_t *frames,
                                                       mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh) {
     std::vector<FrameSrc> s;
-    return submit_frames_heads(as_model(model), "submit_frames_nv12_heads_batch", pool, n, nv12_sources(n, frames, &s), boxes, counts,
-                               maxd, nms_thresh);
+    return submit_batch(model, "submit_frames_nv12_heads_batch", pool, n, SubmitIn{nullptr, 0, true, nv12_sources(n, frames, &s), nullptr},
+                        SubmitOut{SubmitOut::BOXES, boxes, counts, maxd, 0}, nms_thresh);
 }
 
 /* the tiled flow of mars_b200_submit_frames_heads_batch: regions of the frames letterboxed into the pool's slots, their boxes
  * merged per frame (k_merge_rois) and read back per frame */
-static mars_error_t submit_rois_heads(Model *m, const char *what, int pool, const std::vector<FrameSrc> *frames, int n_rois, const mars_b200_roi_t *rois,
-                                      mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh, float merge_thresh) {
-    if (m && m->heads.empty()) { set_last_error("%s: no detection heads configured (mars_b200_set_yolo_heads / mars_b200_set_gfl_heads)", what); return MARS_ERR_INVALID_TENSOR; }
-    if (m && !frames) { set_last_error("%s: no frame table", what); return MARS_ERR_INVALID_FILE; }
-    const RoiList rl{n_rois, rois};
-    return submit_batch(m, pool, n_rois, nullptr, 0, boxes, counts, maxd, nms_thresh, STEP_HEADS, frames, what, &rl, merge_thresh);
-}
 mars_error_t mars_b200_submit_rois_heads_batch(mars_model_t *model, int pool, int n_frames, const mars_b200_frame_t *frames, int n_rois,
                                                const mars_b200_roi_t *rois, mars_box_t *boxes, int32_t *counts, int maxd, float nms_thresh,
                                                float merge_thresh) {
     std::vector<FrameSrc> s;
-    return submit_rois_heads(as_model(model), "submit_rois_heads_batch", pool, rgb_sources(n_frames, frames, &s), n_rois, rois, boxes, counts,
-                             maxd, nms_thresh, merge_thresh);
+    const RoiList rl{n_rois, rois};
+    return submit_batch(model, "submit_rois_heads_batch", pool, n_rois, SubmitIn{nullptr, 0, true, rgb_sources(n_frames, frames, &s), &rl},
+                        SubmitOut{SubmitOut::FRAME_BOXES, boxes, counts, maxd, 0}, nms_thresh, merge_thresh);
 }
 mars_error_t mars_b200_submit_rois_nv12_heads_batch(mars_model_t *model, int pool, int n_frames, const mars_b200_nv12_frame_t *frames,
                                                     int n_rois, const mars_b200_roi_t *rois, mars_box_t *boxes, int32_t *counts, int maxd,
                                                     float nms_thresh, float merge_thresh) {
     std::vector<FrameSrc> s;
-    return submit_rois_heads(as_model(model), "submit_rois_nv12_heads_batch", pool, nv12_sources(n_frames, frames, &s), n_rois, rois, boxes,
-                             counts, maxd, nms_thresh, merge_thresh);
+    const RoiList rl{n_rois, rois};
+    return submit_batch(model, "submit_rois_nv12_heads_batch", pool, n_rois,
+                        SubmitIn{nullptr, 0, true, nv12_sources(n_frames, frames, &s), &rl},
+                        SubmitOut{SubmitOut::FRAME_BOXES, boxes, counts, maxd, 0}, nms_thresh, merge_thresh);
 }
 
 /* mars_b200_submit_batch without the YOLO post-process: the raw output tensor 0 of every image is read back instead
  * (models whose output is not a [1, N, 85] head: NanoDet-style heads, float32 models).  Same pools, same wait. */
 mars_error_t mars_b200_submit_run_batch(mars_model_t *model, int pool, int n, const void *inputs, size_t in_stride, void *outputs, size_t out_stride) {
-    Model *m = as_model(model);
-    if (!m || !inputs || !outputs || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
-    const int half = m->capacity / 2;
-    if (half < 1 || n < 0 || n > half) {
-        set_last_error("submit_run_batch: %d images do not fit half of the slot pool (capacity %d; mars_b200_set_batch)", n, m->capacity);
-        return MARS_ERR_INVALID_TENSOR;
-    }
-    if (m->pending[pool].active) {
-        set_last_error("submit_run_batch: pool %d still has a batch in flight (mars_b200_wait_batch first)", pool);
-        return MARS_ERR_LAYER_FAILED;
-    }
-    const size_t in_bytes = io_bytes(&m->pub, 0), out_bytes = io_bytes(&m->pub, 1);
-    if (in_stride < in_bytes) in_stride = in_bytes;
-    if (out_stride < out_bytes) out_stride = out_bytes;
-    const int first = pool * half;
-    mars_error_t e = compile_model(m);
-    if (e != MARS_OK) return e;
-    if (n > 0) {
-        e = copy_io(m, first, n, const_cast<void *>(inputs), in_stride, 0, m->h2d_stream);
-        if (e != MARS_OK) return e;
-        cudaEventRecord(m->ev_in[pool], m->h2d_stream);
-        cudaStreamWaitEvent(m->stream, m->ev_in[pool], 0);
-        e = enqueue_step_graphed(m, first, n, 0.0f, 0);
-        if (e != MARS_OK) { cudaStreamSynchronize(m->stream); return e; }
-        cudaEventRecord(m->ev_done[pool], m->stream);
-        cudaStreamWaitEvent(m->d2h_stream, m->ev_done[pool], 0);
-        e = copy_io(m, first, n, outputs, out_stride, 1, m->d2h_stream);
-        if (e != MARS_OK) return e;
-    }
-    cudaEventRecord(m->ev_out[pool], m->d2h_stream);
-    m->pending[pool].active = true;
-    m->pending[pool].n = 0; m->pending[pool].maxd = 0; m->pending[pool].counts = nullptr;
-    return MARS_OK;
+    return submit_batch(model, "submit_run_batch", pool, n, SubmitIn{inputs, in_stride, false, nullptr, nullptr},
+                        SubmitOut{SubmitOut::TENSOR, outputs, nullptr, 0, out_stride}, 0.0f);
 }
 
 mars_error_t mars_b200_wait_batch(mars_model_t *model, int pool) {
-    Model *m = as_model(model);
-    if (!m || pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
-    if (!m->pending[pool].active) return MARS_OK;
-    CU_OK(cudaSetDevice(m->device), MARS_ERR_NNA_INIT_FAILED);
+    if (pool < 0 || pool > 1) return MARS_ERR_INVALID_FILE;
+    Model *m;
+    mars_error_t e = enter(model, &m);
+    if (e != MARS_OK || !m->pending[pool].active) return e;
     cudaError_t ce = cudaEventSynchronize(m->ev_out[pool]);
     Model::Pending &pd = m->pending[pool];
     pd.active = false;
@@ -2183,8 +2085,8 @@ uint64_t mars_b200_launch_count(mars_model_t *model) {
  * dets = mars_det_t[capacity][1024], counts = int32[capacity] */
 void mars_b200_detections_device(mars_model_t *model, void **dets, void **counts, int *stride_dets) {
     Model *m = as_model(model);
-    if (dets) *dets = m ? m->d_det : nullptr;
-    if (counts) *counts = m ? m->d_det_cnt : nullptr;
+    if (dets) *dets = m ? m->rec.det.rec.p : nullptr;
+    if (counts) *counts = m ? m->rec.det.cnt.p : nullptr;
     if (stride_dets) *stride_dets = MARS_MAX_DETS;
 }
 float mars_b200_last_gpu_ms(mars_model_t *model) {
