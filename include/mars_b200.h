@@ -255,6 +255,55 @@ mars_error_t mars_b200_submit_rois_nv12_heads_batch(mars_model_t *m, int pool, i
                                                     int n_rois, const mars_b200_roi_t *rois, mars_box_t *boxes, int32_t *counts,
                                                     int maxd, float nms_thresh, float merge_thresh);
 
+/* ---- multi-object tracking of camera streams -------------------------------------------------------------------------------
+ * A tracker per camera stream whose state stays on the device: after a heads step, one CTA per stream turns the frame's kept
+ * corner boxes into tracked boxes with persistent IDs.  The schedule is ByteTrack's (Zhang et al., ECCV 2022): high-score
+ * detections (conf > high_thresh) are matched first to the Tracked and Lost tracks predicted by ByteTrack's Kalman filter, with
+ * similarity IoU * conf; low-score detections (low_thresh < conf < high_thresh) then keep the still unmatched Tracked tracks
+ * alive, with similarity IoU; the high-score detections left over are matched to the unconfirmed tracks (born on an earlier frame
+ * but not yet matched again), and the rest with conf >= new_thresh start tracks.  Matching is greedy under a strict total order
+ * -- the admissible pair (similarity > gate, both unused, equal classes with class_aware) with the largest similarity first,
+ * ties by the smaller track_id, then the smaller detection index -- where ByteTrack solves an optimal assignment.  A track lost
+ * for more than max_lost frames is removed; an unconfirmed track that misses once is removed.  All arithmetic is float32 with
+ * one rounding per operation: the results are bit-exact to the C statement of the definition (tests/track_oracle.c).  Boxes with
+ * a non-finite value or a non-positive width or height are ignored.  Track IDs start at 1 per stream. */
+#define MARS_B200_MAX_TRACKS 256
+/* one tracked object of a frame: the filter's box after this frame's update, and the confidence, class and index (in the frame's
+ * kept boxes) of the detection it was matched to (32 bytes) */
+typedef struct { float x0, y0, x1, y1, confidence; int32_t class_id, track_id, det_index; } mars_b200_track_box_t;
+typedef struct {
+    float high_thresh, low_thresh, new_thresh; /* detection classes and the birth threshold */
+    float sim_high, sim_low, sim_unconfirmed;  /* gates of the three matchings, in [0, 1) */
+    int32_t max_lost, class_aware;             /* frames a lost track survives (>= 0); 1: only equal classes match */
+} mars_b200_track_params_t;
+#define MARS_B200_TRACK_PARAMS_DEFAULT {0.5f, 0.1f, 0.6f, 0.2f, 0.5f, 0.3f, 30, 0}
+/* tracker state for n_streams streams, all reset (frame 0, next ID 1); n_streams = 0 frees it; p = NULL: the defaults.
+ * MARS_ERR_INVALID_TENSOR when a parameter is not finite, low_thresh < 0 or > high_thresh, a gate is outside [0, 1), max_lost < 0 or
+ * class_aware is not 0 or 1.  Waits for the compute stream. */
+mars_error_t mars_b200_set_tracking(mars_model_t *m, int n_streams, const mars_b200_track_params_t *p);
+/* streams [first_stream, first_stream + n) start over (frame 0, next ID 1); enqueued on the compute stream */
+mars_error_t mars_b200_reset_tracks(mars_model_t *m, int first_stream, int n);
+/* after a heads step on slots [first, first+n): the kept boxes of slot first + i are the next frame of stream streams[i]; its
+ * tracked boxes go to track record first + i (mars_b200_download_tracks).  Enqueued on the compute stream.  Every call checks
+ * first that tracking is set, the slots are in range, heads are configured and every stream id is in [0, n_streams) and named
+ * once; a rejected call changes no stream (mars_b200_last_error names the entry). */
+mars_error_t mars_b200_track_resident(mars_model_t *m, int first, int n, const int32_t *streams);
+/* tracked boxes of track records [first, first+n): out[n][maxd] (maxd <= 256), counts[n] */
+mars_error_t mars_b200_download_tracks(mars_model_t *m, int first, int n, mars_b200_track_box_t *out, int32_t *counts, int maxd);
+/* the same kernel on detections from the host: entry i is the next frame of stream streams[i], with counts[i] (0..min(box_stride,
+ * 1000)) boxes at boxes + i * box_stride; out[n][maxd], out_counts[n].  Synchronous; needs no heads and no slots. */
+mars_error_t mars_b200_track_boxes(mars_model_t *m, int n, const int32_t *streams, const mars_box_t *boxes, const int32_t *counts,
+                                   int box_stride, mars_b200_track_box_t *out, int32_t *out_counts, int maxd);
+/* mars_b200_submit_frames_heads_batch followed by the tracker on the pool's slots (frame i = the next frame of stream streams[i]):
+ * out[n][maxd] tracked boxes in frame coordinates and counts[n] are read back instead of the boxes; waited for with
+ * mars_b200_wait_batch.  The stream table travels in the pool's pinned upload.  Both pools use the compute stream, so the track
+ * kernels run in submit order and a stream may appear in consecutive submits on alternating pools. */
+mars_error_t mars_b200_submit_frames_track_batch(mars_model_t *m, int pool, int n, const mars_b200_frame_t *frames, const int32_t *streams,
+                                                 mars_b200_track_box_t *out, int32_t *counts, int maxd, float nms_thresh);
+mars_error_t mars_b200_submit_frames_nv12_track_batch(mars_model_t *m, int pool, int n, const mars_b200_nv12_frame_t *frames,
+                                                      const int32_t *streams, mars_b200_track_box_t *out, int32_t *counts, int maxd,
+                                                      float nms_thresh);
+
 /* ---- several GPUs of one box behind one call (batch sharded over the devices, no inter-GPU traffic on the path) ---------- */
 typedef struct mars_b200_group mars_b200_group_t;
 /* one replica of the model per device (devices = NULL: ordinals 0 .. n_devices-1), `per_gpu_batch` image slots each */

@@ -97,6 +97,22 @@ class ROI(C.Structure):
 
 ROI_DTYPE = np.dtype([("frame", "<i4"), ("x", "<i4"), ("y", "<i4"), ("w", "<i4"), ("h", "<i4")])
 
+# mars_b200_track_box_t: a tracked box of a frame (the filter's box, the matched detection's confidence, class and index)
+TRACK_DTYPE = np.dtype([("x0", "<f4"), ("y0", "<f4"), ("x1", "<f4"), ("y1", "<f4"), ("confidence", "<f4"), ("class_id", "<i4"),
+                        ("track_id", "<i4"), ("det_index", "<i4")])
+MAX_TRACKS = 256  # MARS_B200_MAX_TRACKS
+
+
+class TRACK_PARAMS(C.Structure):
+    """mars_b200_track_params_t; TRACK_PARAMS() holds MARS_B200_TRACK_PARAMS_DEFAULT"""
+    _fields_ = [("high_thresh", C.c_float), ("low_thresh", C.c_float), ("new_thresh", C.c_float), ("sim_high", C.c_float),
+                ("sim_low", C.c_float), ("sim_unconfirmed", C.c_float), ("max_lost", C.c_int32), ("class_aware", C.c_int32)]
+    DEFAULTS = dict(high_thresh=0.5, low_thresh=0.1, new_thresh=0.6, sim_high=0.2, sim_low=0.5, sim_unconfirmed=0.3, max_lost=30,
+                    class_aware=0)
+
+    def __init__(self, **kw):
+        super().__init__(**{**self.DEFAULTS, **kw})
+
 
 # every symbol include/*.h declares: name -> (restype, argtypes)
 SIGNATURES = {
@@ -250,6 +266,15 @@ SIGNATURES = {
                                                     C.c_int, C.c_float, C.c_float]),
     "mars_b200_submit_rois_nv12_heads_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME), C.c_int, C.c_void_p, C.c_void_p,
                                                          C.c_void_p, C.c_int, C.c_float, C.c_float]),
+    "mars_b200_set_tracking": (C.c_int, [PM, C.c_int, C.POINTER(TRACK_PARAMS)]),
+    "mars_b200_reset_tracks": (C.c_int, [PM, C.c_int, C.c_int]),
+    "mars_b200_track_resident": (C.c_int, [PM, C.c_int, C.c_int, C.c_void_p]),
+    "mars_b200_download_tracks": (C.c_int, [PM, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "mars_b200_track_boxes": (C.c_int, [PM, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "mars_b200_submit_frames_track_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(FRAME), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                                      C.c_float]),
+    "mars_b200_submit_frames_nv12_track_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME), C.c_void_p, C.c_void_p, C.c_void_p,
+                                                           C.c_int, C.c_float]),
 }
 
 _lib = None
@@ -536,6 +561,62 @@ class MarsModel:
         self._check(lib().mars_b200_submit_rois_nv12_heads_batch(self.m, pool, len(frames), table, len(r), r.ctypes.data, _addr(boxes),
                                                                  _addr(counts), maxd, thresh, merge_thresh), "submit_rois_nv12_heads_batch")
         self._inflight[pool] = (table, keep, r)
+
+    # ---- multi-object tracking of camera streams (include/mars_b200.h) --------------------------------
+    def set_tracking(self, n_streams, params=None, **kw):
+        """tracker state for n_streams streams, all reset; params: TRACK_PARAMS, or its fields as keywords (the rest default);
+        n_streams = 0 frees it"""
+        p = params if params is not None else TRACK_PARAMS(**kw)
+        self._check(lib().mars_b200_set_tracking(self.m, n_streams, C.byref(p)), "set_tracking")
+
+    def reset_tracks(self, first_stream, n):
+        """streams [first_stream, first_stream + n) start over; enqueued on compute_stream()"""
+        self._check(lib().mars_b200_reset_tracks(self.m, first_stream, n), "reset_tracks")
+
+    def track_resident(self, first, streams):
+        """after a heads step on slots [first, first + len(streams)): slot first + i is the next frame of stream streams[i];
+        enqueued on compute_stream()"""
+        s = np.ascontiguousarray(streams, dtype=np.int32)
+        self._check(lib().mars_b200_track_resident(self.m, first, s.size, s.ctypes.data), "track_resident")
+
+    def download_tracks(self, first, n, maxd=MAX_TRACKS):
+        out = np.zeros((n, maxd), dtype=TRACK_DTYPE)
+        counts = np.zeros(n, dtype=np.int32)
+        self._check(lib().mars_b200_download_tracks(self.m, first, n, out.ctypes.data, counts.ctypes.data, maxd), "download_tracks")
+        return out, counts
+
+    def track_boxes(self, streams, boxes, maxd=MAX_TRACKS):
+        """boxes: one BOX_DTYPE array per entry, the next frame of stream streams[i] -> (TRACK_DTYPE [n, maxd], counts [n]);
+        synchronous"""
+        s = np.ascontiguousarray(streams, dtype=np.int32)
+        n = s.size
+        counts = np.array([len(b) for b in boxes], dtype=np.int32)
+        stride = max(1, int(counts.max()) if n else 1)
+        table = np.zeros((n, stride), dtype=BOX_DTYPE)
+        for i, b in enumerate(boxes):
+            table[i, : len(b)] = b
+        out = np.zeros((n, maxd), dtype=TRACK_DTYPE)
+        oc = np.zeros(n, dtype=np.int32)
+        self._check(lib().mars_b200_track_boxes(self.m, n, s.ctypes.data, table.ctypes.data, counts.ctypes.data, stride, out.ctypes.data,
+                                                oc.ctypes.data, maxd), "track_boxes")
+        return out, oc
+
+    def submit_frames_track_batch(self, pool, frames, streams, out, counts, maxd=MAX_TRACKS, thresh=0.45):
+        """submit_frames_heads_batch followed by the tracker: frame i is the next frame of stream streams[i]; out [n, maxd] TRACK_DTYPE.
+        The frames and the stream table are kept alive until wait_batch(pool); out and counts must be kept alive by the caller"""
+        table, keep = host_frames(frames)
+        s = np.ascontiguousarray(streams, dtype=np.int32)
+        self._check(lib().mars_b200_submit_frames_track_batch(self.m, pool, len(frames), table, s.ctypes.data, _addr(out), _addr(counts), maxd,
+                                                              thresh), "submit_frames_track_batch")
+        self._inflight[pool] = (table, keep, s)
+
+    def submit_frames_nv12_track_batch(self, pool, frames, streams, out, counts, maxd=MAX_TRACKS, thresh=0.45):
+        """submit_frames_track_batch from (y, uv, colour) NV12 host frames (host_nv12_frames)"""
+        table, keep = host_nv12_frames(frames)
+        s = np.ascontiguousarray(streams, dtype=np.int32)
+        self._check(lib().mars_b200_submit_frames_nv12_track_batch(self.m, pool, len(frames), table, s.ctypes.data, _addr(out), _addr(counts),
+                                                                   maxd, thresh), "submit_frames_nv12_track_batch")
+        self._inflight[pool] = (table, keep, s)
 
     def download_outputs(self, first, n, host=None, stride=0):
         if host is None:

@@ -356,7 +356,8 @@ struct PreTable {
     std::vector<size_t> stage; /* byte offset of each source frame in a tightly packed staging buffer (pre_frame_bytes each) */
     std::vector<int> start, src;
     std::vector<float> w;
-    std::vector<int> merge;         /* optional trailer: the region merge table of k_merge_rois, carried in the same upload */
+    std::vector<int> merge;         /* optional trailer carried in the same upload: the region merge table of k_merge_rois, or the
+                                     * stream table of k_track */
     std::vector<int> first, blocks; /* launch k covers entries [first[k], first[k + 1]) with blocks[k] horizontal blocks */
     size_t h_floats = 0;            /* H scratch of the largest launch */
     size_t stage_bytes = 0;         /* staging of the largest launch (per_launch staging) or of every frame */

@@ -40,6 +40,7 @@
 #include "postproc.cuh"
 #include "preproc.cuh"
 #include "nna_layout.cuh"
+#include "track.cuh"
 
 namespace marsb200 {
 
@@ -175,12 +176,12 @@ int find_tensor(const mars_header_t &h, const mars_runtime_tensor_t *tensors, ui
 /* ---- the private model object ------------------------------------------------ */
 static const uint32_t MODEL_TAG = 0x4232304Du; /* "M02B" */
 
-/* MARS_MAX_DETS records and one count per image slot */
-template <typename R> struct RecordSet {
+/* CAP records and one count per image slot */
+template <typename R, int CAP = MARS_MAX_DETS> struct RecordSet {
     DevBuf<R> rec;
     DevBuf<int32_t> cnt;
-    bool alloc(int slots) { return rec.alloc((size_t)slots * MARS_MAX_DETS) && cnt.alloc((size_t)slots); }
-    R *at(int slot) const { return rec.p + (size_t)slot * MARS_MAX_DETS; }
+    bool alloc(int slots) { return rec.alloc((size_t)slots * CAP) && cnt.alloc((size_t)slots); }
+    R *at(int slot) const { return rec.p + (size_t)slot * CAP; }
 };
 
 /* the per-slot device state besides the slots themselves, (re)allocated together by set_capacity */
@@ -188,6 +189,7 @@ struct SlotRecords {
     RecordSet<mars_det_t> raw, det;      /* the output0 path: parsed candidates, kept detections */
     RecordSet<mars_box_t> box_raw, box;  /* the heads path: decoded candidates, kept corner boxes */
     RecordSet<mars_box_t> fbox;          /* frame records of the region merge (mars_b200_merge_rois_resident) */
+    RecordSet<mars_b200_track_box_t, MARS_B200_MAX_TRACKS> trk; /* tracked boxes (mars_b200_track_resident) */
     DevBuf<unsigned> nms_mask;           /* NMS_SCRATCH_WORDS per slot: suppression bit matrices */
     DevBuf<int2> frame;                  /* original frame size per slot (0 = none), for the letterbox inverse */
 };
@@ -252,6 +254,14 @@ struct Model {
     std::vector<TcPlan> tc;
     bool compiled = false;
     uint64_t weights_hash = 0; /* FNV-1a of the host weight blob the compiled plans were built from */
+    /* multi-object tracking (mars_b200_set_tracking, track.cuh): MARS_B200_MAX_TRACKS track slots and the counters per stream, the
+     * parameters, and the device staging of mars_b200_track_boxes (in: stream table, counts, boxes; out: counts, records) */
+    int track_streams = 0;
+    mars_b200_track_params_t track_params = MARS_B200_TRACK_PARAMS_DEFAULT;
+    DevBuf<TrackSlot> tracks;
+    DevBuf<TrackMeta> track_meta;
+    DevBuf<> track_in, track_out;
+    size_t track_in_cap = 0, track_out_cap = 0;
 };
 
 static Model *as_model(mars_model_t *p) {
@@ -317,11 +327,11 @@ static mars_error_t set_capacity(Model *m, int capacity) {
     SlotRecords r;
     if (!slots.alloc(c * m->slot_stride) || (m->scratch_stride && !scratch.alloc(c * m->scratch_stride)) || !r.raw.alloc(capacity) ||
         !r.det.alloc(capacity) || !r.box_raw.alloc(capacity) || !r.box.alloc(capacity) || !r.fbox.alloc(capacity) ||
-        !r.nms_mask.alloc(c * NMS_SCRATCH_WORDS) || !r.frame.alloc(c))
+        !r.trk.alloc(capacity) || !r.nms_mask.alloc(c * NMS_SCRATCH_WORDS) || !r.frame.alloc(c))
         return MARS_ERR_ALLOC_FAILED;
     CU_OK(cudaMemsetAsync(slots.p, 0, c * m->slot_stride, m->stream), MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaMemsetAsync(r.frame.p, 0, c * sizeof(int2), m->stream), MARS_ERR_ALLOC_FAILED);
-    for (int32_t *cnt : {r.raw.cnt.p, r.det.cnt.p, r.box_raw.cnt.p, r.box.cnt.p, r.fbox.cnt.p})
+    for (int32_t *cnt : {r.raw.cnt.p, r.det.cnt.p, r.box_raw.cnt.p, r.box.cnt.p, r.fbox.cnt.p, r.trk.cnt.p})
         CU_OK(cudaMemsetAsync(cnt, 0, c * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
     if (m->slots.p) {
         CU_OK(cudaMemcpyAsync(slots.p, m->slots.p, keep * m->slot_stride, cudaMemcpyDeviceToDevice, m->stream), MARS_ERR_ALLOC_FAILED);
@@ -737,25 +747,62 @@ template <typename T> static bool pre_grow(Model *m, DevBuf<T> &b, size_t *cap, 
 }
 
 /* kept records of slots [first, first+n) of a record set -> dets[n][maxd], counts[n] on stream s */
-template <typename R>
-static mars_error_t copy_dets(const RecordSet<R> &rs, int first, int n, void *dets, int32_t *counts, int maxd, cudaStream_t s) {
-    if (maxd > 1000) maxd = 1000;
+template <typename R, int CAP>
+static mars_error_t copy_dets(const RecordSet<R, CAP> &rs, int first, int n, void *dets, int32_t *counts, int maxd, cudaStream_t s) {
+    if (maxd > std::min(1000, CAP)) maxd = std::min(1000, CAP);
     if (maxd < 0) maxd = 0;
     CU_OK(cudaMemcpyAsync(counts, rs.cnt.p + first, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
     if (maxd > 0)
-        CU_OK(cudaMemcpy2DAsync(dets, (size_t)maxd * sizeof(R), rs.at(first), (size_t)MARS_MAX_DETS * sizeof(R), (size_t)maxd * sizeof(R),
+        CU_OK(cudaMemcpy2DAsync(dets, (size_t)maxd * sizeof(R), rs.at(first), (size_t)CAP * sizeof(R), (size_t)maxd * sizeof(R),
                                 (size_t)n, cudaMemcpyDeviceToHost, s), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
 }
 
-template <typename R>
-static mars_error_t download_records(mars_model_t *model, RecordSet<R> SlotRecords::*set, int first, int n, R *dets, int32_t *counts, int maxd) {
+template <typename R, int CAP>
+static mars_error_t download_records(mars_model_t *model, RecordSet<R, CAP> SlotRecords::*set, int first, int n, R *dets, int32_t *counts,
+                                     int maxd) {
     Model *m;
     mars_error_t e = dets && counts ? enter(model, &m, first, n) : MARS_ERR_INVALID_FILE;
     if (e == MARS_OK) e = copy_dets(m->rec.*set, first, n, dets, counts, maxd, m->stream);
     if (e != MARS_OK) return e;
     CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
     for (int i = 0; i < n; i++) if (counts[i] > maxd) counts[i] = maxd;
+    return MARS_OK;
+}
+
+/* ---- multi-object tracking (track.cuh) ----------------------------------------------------------------------------------- */
+static mars_error_t need_tracking(Model *m, const char *what) {
+    if (m->track_streams > 0) return MARS_OK;
+    set_last_error("%s: tracking is not set (mars_b200_set_tracking)", what);
+    return MARS_ERR_INVALID_TENSOR;
+}
+
+/* tracking is set and the n entries of a call name streams of it, each at most once */
+static mars_error_t check_streams(Model *m, const char *what, int n, const int32_t *streams) {
+    mars_error_t e = need_tracking(m, what);
+    if (e != MARS_OK) return e;
+    if (n > 0 && !streams) { set_last_error("%s: no stream table", what); return MARS_ERR_INVALID_FILE; }
+    std::vector<uint8_t> seen((size_t)m->track_streams, 0);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        if (s < 0 || s >= m->track_streams) {
+            set_last_error("%s: entry %d: stream %d outside [0, %d) (mars_b200_set_tracking)", what, i, s, m->track_streams);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        if (seen[s]++) { set_last_error("%s: entry %d: stream %d named twice in one call", what, i, s); return MARS_ERR_INVALID_TENSOR; }
+    }
+    return MARS_OK;
+}
+
+/* the tracker on the compute stream: entry i = the detections at boxes + i * box_stride (counts[i]) as the next frame of stream
+ * streams[i] (a device table), tracked boxes to out + i * out_stride and out_counts[i] */
+static mars_error_t enqueue_track(Model *m, const mars_box_t *boxes, const int32_t *counts, int box_stride, const int32_t *streams, int n,
+                                  mars_b200_track_box_t *out, int32_t *out_counts, int out_stride) {
+    if (n <= 0) return MARS_OK;
+    k_track<<<n, TRK_THREADS, 0, m->stream>>>(boxes, counts, box_stride, streams, m->tracks.p, m->track_meta.p, m->track_params, out,
+                                             out_counts, out_stride);
+    m->launches++;
+    CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
 }
 } // namespace marsb200
@@ -1553,13 +1600,14 @@ static mars_error_t pre_upload(Model *m, Model::PreStage &st, const PreTable &t,
 /* Letterboxes validated frames into input tensor ti of slots first, first+1, ... and records each slot's source size for the
  * letterbox inverse; the launches go on the compute stream.  Without rois slot first + f gets frame f (geometry g[f]); with
  * rois slot first + r gets region r (geometry g[r]) of frame rois[r].frame -- each frame staged once, whatever its number of
- * regions.  merge_tab (with rois): receives the device address of the merge table (merge_table), carried in the same upload.
+ * regions.  tail: an int table carried in the same upload (the region merge table, or the stream table of the tracker), whose
+ * device address goes to *tail_dev.
  *   PRE_HOST_SYNC : host frames staged on the compute stream, launch by launch without regions (the caller synchronises);
  *   PRE_DEVICE    : device frames read in place;
  *   PRE_HOST_POOL : host frames and the table copied on the copy stream, then ev_in, which the compute stream waits for. */
 static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, const std::vector<FrameSrc> &frames,
                                       const std::vector<LetterboxGeom> &g, uint32_t ti, int nhwc, PreSource how, cudaEvent_t ev_in,
-                                      const RoiList *rois = nullptr, const int **merge_tab = nullptr) {
+                                      const RoiList *rois = nullptr, const std::vector<int> *tail = nullptr, const int **tail_dev = nullptr) {
     const int n = (int)g.size(), nfr = (int)frames.size();
     if (n == 0) return MARS_OK;
     if (m->pre_taps.size() > 64) m->pre_taps.clear();
@@ -1572,7 +1620,7 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
     for (int f = 0; f < nfr; f++) fbytes[f] = pre_frame_bytes(frames[f].fmt, frames[f].w, frames[f].h);
     const bool per_launch = how == PRE_HOST_SYNC && !rois;
     pre_table_stage(&t, fbytes.data(), nfr, per_launch);
-    if (rois && merge_tab) merge_table(nfr, *rois, &t.merge);
+    if (tail) t.merge = *tail;
     if ((how != PRE_DEVICE && !pre_grow(m, st.frames, &st.frames_cap, t.stage_bytes)) || !pre_grow(m, m->preH, &m->preH_cap, t.h_floats)) {
         set_last_error("preprocess: out of device memory for %d frames", n);
         return MARS_ERR_ALLOC_FAILED;
@@ -1597,7 +1645,7 @@ static mars_error_t enqueue_letterbox(Model *m, Model::PreStage &st, int first, 
     cudaStream_t cs = how == PRE_HOST_POOL ? m->h2d_stream : m->stream;
     mars_error_t e = pre_upload(m, st, t, cs);
     if (e != MARS_OK) return e;
-    if (merge_tab) *merge_tab = reinterpret_cast<const int *>(st.tab.p + t.merge_offset());
+    if (tail_dev) *tail_dev = reinterpret_cast<const int *>(st.tab.p + t.merge_offset());
     if (how == PRE_HOST_POOL || (how == PRE_HOST_SYNC && !per_launch)) {
         CU_OK(pre_stage_frames(t, frames.data(), 0, nfr, st.frames.p, cs), MARS_ERR_LAYER_FAILED);
         if (how == PRE_HOST_POOL) {
@@ -1841,6 +1889,121 @@ mars_error_t mars_b200_download_frame_boxes(mars_model_t *model, int first, int 
     return download_records(model, &SlotRecords::fbox, first, n, boxes, counts, maxd);
 }
 
+mars_error_t mars_b200_set_tracking(mars_model_t *model, int n_streams, const mars_b200_track_params_t *p) {
+    Model *m;
+    mars_error_t e = enter(model, &m);
+    if (e != MARS_OK) return e;
+    const mars_b200_track_params_t q = p ? *p : mars_b200_track_params_t MARS_B200_TRACK_PARAMS_DEFAULT;
+    if (n_streams < 0 || n_streams > (1 << 20)) {
+        set_last_error("set_tracking: %d streams (0 .. %d)", n_streams, 1 << 20);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    const float th[6] = {q.high_thresh, q.low_thresh, q.new_thresh, q.sim_high, q.sim_low, q.sim_unconfirmed};
+    bool ok = q.low_thresh >= 0.0f && q.low_thresh <= q.high_thresh && q.max_lost >= 0 && (q.class_aware == 0 || q.class_aware == 1);
+    for (int i = 0; i < 6; i++) ok = ok && std::isfinite(th[i]) && (i < 3 || (th[i] >= 0.0f && th[i] < 1.0f));
+    if (!ok) {
+        set_last_error("set_tracking: parameters (high %g, low %g, new %g, gates %g %g %g, max_lost %d, class_aware %d) need finite "
+                       "values, 0 <= low <= high, gates in [0, 1), max_lost >= 0, class_aware 0 or 1",
+                       q.high_thresh, q.low_thresh, q.new_thresh, q.sim_high, q.sim_low, q.sim_unconfirmed, q.max_lost, q.class_aware);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED); /* the old tables may still be in use */
+    DevBuf<TrackSlot> tracks;
+    DevBuf<TrackMeta> meta;
+    if (n_streams > 0) {
+        if (!tracks.alloc((size_t)n_streams * MARS_B200_MAX_TRACKS) || !meta.alloc((size_t)n_streams)) return MARS_ERR_ALLOC_FAILED;
+        CU_OK(cudaMemsetAsync(meta.p, 0, (size_t)n_streams * sizeof(TrackMeta), m->stream), MARS_ERR_ALLOC_FAILED);
+        CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
+    }
+    m->tracks = std::move(tracks);
+    m->track_meta = std::move(meta);
+    m->track_streams = n_streams;
+    m->track_params = q;
+    return MARS_OK;
+}
+
+mars_error_t mars_b200_reset_tracks(mars_model_t *model, int first_stream, int n) {
+    Model *m;
+    mars_error_t e = enter(model, &m);
+    if (e == MARS_OK) e = need_tracking(m, "reset_tracks");
+    if (e != MARS_OK) return e;
+    if (first_stream < 0 || n < 0 || (long long)first_stream + n > m->track_streams) {
+        set_last_error("reset_tracks: streams [%d, %lld) outside [0, %d)", first_stream, (long long)first_stream + n, m->track_streams);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    if (n > 0) CU_OK(cudaMemsetAsync(m->track_meta.p + first_stream, 0, (size_t)n * sizeof(TrackMeta), m->stream), MARS_ERR_LAYER_FAILED);
+    return MARS_OK;
+}
+
+/* the stream table goes through the synchronous calls' pinned staging, as mars_b200_merge_rois_resident's merge table does */
+mars_error_t mars_b200_track_resident(mars_model_t *model, int first, int n, const int32_t *streams) {
+    Model *m;
+    mars_error_t e = enter(model, &m, first, n);
+    if (e == MARS_OK) e = check_streams(m, "track_resident", n, streams);
+    if (e == MARS_OK) e = need_heads(m, "track_resident");
+    if (e != MARS_OK || n == 0) return e;
+    PreTable t;
+    t.merge.assign(streams, streams + n);
+    Model::PreStage &st = m->pre_stage[PRE_SYNC];
+    e = pre_upload(m, st, t, m->stream);
+    if (e != MARS_OK) return e;
+    return enqueue_track(m, m->rec.box.at(first), m->rec.box.cnt.p + first, MARS_MAX_DETS, reinterpret_cast<const int32_t *>(st.tab.p), n,
+                         m->rec.trk.at(first), m->rec.trk.cnt.p + first, MARS_B200_MAX_TRACKS);
+}
+
+mars_error_t mars_b200_download_tracks(mars_model_t *model, int first, int n, mars_b200_track_box_t *out, int32_t *counts, int maxd) {
+    Model *m = as_model(model);
+    if (m && need_tracking(m, "download_tracks") != MARS_OK) return MARS_ERR_INVALID_TENSOR;
+    return download_records(model, &SlotRecords::trk, first, n, out, counts, maxd);
+}
+
+mars_error_t mars_b200_track_boxes(mars_model_t *model, int n, const int32_t *streams, const mars_box_t *boxes, const int32_t *counts,
+                                   int box_stride, mars_b200_track_box_t *out, int32_t *out_counts, int maxd) {
+    Model *m;
+    mars_error_t e = enter(model, &m);
+    if (e == MARS_OK) e = check_streams(m, "track_boxes", n, streams);
+    if (e != MARS_OK) return e;
+    if (n < 0 || (n > 0 && (!counts || !out || !out_counts))) { set_last_error("track_boxes: no count or output table"); return MARS_ERR_INVALID_FILE; }
+    int maxc = 1;
+    for (int i = 0; i < n; i++) {
+        if (counts[i] < 0 || counts[i] > TRK_MAX_DETS || counts[i] > box_stride || (counts[i] > 0 && !boxes)) {
+            set_last_error("track_boxes: entry %d: %d boxes (0 .. min(box_stride %d, %d))", i, counts[i], box_stride, TRK_MAX_DETS);
+            return MARS_ERR_INVALID_TENSOR;
+        }
+        maxc = std::max(maxc, (int)counts[i]);
+    }
+    if (n == 0) return MARS_OK;
+    maxd = std::max(0, std::min(maxd, MARS_B200_MAX_TRACKS));
+    /* in: [streams | counts | boxes n x maxc], out: [counts | records n x MARS_B200_MAX_TRACKS], each part 256-byte aligned */
+    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t ints = up((size_t)n * sizeof(int32_t)), in_bytes = 2 * ints + (size_t)n * maxc * sizeof(mars_box_t);
+    const size_t out_bytes = ints + (size_t)n * MARS_B200_MAX_TRACKS * sizeof(mars_b200_track_box_t);
+    if (!pre_grow(m, m->track_in, &m->track_in_cap, in_bytes) || !pre_grow(m, m->track_out, &m->track_out_cap, out_bytes)) return MARS_ERR_ALLOC_FAILED;
+    std::vector<uint8_t> blob(in_bytes, 0);
+    memcpy(blob.data(), streams, (size_t)n * sizeof(int32_t));
+    memcpy(blob.data() + ints, counts, (size_t)n * sizeof(int32_t));
+    for (int i = 0; i < n; i++)
+        memcpy(blob.data() + 2 * ints + (size_t)i * maxc * sizeof(mars_box_t), boxes + (size_t)i * box_stride, (size_t)counts[i] * sizeof(mars_box_t));
+    const int32_t *d_streams = reinterpret_cast<const int32_t *>(m->track_in.p), *d_counts = reinterpret_cast<const int32_t *>(m->track_in.p + ints);
+    const mars_box_t *d_boxes = reinterpret_cast<const mars_box_t *>(m->track_in.p + 2 * ints);
+    int32_t *d_out_counts = reinterpret_cast<int32_t *>(m->track_out.p);
+    mars_b200_track_box_t *d_out = reinterpret_cast<mars_b200_track_box_t *>(m->track_out.p + ints);
+    e = timed_call(m, "track_boxes", [&]() -> mars_error_t {
+        CU_OK(cudaMemcpyAsync(m->track_in.p, blob.data(), in_bytes, cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
+        mars_error_t r = enqueue_track(m, d_boxes, d_counts, maxc, d_streams, n, d_out, d_out_counts, MARS_B200_MAX_TRACKS);
+        if (r != MARS_OK) return r;
+        CU_OK(cudaMemcpyAsync(out_counts, d_out_counts, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, m->stream), MARS_ERR_LAYER_FAILED);
+        if (maxd > 0)
+            CU_OK(cudaMemcpy2DAsync(out, (size_t)maxd * sizeof(mars_b200_track_box_t), d_out, MARS_B200_MAX_TRACKS * sizeof(mars_b200_track_box_t),
+                                    (size_t)maxd * sizeof(mars_b200_track_box_t), (size_t)n, cudaMemcpyDeviceToHost, m->stream),
+                  MARS_ERR_LAYER_FAILED);
+        return MARS_OK;
+    });
+    if (e == MARS_OK)
+        for (int i = 0; i < n; i++) out_counts[i] = std::min(out_counts[i], maxd);
+    return e;
+}
+
 /* end to end from host buffers, double-buffered over the two halves of the slot pool:
  * H2D of chunk c+1 and D2H of chunk c-1 overlap the kernels of chunk c */
 static mars_error_t batch_pipeline(Model *m, int n, const void *inputs, size_t in_stride, void *outputs, size_t out_stride,
@@ -1910,13 +2073,15 @@ struct SubmitIn {
     const RoiList *rois;
 };
 /* what a pooled submit reads back, which also picks the step: the kept detections of output0 (decode + centre NMS), the kept
- * corner boxes of the heads, the frame records of the region merge (rois), or the raw output tensor 0 (the layers alone) */
+ * corner boxes of the heads, the frame records of the region merge (rois), the tracked boxes of the heads' boxes (frames only:
+ * the stream table travels in the letterbox upload), or the raw output tensor 0 (the layers alone) */
 struct SubmitOut {
-    enum Kind { DETS, BOXES, FRAME_BOXES, TENSOR } kind;
+    enum Kind { DETS, BOXES, FRAME_BOXES, TRACKS, TENSOR } kind;
     void *dst; /* records [records][maxd], or output tensors `stride` bytes apart */
     int32_t *counts;
     int maxd;
     size_t stride;
+    const int32_t *streams = nullptr; /* TRACKS: the tracker stream of each image */
 };
 
 /* Asynchronous form of mars_b200_detect_batch: the slot pool is split into two halves ("pools" 0 and 1); a batch of up to
@@ -1952,6 +2117,11 @@ static mars_error_t submit_batch(mars_model_t *model, const char *what, int pool
         set_last_error("%s: pool %d still has a batch in flight (mars_b200_wait_batch first)", what, pool);
         return MARS_ERR_LAYER_FAILED;
     }
+    if (out.kind == SubmitOut::TRACKS) {
+        e = in.from_frames ? check_streams(m, what, n, out.streams) : MARS_ERR_INVALID_FILE;
+        if (e != MARS_OK) return e;
+        if (out.maxd > MARS_B200_MAX_TRACKS) out.maxd = MARS_B200_MAX_TRACKS;
+    }
     if (out.maxd > 1000) out.maxd = 1000;
     if (out.maxd < 0) out.maxd = 0;
     const size_t in_stride = std::max(in.stride, io_bytes(&m->pub, 0)), out_stride = std::max(out.stride, io_bytes(&m->pub, 1));
@@ -1967,10 +2137,13 @@ static mars_error_t submit_batch(mars_model_t *model, const char *what, int pool
     if (e != MARS_OK) return e;
     if (n > 0) {
         /* the half is free: its previous batch was waited for (read-back complete) before this call -- its staging too */
-        const int *merge_tab = nullptr;
+        std::vector<int> tail;
+        if (in.rois) merge_table(nrec, *in.rois, &tail);
+        if (out.kind == SubmitOut::TRACKS) tail.assign(out.streams, out.streams + n);
+        const int *tail_dev = nullptr;
         if (in.from_frames) {
-            e = enqueue_letterbox(m, m->pre_stage[pool], first, *in.frames, g, ti, nhwc, PRE_HOST_POOL, m->ev_in[pool], in.rois,
-                                  in.rois ? &merge_tab : nullptr);
+            e = enqueue_letterbox(m, m->pre_stage[pool], first, *in.frames, g, ti, nhwc, PRE_HOST_POOL, m->ev_in[pool], in.rois, &tail,
+                                  &tail_dev);
             if (e != MARS_OK) return e;
         } else {
             e = copy_io(m, first, n, const_cast<void *>(in.tensors), in_stride, 0, m->h2d_stream);
@@ -1979,7 +2152,10 @@ static mars_error_t submit_batch(mars_model_t *model, const char *what, int pool
             cudaStreamWaitEvent(m->stream, m->ev_in[pool], 0);
         }
         e = enqueue_step_graphed(m, first, n, nms_thresh, flavour);
-        if (e == MARS_OK && in.rois) e = enqueue_merge(m, first, nrec, merge_tab, merge_thresh);
+        if (e == MARS_OK && in.rois) e = enqueue_merge(m, first, nrec, tail_dev, merge_thresh);
+        if (e == MARS_OK && out.kind == SubmitOut::TRACKS)
+            e = enqueue_track(m, m->rec.box.at(first), m->rec.box.cnt.p + first, MARS_MAX_DETS, tail_dev, n, m->rec.trk.at(first),
+                              m->rec.trk.cnt.p + first, MARS_B200_MAX_TRACKS);
         if (e != MARS_OK) { cudaStreamSynchronize(m->stream); return e; }
         cudaEventRecord(m->ev_done[pool], m->stream);
         cudaStreamWaitEvent(m->d2h_stream, m->ev_done[pool], 0);
@@ -1987,6 +2163,7 @@ static mars_error_t submit_batch(mars_model_t *model, const char *what, int pool
             case SubmitOut::DETS: e = copy_dets(m->rec.det, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
             case SubmitOut::BOXES: e = copy_dets(m->rec.box, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
             case SubmitOut::FRAME_BOXES: e = copy_dets(m->rec.fbox, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
+            case SubmitOut::TRACKS: e = copy_dets(m->rec.trk, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
             case SubmitOut::TENSOR: e = copy_io(m, first, n, out.dst, out_stride, 1, m->d2h_stream); break;
         }
         if (e != MARS_OK) return e;
@@ -2046,6 +2223,21 @@ mars_error_t mars_b200_submit_rois_nv12_heads_batch(mars_model_t *model, int poo
     return submit_batch(model, "submit_rois_nv12_heads_batch", pool, n_rois,
                         SubmitIn{nullptr, 0, true, nv12_sources(n_frames, frames, &s), &rl},
                         SubmitOut{SubmitOut::FRAME_BOXES, boxes, counts, maxd, 0}, nms_thresh, merge_thresh);
+}
+
+/* mars_b200_submit_frames[_nv12]_heads_batch, then the tracker on the pool's slots; the tracked boxes are read back */
+mars_error_t mars_b200_submit_frames_track_batch(mars_model_t *model, int pool, int n, const mars_b200_frame_t *frames, const int32_t *streams,
+                                                 mars_b200_track_box_t *out, int32_t *counts, int maxd, float nms_thresh) {
+    std::vector<FrameSrc> s;
+    return submit_batch(model, "submit_frames_track_batch", pool, n, SubmitIn{nullptr, 0, true, rgb_sources(n, frames, &s), nullptr},
+                        SubmitOut{SubmitOut::TRACKS, out, counts, maxd, 0, streams}, nms_thresh);
+}
+mars_error_t mars_b200_submit_frames_nv12_track_batch(mars_model_t *model, int pool, int n, const mars_b200_nv12_frame_t *frames,
+                                                      const int32_t *streams, mars_b200_track_box_t *out, int32_t *counts, int maxd,
+                                                      float nms_thresh) {
+    std::vector<FrameSrc> s;
+    return submit_batch(model, "submit_frames_nv12_track_batch", pool, n, SubmitIn{nullptr, 0, true, nv12_sources(n, frames, &s), nullptr},
+                        SubmitOut{SubmitOut::TRACKS, out, counts, maxd, 0, streams}, nms_thresh);
 }
 
 /* mars_b200_submit_batch without the YOLO post-process: the raw output tensor 0 of every image is read back instead
