@@ -304,6 +304,88 @@ mars_error_t mars_b200_submit_frames_nv12_track_batch(mars_model_t *m, int pool,
                                                       const int32_t *streams, mars_b200_track_box_t *out, int32_t *counts, int maxd,
                                                       float nms_thresh);
 
+/* ---- zones and counting lines on tracked streams ----------------------------------------------------------------------------
+ * Line-crossing counts, zone occupancy and enter / dwell / exit events per tracker stream, computed on the device right after the
+ * tracker, with the per-track state in HBM.  This is the library's own definition; the C statement is tests/zones_oracle.c and
+ * the device equals it byte for byte.
+ *
+ * Geometry is set per tracker stream (mars_b200_set_zones), in the coordinates of the tracked boxes: frame coordinates for slots
+ * with a frame size, network coordinates otherwise.  A zone is a polygon of 3..16 vertices with a class (-1: any), an anchor and
+ * min_dwell (frames; 0: no dwell events).  A line is a directed segment (x0, y0) -> (x1, y1) with distinct ends, a class and an
+ * anchor.  A track is "shown" in a frame when the tracker outputs it in that frame (Tracked and confirmed); its anchor is taken
+ * from its tracked box (mars_b200_track_box_t after this frame's update):
+ *   MARS_B200_ANCHOR_BOTTOM  ((x0 + x1) * 0.5f, y1)        MARS_B200_ANCHOR_CENTRE  ((x0 + x1) * 0.5f, (y0 + y1) * 0.5f)
+ * All arithmetic is float32, one rounding per operation, in the order written.  A class matches when the geometry's class is -1
+ * or equals the track's class in this frame.
+ *   inside(P, px, py) (crossing number, even-odd): for i = 0 .. n-1 and j = (i + n - 1) mod n, toggle when (yi > py) != (yj > py)
+ *     and px < xi + ((xj - xi) * (py - yi)) / (yj - yi).
+ *   side(L, px, py): the sign (+1, -1, 0) of (x1 - x0) * (py - y0) - (y1 - y0) * (px - x0); +1 is the right-hand side walking
+ *     from end 0 to end 1 on screen (y down).
+ *   crossing: per (track, line) sigma is the last non-zero side seen at a shown frame (0: none yet).  At a shown frame with anchor
+ *     q, the track shown before with anchor p, a crossing counts when side(q) != 0, sigma == -side(q), the class matches, and the
+ *     step meets the closed segment: o_a = (qx - px) * (ay - py) - (qy - py) * (ax - px) and o_b (the same with end b) are not both
+ *     > 0 and not both < 0.  A crossing to +1 is CROSS_POS, to -1 CROSS_NEG.  Then sigma = side(q) when that is non-zero, whatever
+ *     the class.  So walking around a line's end never counts, stopping on the line and going on counts once, and a crossing made
+ *     during a lost gap counts when the track is shown again.  There is no debouncing: a track jittering over a line counts each
+ *     crossing.
+ *   zones: membership is evaluated at shown frames only: inside(anchor) and the class matches.  A track not shown in a frame
+ *     (Lost, or not confirmed yet) keeps its state.  ENTER: inside now and not at the previous shown frame (value 1 at the track's
+ *     first shown frame since the stream's analytics started, else 0); the entry frame is recorded.  DWELL: once per stay, at the
+ *     first shown frame with frame - entry + 1 >= min_dwell > 0 (value: that number).  EXIT: inside before, shown outside now
+ *     (value frame - entry).  GONE: the tracker removed a track that was inside (value frame - entry, the last class known); its
+ *     analytics state is then dropped.
+ *   occupancy of a zone: the tracks shown in the frame that are inside it.  Line totals: CROSS_POS and CROSS_NEG counts since
+ *     mars_b200_set_zones or mars_b200_reset_tracks on that stream.
+ *   events of a frame in order: ascending track_id (removed tracks included); within a track its crossings in line order, then its
+ *     zone events in zone order; within a zone ENTER before DWELL (both in one frame when min_dwell == 1).  The first
+ *     MARS_B200_MAX_ZONE_EVENTS are written; n_events is the full count.  A crossing's value is the line's total of that
+ *     direction after it; GONE, EXIT, ENTER and DWELL have index = the zone, crossings index = the line.
+ * `frame` of a record is the tracker's frame number of the stream.  A record of a stream without geometry has its frame number,
+ * zeros and no events. */
+#define MARS_B200_MAX_ZONES 8
+#define MARS_B200_MAX_ZONE_VERTS 16
+#define MARS_B200_MAX_LINES 8
+#define MARS_B200_MAX_ZONE_EVENTS 128
+enum { MARS_B200_ANCHOR_BOTTOM = 0, MARS_B200_ANCHOR_CENTRE = 1 };
+enum { MARS_B200_ZONE_ENTER = 0, MARS_B200_ZONE_DWELL = 1, MARS_B200_ZONE_EXIT = 2, MARS_B200_ZONE_GONE = 3, MARS_B200_CROSS_POS = 4,
+       MARS_B200_CROSS_NEG = 5 };
+typedef struct {
+    float x[MARS_B200_MAX_ZONE_VERTS], y[MARS_B200_MAX_ZONE_VERTS]; /* vertices 0 .. n_verts-1 */
+    int32_t n_verts, class_id, anchor, min_dwell;
+} mars_b200_zone_t; /* 144 bytes */
+typedef struct { float x0, y0, x1, y1; int32_t class_id, anchor; } mars_b200_line_t; /* 24 bytes */
+typedef struct { int32_t track_id, class_id; int16_t kind, index; int32_t value; } mars_b200_zone_event_t; /* 16 bytes */
+typedef struct {
+    int32_t frame, n_events;
+    int32_t occupancy[MARS_B200_MAX_ZONES];                      /* this frame */
+    int32_t crossed_pos[MARS_B200_MAX_LINES], crossed_neg[MARS_B200_MAX_LINES]; /* line totals after this frame */
+    mars_b200_zone_event_t events[MARS_B200_MAX_ZONE_EVENTS];
+} mars_b200_zone_frame_t; /* 2152 bytes */
+/* geometry of tracker stream `stream`; its analytics state and line totals start over.  n_zones = n_lines = 0 switches the stream
+ * off.  Needs tracking set (mars_b200_set_tracking, which drops all geometry); waits for the compute stream.  Everything is checked
+ * first (stream in range, counts within the limits, 3..16 vertices, finite coordinates, class_id >= -1, a known anchor, min_dwell >=
+ * 0, distinct line ends): a rejected call changes nothing and mars_b200_last_error names the zone or line and the field.  While any
+ * stream has geometry, every tracker call (resident, host boxes, submits) runs the analytics after the tracker, so each stream's
+ * analytics see every frame; mars_b200_reset_tracks clears the analytics state and totals of its streams, not their geometry. */
+mars_error_t mars_b200_set_zones(mars_model_t *m, int stream, const mars_b200_zone_t *zones, int n_zones, const mars_b200_line_t *lines,
+                                 int n_lines);
+/* zone records of track records [first, first+n), as the last mars_b200_track_resident or track submit on those slots wrote them.
+ * Those calls write the records only while some stream has geometry (so that, with none, they launch what they launched before
+ * zones existed); a slot not written since keeps its earlier record, or zeros from mars_b200_set_batch */
+mars_error_t mars_b200_download_zones(mars_model_t *m, int first, int n, mars_b200_zone_frame_t *out);
+/* mars_b200_track_boxes, plus zone_out[n] (NULL: none): the analytics run in this call even when no stream has geometry */
+mars_error_t mars_b200_track_boxes_zones(mars_model_t *m, int n, const int32_t *streams, const mars_box_t *boxes, const int32_t *counts,
+                                         int box_stride, mars_b200_track_box_t *out, int32_t *out_counts, int maxd,
+                                         mars_b200_zone_frame_t *zone_out);
+/* mars_b200_submit_frames[_nv12]_track_batch, plus zones[n]: the zone record of every frame, in the same read-back (waited for with
+ * mars_b200_wait_batch) */
+mars_error_t mars_b200_submit_frames_zones_batch(mars_model_t *m, int pool, int n, const mars_b200_frame_t *frames, const int32_t *streams,
+                                                 mars_b200_track_box_t *out, int32_t *counts, int maxd, mars_b200_zone_frame_t *zones,
+                                                 float nms_thresh);
+mars_error_t mars_b200_submit_frames_nv12_zones_batch(mars_model_t *m, int pool, int n, const mars_b200_nv12_frame_t *frames,
+                                                      const int32_t *streams, mars_b200_track_box_t *out, int32_t *counts, int maxd,
+                                                      mars_b200_zone_frame_t *zones, float nms_thresh);
+
 /* ---- several GPUs of one box behind one call (batch sharded over the devices, no inter-GPU traffic on the path) ---------- */
 typedef struct mars_b200_group mars_b200_group_t;
 /* one replica of the model per device (devices = NULL: ordinals 0 .. n_devices-1), `per_gpu_batch` image slots each */

@@ -114,6 +114,37 @@ class TRACK_PARAMS(C.Structure):
         super().__init__(**{**self.DEFAULTS, **kw})
 
 
+# zones and counting lines on tracked streams (mars_b200_set_zones)
+MAX_ZONES, MAX_ZONE_VERTS, MAX_LINES, MAX_ZONE_EVENTS = 8, 16, 8, 128
+ANCHOR_BOTTOM, ANCHOR_CENTRE = 0, 1
+ZONE_ENTER, ZONE_DWELL, ZONE_EXIT, ZONE_GONE, CROSS_POS, CROSS_NEG = 0, 1, 2, 3, 4, 5
+
+
+class ZONE(C.Structure):
+    """mars_b200_zone_t: ZONE([(x, y), ...], class_id=-1, anchor=ANCHOR_BOTTOM, min_dwell=0)"""
+    _fields_ = [("x", C.c_float * MAX_ZONE_VERTS), ("y", C.c_float * MAX_ZONE_VERTS), ("n_verts", C.c_int32), ("class_id", C.c_int32),
+                ("anchor", C.c_int32), ("min_dwell", C.c_int32)]
+
+    def __init__(self, points=(), class_id=-1, anchor=ANCHOR_BOTTOM, min_dwell=0):
+        super().__init__(n_verts=len(points), class_id=class_id, anchor=anchor, min_dwell=min_dwell)
+        for i, (x, y) in enumerate(points[:MAX_ZONE_VERTS]):
+            self.x[i], self.y[i] = x, y
+
+
+class LINE(C.Structure):
+    """mars_b200_line_t: LINE(x0, y0, x1, y1, class_id=-1, anchor=ANCHOR_BOTTOM), directed from (x0, y0) to (x1, y1)"""
+    _fields_ = [("x0", C.c_float), ("y0", C.c_float), ("x1", C.c_float), ("y1", C.c_float), ("class_id", C.c_int32), ("anchor", C.c_int32)]
+
+    def __init__(self, x0=0.0, y0=0.0, x1=0.0, y1=0.0, class_id=-1, anchor=ANCHOR_BOTTOM):
+        super().__init__(x0, y0, x1, y1, class_id, anchor)
+
+
+# mars_b200_zone_event_t and mars_b200_zone_frame_t
+ZONE_EVENT_DTYPE = np.dtype([("track_id", "<i4"), ("class_id", "<i4"), ("kind", "<i2"), ("index", "<i2"), ("value", "<i4")])
+ZONE_FRAME_DTYPE = np.dtype([("frame", "<i4"), ("n_events", "<i4"), ("occupancy", "<i4", MAX_ZONES), ("crossed_pos", "<i4", MAX_LINES),
+                             ("crossed_neg", "<i4", MAX_LINES), ("events", ZONE_EVENT_DTYPE, MAX_ZONE_EVENTS)])
+assert C.sizeof(ZONE) == 144 and C.sizeof(LINE) == 24 and ZONE_FRAME_DTYPE.itemsize == 2152
+
 # every symbol include/*.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     # include/mars_runtime.h
@@ -275,6 +306,14 @@ SIGNATURES = {
                                                       C.c_float]),
     "mars_b200_submit_frames_nv12_track_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME), C.c_void_p, C.c_void_p, C.c_void_p,
                                                            C.c_int, C.c_float]),
+    "mars_b200_set_zones": (C.c_int, [PM, C.c_int, C.POINTER(ZONE), C.c_int, C.POINTER(LINE), C.c_int]),
+    "mars_b200_download_zones": (C.c_int, [PM, C.c_int, C.c_int, C.c_void_p]),
+    "mars_b200_track_boxes_zones": (C.c_int, [PM, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
+                                              C.c_void_p]),
+    "mars_b200_submit_frames_zones_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(FRAME), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                                      C.c_void_p, C.c_float]),
+    "mars_b200_submit_frames_nv12_zones_batch": (C.c_int, [PM, C.c_int, C.c_int, C.POINTER(NV12_FRAME), C.c_void_p, C.c_void_p, C.c_void_p,
+                                                           C.c_int, C.c_void_p, C.c_float]),
 }
 
 _lib = None
@@ -588,6 +627,13 @@ class MarsModel:
     def track_boxes(self, streams, boxes, maxd=MAX_TRACKS):
         """boxes: one BOX_DTYPE array per entry, the next frame of stream streams[i] -> (TRACK_DTYPE [n, maxd], counts [n]);
         synchronous"""
+        return self._track_boxes(streams, boxes, maxd, False)
+
+    def track_boxes_zones(self, streams, boxes, maxd=MAX_TRACKS):
+        """track_boxes plus the zone record of every entry -> (TRACK_DTYPE [n, maxd], counts [n], ZONE_FRAME_DTYPE [n])"""
+        return self._track_boxes(streams, boxes, maxd, True)
+
+    def _track_boxes(self, streams, boxes, maxd, zones):
         s = np.ascontiguousarray(streams, dtype=np.int32)
         n = s.size
         counts = np.array([len(b) for b in boxes], dtype=np.int32)
@@ -597,9 +643,21 @@ class MarsModel:
             table[i, : len(b)] = b
         out = np.zeros((n, maxd), dtype=TRACK_DTYPE)
         oc = np.zeros(n, dtype=np.int32)
-        self._check(lib().mars_b200_track_boxes(self.m, n, s.ctypes.data, table.ctypes.data, counts.ctypes.data, stride, out.ctypes.data,
-                                                oc.ctypes.data, maxd), "track_boxes")
-        return out, oc
+        zo = np.zeros(n, dtype=ZONE_FRAME_DTYPE) if zones else None
+        self._check(lib().mars_b200_track_boxes_zones(self.m, n, s.ctypes.data, table.ctypes.data, counts.ctypes.data, stride, out.ctypes.data,
+                                                      oc.ctypes.data, maxd, None if zo is None else zo.ctypes.data), "track_boxes")
+        return (out, oc, zo) if zones else (out, oc)
+
+    def set_zones(self, stream, zones=(), lines=()):
+        """geometry of tracker stream `stream` (ZONE and LINE sequences); its analytics start over; empty: the stream is off"""
+        za, la = (ZONE * max(1, len(zones)))(*zones), (LINE * max(1, len(lines)))(*lines)
+        self._check(lib().mars_b200_set_zones(self.m, stream, za, len(zones), la, len(lines)), "set_zones")
+
+    def download_zones(self, first, n):
+        """zone records of track records [first, first + n) -> ZONE_FRAME_DTYPE [n]"""
+        out = np.zeros(n, dtype=ZONE_FRAME_DTYPE)
+        self._check(lib().mars_b200_download_zones(self.m, first, n, out.ctypes.data), "download_zones")
+        return out
 
     def submit_frames_track_batch(self, pool, frames, streams, out, counts, maxd=MAX_TRACKS, thresh=0.45):
         """submit_frames_heads_batch followed by the tracker: frame i is the next frame of stream streams[i]; out [n, maxd] TRACK_DTYPE.
@@ -616,6 +674,23 @@ class MarsModel:
         s = np.ascontiguousarray(streams, dtype=np.int32)
         self._check(lib().mars_b200_submit_frames_nv12_track_batch(self.m, pool, len(frames), table, s.ctypes.data, _addr(out), _addr(counts),
                                                                    maxd, thresh), "submit_frames_nv12_track_batch")
+        self._inflight[pool] = (table, keep, s)
+
+    def submit_frames_zones_batch(self, pool, frames, streams, out, counts, zones, maxd=MAX_TRACKS, thresh=0.45):
+        """submit_frames_track_batch plus the zone record of every frame into zones [n] ZONE_FRAME_DTYPE, read back in the same
+        batch; out, counts and zones must be kept alive by the caller until wait_batch(pool)"""
+        table, keep = host_frames(frames)
+        s = np.ascontiguousarray(streams, dtype=np.int32)
+        self._check(lib().mars_b200_submit_frames_zones_batch(self.m, pool, len(frames), table, s.ctypes.data, _addr(out), _addr(counts), maxd,
+                                                              _addr(zones), thresh), "submit_frames_zones_batch")
+        self._inflight[pool] = (table, keep, s)
+
+    def submit_frames_nv12_zones_batch(self, pool, frames, streams, out, counts, zones, maxd=MAX_TRACKS, thresh=0.45):
+        """submit_frames_zones_batch from (y, uv, colour) NV12 host frames (host_nv12_frames)"""
+        table, keep = host_nv12_frames(frames)
+        s = np.ascontiguousarray(streams, dtype=np.int32)
+        self._check(lib().mars_b200_submit_frames_nv12_zones_batch(self.m, pool, len(frames), table, s.ctypes.data, _addr(out), _addr(counts),
+                                                                   maxd, _addr(zones), thresh), "submit_frames_nv12_zones_batch")
         self._inflight[pool] = (table, keep, s)
 
     def download_outputs(self, first, n, host=None, stride=0):

@@ -41,6 +41,7 @@
 #include "preproc.cuh"
 #include "nna_layout.cuh"
 #include "track.cuh"
+#include "zones.cuh"
 
 namespace marsb200 {
 
@@ -190,6 +191,7 @@ struct SlotRecords {
     RecordSet<mars_box_t> box_raw, box;  /* the heads path: decoded candidates, kept corner boxes */
     RecordSet<mars_box_t> fbox;          /* frame records of the region merge (mars_b200_merge_rois_resident) */
     RecordSet<mars_b200_track_box_t, MARS_B200_MAX_TRACKS> trk; /* tracked boxes (mars_b200_track_resident) */
+    DevBuf<mars_b200_zone_frame_t> zone; /* one zone record per slot, beside its tracked boxes (k_zones) */
     DevBuf<unsigned> nms_mask;           /* NMS_SCRATCH_WORDS per slot: suppression bit matrices */
     DevBuf<int2> frame;                  /* original frame size per slot (0 = none), for the letterbox inverse */
 };
@@ -262,6 +264,13 @@ struct Model {
     DevBuf<TrackMeta> track_meta;
     DevBuf<> track_in, track_out;
     size_t track_in_cap = 0, track_out_cap = 0;
+    /* zones and counting lines (mars_b200_set_zones, zones.cuh): per tracker stream its geometry, the analytics state of its
+     * tracks and its line totals, allocated by the first set_zones; which streams have geometry, and how many */
+    DevBuf<ZoneGeom> zone_geom;
+    DevBuf<ZoneTrack> zone_state;
+    DevBuf<ZoneMeta> zone_meta;
+    std::vector<uint8_t> zone_on;
+    int zone_streams = 0;
 };
 
 static Model *as_model(mars_model_t *p) {
@@ -327,10 +336,11 @@ static mars_error_t set_capacity(Model *m, int capacity) {
     SlotRecords r;
     if (!slots.alloc(c * m->slot_stride) || (m->scratch_stride && !scratch.alloc(c * m->scratch_stride)) || !r.raw.alloc(capacity) ||
         !r.det.alloc(capacity) || !r.box_raw.alloc(capacity) || !r.box.alloc(capacity) || !r.fbox.alloc(capacity) ||
-        !r.trk.alloc(capacity) || !r.nms_mask.alloc(c * NMS_SCRATCH_WORDS) || !r.frame.alloc(c))
+        !r.trk.alloc(capacity) || !r.zone.alloc(c) || !r.nms_mask.alloc(c * NMS_SCRATCH_WORDS) || !r.frame.alloc(c))
         return MARS_ERR_ALLOC_FAILED;
     CU_OK(cudaMemsetAsync(slots.p, 0, c * m->slot_stride, m->stream), MARS_ERR_ALLOC_FAILED);
     CU_OK(cudaMemsetAsync(r.frame.p, 0, c * sizeof(int2), m->stream), MARS_ERR_ALLOC_FAILED);
+    CU_OK(cudaMemsetAsync(r.zone.p, 0, c * sizeof(mars_b200_zone_frame_t), m->stream), MARS_ERR_ALLOC_FAILED);
     for (int32_t *cnt : {r.raw.cnt.p, r.det.cnt.p, r.box_raw.cnt.p, r.box.cnt.p, r.fbox.cnt.p, r.trk.cnt.p})
         CU_OK(cudaMemsetAsync(cnt, 0, c * sizeof(int32_t), m->stream), MARS_ERR_ALLOC_FAILED);
     if (m->slots.p) {
@@ -795,14 +805,22 @@ static mars_error_t check_streams(Model *m, const char *what, int n, const int32
 }
 
 /* the tracker on the compute stream: entry i = the detections at boxes + i * box_stride (counts[i]) as the next frame of stream
- * streams[i] (a device table), tracked boxes to out + i * out_stride and out_counts[i] */
+ * streams[i] (a device table), tracked boxes to out + i * out_stride and out_counts[i].  The zone analytics follow while any
+ * stream has geometry, or always when with_zones; their records go to zones[i] (null: none) */
 static mars_error_t enqueue_track(Model *m, const mars_box_t *boxes, const int32_t *counts, int box_stride, const int32_t *streams, int n,
-                                  mars_b200_track_box_t *out, int32_t *out_counts, int out_stride) {
+                                  mars_b200_track_box_t *out, int32_t *out_counts, int out_stride, mars_b200_zone_frame_t *zones = nullptr,
+                                  bool with_zones = false) {
     if (n <= 0) return MARS_OK;
     k_track<<<n, TRK_THREADS, 0, m->stream>>>(boxes, counts, box_stride, streams, m->tracks.p, m->track_meta.p, m->track_params, out,
                                              out_counts, out_stride);
     m->launches++;
     CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
+    if (m->zone_streams > 0 || with_zones) {
+        k_zones<<<n, ZN_THREADS, 0, m->stream>>>(streams, m->tracks.p, m->track_meta.p, out, out_counts, out_stride, m->zone_geom.p,
+                                                m->zone_state.p, m->zone_meta.p, zones);
+        m->launches++;
+        CU_OK(cudaGetLastError(), MARS_ERR_LAYER_FAILED);
+    }
     return MARS_OK;
 }
 } // namespace marsb200
@@ -1919,6 +1937,11 @@ mars_error_t mars_b200_set_tracking(mars_model_t *model, int n_streams, const ma
     m->track_meta = std::move(meta);
     m->track_streams = n_streams;
     m->track_params = q;
+    m->zone_geom.reset();
+    m->zone_state.reset();
+    m->zone_meta.reset();
+    m->zone_on.assign((size_t)n_streams, 0);
+    m->zone_streams = 0;
     return MARS_OK;
 }
 
@@ -1932,6 +1955,9 @@ mars_error_t mars_b200_reset_tracks(mars_model_t *model, int first_stream, int n
         return MARS_ERR_INVALID_TENSOR;
     }
     if (n > 0) CU_OK(cudaMemsetAsync(m->track_meta.p + first_stream, 0, (size_t)n * sizeof(TrackMeta), m->stream), MARS_ERR_LAYER_FAILED);
+    /* the track IDs start over, so the analytics state of these streams would name other tracks: it goes too, the geometry stays */
+    if (n > 0 && m->zone_meta.p)
+        CU_OK(cudaMemsetAsync(m->zone_meta.p + first_stream, 0, (size_t)n * sizeof(ZoneMeta), m->stream), MARS_ERR_LAYER_FAILED);
     return MARS_OK;
 }
 
@@ -1948,7 +1974,7 @@ mars_error_t mars_b200_track_resident(mars_model_t *model, int first, int n, con
     e = pre_upload(m, st, t, m->stream);
     if (e != MARS_OK) return e;
     return enqueue_track(m, m->rec.box.at(first), m->rec.box.cnt.p + first, MARS_MAX_DETS, reinterpret_cast<const int32_t *>(st.tab.p), n,
-                         m->rec.trk.at(first), m->rec.trk.cnt.p + first, MARS_B200_MAX_TRACKS);
+                         m->rec.trk.at(first), m->rec.trk.cnt.p + first, MARS_B200_MAX_TRACKS, m->rec.zone.p + first);
 }
 
 mars_error_t mars_b200_download_tracks(mars_model_t *model, int first, int n, mars_b200_track_box_t *out, int32_t *counts, int maxd) {
@@ -1957,8 +1983,104 @@ mars_error_t mars_b200_download_tracks(mars_model_t *model, int first, int n, ma
     return download_records(model, &SlotRecords::trk, first, n, out, counts, maxd);
 }
 
+/* the checks of mars_b200_set_zones; the message names the zone or line and the field */
+static bool zones_valid(const mars_b200_zone_t *zones, int n_zones, const mars_b200_line_t *lines, int n_lines) {
+    auto anchor_ok = [](int a) { return a == MARS_B200_ANCHOR_BOTTOM || a == MARS_B200_ANCHOR_CENTRE; };
+    for (int k = 0; k < n_zones; k++) {
+        const mars_b200_zone_t &z = zones[k];
+        if (z.n_verts < 3 || z.n_verts > MARS_B200_MAX_ZONE_VERTS) {
+            set_last_error("set_zones: zone %d: n_verts %d (3 .. %d)", k, z.n_verts, MARS_B200_MAX_ZONE_VERTS);
+            return false;
+        }
+        for (int i = 0; i < z.n_verts; i++)
+            if (!std::isfinite(z.x[i]) || !std::isfinite(z.y[i])) {
+                set_last_error("set_zones: zone %d: vertex %d (%g, %g) is not finite", k, i, z.x[i], z.y[i]);
+                return false;
+            }
+        if (z.class_id < -1) { set_last_error("set_zones: zone %d: class_id %d (-1: any, or >= 0)", k, z.class_id); return false; }
+        if (!anchor_ok(z.anchor)) { set_last_error("set_zones: zone %d: anchor %d (0 bottom, 1 centre)", k, z.anchor); return false; }
+        if (z.min_dwell < 0) { set_last_error("set_zones: zone %d: min_dwell %d (>= 0)", k, z.min_dwell); return false; }
+    }
+    for (int k = 0; k < n_lines; k++) {
+        const mars_b200_line_t &l = lines[k];
+        if (!std::isfinite(l.x0) || !std::isfinite(l.y0) || !std::isfinite(l.x1) || !std::isfinite(l.y1)) {
+            set_last_error("set_zones: line %d: ends (%g, %g) (%g, %g) are not finite", k, l.x0, l.y0, l.x1, l.y1);
+            return false;
+        }
+        if (l.x0 == l.x1 && l.y0 == l.y1) { set_last_error("set_zones: line %d: ends coincide at (%g, %g)", k, l.x0, l.y0); return false; }
+        if (l.class_id < -1) { set_last_error("set_zones: line %d: class_id %d (-1: any, or >= 0)", k, l.class_id); return false; }
+        if (!anchor_ok(l.anchor)) { set_last_error("set_zones: line %d: anchor %d (0 bottom, 1 centre)", k, l.anchor); return false; }
+    }
+    return true;
+}
+
+mars_error_t mars_b200_set_zones(mars_model_t *model, int stream, const mars_b200_zone_t *zones, int n_zones, const mars_b200_line_t *lines,
+                                 int n_lines) {
+    Model *m;
+    mars_error_t e = enter(model, &m);
+    if (e == MARS_OK) e = need_tracking(m, "set_zones");
+    if (e != MARS_OK) return e;
+    if (stream < 0 || stream >= m->track_streams) {
+        set_last_error("set_zones: stream %d outside [0, %d) (mars_b200_set_tracking)", stream, m->track_streams);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    if (n_zones < 0 || n_zones > MARS_B200_MAX_ZONES || n_lines < 0 || n_lines > MARS_B200_MAX_LINES || (n_zones > 0 && !zones) ||
+        (n_lines > 0 && !lines)) {
+        set_last_error("set_zones: %d zones (0 .. %d) and %d lines (0 .. %d), each table present when its count is positive", n_zones,
+                       MARS_B200_MAX_ZONES, n_lines, MARS_B200_MAX_LINES);
+        return MARS_ERR_INVALID_TENSOR;
+    }
+    if (!zones_valid(zones, n_zones, lines, n_lines)) return MARS_ERR_INVALID_TENSOR;
+    CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED); /* tracker calls in flight read the geometry and the state */
+    if (!m->zone_geom.p) {
+        const size_t ns = (size_t)m->track_streams;
+        DevBuf<ZoneGeom> geom;
+        DevBuf<ZoneTrack> state;
+        DevBuf<ZoneMeta> meta;
+        if (!geom.alloc(ns) || !state.alloc(ns * MARS_B200_MAX_TRACKS) || !meta.alloc(ns)) return MARS_ERR_ALLOC_FAILED;
+        CU_OK(cudaMemsetAsync(geom.p, 0, ns * sizeof(ZoneGeom), m->stream), MARS_ERR_ALLOC_FAILED);
+        CU_OK(cudaMemsetAsync(meta.p, 0, ns * sizeof(ZoneMeta), m->stream), MARS_ERR_ALLOC_FAILED);
+        CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_ALLOC_FAILED);
+        m->zone_geom = std::move(geom);
+        m->zone_state = std::move(state);
+        m->zone_meta = std::move(meta);
+    }
+    ZoneGeom g;
+    memset(&g, 0, sizeof g);
+    g.n_zones = n_zones;
+    g.n_lines = n_lines;
+    if (n_zones) memcpy(g.zone, zones, (size_t)n_zones * sizeof(mars_b200_zone_t));
+    if (n_lines) memcpy(g.line, lines, (size_t)n_lines * sizeof(mars_b200_line_t));
+    /* on the compute stream, so that the tracker calls that follow see the new geometry and the cleared state; g is a stack
+     * object, so the call waits for the copy */
+    CU_OK(cudaMemcpyAsync(m->zone_geom.p + stream, &g, sizeof g, cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
+    CU_OK(cudaMemsetAsync(m->zone_meta.p + stream, 0, sizeof(ZoneMeta), m->stream), MARS_ERR_LAYER_FAILED);
+    CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
+    const uint8_t on = n_zones > 0 || n_lines > 0;
+    m->zone_streams += (int)on - (int)m->zone_on[stream];
+    m->zone_on[stream] = on;
+    return MARS_OK;
+}
+
+mars_error_t mars_b200_download_zones(mars_model_t *model, int first, int n, mars_b200_zone_frame_t *out) {
+    Model *m;
+    mars_error_t e = out || n == 0 ? enter(model, &m, first, n) : MARS_ERR_INVALID_FILE;
+    if (e == MARS_OK) e = need_tracking(m, "download_zones");
+    if (e != MARS_OK || n == 0) return e;
+    CU_OK(cudaMemcpyAsync(out, m->rec.zone.p + first, (size_t)n * sizeof(mars_b200_zone_frame_t), cudaMemcpyDeviceToHost, m->stream),
+          MARS_ERR_LAYER_FAILED);
+    CU_OK(cudaStreamSynchronize(m->stream), MARS_ERR_LAYER_FAILED);
+    return MARS_OK;
+}
+
 mars_error_t mars_b200_track_boxes(mars_model_t *model, int n, const int32_t *streams, const mars_box_t *boxes, const int32_t *counts,
                                    int box_stride, mars_b200_track_box_t *out, int32_t *out_counts, int maxd) {
+    return mars_b200_track_boxes_zones(model, n, streams, boxes, counts, box_stride, out, out_counts, maxd, nullptr);
+}
+
+mars_error_t mars_b200_track_boxes_zones(mars_model_t *model, int n, const int32_t *streams, const mars_box_t *boxes, const int32_t *counts,
+                                         int box_stride, mars_b200_track_box_t *out, int32_t *out_counts, int maxd,
+                                         mars_b200_zone_frame_t *zone_out) {
     Model *m;
     mars_error_t e = enter(model, &m);
     if (e == MARS_OK) e = check_streams(m, "track_boxes", n, streams);
@@ -1974,10 +2096,12 @@ mars_error_t mars_b200_track_boxes(mars_model_t *model, int n, const int32_t *st
     }
     if (n == 0) return MARS_OK;
     maxd = std::max(0, std::min(maxd, MARS_B200_MAX_TRACKS));
-    /* in: [streams | counts | boxes n x maxc], out: [counts | records n x MARS_B200_MAX_TRACKS], each part 256-byte aligned */
+    /* in: [streams | counts | boxes n x maxc], out: [counts | records n x MARS_B200_MAX_TRACKS | (zone records n)], each part
+     * 256-byte aligned */
     auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const size_t ints = up((size_t)n * sizeof(int32_t)), in_bytes = 2 * ints + (size_t)n * maxc * sizeof(mars_box_t);
-    const size_t out_bytes = ints + (size_t)n * MARS_B200_MAX_TRACKS * sizeof(mars_b200_track_box_t);
+    const size_t rec_bytes = (size_t)n * MARS_B200_MAX_TRACKS * sizeof(mars_b200_track_box_t);
+    const size_t out_bytes = ints + rec_bytes + (zone_out ? (size_t)n * sizeof(mars_b200_zone_frame_t) : 0);
     if (!pre_grow(m, m->track_in, &m->track_in_cap, in_bytes) || !pre_grow(m, m->track_out, &m->track_out_cap, out_bytes)) return MARS_ERR_ALLOC_FAILED;
     std::vector<uint8_t> blob(in_bytes, 0);
     memcpy(blob.data(), streams, (size_t)n * sizeof(int32_t));
@@ -1988,10 +2112,15 @@ mars_error_t mars_b200_track_boxes(mars_model_t *model, int n, const int32_t *st
     const mars_box_t *d_boxes = reinterpret_cast<const mars_box_t *>(m->track_in.p + 2 * ints);
     int32_t *d_out_counts = reinterpret_cast<int32_t *>(m->track_out.p);
     mars_b200_track_box_t *d_out = reinterpret_cast<mars_b200_track_box_t *>(m->track_out.p + ints);
+    mars_b200_zone_frame_t *d_zones = zone_out ? reinterpret_cast<mars_b200_zone_frame_t *>(m->track_out.p + ints + rec_bytes) : nullptr;
     e = timed_call(m, "track_boxes", [&]() -> mars_error_t {
         CU_OK(cudaMemcpyAsync(m->track_in.p, blob.data(), in_bytes, cudaMemcpyHostToDevice, m->stream), MARS_ERR_LAYER_FAILED);
-        mars_error_t r = enqueue_track(m, d_boxes, d_counts, maxc, d_streams, n, d_out, d_out_counts, MARS_B200_MAX_TRACKS);
+        mars_error_t r = enqueue_track(m, d_boxes, d_counts, maxc, d_streams, n, d_out, d_out_counts, MARS_B200_MAX_TRACKS, d_zones,
+                                       zone_out != nullptr);
         if (r != MARS_OK) return r;
+        if (zone_out)
+            CU_OK(cudaMemcpyAsync(zone_out, d_zones, (size_t)n * sizeof(mars_b200_zone_frame_t), cudaMemcpyDeviceToHost, m->stream),
+                  MARS_ERR_LAYER_FAILED);
         CU_OK(cudaMemcpyAsync(out_counts, d_out_counts, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, m->stream), MARS_ERR_LAYER_FAILED);
         if (maxd > 0)
             CU_OK(cudaMemcpy2DAsync(out, (size_t)maxd * sizeof(mars_b200_track_box_t), d_out, MARS_B200_MAX_TRACKS * sizeof(mars_b200_track_box_t),
@@ -2082,6 +2211,7 @@ struct SubmitOut {
     int maxd;
     size_t stride;
     const int32_t *streams = nullptr; /* TRACKS: the tracker stream of each image */
+    mars_b200_zone_frame_t *zones = nullptr; /* TRACKS: the zone record of each image (null: not read back) */
 };
 
 /* Asynchronous form of mars_b200_detect_batch: the slot pool is split into two halves ("pools" 0 and 1); a batch of up to
@@ -2155,7 +2285,7 @@ static mars_error_t submit_batch(mars_model_t *model, const char *what, int pool
         if (e == MARS_OK && in.rois) e = enqueue_merge(m, first, nrec, tail_dev, merge_thresh);
         if (e == MARS_OK && out.kind == SubmitOut::TRACKS)
             e = enqueue_track(m, m->rec.box.at(first), m->rec.box.cnt.p + first, MARS_MAX_DETS, tail_dev, n, m->rec.trk.at(first),
-                              m->rec.trk.cnt.p + first, MARS_B200_MAX_TRACKS);
+                              m->rec.trk.cnt.p + first, MARS_B200_MAX_TRACKS, m->rec.zone.p + first, out.zones != nullptr);
         if (e != MARS_OK) { cudaStreamSynchronize(m->stream); return e; }
         cudaEventRecord(m->ev_done[pool], m->stream);
         cudaStreamWaitEvent(m->d2h_stream, m->ev_done[pool], 0);
@@ -2163,7 +2293,12 @@ static mars_error_t submit_batch(mars_model_t *model, const char *what, int pool
             case SubmitOut::DETS: e = copy_dets(m->rec.det, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
             case SubmitOut::BOXES: e = copy_dets(m->rec.box, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
             case SubmitOut::FRAME_BOXES: e = copy_dets(m->rec.fbox, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
-            case SubmitOut::TRACKS: e = copy_dets(m->rec.trk, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream); break;
+            case SubmitOut::TRACKS:
+                e = copy_dets(m->rec.trk, first, nrec, out.dst, out.counts, out.maxd, m->d2h_stream);
+                if (e == MARS_OK && out.zones)
+                    CU_OK(cudaMemcpyAsync(out.zones, m->rec.zone.p + first, (size_t)n * sizeof(mars_b200_zone_frame_t), cudaMemcpyDeviceToHost,
+                                          m->d2h_stream), MARS_ERR_LAYER_FAILED);
+                break;
             case SubmitOut::TENSOR: e = copy_io(m, first, n, out.dst, out_stride, 1, m->d2h_stream); break;
         }
         if (e != MARS_OK) return e;
@@ -2238,6 +2373,29 @@ mars_error_t mars_b200_submit_frames_nv12_track_batch(mars_model_t *model, int p
     std::vector<FrameSrc> s;
     return submit_batch(model, "submit_frames_nv12_track_batch", pool, n, SubmitIn{nullptr, 0, true, nv12_sources(n, frames, &s), nullptr},
                         SubmitOut{SubmitOut::TRACKS, out, counts, maxd, 0, streams}, nms_thresh);
+}
+/* the track submits with the zone record of every frame read back too */
+mars_error_t mars_b200_submit_frames_zones_batch(mars_model_t *model, int pool, int n, const mars_b200_frame_t *frames, const int32_t *streams,
+                                                 mars_b200_track_box_t *out, int32_t *counts, int maxd, mars_b200_zone_frame_t *zones,
+                                                 float nms_thresh) {
+    std::vector<FrameSrc> s;
+    if (!zones) {
+        set_last_error("submit_frames_zones_batch: no zone record table (zones is NULL; mars_b200_submit_frames_track_batch reads back no zone records)");
+        return MARS_ERR_INVALID_FILE;
+    }
+    return submit_batch(model, "submit_frames_zones_batch", pool, n, SubmitIn{nullptr, 0, true, rgb_sources(n, frames, &s), nullptr},
+                        SubmitOut{SubmitOut::TRACKS, out, counts, maxd, 0, streams, zones}, nms_thresh);
+}
+mars_error_t mars_b200_submit_frames_nv12_zones_batch(mars_model_t *model, int pool, int n, const mars_b200_nv12_frame_t *frames,
+                                                      const int32_t *streams, mars_b200_track_box_t *out, int32_t *counts, int maxd,
+                                                      mars_b200_zone_frame_t *zones, float nms_thresh) {
+    std::vector<FrameSrc> s;
+    if (!zones) {
+        set_last_error("submit_frames_nv12_zones_batch: no zone record table (zones is NULL; mars_b200_submit_frames_nv12_track_batch reads back no zone records)");
+        return MARS_ERR_INVALID_FILE;
+    }
+    return submit_batch(model, "submit_frames_nv12_zones_batch", pool, n, SubmitIn{nullptr, 0, true, nv12_sources(n, frames, &s), nullptr},
+                        SubmitOut{SubmitOut::TRACKS, out, counts, maxd, 0, streams, zones}, nms_thresh);
 }
 
 /* mars_b200_submit_batch without the YOLO post-process: the raw output tensor 0 of every image is read back instead
